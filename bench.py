@@ -53,14 +53,60 @@ NB_ITER_MAX = 10
 SYND = {20: (19, 15, 5, 1000, 25), 16: (15, 15, 5, 1000, 25)}
 SYND_FRAMES = {"AD_64800_R12_GF256": 592, "MatDeclercq_R12_GF64": 592, "Mat24_N480_M240": 16384, "N96_K48_GF64": 1 << 18}
 REF_DIR = os.path.join(ROOT, "oracle", "_ref")
+# (N, M, GF, dc) of each workload's code, all with column degree 2.  Only the small matrices ship in matrices/ (see its README);
+# a workload whose file is absent decodes a seeded random code of this shape instead, so that the kernels see the same sizes,
+# degrees and field.  The JSON line names the code that ran under "matrix".
+STANDIN = {"AD_64800_R12_GF256": (8100, 4050, 256, 4), "Ahmed_64800_R34_GF16": (16200, 4050, 16, 8),
+           "MatDeclercq_R12_GF64": (10800, 5400, 64, 4), "Mat24_N480_M240": (480, 240, 64, 4),
+           "KN_64800_R34_GF256": (8100, 2025, 256, 8)}
+STANDIN_SEED = 2024
+_standin_dir = None
 
 
 def find_matrix(rel):
-    for d in (REF_DIR, "/root/reference"):
+    for d in (ROOT, REF_DIR):
         p = os.path.join(d, rel)
         if os.path.exists(p):
             return p
-    raise FileNotFoundError("%s not found under oracle/_ref (run __graft_entry__.build() where /root/reference exists)" % rel)
+    raise FileNotFoundError("%s found neither in matrices/ nor in oracle/_ref" % rel)
+
+
+def write_standin(path, N, M, q, dc, seed):
+    """UBS alist of a random code, every column in 2 checks, no column twice in a check, non-zero coefficients."""
+    rng = np.random.default_rng(seed)
+    rows = rng.permutation(np.repeat(np.arange(N), 2)).reshape(M, dc)
+    while True:
+        bad = [m for m in range(M) if len(set(rows[m])) < dc]
+        if not bad:
+            break
+        for m in bad:                                  # swap one slot of the row with a random slot anywhere
+            k, m2, k2 = int(rng.integers(dc)), int(rng.integers(M)), int(rng.integers(dc))
+            rows[m, k], rows[m2, k2] = rows[m2, k2], rows[m, k]
+    val = rng.integers(1, q, (M, dc))
+    with open(path, "w") as f:
+        f.write("%d %d %d\n%s\n%s\n" % (N, M, q, " ".join(["2"] * N), " ".join([str(dc)] * M)))
+        f.write("".join(" ".join(map(str, r)) + "\n" for r in rows))
+        f.write("".join(" ".join(map(str, r)) + "\n" for r in val))
+
+
+def workload_matrix(wl):
+    """(path, description) of the code of workload wl: its matrix file, or the seeded stand-in written to a temporary directory."""
+    rel = WORKLOADS[wl][0]
+    try:
+        return find_matrix(rel), rel
+    except FileNotFoundError:
+        pass
+    global _standin_dir
+    if _standin_dir is None:
+        import atexit
+        import shutil
+        _standin_dir = tempfile.mkdtemp(prefix="nbldpc_bench_")
+        atexit.register(shutil.rmtree, _standin_dir, True)
+    N, M, q, dc = STANDIN[wl]
+    path = os.path.join(_standin_dir, wl)
+    if not os.path.exists(path):
+        write_standin(path, N, M, q, dc, STANDIN_SEED)
+    return path, "random stand-in for %s (absent): N=%d, M=%d, GF(%d), dv=2, dc=%d, seed %d" % (rel, N, M, q, dc, STANDIN_SEED)
 
 
 def bytes_per_frame(N, E, q, n_m, passes, ecn="bubble"):
@@ -170,7 +216,7 @@ def _port_worker(arg):
     sys.path.insert(0, os.path.join(ROOT, "tests"))          # the oracle port: cpu_baseline fallback only, never the product arm
     import oracle_lib as ol
     matrix, n_m, nb_oper, offset, ebn, _ = WORKLOADS[wl]
-    o = ol.Oracle(find_matrix(matrix))
+    o = ol.Oracle(workload_matrix(wl)[0])
     kw = {}
     if ecn == "syndrome":
         d1, d2, d3, trunc, n_cv = SYND[n_m]
@@ -213,7 +259,7 @@ def reference_arm(args, rank, world):
         return
     wl = args.workload
     matrix, n_m, nb_oper, offset, ebn, _ = WORKLOADS[wl]
-    code = AlistHeader(find_matrix(matrix))
+    code = AlistHeader(workload_matrix(wl)[0])
     cores = host_cores()
     budget_s = float(os.environ.get("NBLDPC_REF_BUDGET_S", "240"))
     # calibration (also the first warm-up step): one frame per process
@@ -369,6 +415,7 @@ def measure_leg(nbldpc, code, wl, ecn, B, args, rank, local_rank, world, dist, n
     ms = dec.timer_end()
     t1 = time.time()
     barrier()
+    d_res, s_res, it_res = dec.download()              # what the last timed step computed
     launches = dec.launch_count() - l0
     clocks = sampler.stop(t0, t1) if sampler else None
     ms = maxr(ms)
@@ -377,7 +424,6 @@ def measure_leg(nbldpc, code, wl, ecn, B, args, rank, local_rank, world, dist, n
         dec.run()
         kms.append(dec.last_kernel_ms())
     kernel_ms = statistics.mean(kms)
-    d_res, s_res, it_res = dec.download()
     frames_total = world * B * args.steps
     fps = frames_total / (ms / 1e3)
     value = fps * code.info_bits / 1e6
@@ -469,6 +515,7 @@ def measure_leg(nbldpc, code, wl, ecn, B, args, rank, local_rank, world, dist, n
                             "slow_path_selects": dec.slow_selects()}}
         if shard is not None:
             leg["sharding_check"] = shard
+        leg["outputs"] = {"decide": d_res, "syndrome": s_res, "iterations": it_res}
     dec.close()
     return leg
 
@@ -485,7 +532,8 @@ def ours(args, rank, local_rank, world):
         raise RuntimeError("bench.py needs a B200: the product has no CPU fallback")
     wl = args.workload
     matrix, n_m, nb_oper, offset, ebn, dflt_B = WORKLOADS[wl]
-    code = nbldpc.Code(find_matrix(matrix))
+    path, matrix_desc = workload_matrix(wl)
+    code = nbldpc.Code(path)
     synd_ok = n_m in SYND and code.dc_min == code.dc_max and 4 <= code.dc_max <= 8
     B_of = {"bubble": args.frames or dflt_B, "syndrome": args.frames or SYND_FRAMES.get(wl, dflt_B)}
     # the headline leg is the check node asked for; the default run carries the other one of the workload as a second, complete leg
@@ -505,7 +553,7 @@ def ours(args, rank, local_rank, world):
         line = {"metric": "decoded info Mbit/s at fixed iterations (%d passes)" % passes, "value": head["value"], "unit": "Mbit/s", "n_gpus": world,
                 "steps": args.steps, "warmup": args.warmup, "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak",
                 "vs_baseline": None, "dtype": "f32", "data": "synthetic (encoder codewords + numpy Gaussian noise at the reference's sigma)",
-                "git": git_head(), "source_id": source_id()}
+                "git": git_head(), "source_id": source_id(), "matrix": matrix_desc}
         for k in ("frames_per_s", "config", "geometry", "e2e", "gpu_launches", "roofline", "clocks", "simulation", "counters", "sharding_check"):
             if k in head:
                 line[k] = head[k]
@@ -521,13 +569,32 @@ def ours(args, rank, local_rank, world):
             other["note"] = "the same workload and frames through the reference's other check node (NB_LDPC.c:%s instead of :%s), measured like the " \
                             "headline leg (same steps and warm-up); `bench.py --ecn %s` makes it the headline" % (
                                 ("388", "392", "syndrome") if legs[1] == "syndrome" else ("392", "388", "bubble"))
+            other.pop("outputs")
             line["config5_as_written" if (legs[1] == "syndrome" and BASELINE_CONFIG.get(wl) == 5) else "other_check_node"] = other
+        outputs = head.pop("outputs")
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         emit(line)
     nbldpc.unpin(noisy)
     for o in out:
         nbldpc.unpin(o)
     if dist is not None:
         dist.destroy_process_group()
+
+
+def dump_outputs(d, outputs, limit=48 << 20):
+    """The arrays the decode call returns (decisions [B, N], syndromes [B], iteration counts [B]) as float32 .npy files.  When the
+    decisions exceed `limit` bytes, a fixed seeded sample of frames is written and decide_frames.npy names them."""
+    os.makedirs(d, exist_ok=True)
+    dec = outputs["decide"]
+    B, N = dec.shape
+    keep = np.arange(B)
+    if B * N * 4 > limit:
+        keep = np.sort(np.random.default_rng(0).choice(B, limit // (N * 4), replace=False))
+    np.save(os.path.join(d, "decide.npy"), dec[keep].astype(np.float32))
+    np.save(os.path.join(d, "decide_frames.npy"), keep.astype(np.float64))
+    np.save(os.path.join(d, "syndrome.npy"), outputs["syndrome"].astype(np.float32))
+    np.save(os.path.join(d, "iterations.npy"), outputs["iterations"].astype(np.float32))
 
 
 def code_bits(code, syms):
@@ -572,6 +639,7 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-also", action="store_true", help="skip the short syndrome_ems leg of the default run")
     ap.add_argument("--count-errors", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -10,7 +10,7 @@ import oracle_lib as ol
 
 ROOT = ol.ROOT
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
-MATRIX_DIRS = [os.path.join(ol.REF_DIR), "/root/reference"]
+MATRIX_DIRS = [ROOT, ol.REF_DIR]
 
 
 def sha(a):
@@ -18,12 +18,44 @@ def sha(a):
 
 
 def matrix_path(rel):
-    """rel = 'matrices/...' as in the reference tree; the copies made by oracle/Makefile travel to the GPU box."""
+    """rel = 'matrices/...' as in the reference tree: the repository's matrices/, then the copies oracle/Makefile makes."""
     for d in MATRIX_DIRS:
         p = os.path.join(d, rel)
         if os.path.exists(p):
             return p
-    pytest.skip("matrix %s not available (build oracle/_ref where /root/reference exists)" % rel)
+    pytest.skip("matrix %s not available (neither in matrices/ nor in oracle/_ref)" % rel)
+
+
+# (N, M, GF, check degree) of the reference's matrices that matrices/ lacks; every one has column degree 2
+SHAPES = {"matrices/AD_64800_R12_GF256": (8100, 4050, 256, 4), "matrices/Ahmed_64800_R34_GF16": (16200, 4050, 16, 8),
+          "matrices/MatDeclercq_R12_GF64": (10800, 5400, 64, 4), "matrices/Mat24_N480_M240": (480, 240, 64, 4),
+          "matrices/Mat26_N48_M16": (48, 16, 64, 6),
+          "matrices/Mat212_N96_M16": (96, 16, 64, 12), "matrices/Mat212_N480_M80": (480, 80, 64, 12),
+          "matrices/KN/N576_K480_GF64.txt": (96, 16, 64, 12), "matrices/KN/N128_K64_GF256.txt": (16, 8, 256, 4),
+          "matrices/KN/N64800_K48600_GF256.txt": (8100, 2025, 256, 8)}
+_STANDIN = {}
+
+
+def code_path(rel):
+    """matrix_path(rel) when the file is here; otherwise a seeded random code of the same shape, written in the same layout
+    (UBS, KN, or full alist for N64800_*).  For tests that compare the product with the oracle on a code of that size and
+    field: they need such a code, not that particular one.  Tests against recorded reference runs use matrix_path."""
+    for d in MATRIX_DIRS:
+        if os.path.exists(os.path.join(d, rel)):
+            return os.path.join(d, rel)
+    if rel not in _STANDIN:
+        import tempfile
+        N, M, q, dc = SHAPES[rel]
+        a = random_regular_code(np.random.default_rng(N + M + q + dc), N, M, q, dc)
+        path = os.path.join(tempfile.mkdtemp(prefix="nbldpc_standin_"), os.path.basename(rel))
+        if "N64800" in rel:
+            write_alist_full(path, a)
+        elif rel.startswith("matrices/KN/"):
+            write_alist_kn(path, a)
+        else:
+            write_alist_ubs(path, a)
+        _STANDIN[rel] = path
+    return _STANDIN[rel]
 
 
 def golden_names():
@@ -93,7 +125,15 @@ def random_regular_code(rng, N, M, q, dc, dv=2):
         if all(len(set(r)) == dc for r in rows):
             break
     else:
-        raise RuntimeError("could not build a simple graph")
+        for _ in range(1000):                    # dense rows: repair repeated columns by swapping a slot with a random one
+            bad = [m for m in range(M) if len(set(rows[m])) < dc]
+            if not bad:
+                break
+            for m in bad:
+                k, m2, k2 = rng.integers(dc), rng.integers(M), rng.integers(dc)
+                rows[m, k], rows[m2, k2] = rows[m2, k2], rows[m, k]
+        else:
+            raise RuntimeError("could not build a simple graph")
     col = rows.reshape(-1).astype(np.int32)
     val = rng.integers(1, q, size=M * dc).astype(np.int32)
     return dict(N=N, M=M, q=q, row_deg=np.full(M, dc, np.int32), col=col, val=val)

@@ -8,7 +8,7 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import (Golden, golden_names, matrix_path, oracle_frames, product_frames, random_regular_code, sha,
+from common import (Golden, code_path, golden_names, matrix_path, oracle_frames, product_frames, random_regular_code, sha,
                     write_alist_ubs)
 
 pytestmark = pytest.mark.gpu
@@ -20,7 +20,7 @@ _SYN = {}
 def mpath(rel):
     """reference matrices, plus small synthetic GF(16) codes (the only GF(16) matrix of the reference is the 64800-bit one)"""
     if not rel.startswith("synthetic/"):
-        return matrix_path(rel)
+        return code_path(rel)
     if rel not in _SYN:
         import re
         import tempfile
@@ -135,7 +135,8 @@ def _synd_kw(g):
 @pytest.mark.parametrize("name", [n for n in golden_names() if "cn_node" in Golden(n).z])
 def test_check_node_on_reference_messages(name):
     g = Golden(name)
-    code, d = _dec(g.matrix, g.n_m, g.nb_oper, g.nb_iter_max, g.offset, **_synd_kw(g))
+    code = nbldpc.Code(matrix_path(g.matrix))                 # messages recorded on the reference's own code: no stand-in
+    d = nbldpc.Decoder(code, g.n_m, g.nb_oper, g.nb_iter_max, g.offset, **_synd_kw(g))
     z = g.z
     nodes = z["cn_node"]
     for node in np.unique(nodes):
@@ -337,7 +338,7 @@ def test_streamed_end_to_end_path_equals_resident_launch():
 def test_full_alist_dvb_size_code_equals_oracle(tmp_path):
     """matrices/KN/N64800_K48600_GF256.txt (full alist, rate 3/4 over GF(256), check degree 8): the reference cannot load it;
     the oracle port gets the same graph through a UBS copy"""
-    code = nbldpc.Code(matrix_path("matrices/KN/N64800_K48600_GF256.txt"))
+    code = nbldpc.Code(code_path("matrices/KN/N64800_K48600_GF256.txt"))
     a = dict(N=code.N, M=code.M, q=code.q, row_deg=code.row_deg, col=code.col, val=code.val)
     p = str(tmp_path / "ubs")
     write_alist_ubs(p, a)
@@ -356,7 +357,7 @@ def test_full_alist_dvb_size_code_equals_oracle(tmp_path):
 
 def test_contexts_with_different_geometries_coexist():
     """two decoders of the same kernel (GF(64), closed form) but different shared-memory plans, used alternately"""
-    c1 = nbldpc.Code(matrix_path("matrices/N96_K48_GF64")); c2 = nbldpc.Code(matrix_path("matrices/Mat24_N480_M240"))
+    c1 = nbldpc.Code(matrix_path("matrices/N96_K48_GF64")); c2 = nbldpc.Code(code_path("matrices/Mat24_N480_M240"))
     d1 = nbldpc.Decoder(c1, 20, 25, 10, 0.3, max_batch=64)
     d2 = nbldpc.Decoder(c2, 8, 25, 10, 0.3, max_batch=8, cns_per_step=12)
     assert d1.geometry()["smem_bytes"] != d2.geometry()["smem_bytes"]
@@ -426,7 +427,7 @@ def test_irregular_and_isolated_variables(tmp_path):
 @pytest.mark.parametrize("rel,n_m,ebn_hi", [("matrices/AD_64800_R12_GF256", 20, 3.2), ("matrices/Ahmed_64800_R34_GF16", 16, 4.5),
                                             ("matrices/MatDeclercq_R12_GF64", 20, 2.6)])
 def test_full_size_round_trip_and_invariances(rel, n_m, ebn_hi):
-    code = nbldpc.Code(matrix_path(rel))
+    code = nbldpc.Code(code_path(rel))
     B = 24
     fr, sigma = product_frames(code, B, ebn_hi)
     noisy = np.stack([f["noisy"] for f in fr]); cw = np.stack([f["cw"] for f in fr])
@@ -455,7 +456,7 @@ def test_fixed_iteration_mode_equals_oracle_with_forced_passes(rel, n_m, ebn, ec
     """The metric's mode (early termination off, NbIterMax-1 passes for every frame): Decision and Syndrom run only after the
     last pass on the GPU; decisions, syndrome, iteration count and every APP / CtoV bit must equal the oracle run with the
     break of NB_LDPC.c:470 disabled -- for frames that would have converged early and for frames that never do."""
-    path = matrix_path(rel)
+    path = code_path(rel)
     code = nbldpc.Code(path)
     o = ol.Oracle(path, code.dialect)
     kw, okw = {}, {}
@@ -486,7 +487,7 @@ def test_full_size_multi_wave_batch_spot_checked_against_oracle():
     """BASELINE config 5 at the operating point of the bench (Eb/N0 2.0 dB, some frames never converge): a batch larger than
     the persistent grid (several frames per CTA, streamed end-to-end path), six frames spot-checked against the oracle"""
     rel, n_m = "matrices/AD_64800_R12_GF256", 20
-    code = nbldpc.Code(matrix_path(rel))
+    code = nbldpc.Code(code_path(rel))
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=1400)
     geo = d.geometry()
     B = min(1400, 4 * geo["grid"] * geo["frames_per_cta"] + 13)
@@ -497,7 +498,7 @@ def test_full_size_multi_wave_batch_spot_checked_against_oracle():
     noisy = noisy + (rng.standard_normal(noisy.shape) * 0.02).astype(np.float32)       # every frame differs
     dec, synd, it = d.decode_noisy(noisy, sigma)
     assert len(set(it.tolist())) > 1, "the batch should mix converging and non-converging frames"
-    o = ol.Oracle(matrix_path(rel), code.dialect)
+    o = ol.Oracle(code_path(rel), code.dialect)
     for f in [0, 1, B // 3, B // 2, B - 2, B - 1]:
         r = o.decode_frame(o.channel_llr(noisy[f], sigma), n_m, 25, 10, 0.3)
         assert (dec[f] == r["decide"]).all() and synd[f] == r["synd"] and it[f] == r["iters"], f
@@ -508,8 +509,8 @@ def _multi_wave_case(rel, n_m, ebn, ecn, frames_checked, state_frames=2, fpc=1):
     """A batch of at least four waves of the persistent grid through the streamed end-to-end path at a benched operating
     point; `frames_checked` frames compared with the oracle (decisions, syndrome, iterations), the last `state_frames` of
     them -- they sit in the last wave, so their slots still hold their state -- also on every APP and CtoV bit."""
-    code = nbldpc.Code(matrix_path(rel))
-    o = ol.Oracle(matrix_path(rel), code.dialect)
+    code = nbldpc.Code(code_path(rel))
+    o = ol.Oracle(code_path(rel), code.dialect)
     kw, okw = {}, {}
     if ecn:
         cfg = o.build_config_table(int(code.row_deg[0]), min(19, n_m - 1), 15, 5, 1000)
@@ -587,7 +588,7 @@ def test_apsk64_intake_kernel_equals_oracle_and_reference_vectors():
 def test_apsk64_decode_equals_oracle(rel, ebn):
     """nbgpu_decode_apsk64 (intake fused into the decoder) against the oracle's 64-APSK LLR + decode loop, frames that converge
     and frames that do not."""
-    path = matrix_path(rel)
+    path = code_path(rel)
     code = nbldpc.Code(path)
     o = ol.Oracle(path, code.dialect)
     code.prepare_encoder(); code.rng_default()

@@ -4,7 +4,7 @@ import numpy as np
 import pytest
 
 import nbldpc
-from common import matrix_path
+from common import code_path
 
 multigpu = __import__("importlib").import_module("ems-decoder-of-nb-ldpc-codes_b200.multigpu")
 
@@ -27,7 +27,7 @@ def _host_frames(code, frame0, B, ebn):
 
 @pytest.mark.parametrize("rel,n_m", CODES)
 def test_generated_frames_equal_the_host_stream(rel, n_m):
-    code = nbldpc.Code(matrix_path(rel))
+    code = nbldpc.Code(code_path(rel))
     big = code.N > 5000
     B = 6 if big else 200
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=B)
@@ -42,7 +42,7 @@ def test_generated_frames_equal_the_host_stream(rel, n_m):
 
 def test_flagged_samples_are_recomputed_by_the_host():
     """with the widest margin a large share of the samples takes the host path; the stream must not change"""
-    code = nbldpc.Code(matrix_path("matrices/Mat24_N480_M240"))
+    code = nbldpc.Code(code_path("matrices/Mat24_N480_M240"))
     d = nbldpc.Decoder(code, 16, 25, 10, 0.3, max_batch=64)
     cw, _, noisy = _host_frames(code, 7, 64, 1.5)
     d.source_frames(7, 64, 1.5)
@@ -58,7 +58,7 @@ def test_flagged_samples_are_recomputed_by_the_host():
 
 
 def test_default_margin_flags_about_one_sample_in_a_million():
-    code = nbldpc.Code(matrix_path("matrices/AD_64800_R12_GF256"))
+    code = nbldpc.Code(code_path("matrices/AD_64800_R12_GF256"))
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=256)
     d.source_frames(100, 256, 2.0)                       # 16.6 M samples
     n = d.source_fixups()
@@ -70,7 +70,7 @@ def test_default_margin_flags_about_one_sample_in_a_million():
                                                      ("matrices/Mat24_N480_M240", 16, 1.5, 200, 64)])
 def test_results_equal_the_host_driven_run(rel, n_m, ebn, frames, batch):
     """source -> run -> results reproduces (bit errors, syndrome, iterations) of host frames through decode_noisy"""
-    code = nbldpc.Code(matrix_path(rel))
+    code = nbldpc.Code(code_path(rel))
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=batch)
     bing = code.tables()[0]
     sigma = code.sigma(ebn)
@@ -89,7 +89,7 @@ def test_results_equal_the_host_driven_run(rel, n_m, ebn, frames, batch):
 
 
 def test_source_argument_errors():
-    c1 = nbldpc.Code(matrix_path("matrices/N96_K48_GF64")); c2 = nbldpc.Code(matrix_path("matrices/Mat24_N480_M240"))
+    c1 = nbldpc.Code(code_path("matrices/N96_K48_GF64")); c2 = nbldpc.Code(code_path("matrices/Mat24_N480_M240"))
     d = nbldpc.Decoder(c1, 20, 25, 10, 0.3, max_batch=8)
     with pytest.raises(nbldpc.NbgpuError):
         d.source_results()                               # nothing generated

@@ -10,7 +10,7 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import Golden, golden_names, matrix_path, oracle_frames, product_frames, random_regular_code, write_alist_full, write_alist_kn, write_alist_ubs, ROOT
+from common import Golden, code_path, golden_names, matrix_path, oracle_frames, product_frames, random_regular_code, write_alist_full, write_alist_kn, write_alist_ubs, ROOT
 
 
 def test_library_exports_every_declared_symbol():
@@ -40,7 +40,7 @@ def test_no_gpu_means_error_not_fallback():
                                          ("matrices/AD_64800_R12_GF256", 1), ("matrices/MatDeclercq_R12_GF64", 1),
                                          ("matrices/KN/N576_K480_GF64.txt", 2), ("matrices/Mat212_N480_M80", 1)])
 def test_loader_and_tables_equal_oracle(rel, dialect):
-    p = matrix_path(rel)
+    p = code_path(rel)
     o = ol.Oracle(p, dialect)
     for d in (dialect, nbldpc.ALIST_AUTO):
         c = nbldpc.Code(p, d)
@@ -112,7 +112,7 @@ def test_three_layouts_of_one_random_code_load_identically(tmp_path, seed):
 
 
 def test_shipped_full_alist_matrix_loads_and_encodes():
-    c = nbldpc.Code(matrix_path("matrices/KN/N64800_K48600_GF256.txt"))
+    c = nbldpc.Code(code_path("matrices/KN/N64800_K48600_GF256.txt"))
     assert (c.dialect, c.N, c.M, c.q, c.dc_min, c.dc_max) == (nbldpc.ALIST_FULL, 8100, 2025, 256, 8, 8)
     c.prepare_encoder()
     cw, _ = c.random_codeword()
