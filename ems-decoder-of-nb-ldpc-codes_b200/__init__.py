@@ -19,6 +19,7 @@ LIB_PATH = os.environ.get("NBLDPC_B200_LIB") or os.path.join(HERE, "libnbldpc_b2
 
 OK, EINVAL, EIO, ENOMEM, ECUDA, ESTATE, ERANK = 0, -1, -2, -3, -4, -5, -6
 ALIST_AUTO, ALIST_UBS, ALIST_KN, ALIST_FULL = 0, 1, 2, 3
+SOFT_NONE, SOFT_LIST, SOFT_BITS = 0, 1, 2
 
 _ip = C.POINTER(C.c_int)
 _fp = C.POINTER(C.c_float)
@@ -116,6 +117,9 @@ def lib():
         "nbgpu_geometry": (C.c_int, [vp, _ip]),
         "nbgpu_slow_selects": (C.c_long, [vp]),
         "nbgpu_get_state": (C.c_int, [vp, C.c_int, _fp, _fp]),
+        "nbgpu_set_soft_output": (C.c_int, [vp, C.c_int, C.c_int]),
+        "nbgpu_download_soft_list": (C.c_int, [vp, _fp, _ip]),
+        "nbgpu_download_soft_bits": (C.c_int, [vp, _fp]),
         "nbgpu_source_frames": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_download": (C.c_int, [vp, _ip, _fp]),
         "nbgpu_source_results": (C.c_int, [vp, _ip, _ip, _ip]),
@@ -260,6 +264,7 @@ class Decoder:
         self.max_batch = max_batch
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
+        self.soft_k = 0
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
@@ -307,13 +312,13 @@ class Decoder:
 
     def upload_noisy(self, noisy, sigma):
         noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, self.code.logq)
-        self.B = noisy.shape[0]
-        _check(lib().nbgpu_upload_noisy(self.h, _f(noisy), C.c_float(sigma), self.B), self.h)
+        _check(lib().nbgpu_upload_noisy(self.h, _f(noisy), C.c_float(sigma), noisy.shape[0]), self.h)
+        self.B = noisy.shape[0]                               # only once the batch is resident: it sizes every download
 
     def upload_llr(self, llr):
         llr = np.ascontiguousarray(llr, np.float32).reshape(-1, self.code.N, self.code.q)
+        _check(lib().nbgpu_upload_llr(self.h, _f(llr), llr.shape[0]), self.h)
         self.B = llr.shape[0]
-        _check(lib().nbgpu_upload_llr(self.h, _f(llr), self.B), self.h)
 
     def run(self):
         _check(lib().nbgpu_run(self.h), self.h)
@@ -384,6 +389,27 @@ class Decoder:
         ctov = np.zeros((self.code.E, self.code.q), np.float32)
         _check(lib().nbgpu_get_state(self.h, frame, _f(app), _f(ctov)), self.h)
         return app, ctov
+
+    def set_soft_output(self, kind, k=0):
+        """nbgpu_set_soft_output: every later decode launch also returns SOFT_LIST (the k most likely symbols per variable)
+        or SOFT_BITS (log2 q bit reliabilities per variable); SOFT_NONE turns it off."""
+        rc = lib().nbgpu_set_soft_output(self.h, kind, k)
+        if rc in (OK, ENOMEM):                                # ENOMEM leaves soft output off
+            self.soft_k = k if rc == OK else 0
+        _check(rc, self.h)
+
+    def soft_list(self):
+        """(llr [B,N,k] f32, sym [B,N,k] i32) of the last decode launch, armed with SOFT_LIST"""
+        llr = np.zeros((self.B, self.code.N, self.soft_k), np.float32)
+        sym = np.zeros(llr.shape, np.int32)
+        _check(lib().nbgpu_download_soft_list(self.h, _f(llr), _i(sym)), self.h)
+        return llr, sym
+
+    def soft_bits(self):
+        """bit reliabilities [B,N,logq] f32 of the last decode launch, armed with SOFT_BITS (> 0 favours bit 0)"""
+        llr = np.zeros((self.B, self.code.N, self.code.logq), np.float32)
+        _check(lib().nbgpu_download_soft_bits(self.h, _f(llr)), self.h)
+        return llr
 
     def channel(self, noisy, sigma, want_sorted=False):
         noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, self.code.logq)

@@ -109,6 +109,11 @@ struct KArgs {
     const uint8_t *cfg;                 /* [S][dc_max] u8 */
     float *ctov_dense;                  /* [slots][E][q] f32 */
     int off_cfg, sw_key, sw_pay, sw_gf, sw_hist, sw_cand, sw_M, sw_rows, sw_perm;   /* sw_*: offsets inside a warp's list area */
+    /* soft output (nbgpu_set_soft_output), read by decode_kernel<..., SOFT = true> only.  Kept at the end of the struct so
+     * that the fields above keep their parameter offsets in every kernel. */
+    int soft_kind, soft_k;              /* NBGPU_SOFT_LIST with k symbols per variable, or NBGPU_SOFT_BITS (k = 0)  */
+    float *soft_llr;                    /* [B][N][k] (LIST) or [B][N][logq] (BITS)                                  */
+    uint8_t *soft_sym;                  /* [B][N][k] symbols (LIST)                                                 */
 };
 
 /* Lists of a warp's tile in shared memory, by 32-bit shared-window address: one array of cpw * L lists, the input lists
@@ -654,7 +659,56 @@ __device__ __forceinline__ void tile_phase3(const KArgs &a, const WarpMem<Q> &wm
     }
 }
 
-template <int Q, bool CLOSED, int ECN>
+/* Soft output of the nf frames of a finished group (include/nbldpc_b200.h), one warp per variable, from the final APP rows
+ * in the group's slots (app = the CTA's slot block).  Runs after the last pass, where the phase-1 scratch of the warp is
+ * free; the slots are reused by the next group, so this is the last moment the rows exist. */
+template <int Q, int ECN>
+__device__ __forceinline__ void soft_output(const KArgs &a, const WarpMem<Q, ECN> &wm, const GFTab &gf, const float *app, int base, int nf,
+                                         int warp, int nw, int lane)
+{
+    constexpr int VPL = QTraits<Q>::VPL, LOGQ = QTraits<Q>::LOGQ;
+    const bool active = (Q >= 32) || lane < Q;
+    const int k = a.soft_k;
+    for (int w = warp; w < nf * a.N; w += nw) {          /* w = f * N + n: row w of the slot block, variable base * N + w */
+        const size_t var = (size_t)base * a.N + w;
+        float v[1][VPL];
+        load_row<Q>(app + (size_t)w * Q, lane, v[0]);
+        if (a.soft_kind == NBGPU_SOFT_LIST) {
+            /* the truncation NB_LDPC.c:354-374 with n_m = k; the decoder's slow-path counter is not touched */
+            const uint32_t scr[1] = { wm.scra(0) }, sel[1] = { wm.sela(0) };
+            float llr[1]; int sym[1];
+            select_edges<Q, 1>(v, lane, scr, sel, k, llr, sym, nullptr);
+            if (lane < k) { a.soft_llr[var * k + lane] = llr[0]; a.soft_sym[var * k + lane] = (uint8_t)sym[0]; }
+        } else {
+            /* per bit the two minima, split by the binary image; keys in the total order of the floats (the APP may be
+             * negative with a negative offset), so one integer REDUX per minimum gives the exact value back */
+            uint32_t m0[LOGQ], m1[LOGQ];
+#pragma unroll
+            for (int l = 0; l < LOGQ; l++) { m0[l] = NB_KEY_INF; m1[l] = NB_KEY_INF; }
+#pragma unroll
+            for (int j = 0; j < VPL; j++) {
+                const uint32_t b = __float_as_uint(v[0][j]);
+                const uint32_t key = active ? b ^ ((uint32_t)((int)b >> 31) | 0x80000000u) : NB_KEY_INF;
+                const uint32_t im = gf.img[QTraits<Q>::sym(lane, j) & (Q - 1)];
+#pragma unroll
+                for (int l = 0; l < LOGQ; l++) {
+                    if ((im >> l) & 1u) m1[l] = min(m1[l], key); else m0[l] = min(m0[l], key);
+                }
+            }
+            float out = 0.0f;
+#pragma unroll
+            for (int l = 0; l < LOGQ; l++) {
+                const uint32_t k0 = __reduce_min_sync(NB_FULL, m0[l]), k1 = __reduce_min_sync(NB_FULL, m1[l]);
+                const float x0 = __uint_as_float((k0 & 0x80000000u) ? k0 ^ 0x80000000u : ~k0);
+                const float x1 = __uint_as_float((k1 & 0x80000000u) ? k1 ^ 0x80000000u : ~k1);
+                if (lane == l) out = __fsub_rn(x1, x0);
+            }
+            if (lane < LOGQ) a.soft_llr[var * LOGQ + lane] = out;
+        }
+    }
+}
+
+template <int Q, bool CLOSED, int ECN, bool SOFT>
 __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_kernel(const KArgs a)
 {
     constexpr int VPL = QTraits<Q>::VPL;
@@ -887,6 +941,7 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
             a.out_synd[base + tid] = s_synd[tid];
             a.out_iters[base + tid] = s_done[tid] > 0 ? s_done[tid] : a.nb_iter_max;      /* NB_LDPC.c:474 */
         }
+        if constexpr (SOFT) soft_output<Q, ECN>(a, wm, gf, app, base, nf, warp, nw, lane);
     }
 }
 
@@ -1093,13 +1148,18 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
     }
 }
 
-template <int ECN> static const void *decode_fn_e(int q, int closed)
+template <int ECN, bool SOFT> static const void *decode_fn_e(int q, int closed)
 {
-    if (closed) return q == 16 ? (const void *)decode_kernel<16, true, ECN> : q == 64 ? (const void *)decode_kernel<64, true, ECN> : (const void *)decode_kernel<256, true, ECN>;
-    return q == 16 ? (const void *)decode_kernel<16, false, ECN> : q == 64 ? (const void *)decode_kernel<64, false, ECN> : (const void *)decode_kernel<256, false, ECN>;
+    if (closed) return q == 16 ? (const void *)decode_kernel<16, true, ECN, SOFT> : q == 64 ? (const void *)decode_kernel<64, true, ECN, SOFT> : (const void *)decode_kernel<256, true, ECN, SOFT>;
+    return q == 16 ? (const void *)decode_kernel<16, false, ECN, SOFT> : q == 64 ? (const void *)decode_kernel<64, false, ECN, SOFT> : (const void *)decode_kernel<256, false, ECN, SOFT>;
 }
-/* q is validated in nbgpu_create (16, 64 or 256); anything else never reaches a launch */
-static const void *decode_fn(int q, int closed, int ecn) { if (q != 16 && q != 64 && q != 256) return nullptr; return ecn ? decode_fn_e<1>(q, closed) : decode_fn_e<0>(q, closed); }
+/* q is validated in nbgpu_create (16, 64 or 256); anything else never reaches a launch.  soft: a soft-output kind is armed */
+static const void *decode_fn(int q, int closed, int ecn, bool soft)
+{
+    if (q != 16 && q != 64 && q != 256) return nullptr;
+    if (soft) return ecn ? decode_fn_e<1, true>(q, closed) : decode_fn_e<0, true>(q, closed);
+    return ecn ? decode_fn_e<1, false>(q, closed) : decode_fn_e<0, false>(q, closed);
+}
 static const void *checknode_fn(int q, int closed, int ecn)
 {
     if (ecn) {
@@ -1136,6 +1196,10 @@ struct nbgpu_ctx {
     unsigned *d_queue, *d_slow, *d_ready, *d_fault;
     unsigned *h_ready;                       /* pinned: cumulative frame counts of the input pieces of decode_host */
     int resident_B, resident_kind;
+    /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
+     * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
+     * kernel was launched at least once */
+    int soft_made, soft_B, decoded;
     /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames */
     struct {
         int ready, nlevels, B;
@@ -1414,10 +1478,11 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     k.hval = c->d_hval; k.rotin = c->d_rotin; k.rotout = c->d_rotout; k.img = c->d_img; k.inv = c->d_inv;
 
     /* persistent grid: one CTA per SM */
-    const void *fn = decode_fn(q, k.gf_closed, k.ecn);
+    const void *fn = decode_fn(q, k.gf_closed, k.ecn, false);
     /* opt in to the device maximum, not to this context's size: the attribute is per function and several contexts with
      * different geometries may share a kernel */
     CKF(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
+    CKF(cudaFuncSetAttribute(decode_fn(q, k.gf_closed, k.ecn, true), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     const void *fn2 = checknode_fn(q, k.gf_closed, k.ecn);
     CKF(cudaFuncSetAttribute(fn2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prop.sharedMemPerBlockOptin));
     int per_sm = 0;
@@ -1462,7 +1527,7 @@ extern "C" void nbgpu_destroy(nbgpu_ctx *c)
     cudaSetDevice(c->device);
     void *bufs[] = { c->d_cfg, c->d_ctov_dense, c->d_row_ptr, c->d_col, c->d_cninfo, c->d_einfo, c->d_step_ptr, c->d_isolated, c->d_hval, c->d_rotin,
                      c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
-                     c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue };
+                     c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue, c->k.soft_llr, c->k.soft_sym };
     for (void *b : bufs) if (b) cudaFree(b);
     if (c->h_ready) cudaFreeHost(c->h_ready);
     source_teardown(c);
@@ -1490,6 +1555,7 @@ static int ensure_input(nbgpu_ctx *c, size_t floats)
 static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B, int kind)
 {
     if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    c->soft_made = NBGPU_SOFT_NONE;                           /* even a rejected batch: the caller moved on from the last one */
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     int rc = ensure_input(c, per_frame * (size_t)B);          /* grows on demand: dense-LLR batches are q/log2(q) times larger */
@@ -1536,11 +1602,13 @@ extern "C" int nbgpu_run(nbgpu_ctx *c)
     CK(c, cudaEventRecord(c->ev0, c->stream));
     {
         void *args[] = { (void *)&k };
-        CK(c, cudaLaunchKernel(decode_fn(c->q, k.gf_closed, k.ecn), dim3(grid), dim3(k.nw * 32), args, k.smem_bytes, c->stream));
+        c->soft_made = NBGPU_SOFT_NONE;
+        CK(c, cudaLaunchKernel(decode_fn(c->q, k.gf_closed, k.ecn, k.soft_kind != NBGPU_SOFT_NONE), dim3(grid), dim3(k.nw * 32), args, k.smem_bytes, c->stream));
     }
     CK(c, cudaGetLastError());
     CK(c, cudaEventRecord(c->ev1, c->stream));
     c->launches += 1;
+    c->decoded = 1; c->soft_made = k.soft_kind; c->soft_B = k.B;
     if (c->src.state == 1) c->src.state = 2;
     return NBGPU_OK;
 }
@@ -1628,6 +1696,7 @@ extern "C" int nbgpu_download(nbgpu_ctx *c, int *decide, int *synd, int *iters)
 static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kind, int B, int *decide, int *synd, int *iters)
 {
     if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     const int wave = c->grid * c->k.F;
     if (B < 2 * wave || getenv("NBGPU_NO_CHUNKS")) {
@@ -1664,11 +1733,12 @@ static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kin
     CK(c, cudaEventRecord(c->ev0, c->stream));
     {
         void *args[] = { (void *)&k };
-        CK(c, cudaLaunchKernel(decode_fn(c->q, k.gf_closed, k.ecn), dim3(c->grid), dim3(k.nw * 32), args, k.smem_bytes, c->stream));
+        CK(c, cudaLaunchKernel(decode_fn(c->q, k.gf_closed, k.ecn, k.soft_kind != NBGPU_SOFT_NONE), dim3(c->grid), dim3(k.nw * 32), args, k.smem_bytes, c->stream));
     }
     CK(c, cudaGetLastError());
     CK(c, cudaEventRecord(c->ev1, c->stream));
     c->launches += 1;
+    c->decoded = 1;
     unsigned fault = 0;
     if (decide) CK(c, cudaMemcpyAsync(decide, c->d_decide, (size_t)B * c->N * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     if (synd) CK(c, cudaMemcpyAsync(synd, c->d_synd, (size_t)B * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
@@ -1677,6 +1747,7 @@ static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kin
     CK(c, cudaStreamSynchronize(c->copy_stream));
     CK(c, cudaStreamSynchronize(c->stream));
     if (fault) { ctx_err(c, "decode: the kernel gave up waiting for its input frames (host-to-device copy did not arrive)"); return NBGPU_ECUDA; }
+    c->soft_made = k.soft_kind; c->soft_B = B;                /* only a launch that saw all its frames leaves soft output */
     return NBGPU_OK;
 }
 
@@ -1800,6 +1871,7 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
 extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
     if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     if ((double)B * c->N * c->logq >= 2147483648.0) { ctx_err(c, "frame source: B*N*log2(q) must stay below 2^31"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
@@ -1913,6 +1985,75 @@ extern "C" int nbgpu_get_state(nbgpu_ctx *c, int frame, float *APP, float *CtoV)
             for (int kk = 0; kk < stp; kk++) { float l; memcpy(&l, r + 4 * kk, 4); CtoV[(size_t)e * q + r[tail + 8 + kk]] = l; }
         }
     }
+    return NBGPU_OK;
+}
+
+/* ---- soft output (include/nbldpc_b200.h; computed by soft_output at the end of every group of decode_kernel<..., true>) ---- */
+extern "C" int nbgpu_set_soft_output(nbgpu_ctx *c, int kind, int k)
+{
+    if (!c) { ctx_err(NULL, "nbgpu_set_soft_output: NULL context"); return NBGPU_EINVAL; }
+    const int kmax = std::min(c->q, 32);
+    const bool ok = kind == NBGPU_SOFT_LIST ? (k >= 1 && k <= kmax) : (kind == NBGPU_SOFT_NONE || kind == NBGPU_SOFT_BITS) && k == 0;
+    if (!ok) {
+        ctx_err(c, "nbgpu_set_soft_output: kind %d with k = %d (NBGPU_SOFT_LIST: 1 <= k <= min(q, 32) = %d; NBGPU_SOFT_BITS, NBGPU_SOFT_NONE: k = 0)", kind, k, kmax);
+        return NBGPU_EINVAL;
+    }
+    CK(c, cudaSetDevice(c->device));
+    CK(c, cudaStreamSynchronize(c->stream));               /* a launch in flight may still write the old buffers */
+    KArgs &ka = c->k;
+    CK(c, cudaFree(ka.soft_llr)); CK(c, cudaFree(ka.soft_sym));
+    ka.soft_llr = nullptr; ka.soft_sym = nullptr; ka.soft_kind = NBGPU_SOFT_NONE; ka.soft_k = 0;
+    c->soft_made = NBGPU_SOFT_NONE;
+    if (kind == NBGPU_SOFT_NONE) return NBGPU_OK;
+    const size_t n = (size_t)c->max_batch * c->N * (kind == NBGPU_SOFT_LIST ? k : c->logq);
+    float *llr = nullptr; uint8_t *sym = nullptr;
+    cudaError_t e = cudaMalloc((void **)&llr, n * sizeof(float));
+    if (e == cudaSuccess && kind == NBGPU_SOFT_LIST) e = cudaMalloc((void **)&sym, n);
+    if (e != cudaSuccess) {
+        cudaGetLastError();
+        cudaFree(llr);
+        ctx_err(c, "nbgpu_set_soft_output: %zu bytes of soft output for max_batch = %d frames do not fit on device %d (%s); soft output is off",
+                n * (kind == NBGPU_SOFT_LIST ? 5 : 4), c->max_batch, c->device, cudaGetErrorString(e));
+        return NBGPU_ENOMEM;
+    }
+    ka.soft_llr = llr; ka.soft_sym = sym; ka.soft_kind = kind; ka.soft_k = k;
+    return NBGPU_OK;
+}
+
+static int soft_available(nbgpu_ctx *c, int kind, const char *fn)
+{
+    if (!c->decoded) { ctx_err(c, "%s: nothing decoded", fn); return NBGPU_EINVAL; }
+    if (c->soft_made != kind) {
+        ctx_err(c, "%s: the last decode launch left no %s soft output (armed kind %d; re-arming or a new batch invalidates it)", fn,
+                kind == NBGPU_SOFT_LIST ? "NBGPU_SOFT_LIST" : "NBGPU_SOFT_BITS", c->k.soft_kind);
+        return NBGPU_ESTATE;
+    }
+    return NBGPU_OK;
+}
+
+extern "C" int nbgpu_download_soft_list(nbgpu_ctx *c, float *llr, int *sym)
+{
+    if (!c || !llr || !sym) { ctx_err(c, "nbgpu_download_soft_list: NULL argument"); return NBGPU_EINVAL; }
+    int rc = soft_available(c, NBGPU_SOFT_LIST, "nbgpu_download_soft_list");
+    if (rc) return rc;
+    CK(c, cudaSetDevice(c->device));
+    const size_t n = (size_t)c->soft_B * c->N * c->k.soft_k;
+    std::vector<uint8_t> s(n);
+    CK(c, cudaMemcpyAsync(llr, c->k.soft_llr, n * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaMemcpyAsync(s.data(), c->k.soft_sym, n, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    for (size_t i = 0; i < n; i++) sym[i] = s[i];
+    return NBGPU_OK;
+}
+
+extern "C" int nbgpu_download_soft_bits(nbgpu_ctx *c, float *llr)
+{
+    if (!c || !llr) { ctx_err(c, "nbgpu_download_soft_bits: NULL argument"); return NBGPU_EINVAL; }
+    int rc = soft_available(c, NBGPU_SOFT_BITS, "nbgpu_download_soft_bits");
+    if (rc) return rc;
+    CK(c, cudaSetDevice(c->device));
+    CK(c, cudaMemcpyAsync(llr, c->k.soft_llr, (size_t)c->soft_B * c->N * c->logq * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
     return NBGPU_OK;
 }
 

@@ -192,6 +192,34 @@ int  nbgpu_source_set_margin(nbgpu_ctx *ctx, double margin);
  * the last batch.  Only frames whose working set is still resident can be read (NBGPU_ESTATE). */
 int nbgpu_get_state(nbgpu_ctx *ctx, int frame, float *APP, float *CtoV);
 
+/* ---- Soft output of every frame of a batch ----
+ * Computed by the decode kernel from the final APP[N][q] of each frame: the APP at the early stop (NB_LDPC.c:470) for a
+ * frame that stopped early, else the APP after the last pass -- exactly the array nbgpu_get_state returns.  Isolated
+ * variables report their intake row.  A context produces at most one kind per launch.
+ *
+ * NBGPU_SOFT_LIST, 1 <= k <= min(q, 32): per variable the k most likely symbols, by the truncation rule NB_LDPC.c:354-374
+ *   with n_m = k applied to the APP row: ascending, ties -> lowest symbol; values >= 1e5 are never selected and such a
+ *   slot keeps (1e5, symbol 0); then llr[i] -= llr[0], llr[0] = 0.  llr[B][N][k] f32 and sym[B][N][k] symbols in GF
+ *   order (0 = zero, s = alpha^(s-1)), as nbgpu_select_nm would return for the row; sym[..][0] equals the decision.
+ * NBGPU_SOFT_BITS, k = 0: per variable log2(q) bit reliabilities in the distance convention,
+ *   b[l] = min{APP[s] : bingf[s][l] = 1} - min{APP[s] : bingf[s][l] = 0}, one f32 subtraction (round to nearest) of two
+ *   exact minima; b[l] > 0 favours bit 0.  llr[B][N][log2 q] f32, the layout of the `noisy` input.
+ * NBGPU_SOFT_NONE, k = 0: no soft output (the default). */
+#define NBGPU_SOFT_NONE 0
+#define NBGPU_SOFT_LIST 1
+#define NBGPU_SOFT_BITS 2
+/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 including their streamed path,
+ * nbgpu_source_frames + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
+ * if that does not fit, after which ctx stays usable with soft output off.  A bad kind or k is NBGPU_EINVAL and leaves
+ * the context as it was.  Invalidates the soft output of the last batch. */
+int nbgpu_set_soft_output(nbgpu_ctx *ctx, int kind, int k);
+/* The soft output of the B frames of the last decode launch: llr/sym [B][N][k] (LIST), llr [B][N][log2 q] (BITS).
+ * NBGPU_EINVAL before any decode launch; NBGPU_ESTATE when the last launch did not produce this kind, or when the
+ * soft output was invalidated since (re-armed, or another batch uploaded / generated).  Unit-boundary calls
+ * (nbgpu_check_node, ...) leave it alone. */
+int nbgpu_download_soft_list(nbgpu_ctx *ctx, float *llr, int *sym);
+int nbgpu_download_soft_bits(nbgpu_ctx *ctx, float *llr);
+
 /* Boundary 1 (unit parity): one check node for B independent input sets.
  * replaces CheckPassLogEMS (bubble_decoder.h:17) / syndrome_ems (syndrome_decoder.h:14):
  * vllr/vgf[B][dc][n_m] = decoder->M_VtoC_LLR/GF before the call, cllr/cgf[B][dc][q] =
