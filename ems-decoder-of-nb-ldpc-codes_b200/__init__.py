@@ -121,6 +121,7 @@ def lib():
         "nbgpu_download_soft_list": (C.c_int, [vp, _fp, _ip]),
         "nbgpu_download_soft_bits": (C.c_int, [vp, _fp]),
         "nbgpu_source_frames": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
+        "nbgpu_source_frames_apsk64": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_download": (C.c_int, [vp, _ip, _fp]),
         "nbgpu_source_results": (C.c_int, [vp, _ip, _ip, _ip]),
         "nbgpu_source_fixups": (C.c_long, [vp]),
@@ -265,6 +266,7 @@ class Decoder:
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
         self.soft_k = 0
+        self.source_channel = None                            # "bpsk" | "apsk64": channel of the generated batch
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
@@ -334,16 +336,28 @@ class Decoder:
     def source_frames(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames: frames [frame0, frame0+B) of the reference's stream generated on the device and left resident
         (origin: drand48 state before frame 0 as an int, default = the reference's unseeded stream)."""
+        self._source(lib().nbgpu_source_frames, frame0, B, ebn, origin)
+        self.source_channel = "bpsk"
+
+    def source_frames_apsk64(self, frame0, B, ebn, origin=None):
+        """nbgpu_source_frames_apsk64: the same for a GF(64) code sent as 64-APSK symbols (ModelChannel_AWGN_64); the batch is
+        resident as after an upload of noisy[B, N, 2] samples."""
+        self._source(lib().nbgpu_source_frames_apsk64, frame0, B, ebn, origin)
+        self.source_channel = "apsk64"
+
+    def _source(self, fn, frame0, B, ebn, origin):
         r = Rng()
         lib().nbgpu_rng_reference_default(C.byref(r))
         if origin is not None:
             r.x = origin
-        _check(lib().nbgpu_source_frames(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn)), self.h)
+        _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn)), self.h)
         self.B = B
 
     def source_download(self, want_noisy=True):
+        """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        noisy = np.zeros((self.B, self.code.N, self.code.logq), np.float32) if want_noisy else None
+        spf = 2 if self.source_channel == "apsk64" else self.code.logq
+        noisy = np.zeros((self.B, self.code.N, spf), np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy
 

@@ -1200,14 +1200,15 @@ struct nbgpu_ctx {
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
     int soft_made, soft_B, decoded;
-    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames */
+    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames / _apsk64 */
     struct {
         int ready, nlevels, B;
+        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 64-APSK */
         int *d_level_ptr, *d_row_order, *d_ut_ptr, *d_ut_col, *d_perm, *d_bit_errors;
-        uint8_t *d_ut_val, *d_piv, *d_mulimg, *d_divimg, *d_cw;
+        uint8_t *d_ut_val, *d_piv, *d_mulimg, *d_divimg, *d_cw, *d_flag_img;
         unsigned *d_flag_count, *d_flags, *d_patch_idx;
         float *d_patch_val;
-        uint64_t D;
+        uint64_t D;              /* draws per frame of the generated batch (depends on the channel) */
         double margin;
         long fixups;
         uint64_t code_hash;      /* graph + coefficients of the code the encoder tables were built from */
@@ -1789,7 +1790,7 @@ static void source_teardown(nbgpu_ctx *c)
 {
     void *sbufs[] = { c->src.d_level_ptr, c->src.d_row_order, c->src.d_ut_ptr, c->src.d_ut_col, c->src.d_perm, c->src.d_bit_errors, c->src.d_ut_val,
                       c->src.d_piv, c->src.d_mulimg, c->src.d_divimg, c->src.d_cw, c->src.d_flag_count, c->src.d_flags, c->src.d_patch_idx,
-                      c->src.d_patch_val };
+                      c->src.d_patch_val, c->src.d_flag_img };
     for (void *b : sbufs) if (b) cudaFree(b);
     const double margin = c->src.margin;
     memset(&c->src, 0, sizeof c->src);
@@ -1835,12 +1836,12 @@ static int source_setup(nbgpu_ctx *c, nbgpu_code *code)
     CK(c, cudaMalloc((void **)&c->src.d_flags, SRC_FLAG_CAP * sizeof(unsigned)));
     CK(c, cudaMalloc((void **)&c->src.d_patch_idx, SRC_FLAG_CAP * sizeof(unsigned)));
     CK(c, cudaMalloc((void **)&c->src.d_patch_val, SRC_FLAG_CAP * sizeof(float)));
+    CK(c, cudaMalloc((void **)&c->src.d_flag_img, SRC_FLAG_CAP));
     uint64_t mul[48], add[48], m_ = SRC_A, a_ = SRC_C;
     for (int j = 0; j < 48; j++) { mul[j] = m_; add[j] = a_; a_ = ((m_ + 1) * a_) & SRC_MASK; m_ = (m_ * m_) & SRC_MASK; }
     CK(c, cudaMemcpyToSymbol(c_src_mul, mul, sizeof mul));
     CK(c, cudaMemcpyToSymbol(c_src_add, add, sizeof add));
     c->src.nlevels = depth;
-    c->src.D = (uint64_t)(code->K + 2 * N) * c->logq;
     if (c->src.margin == 0.0) c->src.margin = 0x1p-46;
     c->src.code_hash = code_hash(code);
     c->src.ready = 1;
@@ -1857,6 +1858,7 @@ static SrcArgs source_args(nbgpu_ctx *c, const nbgpu_code *code, int B)
     a.img = c->d_img; a.cw = c->src.d_cw; a.noisy = c->d_in; a.margin = c->src.margin;
     a.flag_count = c->src.d_flag_count; a.flags = c->src.d_flags; a.flag_cap = SRC_FLAG_CAP;
     a.decide = c->d_decide; a.bit_errors = c->src.d_bit_errors;
+    a.mod = c->d_mod; a.flag_img = c->src.d_flag_img;
     (void)code;
     return a;
 }
@@ -1868,28 +1870,36 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
     return NBGPU_OK;
 }
 
-extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
+/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]) and nbgpu_source_frames_apsk64 (kind 2, 64-APSK:
+ * noisy[B][N][2]).  The channel fixes the draws per frame D, sigma, the noise kernel and the host recomputation of a
+ * flagged sample; encoder, flag read-back and patch are shared. */
+static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind)
 {
-    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
-    if ((double)B * c->N * c->logq >= 2147483648.0) { ctx_err(c, "frame source: B*N*log2(q) must stay below 2^31"); return NBGPU_EINVAL; }
+    const int spf = kind == 2 ? 2 : c->logq;                    /* noisy samples per symbol */
+    if ((double)B * c->N * spf >= 2147483648.0) { ctx_err(c, "frame source: B*N*%s must stay below 2^31", kind == 2 ? "2" : "log2(q)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     int rc;
     /* the encoder tables belong to ONE code: another code of the same size gets its own (the stale tables would encode
      * words of the first code and score the decoder against them) */
     if (c->src.ready && c->src.code_hash != code_hash(code)) { CK(c, cudaStreamSynchronize(c->stream)); source_teardown(c); }
     if (!c->src.ready && (rc = source_setup(c, code))) { source_teardown(c); return rc; }
-    if ((rc = ensure_input(c, (size_t)c->N * c->logq * B))) return rc;
-    const float sigma = nbgpu_sigma(code, EbN);
+    if ((rc = ensure_input(c, (size_t)c->N * spf * B))) return rc;
+    const uint64_t koff = (uint64_t)(c->N - c->M) * c->logq;   /* information-bit draws, tools.c:124-136 */
+    /* K log2 q information bits, then two draws per noisy sample (channel.c:56-57 per bit, channel.c:234-263 per I/Q) */
+    const uint64_t D = koff + 2 * (uint64_t)c->N * spf;
+    const float sigma = kind == 2 ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
     nbgpu_rng r = *origin;
-    nbgpu_rng_skip(&r, frame0 * c->src.D);
+    nbgpu_rng_skip(&r, frame0 * D);
+    c->src.D = D;
     SrcArgs a = source_args(c, code, B);
     a.x0 = r.x; a.sigma = sigma;
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
     const long long threads = (long long)B * c->N;
-    source_noise_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
+    if (kind == 2) source_noise_apsk64_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
+    else source_noise_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
     CK(c, cudaGetLastError());
     c->launches += 2;
     unsigned nflag = 0;
@@ -1898,17 +1908,24 @@ extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_r
     if (nflag > SRC_FLAG_CAP) { ctx_err(c, "frame source: %u samples flagged for host recomputation (capacity %u); margin too wide", nflag, SRC_FLAG_CAP); return NBGPU_EINVAL; }
     c->src.fixups = nflag;
     if (nflag) {
-        /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59) */
+        /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
+         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in both channels. */
         std::vector<unsigned> idx(nflag);
         std::vector<float> val(nflag);
+        std::vector<uint8_t> img(kind == 2 ? nflag : 0);
+        float mod[128];
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        const uint64_t per = (uint64_t)c->N * c->logq, koff = (uint64_t)(c->N - c->M) * c->logq;
+        if (kind == 2) {
+            CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
+            nbgpu_apsk64_table(mod);
+        }
+        const uint64_t per = (uint64_t)c->N * spf;
         for (unsigned i = 0; i < nflag; i++) {
             const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
             nbgpu_rng g; g.x = a.x0;
-            nbgpu_rng_skip(&g, f * c->src.D + koff + 2 * s);
+            nbgpu_rng_skip(&g, f * D + koff + 2 * s);
             const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-            val[i] = nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+            val[i] = kind == 2 ? nbgpu_apsk64_sample(sigma, mod[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
         CK(c, cudaMemcpyAsync(c->src.d_patch_val, val.data(), nflag * sizeof(float), cudaMemcpyHostToDevice, c->stream));
@@ -1917,9 +1934,22 @@ extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_r
         CK(c, cudaStreamSynchronize(c->stream));                 /* idx/val are stack-scoped */
         c->launches += 1;
     }
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);            /* 2.0*SQR(sigma), channel.c:73 */
-    c->resident_B = B; c->resident_kind = 0; c->src.B = B; c->src.state = 1;
+    c->k.den = 2.0 * (double)(float)(sigma * sigma);            /* 2.0*SQR(sigma), channel.c:73 / channel.c:280 */
+    c->resident_B = B; c->resident_kind = kind; c->src.B = B; c->src.kind = kind; c->src.state = 1;
     return NBGPU_OK;
+}
+
+extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
+{
+    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    return source_generate(c, code, origin, frame0, B, EbN, 0);
+}
+
+extern "C" int nbgpu_source_frames_apsk64(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
+{
+    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    if (!apsk64_ok(c)) return NBGPU_EINVAL;
+    return source_generate(c, code, origin, frame0, B, EbN, 2);
 }
 
 extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixups : 0; }
@@ -1936,7 +1966,8 @@ extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
         for (size_t i = 0; i < cw.size(); i++) codeword[i] = c->inv_h[cw[i]];
     }
     if (noisy) {
-        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * c->logq * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        const size_t spf = c->src.kind == 2 ? 2 : c->logq;
+        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * spf * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
     return NBGPU_OK;

@@ -477,10 +477,17 @@ float nbgpu_sigma_apsk64(float EbN)
 {
     return (float)sqrt(1.0 / (2.0 * pow(10, EbN / 10.0)));      /* channel.c:232 (no code rate here) */
 }
+/* one sample of channel.c:234-263 (point = I or Q coordinate of the symbol's constellation point); also the host
+ * recomputation of the 64-APSK samples the device source flags (nbldpc_source.cuh) */
+float nbgpu_apsk64_sample(float sigma, float point, float u, float v)
+{
+    const double pi = NB_PI;
+    return (float)(point + sigma * sqrt(-2.0 * log(u)) * cos(2.0 * pi * v));
+}
+
 /* noisy[N][2]: the constellation point of symbol n (binary image nbin[n][0..5], LSB first) plus Box-Muller noise, channel.c:234-263 */
 int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
 {
-    const double pi = NB_PI;
     const float sigma = nbgpu_sigma_apsk64(EbN);
     float mod[128];
     int n, q;
@@ -493,7 +500,7 @@ int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, 
         for (q = 0; q < 2; q++) {
             float u = draw_float(r);
             float v = draw_float(r);
-            noisy[2 * n + q] = mod[2 * som + q] + sigma * sqrt(-2.0 * log(u)) * cos(2.0 * pi * v);
+            noisy[2 * n + q] = nbgpu_apsk64_sample(sigma, mod[2 * som + q], u, v);
         }
     }
     return NBGPU_OK;

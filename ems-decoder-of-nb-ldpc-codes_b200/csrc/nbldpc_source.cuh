@@ -5,17 +5,20 @@
  *   Encoding                tools.c:232-270   back-substitution on the triangular matrix of GaussianElimination
  *                                             (tools.c:151-218; done once on the host, nbldpc_host.c)
  *   ModelChannel_AWGN_BPSK  channel.c:51-62   y = BPSK(b) + sigma*sqrt(-2 ln u)*cos(2 pi v), f64 -> f32
+ *   ModelChannel_AWGN_64    channel.c:234-263 (GF(64) only) y[c] = mod[som][c] + sigma*sqrt(-2 ln u)*cos(2 pi v), c = I, Q
  *   the error count         NB_LDPC.c:479-485 information-bit errors of the decided word
  *
- * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q, so every thread reaches its own
- * draws by LCG jump-ahead (48 precomputed powers of the affine map in constant memory).
+ * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q for BPSK and 6K + 4N for 64-APSK (two
+ * draws per noisy sample), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of the affine
+ * map in constant memory).  D is a property of the batch: one context may alternate the two channels.
  *
  * Exactness.  Everything except log() and cos() is IEEE arithmetic that the device reproduces bit for bit (explicit
  * __dmul_rn/__dadd_rn so that nothing is contracted into an FMA).  The device's log/cos may differ from glibc's by a
  * few ulp of a double, which changes the f32 sample only when the f64 value sits within that distance of an f32
  * rounding boundary.  Such samples (about one in 10^6) are FLAGGED by a margin test that is ~8x wider than the
- * documented error bounds, and recomputed by the host with glibc (nbgpu_noise_sample, nbldpc_host.c) before the
- * decoder reads them.  tests/test_gpu_source.py checks the stream against the host source sample by sample.
+ * documented error bounds, and recomputed by the host with glibc (nbgpu_noise_sample / nbgpu_apsk64_sample, nbldpc_host.c)
+ * before the decoder reads them.  tests/test_gpu_source.py and tests/test_gpu_source_apsk64.py check the stream against
+ * the host source sample by sample.
  *
  * GF arithmetic of the encoder runs on binary images (addition = XOR): mulimg[h][x] = img(h * sym(x)),
  * divimg[p][x] = img(sym(x) / p), both built on the host from the code's tables.
@@ -50,6 +53,8 @@ struct SrcArgs {
     unsigned flag_cap;
     const int *decide;           /* [B][N] */
     int *bit_errors;             /* [B] */
+    const float *mod;            /* [64][2] 64-APSK constellation by binary image (the decoder's intake table) */
+    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged 64-APSK sample */
 };
 
 __device__ __forceinline__ uint64_t src_skip(uint64_t x, uint64_t n)
@@ -121,6 +126,35 @@ __global__ void __launch_bounds__(256) source_noise_kernel(SrcArgs a)
             if (slot < a.flag_cap) a.flags[slot] = (unsigned)(id * a.logq + l) | ((unsigned)bit << 31);
         }
         out[l] = yf;
+    }
+}
+
+/* 64-APSK (ModelChannel_AWGN_64, channel.c:234-263): one thread per codeword symbol, its 4 draws (u, v for I, then u, v
+ * for Q), the symbol's constellation point plus noise, written as noisy[B][N][2] (the layout of nbgpu_upload_apsk64).
+ * Same arithmetic and margin test as source_noise_kernel; a flagged sample records its symbol's image for the host. */
+__global__ void __launch_bounds__(256) source_noise_apsk64_kernel(SrcArgs a)
+{
+    const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (id >= (long long)a.B * a.N) return;
+    const int f = (int)(id / a.N), n = (int)(id % a.N);
+    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * 4);
+    const int som = a.cw[id];
+    const double sigma = (double)a.sigma;
+    float *out = a.noisy + (size_t)id * 2;
+    for (int c = 0; c < 2; c++) {
+        const float u = src_draw(x);
+        const float v = src_draw(x);
+        const double r = sqrt(-2.0 * log((double)u));
+        const double cs = cos(__dmul_rn(2.0 * 3.1415926536, (double)v));         /* PI of channel.c:18 */
+        const double t = __dmul_rn(__dmul_rn(sigma, r), cs);
+        const double y = __dadd_rn((double)a.mod[2 * som + c], t);               /* point + noise, channel.c:234-263 */
+        const float yf = __double2float_rn(y);
+        const double d = a.margin * (fabs(t) + fabs(y));
+        if (!(__double2float_rn(y + d) == __double2float_rn(y - d))) {            /* also true for inf/NaN */
+            const unsigned slot = atomicAdd(a.flag_count, 1u);
+            if (slot < a.flag_cap) { a.flags[slot] = (unsigned)(id * 2 + c); a.flag_img[slot] = (uint8_t)som; }
+        }
+        out[c] = yf;
     }
 }
 

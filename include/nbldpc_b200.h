@@ -179,7 +179,15 @@ long nbgpu_slow_selects(nbgpu_ctx *ctx);
  * (nbgpu_source_fixups tells how many in the last call).  Afterwards the batch is resident as after
  * nbgpu_upload_noisy: call nbgpu_run, then nbgpu_source_results (or nbgpu_download for the decisions). */
 int  nbgpu_source_frames(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
-/* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq] */
+/* The same for a GF(64) code sent as 64-APSK symbols (ModelChannel_AWGN_64, channel.c:234-263): frame f owns the draws
+ * [f*D, (f+1)*D) with D = 6K + 4N, and its samples are bit-identical to nbgpu_random_codeword + nbgpu_awgn_apsk64_noise
+ * (sigma = nbgpu_sigma_apsk64(EbN)).  Afterwards the batch is resident as after nbgpu_upload_apsk64; nbgpu_run,
+ * nbgpu_source_results, nbgpu_download and the soft output work on it as on a BPSK batch.  One context may alternate BPSK
+ * and 64-APSK batches.  NBGPU_EINVAL: q != 64 (context unchanged); B outside 1..max_batch or B*N*2 >= 2^31 (as for
+ * nbgpu_source_frames, the soft output of the previous batch is dropped; the context stays usable). */
+int  nbgpu_source_frames_apsk64(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
+/* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq]
+ * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 */
 int  nbgpu_source_download(nbgpu_ctx *ctx, int *codeword, float *noisy);
 /* after nbgpu_run: information-bit errors of each frame (NB_LDPC.c:479-485), syndrome value, iteration count;
  * feed them to the frame-order statistics rule (NB_LDPC.c:474-507).  12 bytes per frame cross PCIe. */
@@ -209,7 +217,7 @@ int nbgpu_get_state(nbgpu_ctx *ctx, int frame, float *APP, float *CtoV);
 #define NBGPU_SOFT_LIST 1
 #define NBGPU_SOFT_BITS 2
 /* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 including their streamed path,
- * nbgpu_source_frames + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
+ * nbgpu_source_frames / _apsk64 + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
  * if that does not fit, after which ctx stays usable with soft output off.  A bad kind or k is NBGPU_EINVAL and leaves
  * the context as it was.  Invalidates the soft output of the last batch. */
 int nbgpu_set_soft_output(nbgpu_ctx *ctx, int kind, int k);
