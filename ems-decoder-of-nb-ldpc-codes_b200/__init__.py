@@ -20,6 +20,7 @@ LIB_PATH = os.environ.get("NBLDPC_B200_LIB") or os.path.join(HERE, "libnbldpc_b2
 OK, EINVAL, EIO, ENOMEM, ECUDA, ESTATE, ERANK = 0, -1, -2, -3, -4, -5, -6
 ALIST_AUTO, ALIST_UBS, ALIST_KN, ALIST_FULL = 0, 1, 2, 3
 SOFT_NONE, SOFT_LIST, SOFT_BITS = 0, 1, 2
+MAP_APSK64, MAP_QAM = 1, 2
 
 _ip = C.POINTER(C.c_int)
 _fp = C.POINTER(C.c_float)
@@ -66,6 +67,13 @@ def sigma_apsk64(ebn):
     return float(lib().nbgpu_sigma_apsk64(C.c_float(ebn)))
 
 
+def constellation(kind, q):
+    """nbgpu_constellation: mod[q][2] by binary image; MAP_APSK64 (q = 64) or MAP_QAM (Gray square q-QAM, q = 16, 64, 256)."""
+    mod = np.zeros((q, 2), np.float32)
+    _check(lib().nbgpu_constellation(kind, q, mod.ctypes.data_as(_fp)))
+    return mod
+
+
 def lib():
     """The loaded C-ABI library.  Fails loudly when it has not been built."""
     global _lib
@@ -97,6 +105,12 @@ def lib():
         "nbgpu_channel_awgn_apsk64": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
         "nbgpu_decode_apsk64": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
         "nbgpu_upload_apsk64": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
+        "nbgpu_constellation": (C.c_int, [C.c_int, C.c_int, _fp]),
+        "nbgpu_awgn_mapped_noise": (C.c_int, [vp, C.POINTER(Rng), _ip, _fp, C.c_float, _fp]),
+        "nbgpu_set_constellation": (C.c_int, [vp, _fp]),
+        "nbgpu_channel_awgn_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
+        "nbgpu_decode_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
+        "nbgpu_upload_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
         "nbgpu_create": (C.c_int, [C.POINTER(vp), vp, C.POINTER(Params), C.c_int, C.c_int]),
         "nbgpu_destroy": (None, [vp]),
         "nbgpu_last_error": (C.c_char_p, [vp]),
@@ -122,6 +136,7 @@ def lib():
         "nbgpu_download_soft_bits": (C.c_int, [vp, _fp]),
         "nbgpu_source_frames": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_frames_apsk64": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
+        "nbgpu_source_frames_mapped": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_download": (C.c_int, [vp, _ip, _fp]),
         "nbgpu_source_results": (C.c_int, [vp, _ip, _ip, _ip]),
         "nbgpu_source_fixups": (C.c_long, [vp]),
@@ -231,6 +246,14 @@ class Code:
         _check(lib().nbgpu_awgn_apsk64_noise(self.h, C.byref(self.rng), _i(nb), C.c_float(ebn), _f(noisy)))
         return noisy
 
+    def noise_mapped(self, nbin, mod, ebn):
+        """channel.c:234-263 on the constellation mod[q][2] (by binary image) for one frame: noisy[N][2], sigma_apsk64(ebn)."""
+        noisy = np.zeros((self.N, 2), np.float32)
+        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
+        m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
+        _check(lib().nbgpu_awgn_mapped_noise(self.h, C.byref(self.rng), _i(nb), _f(m), C.c_float(ebn), _f(noisy)))
+        return noisy
+
     def accumulate_stats(self, codeword_bits, decide, synd, iters, stats):
         cb = np.ascontiguousarray(codeword_bits, np.int32)
         d = np.ascontiguousarray(decide, np.int32)
@@ -266,7 +289,7 @@ class Decoder:
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
         self.soft_k = 0
-        self.source_channel = None                            # "bpsk" | "apsk64": channel of the generated batch
+        self.source_channel = None                            # "bpsk" | "apsk64" | "mapped": channel of the generated batch
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
@@ -296,6 +319,34 @@ class Decoder:
         ig = np.zeros(llr.shape, np.int32) if want_sorted else None
         _check(lib().nbgpu_channel_awgn_apsk64(self.h, _f(noisy), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
         return (llr, il, ig) if want_sorted else llr
+
+    def set_constellation(self, mod):
+        """nbgpu_set_constellation: bind mod[q][2] (by binary image) to the *_mapped calls of this context."""
+        m = np.ascontiguousarray(mod, np.float32).reshape(self.code.q, 2)
+        _check(lib().nbgpu_set_constellation(self.h, _f(m)), self.h)
+
+    def decode_mapped(self, noisy, sigma):
+        """nbgpu_decode_mapped: frames received as samples [B, N, 2] of the bound constellation."""
+        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
+        B = noisy.shape[0]
+        d, s, it = self._out(B)
+        _check(lib().nbgpu_decode_mapped(self.h, _f(noisy), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
+        self.B = B
+        return d, s, it
+
+    def channel_mapped(self, noisy, sigma, want_sorted=False):
+        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
+        B = noisy.shape[0]
+        llr = np.zeros((B, self.code.N, self.code.q), np.float32)
+        il = np.zeros_like(llr) if want_sorted else None
+        ig = np.zeros(llr.shape, np.int32) if want_sorted else None
+        _check(lib().nbgpu_channel_awgn_mapped(self.h, _f(noisy), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
+        return (llr, il, ig) if want_sorted else llr
+
+    def upload_mapped(self, noisy, sigma):
+        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
+        _check(lib().nbgpu_upload_mapped(self.h, _f(noisy), C.c_float(sigma), noisy.shape[0]), self.h)
+        self.B = noisy.shape[0]
 
     def decode_noisy_into(self, noisy, sigma, out):
         """nbgpu_decode_noisy on caller-owned (e.g. pinned) buffers, no allocation: noisy [B,N,logq] f32, out = (decide, synd, iters)."""
@@ -345,6 +396,11 @@ class Decoder:
         self._source(lib().nbgpu_source_frames_apsk64, frame0, B, ebn, origin)
         self.source_channel = "apsk64"
 
+    def source_frames_mapped(self, frame0, B, ebn, origin=None):
+        """nbgpu_source_frames_mapped: the same for a code sent on the bound constellation; D = K log2(q) + 4N draws per frame."""
+        self._source(lib().nbgpu_source_frames_mapped, frame0, B, ebn, origin)
+        self.source_channel = "mapped"
+
     def _source(self, fn, frame0, B, ebn, origin):
         r = Rng()
         lib().nbgpu_rng_reference_default(C.byref(r))
@@ -354,9 +410,9 @@ class Decoder:
         self.B = B
 
     def source_download(self, want_noisy=True):
-        """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK"""
+        """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        spf = 2 if self.source_channel == "apsk64" else self.code.logq
+        spf = 2 if self.source_channel in ("apsk64", "mapped") else self.code.logq
         noisy = np.zeros((self.B, self.code.N, spf), np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy

@@ -32,6 +32,7 @@
 #include "nbldpc_synd.cuh"
 #include "nbldpc_source.cuh"
 #include "nbldpc_internal.h"
+#include <cmath>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
@@ -76,7 +77,7 @@ struct KArgs {
     int n_m, nb_oper, passes, early_stop, nb_iter_max;
     float offset;
     int F, nw, cpw, cap, nsteps, L;     /* frames per group, warps per CTA, check nodes per warp, items per step, steps, lists per node */
-    int B, input_kind, frame0;          /* frames of this launch; 0 = BPSK samples, 1 = dense LLR, 2 = 64-APSK samples; batch index of its first frame */
+    int B, input_kind, frame0;          /* frames of this launch; 0 = BPSK samples, 1 = dense LLR, 2 = mapped (I, Q) samples; batch index of its first frame */
     double den;                         /* 2.0 * (double)(float)(sigma*sigma), channel.c:73 */
     const int *step_ptr, *isolated;
     int n_isolated;
@@ -84,7 +85,7 @@ struct KArgs {
     const uint32_t *einfo;              /* [E] variable | coefficient << 20 | last-visit flag << 28 */
     const int *row_ptr, *col;
     const uint8_t *hval, *rotin, *rotout, *img, *inv;
-    const float *mod;                   /* [64][2] normalised 64-APSK constellation by binary image (GF(64) only), input_kind 2 */
+    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, input_kind 2 (set per launch) */
     int gf_closed;
     const float *in;
     float *app; uint8_t *ctov; uint8_t *dec;
@@ -294,17 +295,19 @@ __device__ __forceinline__ void intake_variable(const float *noisy_n, double den
     __syncwarp();
 }
 
-/* LLR intake for one variable of a GF(64) code sent as one 64-APSK symbol (channel.c:268-291): for every symbol k,
- * TMP[k] = (float)( (double)((I - mI)^2) / (2 sigma^2) + (double)((Q - mQ)^2) / (2 sigma^2) ) with (mI, mQ) the constellation point of the
- * symbol's binary image; differences and squares in f32, divisions and the sum in f64, as the reference evaluates them. */
+/* LLR intake for one variable sent as one point of a q-point constellation (the mapped channel; channel.c:268-291 for
+ * 64-APSK): for every symbol k, TMP[k] = (float)( (double)((I - mI)^2) / (2 sigma^2) + (double)((Q - mQ)^2) / (2 sigma^2) )
+ * with (mI, mQ) = mod[binary image of k]; differences and squares in f32, divisions and the sum in f64, as the reference
+ * evaluates them (a reciprocal multiply would round differently).  GF(16): lanes >= 16 hold no symbol. */
 template <int Q>
-__device__ __forceinline__ void intake_apsk64(const float *noisy_n, double den, const float *mod, const uint8_t *img, int lane,
+__device__ __forceinline__ void intake_mapped(const float *noisy_n, double den, const float *mod, const uint8_t *img, int lane,
                                               float (&v)[QTraits<Q>::VPL])
 {
     const float y0 = noisy_n[0], y1 = noisy_n[1];
 #pragma unroll
     for (int j = 0; j < QTraits<Q>::VPL; j++) {
-        const int som = img[QTraits<Q>::sym(lane, j) & 63];
+        if (Q < 32 && lane >= Q) { v[j] = 0.0f; continue; }
+        const int som = img[QTraits<Q>::sym(lane, j)];
         const float d0 = __fsub_rn(y0, mod[2 * som]), d1 = __fsub_rn(y1, mod[2 * som + 1]);
         const double a = __ddiv_rn((double)__fmul_rn(d0, d0), den), b = __ddiv_rn((double)__fmul_rn(d1, d1), den);
         v[j] = __double2float_rn(__dadd_rn(a, b));
@@ -768,7 +771,7 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
             float v[VPL];
             if (a.input_kind == 0) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
                                                       reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
-            else if (Q == 64 && a.input_kind == 2) intake_apsk64<Q>(a.in + ((size_t)(base + f) * N + n) * 2, a.den, a.mod, gf.img, lane, v);
+            else if (a.input_kind == 2) intake_mapped<Q>(a.in + ((size_t)(base + f) * N + n) * 2, a.den, a.mod, gf.img, lane, v);
             else load_row<Q>(a.in + ((size_t)(base + f) * N + n) * Q, lane, v);
             store_row<Q>(app + ((size_t)f * N + n) * Q, lane, v);
         }
@@ -1127,7 +1130,7 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
     const long total = (long)B * a.N;
     for (long r = (long)blockIdx.x * UW + warp; r < total; r += (long)gridDim.x * UW) {
         float v[VPL];
-        if (Q == 64 && kind == 2) intake_apsk64<Q>(noisy + r * 2, a.den, a.mod, a.img, lane, v);
+        if (kind == 2) intake_mapped<Q>(noisy + r * 2, a.den, a.mod, a.img, lane, v);
         else intake_variable<Q>(noisy + r * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
         if (llr) store_row<Q>(llr + r * Q, lane, v);
         if (illr) {
@@ -1189,21 +1192,25 @@ struct nbgpu_ctx {
     uint32_t *d_cninfo, *d_einfo;
     uint8_t *d_cfg; float *d_ctov_dense;
     uint8_t *d_hval, *d_rotin, *d_rotout, *d_img, *d_inv;
-    float *d_mod;
+    float *d_mod;                            /* the 64-APSK table (q = 64), used by every *_apsk64 call */
+    float *d_map;                            /* the bound table of the mapped calls (nbgpu_set_constellation), NULL until bound */
+    float map_h[512];                        /* host copy of the bound table, for the frame source's fix-up */
     float *d_app; uint8_t *d_ctov; uint8_t *d_dec;
     float *d_in; size_t in_capacity;
     int *d_decide, *d_synd, *d_iters, *d_frame_slot, *d_slot_frame;
     unsigned *d_queue, *d_slow, *d_ready, *d_fault;
     unsigned *h_ready;                       /* pinned: cumulative frame counts of the input pieces of decode_host */
     int resident_B, resident_kind;
+    const float *resident_mod;               /* table of the resident batch (kind 2): d_mod or d_map */
+    int mapped_dropped;                      /* the resident mapped batch was dropped by nbgpu_set_constellation */
     /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
     int soft_made, soft_B, decoded;
-    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames / _apsk64 */
+    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames / _apsk64 / _mapped */
     struct {
         int ready, nlevels, B;
-        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 64-APSK */
+        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 mapped (64-APSK or bound table) */
         int *d_level_ptr, *d_row_order, *d_ut_ptr, *d_ut_col, *d_perm, *d_bit_errors;
         uint8_t *d_ut_val, *d_piv, *d_mulimg, *d_divimg, *d_cw, *d_flag_img;
         unsigned *d_flag_count, *d_flags, *d_patch_idx;
@@ -1473,7 +1480,6 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
         std::vector<float> mod(128);
         nbgpu_apsk64_table(mod.data());
         if ((rc = upload(c, &c->d_mod, mod))) { nbgpu_destroy(c); return rc; }
-        k.mod = c->d_mod;
     }
     k.row_ptr = c->d_row_ptr; k.col = c->d_col; k.cninfo = c->d_cninfo; k.einfo = c->d_einfo; k.step_ptr = c->d_step_ptr; k.isolated = c->d_isolated;
     k.hval = c->d_hval; k.rotin = c->d_rotin; k.rotout = c->d_rotout; k.img = c->d_img; k.inv = c->d_inv;
@@ -1527,7 +1533,7 @@ extern "C" void nbgpu_destroy(nbgpu_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     void *bufs[] = { c->d_cfg, c->d_ctov_dense, c->d_row_ptr, c->d_col, c->d_cninfo, c->d_einfo, c->d_step_ptr, c->d_isolated, c->d_hval, c->d_rotin,
-                     c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
+                     c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_map, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
                      c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue, c->k.soft_llr, c->k.soft_sym };
     for (void *b : bufs) if (b) cudaFree(b);
     if (c->h_ready) cudaFreeHost(c->h_ready);
@@ -1553,7 +1559,8 @@ static int ensure_input(nbgpu_ctx *c, size_t floats)
     return NBGPU_OK;
 }
 
-static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B, int kind)
+/* mod: the constellation of a kind-2 batch (d_mod or d_map), nullptr otherwise */
+static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B, int kind, const float *mod)
 {
     if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;                           /* even a rejected batch: the caller moved on from the last one */
@@ -1562,7 +1569,7 @@ static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B
     int rc = ensure_input(c, per_frame * (size_t)B);          /* grows on demand: dense-LLR batches are q/log2(q) times larger */
     if (rc) return rc;
     CK(c, cudaMemcpyAsync(c->d_in, src, per_frame * B * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    c->resident_B = B; c->resident_kind = kind; c->src.state = 0;
+    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod; c->mapped_dropped = 0; c->src.state = 0;
     return NBGPU_OK;
 }
 
@@ -1570,12 +1577,12 @@ extern "C" int nbgpu_upload_noisy(nbgpu_ctx *c, const float *noisy, float sigma,
 {
     if (!c) return NBGPU_EINVAL;
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:73 */
-    return upload_common(c, noisy, (size_t)c->N * c->logq, B, 0);
+    return upload_common(c, noisy, (size_t)c->N * c->logq, B, 0, nullptr);
 }
 extern "C" int nbgpu_upload_llr(nbgpu_ctx *c, const float *llr, int B)
 {
     if (!c) return NBGPU_EINVAL;
-    return upload_common(c, llr, (size_t)c->N * c->q, B, 1);
+    return upload_common(c, llr, (size_t)c->N * c->q, B, 1, nullptr);
 }
 static int apsk64_ok(nbgpu_ctx *c)
 {
@@ -1588,15 +1595,48 @@ extern "C" int nbgpu_upload_apsk64(nbgpu_ctx *c, const float *noisy, float sigma
     if (!c) return NBGPU_EINVAL;
     if (!apsk64_ok(c)) return NBGPU_EINVAL;
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return upload_common(c, noisy, (size_t)c->N * 2, B, 2);
+    return upload_common(c, noisy, (size_t)c->N * 2, B, 2, c->d_mod);
+}
+static int mapped_ok(nbgpu_ctx *c)
+{
+    if (c->d_map) return NBGPU_OK;
+    ctx_err(c, "mapped channel: no constellation bound to this context (call nbgpu_set_constellation first)");
+    return NBGPU_ESTATE;
+}
+extern "C" int nbgpu_upload_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
+    return upload_common(c, noisy, (size_t)c->N * 2, B, 2, c->d_map);
+}
+
+extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
+{
+    if (!c || !mod) { ctx_err(c, "nbgpu_set_constellation: NULL argument"); return NBGPU_EINVAL; }
+    for (int i = 0; i < 2 * c->q; i++)
+        if (!std::isfinite(mod[i])) { ctx_err(c, "nbgpu_set_constellation: mod[%d][%d] = %g is not finite", i / 2, i % 2, (double)mod[i]); return NBGPU_EINVAL; }
+    CK(c, cudaSetDevice(c->device));
+    if (!c->d_map) CK(c, cudaMalloc((void **)&c->d_map, 2 * (size_t)c->q * sizeof(float)));
+    /* stream order: a launch in flight still reads the old table */
+    CK(c, cudaMemcpyAsync(c->d_map, mod, 2 * (size_t)c->q * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    memcpy(c->map_h, mod, 2 * (size_t)c->q * sizeof(float));
+    if (c->resident_B > 0 && c->resident_kind == 2 && c->resident_mod == c->d_map) {
+        /* its samples were made for the old table: decoding them on the new one would be wrong */
+        c->resident_B = 0; c->mapped_dropped = 1; c->soft_made = NBGPU_SOFT_NONE; c->src.state = 0;
+    }
+    return NBGPU_OK;
 }
 
 extern "C" int nbgpu_run(nbgpu_ctx *c)
 {
+    if (c && c->resident_B < 1 && c->mapped_dropped) { ctx_err(c, "nbgpu_run: the mapped batch was dropped when nbgpu_set_constellation bound a new table"); return NBGPU_ESTATE; }
     if (!c || c->resident_B < 1) { ctx_err(c, "nbgpu_run: no resident batch (call nbgpu_upload_* first)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     KArgs k = c->k;
-    k.B = c->resident_B; k.input_kind = c->resident_kind; k.in = c->d_in;
+    k.B = c->resident_B; k.input_kind = c->resident_kind; k.in = c->d_in; k.mod = c->resident_mod;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     const int groups = (k.B + k.F - 1) / k.F;
     const int grid = std::min(c->grid, groups);
@@ -1694,21 +1734,21 @@ extern "C" int nbgpu_download(nbgpu_ctx *c, int *decide, int *synd, int *iters)
  * only the first groups ever wait and the H2D time disappears behind the kernel -- without cutting the batch into several
  * launches, whose starts and tails cost as much as the copies they hid (measured: 340 ms either way against 327.6 ms for the
  * kernel alone on config 5).  Small batches take the plain upload / run / download path (and keep their state readable). */
-static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kind, int B, int *decide, int *synd, int *iters)
+static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kind, const float *mod, int B, int *decide, int *synd, int *iters)
 {
     if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     const int wave = c->grid * c->k.F;
     if (B < 2 * wave || getenv("NBGPU_NO_CHUNKS")) {
-        int rc = upload_common(c, src, per_frame, B, kind);
+        int rc = upload_common(c, src, per_frame, B, kind, mod);
         if (rc || (rc = nbgpu_run(c)) || (rc = nbgpu_download(c, decide, synd, iters))) return rc;
         return NBGPU_OK;
     }
     CK(c, cudaSetDevice(c->device));
     int rc = ensure_input(c, per_frame * (size_t)B);
     if (rc) return rc;
-    c->resident_B = B; c->resident_kind = kind; c->src.state = 0;
+    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod; c->mapped_dropped = 0; c->src.state = 0;
     /* pieces: one wave first, the rest in up to 7 equal runs of whole waves */
     int lo[9], np = 1;
     {
@@ -1728,7 +1768,7 @@ static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kin
         CK(c, cudaMemcpyAsync(c->d_ready, c->h_ready + i, sizeof(unsigned), cudaMemcpyHostToDevice, c->copy_stream));
     }
     KArgs k = c->k;
-    k.B = B; k.input_kind = kind; k.in = c->d_in; k.ready = c->d_ready;
+    k.B = B; k.input_kind = kind; k.in = c->d_in; k.mod = mod; k.ready = c->d_ready;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     CK(c, cudaStreamWaitEvent(c->stream, c->ev_h2d[0], 0));   /* the counter starts at zero */
     CK(c, cudaEventRecord(c->ev0, c->stream));
@@ -1756,19 +1796,27 @@ extern "C" int nbgpu_decode_noisy(nbgpu_ctx *c, const float *noisy, float sigma,
 {
     if (!c) return NBGPU_EINVAL;
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:73 */
-    return decode_host(c, noisy, (size_t)c->N * c->logq, 0, B, decide, synd, iters);
+    return decode_host(c, noisy, (size_t)c->N * c->logq, 0, nullptr, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_llr(nbgpu_ctx *c, const float *llr, int B, int *decide, int *synd, int *iters)
 {
     if (!c) return NBGPU_EINVAL;
-    return decode_host(c, llr, (size_t)c->N * c->q, 1, B, decide, synd, iters);
+    return decode_host(c, llr, (size_t)c->N * c->q, 1, nullptr, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_apsk64(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
 {
     if (!c) return NBGPU_EINVAL;
     if (!apsk64_ok(c)) return NBGPU_EINVAL;
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return decode_host(c, noisy, (size_t)c->N * 2, 2, B, decide, synd, iters);
+    return decode_host(c, noisy, (size_t)c->N * 2, 2, c->d_mod, B, decide, synd, iters);
+}
+extern "C" int nbgpu_decode_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
+    return decode_host(c, noisy, (size_t)c->N * 2, 2, c->d_map, B, decide, synd, iters);
 }
 
 
@@ -1858,7 +1906,7 @@ static SrcArgs source_args(nbgpu_ctx *c, const nbgpu_code *code, int B)
     a.img = c->d_img; a.cw = c->src.d_cw; a.noisy = c->d_in; a.margin = c->src.margin;
     a.flag_count = c->src.d_flag_count; a.flags = c->src.d_flags; a.flag_cap = SRC_FLAG_CAP;
     a.decide = c->d_decide; a.bit_errors = c->src.d_bit_errors;
-    a.mod = c->d_mod; a.flag_img = c->src.d_flag_img;
+    a.flag_img = c->src.d_flag_img;
     (void)code;
     return a;
 }
@@ -1870,10 +1918,11 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
     return NBGPU_OK;
 }
 
-/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]) and nbgpu_source_frames_apsk64 (kind 2, 64-APSK:
- * noisy[B][N][2]).  The channel fixes the draws per frame D, sigma, the noise kernel and the host recomputation of a
- * flagged sample; encoder, flag read-back and patch are shared. */
-static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind)
+/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]) and nbgpu_source_frames_apsk64 / _mapped (kind 2, mapped:
+ * noisy[B][N][2] on the table mod_d, whose host copy is mod_h).  The channel fixes the draws per frame D, sigma, the noise
+ * kernel and the host recomputation of a flagged sample; encoder, flag read-back and patch are shared. */
+static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind,
+                           const float *mod_d, const float *mod_h)
 {
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
@@ -1894,11 +1943,11 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     nbgpu_rng_skip(&r, frame0 * D);
     c->src.D = D;
     SrcArgs a = source_args(c, code, B);
-    a.x0 = r.x; a.sigma = sigma;
+    a.x0 = r.x; a.sigma = sigma; a.mod = mod_d;
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
     const long long threads = (long long)B * c->N;
-    if (kind == 2) source_noise_apsk64_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
+    if (kind == 2) source_noise_mapped_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
     else source_noise_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
     CK(c, cudaGetLastError());
     c->launches += 2;
@@ -1913,19 +1962,15 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         std::vector<unsigned> idx(nflag);
         std::vector<float> val(nflag);
         std::vector<uint8_t> img(kind == 2 ? nflag : 0);
-        float mod[128];
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (kind == 2) {
-            CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
-            nbgpu_apsk64_table(mod);
-        }
+        if (kind == 2) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
         const uint64_t per = (uint64_t)c->N * spf;
         for (unsigned i = 0; i < nflag; i++) {
             const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
             nbgpu_rng g; g.x = a.x0;
             nbgpu_rng_skip(&g, f * D + koff + 2 * s);
             const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-            val[i] = kind == 2 ? nbgpu_apsk64_sample(sigma, mod[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+            val[i] = kind == 2 ? nbgpu_mapped_sample(sigma, mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
         CK(c, cudaMemcpyAsync(c->src.d_patch_val, val.data(), nflag * sizeof(float), cudaMemcpyHostToDevice, c->stream));
@@ -1935,21 +1980,32 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         c->launches += 1;
     }
     c->k.den = 2.0 * (double)(float)(sigma * sigma);            /* 2.0*SQR(sigma), channel.c:73 / channel.c:280 */
-    c->resident_B = B; c->resident_kind = kind; c->src.B = B; c->src.kind = kind; c->src.state = 1;
+    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod_d; c->mapped_dropped = 0;
+    c->src.B = B; c->src.kind = kind; c->src.state = 1;
     return NBGPU_OK;
 }
 
 extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
     if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    return source_generate(c, code, origin, frame0, B, EbN, 0);
+    return source_generate(c, code, origin, frame0, B, EbN, 0, nullptr, nullptr);
 }
 
 extern "C" int nbgpu_source_frames_apsk64(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
     if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    return source_generate(c, code, origin, frame0, B, EbN, 2);
+    float mod[128];
+    nbgpu_apsk64_table(mod);
+    return source_generate(c, code, origin, frame0, B, EbN, 2, c->d_mod, mod);
+}
+
+extern "C" int nbgpu_source_frames_mapped(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
+{
+    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    return source_generate(c, code, origin, frame0, B, EbN, 2, c->d_map, c->map_h);
 }
 
 extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixups : 0; }
@@ -2211,7 +2267,7 @@ extern "C" int nbgpu_decision_syndrome(nbgpu_ctx *c, const float *app, int *deci
     return NBGPU_OK;
 }
 
-static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf, int kind)
+static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf, int kind, const float *mod)
 {
     if (!c || !noisy || B < 1 || ((illr == NULL) != (igf == NULL))) { ctx_err(c, "nbgpu_channel_awgn_*: bad argument"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
@@ -2222,6 +2278,7 @@ static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, 
     CK(c, cudaMemcpyAsync(dn.p, noisy, (size_t)B * N * per * 4, cudaMemcpyHostToDevice, c->stream));
     KArgs k = c->k;
     k.den = 2.0 * (double)(float)(sigma * sigma);
+    k.mod = mod;
     const int grid = (int)std::min<long>(((long)B * N + UNIT_NT / 32 - 1) / (UNIT_NT / 32), 148 * 8);
     if (q == 16) channel_kernel<16><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
     else if (q == 64) channel_kernel<64><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
@@ -2238,11 +2295,18 @@ static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, 
 }
 extern "C" int nbgpu_channel_awgn_bpsk(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    return channel_common(c, noisy, sigma, B, llr, illr, igf, 0);
+    return channel_common(c, noisy, sigma, B, llr, illr, igf, 0, nullptr);
 }
 extern "C" int nbgpu_channel_awgn_apsk64(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
     if (!c) return NBGPU_EINVAL;
     if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    return channel_common(c, noisy, sigma, B, llr, illr, igf, 2);
+    return channel_common(c, noisy, sigma, B, llr, illr, igf, 2, c->d_mod);
+}
+extern "C" int nbgpu_channel_awgn_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    return channel_common(c, noisy, sigma, B, llr, illr, igf, 2, c->d_map);
 }

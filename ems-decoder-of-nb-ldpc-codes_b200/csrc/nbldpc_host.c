@@ -477,33 +477,61 @@ float nbgpu_sigma_apsk64(float EbN)
 {
     return (float)sqrt(1.0 / (2.0 * pow(10, EbN / 10.0)));      /* channel.c:232 (no code rate here) */
 }
-/* one sample of channel.c:234-263 (point = I or Q coordinate of the symbol's constellation point); also the host
- * recomputation of the 64-APSK samples the device source flags (nbldpc_source.cuh) */
-float nbgpu_apsk64_sample(float sigma, float point, float u, float v)
+/* one sample of channel.c:234-263 (point = I or Q coordinate of the symbol's constellation point), for any table; also the
+ * host recomputation of the mapped samples the device source flags (nbldpc_source.cuh) */
+float nbgpu_mapped_sample(float sigma, float point, float u, float v)
 {
     const double pi = NB_PI;
     return (float)(point + sigma * sqrt(-2.0 * log(u)) * cos(2.0 * pi * v));
 }
 
-/* noisy[N][2]: the constellation point of symbol n (binary image nbin[n][0..5], LSB first) plus Box-Muller noise, channel.c:234-263 */
-int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
+int nbgpu_constellation(int kind, int q, float *mod)
+{
+    if (!mod) { nbgpu_set_global_error("nbgpu_constellation: NULL table"); return NBGPU_EINVAL; }
+    if (kind == NBGPU_MAP_APSK64) {
+        if (q != 64) { nbgpu_set_global_error("nbgpu_constellation: 64-APSK has 64 points, not q = %d", q); return NBGPU_EINVAL; }
+        return nbgpu_apsk64_table(mod);
+    }
+    if (kind != NBGPU_MAP_QAM) { nbgpu_set_global_error("nbgpu_constellation: unknown kind %d (NBGPU_MAP_APSK64 = %d, NBGPU_MAP_QAM = %d)", kind, NBGPU_MAP_APSK64, NBGPU_MAP_QAM); return NBGPU_EINVAL; }
+    if (q != 16 && q != 64 && q != 256) { nbgpu_set_global_error("nbgpu_constellation: square QAM for q = 16, 64 or 256, not %d", q); return NBGPU_EINVAL; }
+    const int m = q == 16 ? 2 : q == 64 ? 3 : 4, L = 1 << m;
+    const double scale = sqrt(2.0 * (q - 1) / 3.0);             /* average power 1 */
+    for (int x = 0; x < q; x++)
+        for (int c = 0; c < 2; c++) {
+            const int g = (x >> (c * m)) & (L - 1);                 /* I: bits [0, m), Q: bits [m, 2m) */
+            int level = g;
+            for (int s = g >> 1; s; s >>= 1) level ^= s;            /* inverse binary-reflected Gray code */
+            mod[2 * x + c] = (float)((double)(2 * level - (L - 1)) / scale);
+        }
+    return NBGPU_OK;
+}
+
+/* noisy[N][2]: the point mod[img] of symbol n (binary image nbin[n][0..logq), LSB first) plus Box-Muller noise, channel.c:234-263 */
+int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, float *noisy)
 {
     const float sigma = nbgpu_sigma_apsk64(EbN);
-    float mod[128];
-    int n, q;
-    if (!c || !r || !noisy) { nbgpu_set_global_error("nbgpu_awgn_apsk64_noise: NULL argument"); return NBGPU_EINVAL; }
-    if (c->q != 64) { nbgpu_set_global_error("64-APSK maps one GF(64) symbol to one constellation point (q = %d)", c->q); return NBGPU_EINVAL; }
-    nbgpu_apsk64_table(mod);
+    int n, b;
+    if (!c || !r || !mod || !noisy) { nbgpu_set_global_error("nbgpu_awgn_mapped_noise: NULL argument"); return NBGPU_EINVAL; }
     for (n = 0; n < c->N; n++) {
         int som = 0;
-        for (q = 0; q < 6; q++) som += (nbin ? nbin[n * 6 + q] : 0) << q;
-        for (q = 0; q < 2; q++) {
+        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
+        for (b = 0; b < 2; b++) {
             float u = draw_float(r);
             float v = draw_float(r);
-            noisy[2 * n + q] = nbgpu_apsk64_sample(sigma, mod[2 * som + q], u, v);
+            noisy[2 * n + b] = nbgpu_mapped_sample(sigma, mod[2 * som + b], u, v);
         }
     }
     return NBGPU_OK;
+}
+
+/* noisy[N][2] over the 64-APSK table (nbgpu_apsk64_table) */
+int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
+{
+    float mod[128];
+    if (!c || !r || !noisy) { nbgpu_set_global_error("nbgpu_awgn_apsk64_noise: NULL argument"); return NBGPU_EINVAL; }
+    if (c->q != 64) { nbgpu_set_global_error("64-APSK maps one GF(64) symbol to one constellation point (q = %d)", c->q); return NBGPU_EINVAL; }
+    nbgpu_apsk64_table(mod);
+    return nbgpu_awgn_mapped_noise(c, r, nbin, mod, EbN, noisy);
 }
 
 /* NB_LDPC.c:474-507 */

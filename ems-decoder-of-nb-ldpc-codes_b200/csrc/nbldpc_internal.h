@@ -40,7 +40,7 @@ void nbgpu_set_global_error(const char *fmt, ...);
 const char *nbgpu_get_global_error(void);
 
 float nbgpu_noise_sample(float sigma, float u, float v, int bit);          /* channel.c:59, one sample */
-float nbgpu_apsk64_sample(float sigma, float point, float u, float v);    /* channel.c:234-263, one I or Q sample */
+float nbgpu_mapped_sample(float sigma, float point, float u, float v);    /* channel.c:234-263, one I or Q sample of any table */
 
 /* syndrome_ems configuration table (syndrome_decoder.c:1542, 1661, 2285); returns malloc'd [size*dc] */
 int *nbgpu_build_config_table(int dc, int d1, int d2, int d3, int trunc, int *size_out);

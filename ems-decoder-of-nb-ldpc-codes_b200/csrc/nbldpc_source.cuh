@@ -5,20 +5,21 @@
  *   Encoding                tools.c:232-270   back-substitution on the triangular matrix of GaussianElimination
  *                                             (tools.c:151-218; done once on the host, nbldpc_host.c)
  *   ModelChannel_AWGN_BPSK  channel.c:51-62   y = BPSK(b) + sigma*sqrt(-2 ln u)*cos(2 pi v), f64 -> f32
- *   ModelChannel_AWGN_64    channel.c:234-263 (GF(64) only) y[c] = mod[som][c] + sigma*sqrt(-2 ln u)*cos(2 pi v), c = I, Q
+ *   ModelChannel_AWGN_64    channel.c:234-263 y[c] = mod[som][c] + sigma*sqrt(-2 ln u)*cos(2 pi v), c = I, Q, on the 64-APSK table
+ *                                             or, for the mapped channel of any field, on the context's bound table
  *   the error count         NB_LDPC.c:479-485 information-bit errors of the decided word
  *
- * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q for BPSK and 6K + 4N for 64-APSK (two
- * draws per noisy sample), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of the affine
- * map in constant memory).  D is a property of the batch: one context may alternate the two channels.
+ * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q for BPSK and K log2 q + 4N for a mapped
+ * channel (two draws per noisy sample), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of
+ * the affine map in constant memory).  D is a property of the batch: one context may alternate the channels.
  *
  * Exactness.  Everything except log() and cos() is IEEE arithmetic that the device reproduces bit for bit (explicit
  * __dmul_rn/__dadd_rn so that nothing is contracted into an FMA).  The device's log/cos may differ from glibc's by a
  * few ulp of a double, which changes the f32 sample only when the f64 value sits within that distance of an f32
  * rounding boundary.  Such samples (about one in 10^6) are FLAGGED by a margin test that is ~8x wider than the
- * documented error bounds, and recomputed by the host with glibc (nbgpu_noise_sample / nbgpu_apsk64_sample, nbldpc_host.c)
- * before the decoder reads them.  tests/test_gpu_source.py and tests/test_gpu_source_apsk64.py check the stream against
- * the host source sample by sample.
+ * documented error bounds, and recomputed by the host with glibc (nbgpu_noise_sample / nbgpu_mapped_sample, nbldpc_host.c)
+ * before the decoder reads them.  tests/test_gpu_source.py, tests/test_gpu_source_apsk64.py and tests/test_gpu_mapped.py
+ * check the stream against the host source sample by sample.
  *
  * GF arithmetic of the encoder runs on binary images (addition = XOR): mulimg[h][x] = img(h * sym(x)),
  * divimg[p][x] = img(sym(x) / p), both built on the host from the code's tables.
@@ -53,8 +54,8 @@ struct SrcArgs {
     unsigned flag_cap;
     const int *decide;           /* [B][N] */
     int *bit_errors;             /* [B] */
-    const float *mod;            /* [64][2] 64-APSK constellation by binary image (the decoder's intake table) */
-    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged 64-APSK sample */
+    const float *mod;            /* [q][2] constellation of a mapped batch by binary image (the decoder's intake table) */
+    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged mapped sample (q <= 256) */
 };
 
 __device__ __forceinline__ uint64_t src_skip(uint64_t x, uint64_t n)
@@ -129,10 +130,11 @@ __global__ void __launch_bounds__(256) source_noise_kernel(SrcArgs a)
     }
 }
 
-/* 64-APSK (ModelChannel_AWGN_64, channel.c:234-263): one thread per codeword symbol, its 4 draws (u, v for I, then u, v
- * for Q), the symbol's constellation point plus noise, written as noisy[B][N][2] (the layout of nbgpu_upload_apsk64).
- * Same arithmetic and margin test as source_noise_kernel; a flagged sample records its symbol's image for the host. */
-__global__ void __launch_bounds__(256) source_noise_apsk64_kernel(SrcArgs a)
+/* Mapped channel (ModelChannel_AWGN_64, channel.c:234-263, on any q-point table): one thread per codeword symbol, its 4
+ * draws (u, v for I, then u, v for Q), the symbol's constellation point plus noise, written as noisy[B][N][2] (the layout
+ * of nbgpu_upload_apsk64 / _mapped).  Same arithmetic and margin test as source_noise_kernel; a flagged sample records its
+ * symbol's image for the host. */
+__global__ void __launch_bounds__(256) source_noise_mapped_kernel(SrcArgs a)
 {
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= (long long)a.B * a.N) return;

@@ -2,8 +2,8 @@
 
 Frames of a Monte-Carlo run are independent (SURVEY.md section 8e): frame f consumes the drand48 draws
 [f*D, (f+1)*D) with D = (K + 2N) * log2(q) (K*log2(q) information bits, tools.c:124-136, then two draws per
-transmitted bit, channel.c:56-57; D = 6K + 4N for a GF(64) code sent as 64-APSK symbols, two draws for each of the I and Q
-samples of a symbol, channel.c:234-263), so every rank can generate its own frames by LCG jump-ahead.  There is no
+transmitted bit, channel.c:56-57; D = K*log2(q) + 4N for a code sent one symbol per constellation point, 64-APSK or any
+mapped table, two draws for each of the I and Q samples of a symbol, channel.c:234-263), so every rank can generate its own frames by LCG jump-ahead.  There is no
 collective on the decode path.  Results meet in ONE collective:
 
   * `allreduce_counters` -- sum of the int64 counters (throughput runs: frames, non-zero syndromes, iterations, ...);
@@ -18,12 +18,12 @@ import numpy as np
 
 def draws_per_frame(code, channel="bpsk"):
     """drand48 draws one frame of the reference's main loop consumes: tools.c:124-136, then channel.c:56-57 ("bpsk",
-    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64)"""
+    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table)"""
     if channel == "bpsk":
         return (code.K + 2 * code.N) * code.logq
-    if channel == "apsk64":
+    if channel in ("apsk64", "mapped"):
         return code.K * code.logq + 4 * code.N
-    raise ValueError("channel must be 'bpsk' or 'apsk64', not %r" % (channel,))
+    raise ValueError("channel must be 'bpsk', 'apsk64' or 'mapped', not %r" % (channel,))
 
 
 def frame_range(total, rank, world):
@@ -61,22 +61,30 @@ def gather_rows(rows):
     return np.concatenate(out, axis=0) if out is not None else None
 
 
-def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_err_frames=40, decoder=None, channel="bpsk"):
+def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_err_frames=40, decoder=None, channel="bpsk",
+                constellation=None):
     """The reference's Monte-Carlo loop (NB_LDPC.c:250-511) sharded by frame block over `world` ranks.
 
     Either decode(noisy, sigma) -> (decide[B, N], synd[B], iters[B]) with frames made by the host source, or
     decoder=<Decoder>: frames are generated, decoded and scored on the rank's GPU (nbgpu_source_frames / nbgpu_run /
     nbgpu_source_results) and only 12 bytes per frame reach the host.
     channel="bpsk" (ModelChannel_AWGN_BPSK): noisy[B, N, logq], e.g. Decoder.decode_noisy; "apsk64" (ModelChannel_AWGN_64,
-    GF(64) codes): noisy[B, N, 2] with sigma_apsk64, e.g. Decoder.decode_apsk64, and Decoder.source_frames_apsk64.
+    GF(64) codes): noisy[B, N, 2] with sigma_apsk64, e.g. Decoder.decode_apsk64, and Decoder.source_frames_apsk64; "mapped":
+    the same on constellation=mod[q][2] (any field), e.g. Decoder.decode_mapped on a decoder with mod bound, and
+    Decoder.source_frames_mapped (the decoder gets mod bound here).
     Returns on rank 0 the dict of the reference's statistics, None on the other ranks."""
     lo, hi = frame_range(frames, rank, world)
     D = draws_per_frame(code, channel)
     apsk = channel == "apsk64"
+    mapped = channel == "mapped"
+    if mapped and constellation is None:
+        raise ValueError("channel='mapped' needs constellation=mod[q][2]")
+    if mapped and decoder is not None:
+        decoder.set_constellation(constellation)
     code.prepare_encoder()
     code.rng_default()
     code.rng_skip(lo * D)
-    if apsk:
+    if apsk or mapped:
         from . import sigma_apsk64
         sigma = sigma_apsk64(ebn)
     else:
@@ -86,7 +94,8 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     for b0 in range(lo, hi, batch):
         b1 = min(hi, b0 + batch)
         if decoder is not None:
-            (decoder.source_frames_apsk64 if apsk else decoder.source_frames)(b0, b1 - b0, ebn)
+            src = decoder.source_frames_apsk64 if apsk else decoder.source_frames_mapped if mapped else decoder.source_frames
+            src(b0, b1 - b0, ebn)
             decoder.run()
             rows[b0 - lo:b1 - lo] = np.stack(decoder.source_results(), axis=1)
             continue
@@ -94,7 +103,10 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         for _ in range(b0, b1):
             _, nbin = code.random_codeword()
             bits.append(nbin)
-            noisy.append(code.noise_apsk64(nbin, ebn) if apsk else code.noise(nbin, ebn))
+            if mapped:
+                noisy.append(code.noise_mapped(nbin, constellation, ebn))
+            else:
+                noisy.append(code.noise_apsk64(nbin, ebn) if apsk else code.noise(nbin, ebn))
         dec, synd, it = decode(np.stack(noisy), sigma)
         for i in range(b1 - b0):
             err = int((bing[dec[i, :code.K]] != bits[i][:code.K]).sum())                    # NB_LDPC.c:479-485

@@ -89,6 +89,28 @@ float nbgpu_sigma_apsk64(float EbN);
 int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][6] or NULL = all-zero word*/, float EbN,
                             float *noisy /*[N][2]*/);
 
+/* ---- Mapped channels: one GF(q) symbol = one point of a q-point 2-D constellation mod[q][2] (I, Q), indexed by the
+ * symbol's binary image (LSB first), as nbgpu_apsk64_table is; two noisy reals per symbol, noisy[N][2].  q = 16, 64, 256.
+ * Sigma convention of every mapped call: the one of the reference's 64-APSK channel (channel.c:232),
+ * sigma = nbgpu_sigma_apsk64(EbN) = sqrt(1 / (2 * 10^(EbN/10))), with neither the code rate nor the bits per symbol.  For a
+ * constellation of average power 1 the argument is therefore Es/N0 in dB; converting from Eb/N0 is the caller's job.
+ *
+ * nbgpu_constellation     writes mod[q][2]:
+ *   NBGPU_MAP_APSK64  q = 64 only; equals nbgpu_apsk64_table.
+ *   NBGPU_MAP_QAM     Gray-labelled square q-QAM, q = 16, 64 or 256, L = sqrt(q) levels per axis, m = log2(L): image bits
+ *                     [0, m) give the I level and bits [m, 2m) the Q level; the level index is the inverse binary-reflected
+ *                     Gray code of those bits; the coordinate is (float)((2*level - (L-1)) / sqrt(2*(q-1)/3)), evaluated in
+ *                     double and rounded once (average power 1).
+ *   Anything else is NBGPU_EINVAL with a message.
+ * nbgpu_awgn_mapped_noise  noisy[N][2] = mod[image of symbol n] + Box-Muller noise on the caller's drand48 stream, in the
+ *                     draw order of channel.c:234-263 (per symbol: u, v for I, then u, v for Q: 4N draws).
+ *                     nbgpu_awgn_apsk64_noise is this call on the 64-APSK table. */
+#define NBGPU_MAP_APSK64 1
+#define NBGPU_MAP_QAM    2
+int nbgpu_constellation(int kind, int q, float *mod /*[q][2]*/);
+int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/,
+                            const float *mod /*[q][2]*/, float EbN, float *noisy /*[N][2]*/);
+
 
 /* Configuration table of the syndrome-based check node: replaces build_config_table + sort_config_table
  * (syndrome_decoder.c:1542, 2285) and the truncation NB_LDPC.c:198-201.  Returns the number of
@@ -144,11 +166,25 @@ int nbgpu_channel_awgn_apsk64(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, 
                               float *llr, float *illr, int *igf);
 int nbgpu_decode_apsk64(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B,
                         int *decide, int *synd, int *iters);
+/* The mapped channel (see nbgpu_constellation) on any field: nbgpu_set_constellation copies a caller's mod[q][2] into the
+ * context's bound table (NBGPU_EINVAL for NULL or a non-finite value, context unchanged; no table is bound after
+ * nbgpu_create).  The *_mapped calls then work as their 64-APSK counterparts with that table in place of the 64-APSK one:
+ * LLR[k] = (float)((double)((I - mI)^2) / (2 sigma^2) + (double)((Q - mQ)^2) / (2 sigma^2)), (mI, mQ) = mod[image of k].
+ * A *_mapped call with no bound table is NBGPU_ESTATE.  Every resident batch records the table it was uploaded or generated
+ * with: re-binding while a mapped batch is resident drops that batch (nbgpu_run returns NBGPU_ESTATE; its soft output and
+ * source results are gone); BPSK, LLR and 64-APSK batches are unaffected, and the *_apsk64 calls always use the 64-APSK
+ * table. */
+int nbgpu_set_constellation(nbgpu_ctx *ctx, const float *mod /*[q][2]*/);
+int nbgpu_channel_awgn_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B,
+                              float *llr, float *illr, int *igf);
+int nbgpu_decode_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B,
+                        int *decide, int *synd, int *iters);
 
 /* Same work split into stages so that a caller can keep inputs resident in HBM (bench.py "value"):
  * upload (H2D) -> run (kernel only, asynchronous on the ctx stream) -> download (D2H + sync). */
 int nbgpu_upload_noisy(nbgpu_ctx *ctx, const float *noisy, float sigma, int B);
 int nbgpu_upload_apsk64(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* 64-APSK samples, see below */
+int nbgpu_upload_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* mapped samples, bound table */
 int nbgpu_upload_llr(nbgpu_ctx *ctx, const float *llr, int B);
 int nbgpu_run(nbgpu_ctx *ctx);                  /* decode the resident batch; returns after launch    */
 int nbgpu_sync(nbgpu_ctx *ctx);
@@ -186,8 +222,12 @@ int  nbgpu_source_frames(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *orig
  * and 64-APSK batches.  NBGPU_EINVAL: q != 64 (context unchanged); B outside 1..max_batch or B*N*2 >= 2^31 (as for
  * nbgpu_source_frames, the soft output of the previous batch is dropped; the context stays usable). */
 int  nbgpu_source_frames_apsk64(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
+/* The same for a code over any field sent on the bound table (nbgpu_set_constellation): D = K log2(q) + 4N draws per frame,
+ * samples bit-identical to nbgpu_random_codeword + nbgpu_awgn_mapped_noise with that table; the batch is resident as after
+ * nbgpu_upload_mapped.  NBGPU_ESTATE with no bound table (context unchanged); the other refusals as above. */
+int  nbgpu_source_frames_mapped(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
 /* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq]
- * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 */
+ * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 / _mapped */
 int  nbgpu_source_download(nbgpu_ctx *ctx, int *codeword, float *noisy);
 /* after nbgpu_run: information-bit errors of each frame (NB_LDPC.c:479-485), syndrome value, iteration count;
  * feed them to the frame-order statistics rule (NB_LDPC.c:474-507).  12 bytes per frame cross PCIe. */
@@ -216,8 +256,8 @@ int nbgpu_get_state(nbgpu_ctx *ctx, int frame, float *APP, float *CtoV);
 #define NBGPU_SOFT_NONE 0
 #define NBGPU_SOFT_LIST 1
 #define NBGPU_SOFT_BITS 2
-/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 including their streamed path,
- * nbgpu_source_frames / _apsk64 + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
+/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 / _mapped including their streamed
+ * path, nbgpu_source_frames / _apsk64 / _mapped + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
  * if that does not fit, after which ctx stays usable with soft output off.  A bad kind or k is NBGPU_EINVAL and leaves
  * the context as it was.  Invalidates the soft output of the last batch. */
 int nbgpu_set_soft_output(nbgpu_ctx *ctx, int kind, int k);
