@@ -1185,6 +1185,7 @@ struct nbgpu_ctx {
     KArgs k;
     int N, M, E, q, logq, dc_max;
     int max_batch, nslots, grid;
+    uint64_t code_hash;  /* code_hash() of the code the context was created for: the frame source takes no other */
     int *row_ptr_h;  /* host copies for get_state */
     int *inv_h;
     /* device buffers */
@@ -1218,7 +1219,6 @@ struct nbgpu_ctx {
         uint64_t D;              /* draws per frame of the generated batch (depends on the channel) */
         double margin;
         long fixups;
-        uint64_t code_hash;      /* graph + coefficients of the code the encoder tables were built from */
         int state;               /* 0: nothing generated; 1: batch generated, not decoded; 2: generated batch decoded */
     } src;
     long launches;
@@ -1257,6 +1257,20 @@ template <typename T> static int upload(nbgpu_ctx *c, T **dst, const std::vector
 }
 
 static int align_up(int x, int a) { return (x + a - 1) / a * a; }
+
+/* FNV-1a over sizes, graph, coefficients and the GF tables (ADDGF follows from BINGF): two codes with the same hash
+ * encode, decode and score frames alike, wherever they were loaded */
+static uint64_t code_hash(const nbgpu_code *code)
+{
+    uint64_t h = 1469598103934665603ull;
+    auto mix = [&h](uint64_t x) { h = (h ^ x) * 1099511628211ull; };
+    mix(code->N); mix(code->M); mix(code->q); mix(code->E);
+    for (int e = 0; e < code->E; e++) mix(((uint64_t)code->col[e] << 16) ^ (uint64_t)code->val[e]);
+    for (int m = 0; m <= code->M; m++) mix(code->row_ptr[m]);
+    for (int i = 0; i < code->q * code->logq; i++) mix((uint32_t)code->bingf[i]);
+    for (int i = 0; i < code->q * code->q; i++) mix(((uint64_t)(uint32_t)code->mulgf[i] << 32) | (uint32_t)code->divgf[i]);
+    return h;
+}
 
 static int scr_words(int q) { return q == 16 ? QTraits<16>::SCR_WORDS : q == 64 ? QTraits<64>::SCR_WORDS : QTraits<256>::SCR_WORDS; }
 
@@ -1336,6 +1350,7 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
 #define CKF(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { ctx_err(NULL, "%s failed: %s", #call, cudaGetErrorString(e_)); cudaGetLastError(); nbgpu_destroy(c); return NBGPU_ECUDA; } } while (0)
     c->device = device; c->p = *p; c->max_batch = max_batch;
     c->N = code->N; c->M = code->M; c->E = code->E; c->q = code->q; c->logq = code->logq; c->dc_max = code->dc_max;
+    c->code_hash = code_hash(code);
     CKF(cudaSetDevice(device));
     cudaDeviceProp prop;
     CKF(cudaGetDeviceProperties(&prop, device));
@@ -1825,15 +1840,6 @@ extern "C" int nbgpu_decode_mapped(nbgpu_ctx *c, const float *noisy, float sigma
  * ---------------------------------------------------------------------------------------------- */
 #define SRC_FLAG_CAP (1u << 20)
 
-static uint64_t code_hash(const nbgpu_code *code)
-{
-    uint64_t h = 1469598103934665603ull;                       /* FNV-1a over sizes, graph and coefficients */
-    auto mix = [&h](uint64_t x) { h = (h ^ x) * 1099511628211ull; };
-    mix(code->N); mix(code->M); mix(code->q); mix(code->E);
-    for (int e = 0; e < code->E; e++) mix(((uint64_t)code->col[e] << 16) ^ (uint64_t)code->val[e]);
-    for (int m = 0; m <= code->M; m++) mix(code->row_ptr[m]);
-    return h;
-}
 static void source_teardown(nbgpu_ctx *c)
 {
     void *sbufs[] = { c->src.d_level_ptr, c->src.d_row_order, c->src.d_ut_ptr, c->src.d_ut_col, c->src.d_perm, c->src.d_bit_errors, c->src.d_ut_val,
@@ -1847,7 +1853,6 @@ static void source_teardown(nbgpu_ctx *c)
 
 static int source_setup(nbgpu_ctx *c, nbgpu_code *code)
 {
-    if (code->N != c->N || code->M != c->M || code->q != c->q) { ctx_err(c, "nbgpu_source_frames: the code is not the one the decoder was created for"); return NBGPU_EINVAL; }
     if (c->N > 48 * 1024) { ctx_err(c, "frame source: N=%d symbols do not fit the encoder's shared memory", c->N); return NBGPU_EINVAL; }
     int rc = nbgpu_code_prepare_encoder(code);
     if (rc) { ctx_err(c, "%s", nbgpu_get_global_error()); return rc; }
@@ -1891,7 +1896,6 @@ static int source_setup(nbgpu_ctx *c, nbgpu_code *code)
     CK(c, cudaMemcpyToSymbol(c_src_add, add, sizeof add));
     c->src.nlevels = depth;
     if (c->src.margin == 0.0) c->src.margin = 0x1p-46;
-    c->src.code_hash = code_hash(code);
     c->src.ready = 1;
     return NBGPU_OK;
 }
@@ -1924,15 +1928,16 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
 static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind,
                            const float *mod_d, const float *mod_h)
 {
+    /* the frames are encoded with the code's tables but decoded and scored with the context's: only the context's own code
+     * (by content, so that a copy loaded per thread or rank qualifies) is accepted, and the encoder tables built from it
+     * stay valid for every later call */
+    if (code_hash(code) != c->code_hash) { ctx_err(c, "nbgpu_source_frames: the code is not the one the decoder was created for"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     const int spf = kind == 2 ? 2 : c->logq;                    /* noisy samples per symbol */
     if ((double)B * c->N * spf >= 2147483648.0) { ctx_err(c, "frame source: B*N*%s must stay below 2^31", kind == 2 ? "2" : "log2(q)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     int rc;
-    /* the encoder tables belong to ONE code: another code of the same size gets its own (the stale tables would encode
-     * words of the first code and score the decoder against them) */
-    if (c->src.ready && c->src.code_hash != code_hash(code)) { CK(c, cudaStreamSynchronize(c->stream)); source_teardown(c); }
     if (!c->src.ready && (rc = source_setup(c, code))) { source_teardown(c); return rc; }
     if ((rc = ensure_input(c, (size_t)c->N * spf * B))) return rc;
     const uint64_t koff = (uint64_t)(c->N - c->M) * c->logq;   /* information-bit draws, tools.c:124-136 */

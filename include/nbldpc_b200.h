@@ -213,7 +213,10 @@ long nbgpu_slow_selects(nbgpu_ctx *ctx);
  * The samples are bit-identical to nbgpu_random_codeword + nbgpu_awgn_bpsk_noise: the few samples whose f32 rounding
  * could depend on the last bits of the device's log/cos are detected and recomputed by the host's libm
  * (nbgpu_source_fixups tells how many in the last call).  Afterwards the batch is resident as after
- * nbgpu_upload_noisy: call nbgpu_run, then nbgpu_source_results (or nbgpu_download for the decisions). */
+ * nbgpu_upload_noisy: call nbgpu_run, then nbgpu_source_results (or nbgpu_download for the decisions).
+ * `code` must be the code the context was created for, compared by content (sizes, graph, coefficients, BINGF, MULGF,
+ * DIVGF), so another handle loaded from the same file qualifies; any other code is NBGPU_EINVAL ("the code is not the one
+ * the decoder was created for") and leaves the context as it was.  The same holds for the _apsk64 and _mapped forms. */
 int  nbgpu_source_frames(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
 /* The same for a GF(64) code sent as 64-APSK symbols (ModelChannel_AWGN_64, channel.c:234-263): frame f owns the draws
  * [f*D, (f+1)*D) with D = 6K + 4N, and its samples are bit-identical to nbgpu_random_codeword + nbgpu_awgn_apsk64_noise

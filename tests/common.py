@@ -115,6 +115,117 @@ def product_frames(code, nframes, ebn):
     return out, code.sigma(ebn)
 
 
+# ---- labelled fields: GF(2)[x]/poly with any bijection from symbols to binary images --------------------------------
+REFERENCE_POLY = {16: 0x13, 64: 0x43, 256: 0x11D}           # struct.h:117/145/217
+RECIPROCAL_POLY = {16: 0x19, 64: 0x61, 256: 0x171}          # the same polynomials with their coefficients reversed
+LABELLINGS = ("reference", "reciprocal", "polynomial", "shuffled")
+
+
+def _gf_mul(a, b, poly, q):
+    """carry-less product of binary images a, b (numpy int arrays) reduced modulo poly"""
+    a = np.asarray(a, np.int64); b = np.asarray(b, np.int64)
+    r = np.zeros(np.broadcast(a, b).shape, np.int64)
+    for l in range(q.bit_length() - 1):
+        r ^= np.where((b >> l) & 1, a, 0)
+        a = a << 1
+        a = np.where(a & q, a ^ poly, a)
+    return r
+
+
+def exponent_images(q, poly):
+    """img[0] = 0, img[k] = x^(k-1) mod poly: the reference's labelling (symbol k >= 1 is alpha^(k-1))"""
+    img = np.zeros(q, np.int64)
+    x = 1
+    for k in range(1, q):
+        img[k] = x
+        x <<= 1
+        if x & q:
+            x ^= poly
+    return img
+
+
+def field_tables(q, poly, img):
+    """(bingf, addgf, mulgf, divgf) of GF(2)[x]/poly where symbol s has the binary image img[s] (img[0] = 0), in the layout of
+    nbgpu_code_from_arrays and the oracle (DIVGF[a][0] = -1 as in Table_Div_GF)"""
+    lg = q.bit_length() - 1
+    img = np.asarray(img, np.int64)
+    assert img.shape == (q,) and img[0] == 0 and sorted(img.tolist()) == list(range(q)), "img must be a bijection with img[0] = 0"
+    assert poly >> lg == 1, "poly must have degree log2 q"
+    x, order = 2, 1
+    while x != 1:
+        x = int(_gf_mul(x, 2, poly, q)); order += 1
+    assert order == q - 1, "poly 0x%x is not primitive: x has order %d" % (poly, order)
+    inv = np.zeros(q, np.int64); inv[img] = np.arange(q)
+    bingf = ((img[:, None] >> np.arange(lg)) & 1).astype(np.int32)
+    addgf = inv[img[:, None] ^ img[None, :]].astype(np.int32)
+    mulgf = inv[_gf_mul(img[:, None], img[None, :], poly, q)].astype(np.int32)
+    # a^-1 = a^(q-2) in the multiplicative group
+    recip = np.ones(q, np.int64)
+    for _ in range(q - 2):
+        recip = _gf_mul(recip, img, poly, q)
+    divgf = np.full((q, q), -1, np.int32)
+    divgf[:, 1:] = inv[_gf_mul(img[:, None], recip[None, 1:], poly, q)]
+    # field axioms on the symbol tables, all q^3 triples
+    M = mulgf.astype(np.uint8); A = addgf.astype(np.uint8)
+    a, b, c = np.ix_(np.arange(q), np.arange(q), np.arange(q))
+    assert (M == M.T).all(), "MUL is not commutative"
+    assert (M[M[a, b], c] == M[a, M[b, c]]).all(), "MUL is not associative"
+    assert (M[a, A[b, c]] == A[M[a, b], M[a, c]]).all(), "MUL does not distribute over ADD"
+    one = inv[1]
+    assert (M[one] == np.arange(q)).all() and (M[:, 0] == 0).all()
+    assert (mulgf[divgf[:, 1:], np.arange(1, q)[None, :]] == np.arange(q)[:, None]).all(), "DIV does not invert MUL"
+    return bingf, addgf, mulgf, divgf
+
+
+def labelled_tables(q, labelling, seed=0):
+    """the GF(q) tables of one labelling:
+    reference  -- exponent labelling over the reference's polynomial (the default tables);
+    reciprocal -- exponent labelling over the reciprocal polynomial: the closed-form kernels with other binary images;
+    polynomial -- symbol = binary image over the reference's polynomial: the table-driven kernels;
+    shuffled   -- a seeded random bijection of the non-zero symbols onto the non-zero images: table-driven kernels, and
+                  the images are an arbitrary permutation (the multiplicative identity is not symbol 1)"""
+    if labelling == "reference":
+        return field_tables(q, REFERENCE_POLY[q], exponent_images(q, REFERENCE_POLY[q]))
+    if labelling == "reciprocal":
+        return field_tables(q, RECIPROCAL_POLY[q], exponent_images(q, RECIPROCAL_POLY[q]))
+    if labelling == "polynomial":
+        return field_tables(q, REFERENCE_POLY[q], np.arange(q))
+    assert labelling == "shuffled", labelling
+    img = np.concatenate([[0], 1 + np.random.default_rng(1000 * q + seed).permutation(q - 1)])
+    return field_tables(q, REFERENCE_POLY[q], img)
+
+
+def is_closed(mulgf, divgf):
+    """the predicate of nbgpu_create: MULGF and DIVGF have the exponent closed form, so the kernels compute the rotations
+    instead of reading the q x q tables"""
+    q = mulgf.shape[0]
+    a = np.arange(q)[:, None]; b = np.arange(1, q)[None, :]
+    mul = np.where(a > 0, (a + b - 2) % (q - 1) + 1, 0)
+    dv = np.where(a > 0, (a - b + (q - 1)) % (q - 1) + 1, 0)
+    return bool((mulgf[:, 1:] == mul).all() and (divgf[:, 1:] == dv).all())
+
+
+def code_arrays(code, tables):
+    """nbgpu_code_from_arrays arguments: the graph of `code` (an nbldpc.Code) with the given GF tables"""
+    bingf, addgf, mulgf, divgf = tables
+    return dict(N=code.N, M=code.M, q=code.q, row_deg=code.row_deg, col=code.col, val=code.val,
+                bingf=bingf, addgf=addgf, mulgf=mulgf, divgf=divgf)
+
+
+def oracle_with_tables(path, dialect, tables):
+    """the oracle on the code at `path` with its GF tables overwritten in place (before any encoder is prepared): every
+    oracle function reads only these tables once they are built"""
+    import ctypes as C
+    o = ol.Oracle(path, dialect)
+    c = o.h.contents
+    for name, t in zip(("bingf", "addgf", "mulgf", "divgf"), tables):
+        t = np.ascontiguousarray(t, np.int32)
+        assert t.shape == getattr(o, name).shape
+        C.memmove(getattr(c, name), t.ctypes.data, t.nbytes)
+        setattr(o, name, t.copy())
+    return o
+
+
 def random_regular_code(rng, N, M, q, dc, dv=2):
     """A random check-regular Tanner graph without repeated columns in a row (arrays for nbgpu_code_from_arrays)."""
     assert N * dv == M * dc

@@ -5,7 +5,7 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import write_alist_ubs
+from common import code_arrays, labelled_tables, oracle_with_tables, write_alist_ubs
 
 pytestmark = pytest.mark.gpu
 
@@ -43,7 +43,15 @@ def test_random_configuration_with_negative_offset_equals_oracle(seed, tmp_path)
     _random_configuration(seed, tmp_path, -0.4 if seed % 2 else -1.5)
 
 
-def _random_configuration(seed, tmp_path, offset_override):
+@pytest.mark.parametrize("labelling", ["polynomial", "shuffled"])
+@pytest.mark.parametrize("seed", list(range(8)) + [11, 15, 19, 23])
+def test_random_configuration_with_relabelled_field_equals_oracle(seed, labelling, tmp_path):
+    """the same configurations over fields whose MULGF/DIVGF lack the exponent form: the table-driven kernels, against the
+    oracle with the same tables"""
+    _random_configuration(seed, tmp_path, None, labelling)
+
+
+def _random_configuration(seed, tmp_path, offset_override, labelling="reference"):
     rng = np.random.default_rng(1000 + seed)
     q = int(rng.choice([16, 64, 256]))
     syndrome = seed % 4 == 3
@@ -61,6 +69,11 @@ def _random_configuration(seed, tmp_path, offset_override):
     write_alist_ubs(path, a)
     code = nbldpc.Code(path)
     o = ol.Oracle(path, code.dialect)
+    if labelling != "reference":
+        t = labelled_tables(q, labelling, seed)
+        o.close()
+        o = oracle_with_tables(path, code.dialect, t)
+        code = nbldpc.Code(arrays=code_arrays(code, t))
     n_m = int(rng.integers(5, min(q, 32) + 1))
     nb_oper = int(rng.integers(1, 61))
     offset = float(rng.choice([0.0, 0.3, 1.0, 2.5]))
