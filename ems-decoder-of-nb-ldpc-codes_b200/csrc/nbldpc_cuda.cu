@@ -13,8 +13,7 @@
  *            normalisation (:354-374), rotation by the edge coefficient (bubble_decoder.c:133)
  *   phase 2  THREAD per ElementaryStep, 4 task slots per check node: forward/backward chains with the
  *            merges folded into the rounds where their inputs are ready (bubble_decoder.c:157-227, 316-593)
- *   phase 3  warp per edge, NE edges interleaved:  Mvc again (parked in the APP row by phase 1, NB_PARK_MVC = 1, or
- *            recomputed from the untouched APP row and the old record, NB_PARK_MVC = 0), saturation + offset +
+ *   phase 3  warp per edge, NE edges interleaved:  Mvc again (parked in the APP row by phase 1), saturation + offset +
  *            expansion to the dense q-vector (bubble_decoder.c:231-281), CtoV store, APP = Mcv + Mvc
  *            (NB_LDPC.c:415-450), fused Decision (tools.c:312)
  * With ecn = 1 the tile is processed one check node at a time through the syndrome-based node (nbldpc_synd.cuh).
@@ -40,35 +39,10 @@
 #include <algorithm>
 #include <vector>
 
-#ifndef NT_MAX
-#define NT_MAX 384
-#endif
-#ifndef NT_SYND
-#define NT_SYND 256              /* syndrome check node: at most 8 warps per CTA (its shared memory allows 7 at 945 configurations), 128 registers */        /* threads per CTA (upper bound; the plan may use fewer warps) */
-#endif
-#ifndef CTAS_PER_SM
+#define NT_MAX 384         /* threads per CTA (upper bound; the plan may use fewer warps) */
+#define NT_SYND 256        /* syndrome check node: at most 8 warps per CTA (its shared memory allows 7 at 945 configurations), 128 registers */
 #define CTAS_PER_SM 2      /* resident CTAs per SM the decode kernel is compiled for (register cap 65536 / (NT_MAX * CTAS_PER_SM)) */
-#endif
-#ifndef NE
-#define NE 2              /* edges interleaved per warp in phases 1 and 3 */
-#endif
-#ifndef NB_L2_PREFETCH
-#define NB_L2_PREFETCH 1   /* phase 1 pulls the next node's APP rows and records into L2 while the current one is selected: 0 never,
-                              1 where it pays (GF(64): two lines per row, little work per row to hide the latency; measured +1.4 % /
-                              +3.3 % on configs 3 / 2, but -0.7 .. -1.3 % on GF(256) and GF(16), where the 24 / 16 warps hide the
-                              latency already and the extra L2 traffic costs board power -- config 5 runs at the 1 kW cap), 2 always */
-#endif
-
-#define NB_PF(Q) (NB_L2_PREFETCH == 2 || (NB_L2_PREFETCH == 1 && (Q) == 64))
-#ifndef NB_P3_PREFETCH
-#define NB_P3_PREFETCH 0     /* phase 3 pulls the next node's parked rows into L2 one node ahead */
-#endif
-#ifndef NB_PIN_BASES
-#define NB_PIN_BASES 0      /* 1: list base addresses opaque (kept in registers); 2: also the tile meta / edge words / mask pointers */
-#endif
-#ifndef NB_PARK_MVC
-#define NB_PARK_MVC 1      /* 1: phase 1 parks Mvc in the APP row, phase 3 reloads it; 0: phase 3 recomputes it from the APP row + old record */
-#endif
+#define NE 2               /* edges interleaved per warp in phases 1 and 3 */
 
 #define UNIT_NT 256       /* block size of the small unit-boundary kernels */
 
@@ -98,7 +72,7 @@ struct KArgs {
     int off_tab, off_misc, off_wa, wa_bytes, off_wb, wb_bytes;
     int wa_mask, wa_meta, wa_einfo, wa_len;   /* offsets inside a warp's small private area: ES mask | tile meta | tile edge words | list lengths */
     int wb_scr1, wb_scr3, wb_U, wb_R;   /* offsets inside a warp's list area: phase-1 scratch (clean rows[NE] | key queues[NE] |
-                                           sel[NE]), phase-3 scratch (clean rows[NE]), input lists U[cpw][dc_max], other lists
+                                           36 unused words[NE]), phase-3 scratch (clean rows[NE]), input lists U[cpw][dc_max], other lists
                                            R[cpw][L - dc_max] directly behind them (one array of lists).
                                            Bubble path: the phase-1 scratch aliases R (unused until phase 2) and the phase-3
                                            scratch aliases U (dead after phase 2).                                         */
@@ -161,16 +135,15 @@ struct TileMeta {
  * keep in registers and ptxas rebuilt them from the kernel parameters at every use (~100 instructions per check node). */
 template <int Q, int ECN = 0> struct WarpMem {
     static constexpr int ROWS = ECN == 0 ? NE * Q : 0;     /* floats of clean rows in front of the queues (bubble path only) */
-    uint32_t s1, s3;         /* shared-window addresses of the phase-1 scratch (clean rows | queues | winners) and the phase-3 rows */
+    uint32_t s1, s3;         /* shared-window addresses of the phase-1 scratch (clean rows | queues) and the phase-3 rows */
     unsigned char *p1, *p3;  /* the same as generic pointers (cold paths)                                    */
     uint32_t mask;           /* q = 256: ElementaryStep "seen" bits, [8][32] lane-strided (shared address)  */
     TileMeta meta;           /* [cpw] {first edge | degree << 24 (0 = skip), frame}                         */
     uint32_t *ew;            /* [cpw][dc_max] einfo words of the tile's edges (one coalesced load per tile) */
     Lists ls;
-    /* phase 1, per in-flight edge: clean row for the record expansion | selection queue (sorted keys) | winners of the rounds */
+    /* phase 1, per in-flight edge: clean row for the record expansion | selection queue (sorted keys) */
     __device__ __forceinline__ uint32_t rowa(int e) const { return s1 + (uint32_t)(e * Q * 4); }
     __device__ __forceinline__ uint32_t scra(int e) const { return s1 + (uint32_t)((ROWS + e * QTraits<Q>::SCR_WORDS) * 4); }
-    __device__ __forceinline__ uint32_t sela(int e) const { return s1 + (uint32_t)((ROWS + NE * QTraits<Q>::SCR_WORDS + e * 36) * 4); }
     /* phase 3, per in-flight edge: clean row */
     __device__ __forceinline__ uint32_t row3a(int e) const { return s3 + (uint32_t)(e * Q * 4); }
     __device__ __forceinline__ float *row(int e) const { return reinterpret_cast<float *>(p1) + e * Q; }
@@ -188,12 +161,6 @@ template <int Q, int ECN = 0> struct WarpMem {
         ew = reinterpret_cast<uint32_t *>(wa + a.wa_einfo);
         ls.base = smem_u32(wb + a.wb_U); ls.lenb = smem_u32(wa + a.wa_len);
         ls.lstride = a.lstride; ls.n_m = a.n_m; ls.dcm = a.dc_max; ls.lr = a.L - a.dc_max; ls.r0 = a.cpw * a.dc_max;
-#if NB_PIN_BASES >= 1
-        asm volatile("" : "+r"(ls.base), "+r"(ls.lenb));
-#endif
-#if NB_PIN_BASES >= 2
-        asm volatile("" : "+r"(mask), "+l"(ew), "+l"(meta.p));
-#endif
     }
 };
 
@@ -353,22 +320,6 @@ __device__ __forceinline__ void synd_dense_row(uint32_t out, const GFTab &gf, in
     }
 }
 
-/* L2 prefetch of the APP rows and CtoV records of up to NE consecutive edges (one instruction) -- GF(16) path */
-template <int Q>
-__device__ __forceinline__ void prefetch_edges(const float *app_f, const uint8_t *ctov_f, const uint32_t *einfo, int ed, int n,
-                                               int rec_stride, int lane)
-{
-    constexpr int LPR = (Q * 4 + 127) / 128;               /* 128-byte lines per row */
-    const char *p = nullptr;
-    if (lane < NE * LPR) {
-        const int e = lane / LPR;
-        if (e < n) p = reinterpret_cast<const char *>(app_f + (size_t)(einfo[ed + e] & 0xfffff) * Q) + (lane % LPR) * 128;
-    } else if (lane < NE * LPR + 3) {
-        const int off = (lane - NE * LPR) * 128;
-        if (off < n * rec_stride) p = reinterpret_cast<const char *>(ctov_f + (size_t)ed * rec_stride) + off;
-    }
-    if (p) asm volatile("prefetch.global.L2 [%0];" :: "l"(p));
-}
 /* L2 prefetch of everything phase 1 reads for ONE check node of the tile: its dc APP rows (edge words already in shared memory)
  * and its dc consecutive records.  Issued one node ahead: two or three instructions per node instead of address arithmetic per
  * edge pair. */
@@ -388,19 +339,6 @@ __device__ __forceinline__ void prefetch_node(const char *app, const char *ctov,
     }
 }
 
-/* the parked rows of ONE check node back into L2 ahead of phase 3 (a good third of them has been evicted by then) */
-template <int Q>
-__device__ __forceinline__ void prefetch_rows(const char *app, const uint32_t *ew, const int4 &m, int lane)
-{
-    constexpr int LPR = (Q * 4) / 128;
-    const int dc = TileMeta::dc(m);
-    for (int i = lane; i < dc * LPR; i += 32) {
-        const uint32_t ei = ew[i / LPR];
-        const char *p = app + (uint32_t)m.y + (ei & 0xfffffu) * (uint32_t)(Q * 4) + (uint32_t)(i % LPR) * 128u;
-        asm volatile("prefetch.global.L2 [%0];" :: "l"(p));
-    }
-}
-
 /* ------------------------------------------------------------------------------------------------
  * GF(16): a row is 16 values, so one warp carries TWO edges of a check node side by side -- edge t in
  * lanes 0-15, edge t+1 in lanes 16-31, lane & 15 = symbol / list entry -- instead of two half-empty
@@ -408,7 +346,7 @@ __device__ __forceinline__ void prefetch_rows(const char *app, const uint32_t *e
  * ---------------------------------------------------------------------------------------------- */
 template <bool CLOSED>
 __device__ __forceinline__ void gf16_phase1(const WarpMem<16> &wm, const GFTab &gf, int c, int e0, int dc, int dcm, float *app_f,
-                                            const uint8_t *ctov_f, const uint32_t *einfo, int n_m, int rs, int lane, unsigned *slow_counter)
+                                            const uint8_t *ctov_f, int n_m, int rs, int lane, unsigned *slow_counter)
 {
     const Lists &ls = wm.ls;
     const int h = lane >> 4, idx = lane & 15, hb = lane & 16;
@@ -423,7 +361,6 @@ __device__ __forceinline__ void gf16_phase1(const WarpMem<16> &wm, const GFTab &
         float *prow = app_f + (size_t)((ei & 0xfffffu) * 16u);
         float v = prow[idx];
         const RecView r = load_record(ctov_f, (uint32_t)(e0 + te), rlh);
-        if (NB_PF(16) && t + 2 < dc) prefetch_edges<16>(app_f, ctov_f, einfo, e0 + t + 2, min(2, dc - t - 2), rs, lane);
         scr[idx] = r.sat;                                        /* dense CtoV row, bubble_decoder.c:262-270 */
         __syncwarp();
         if (idx < r.stp) scr[r.sym] = r.llr;
@@ -556,7 +493,10 @@ __device__ __forceinline__ void tile_phase1(const KArgs &a, const WarpMem<Q> &wm
     for (int c = 0; c < cnt; c++) {
         const int4 mt = wm.meta[c];
         const int dc = TileMeta::dc(mt);
-        if (NB_PF(Q) && c + 1 < cnt) prefetch_node<Q>(app, ctov, wm.ew + (c + 1) * dcm, wm.meta[c + 1], rs, lane);
+        /* GF(64) only: GF(256) and GF(16) hide the latency already and pay for the extra L2 traffic at the power cap */
+        if constexpr (Q == 64) {
+            if (c + 1 < cnt) prefetch_node<Q>(app, ctov, wm.ew + (c + 1) * dcm, wm.meta[c + 1], rs, lane);
+        }
         const char *app_f = app + (uint32_t)mt.y;
         const uint8_t *rec0 = reinterpret_cast<const uint8_t *>(ctov) + (uint32_t)mt.z;      /* record of the node's edge 0 */
         for (int t = 0; t < dc; t += NE) {
@@ -570,8 +510,8 @@ __device__ __forceinline__ void tile_phase1(const KArgs &a, const WarpMem<Q> &wm
                 const uint32_t ei = wm.ew[c * dcm + te];
                 hv[e] = (ei >> 20) & 0xff;
                 prow[e] = reinterpret_cast<float *>(const_cast<char *>(app_f) + (ei & 0xfffffu) * (uint32_t)(Q * 4));
-                /* the row comes back in phase 3 (as the parked Mvc or as itself): keep it in L2 */
-                load_row_hint<Q>(prow[e], lane, v[e], NB_PARK_MVC ? pol_first : pol_keep);
+                /* the row is not read again: phase 3 reads the parked Mvc stored over it below */
+                load_row_hint<Q>(prow[e], lane, v[e], pol_first);
                 r[e] = load_record(rec0, (uint32_t)te, rl);
             }
 #pragma unroll
@@ -580,13 +520,13 @@ __device__ __forceinline__ void tile_phase1(const KArgs &a, const WarpMem<Q> &wm
                 expand_record<Q>(r[e], lane, wm.rowa(e), cv, minform);
 #pragma unroll
                 for (int j = 0; j < VPL; j++) v[e][j] = __fsub_rn(v[e][j], cv[j]);      /* NB_LDPC.c:334 */
-                if (NB_PARK_MVC && t + e < dc) store_row_hint<Q>(prow[e], lane, v[e], pol_keep);     /* parked for phase 3 (NB_LDPC.c:448 adds this vector) */
+                if (t + e < dc) store_row_hint<Q>(prow[e], lane, v[e], pol_keep);     /* parked for phase 3 (NB_LDPC.c:448 adds this vector) */
             }
             float llr[NE]; int sym[NE];
-            uint32_t scra[NE], sela[NE];
+            uint32_t scra[NE];
 #pragma unroll
-            for (int e = 0; e < NE; e++) { scra[e] = wm.scra(e); sela[e] = wm.sela(e); }
-            select_edges<Q, NE>(v, lane, scra, sela, n_m, llr, sym, a.slow_counter);
+            for (int e = 0; e < NE; e++) scra[e] = wm.scra(e);
+            select_edges<Q, NE>(v, lane, scra, n_m, llr, sym, a.slow_counter);
 #pragma unroll
             for (int e = 0; e < NE; e++) {
                 if (t + e < dc) {
@@ -621,28 +561,19 @@ __device__ __forceinline__ void tile_phase3(const KArgs &a, const WarpMem<Q> &wm
         uint8_t *rec0 = reinterpret_cast<uint8_t *>(ctov) + (uint32_t)mt.z;
         /* output list of edge t (id_out): t = dc-1 -> F after dc-2 steps, else B / merge number 3dc-5+t; as an index into the tile's lists */
         const int obase = dc > 2 ? ls.r0 + c * ls.lr - dc : c * dcm;
-        if (NB_P3_PREFETCH && c + 1 < cnt) prefetch_rows<Q>(app, wm.ew + (c + 1) * dcm, wm.meta[c + 1], lane);
         for (int t = 0; t < dc; t += NE) {
             float v[NE][VPL];
             uint32_t ei[NE];
-            RecView old[NE];
 #pragma unroll
             for (int e = 0; e < NE; e++) {
                 const int te = min(t + e, dc - 1);
                 ei[e] = wm.ew[c * dcm + te];
-                load_row_hint<Q>(reinterpret_cast<const float *>(app_f + (ei[e] & 0xfffffu) * (uint32_t)(Q * 4)), lane, v[e], pol_first);    /* parked Mvc, or the APP row again */
-                if (!NB_PARK_MVC) old[e] = load_record(rec0, (uint32_t)te, rl);
+                load_row_hint<Q>(reinterpret_cast<const float *>(app_f + (ei[e] & 0xfffffu) * (uint32_t)(Q * 4)), lane, v[e], pol_first);    /* parked Mvc */
             }
 #pragma unroll
             for (int e = 0; e < NE; e++) {
                 if (t + e < dc) {
                     const uint32_t var = ei[e] & 0xfffffu;
-                    if (!NB_PARK_MVC) {
-                        float cv[VPL];
-                        expand_record<Q>(old[e], lane, wm.row3a(e), cv, minform);
-#pragma unroll
-                        for (int j = 0; j < VPL; j++) v[e][j] = __fsub_rn(v[e][j], cv[j]);      /* NB_LDPC.c:334, same operands as phase 1 */
-                    }
                     const int te = t + e;
                     const int li = dc > 2 ? obase + (te == dc - 1 ? 2 * dc - 3 : 3 * dc - 5 + te) : obase + (1 - te);
                     const RecView nr = finish_list<Q, CLOSED>(ls, li, (ei[e] >> 20) & 0xff, gf, a.offset, lane);
@@ -678,9 +609,9 @@ __device__ __forceinline__ void soft_output(const KArgs &a, const WarpMem<Q, ECN
         load_row<Q>(app + (size_t)w * Q, lane, v[0]);
         if (a.soft_kind == NBGPU_SOFT_LIST) {
             /* the truncation NB_LDPC.c:354-374 with n_m = k; the decoder's slow-path counter is not touched */
-            const uint32_t scr[1] = { wm.scra(0) }, sel[1] = { wm.sela(0) };
+            const uint32_t scr[1] = { wm.scra(0) };
             float llr[1]; int sym[1];
-            select_edges<Q, 1>(v, lane, scr, sel, k, llr, sym, nullptr);
+            select_edges<Q, 1>(v, lane, scr, k, llr, sym, nullptr);
             if (lane < k) { a.soft_llr[var * k + lane] = llr[0]; a.soft_sym[var * k + lane] = (uint8_t)sym[0]; }
         } else {
             /* per bit the two minima, split by the binary image; keys in the total order of the floats (the APP may be
@@ -819,21 +750,14 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                 }
                 __syncwarp();
                 if constexpr (ECN == 0) {
-                    if constexpr (Q == 16 && NE == 2) {
+                    if constexpr (Q == 16) {
                         const Lists &ls = wm.ls;
                         for (int c = 0; c < cnt; c++) {
                             const int4 mt = wm.meta[c];
                             const int e0 = TileMeta::e0(mt), dc = TileMeta::dc(mt);
                             float *app_f = reinterpret_cast<float *>(reinterpret_cast<char *>(app) + (uint32_t)mt.y);
                             const uint8_t *ctov_f = ctov + (uint32_t)mt.z - (size_t)e0 * rs;
-                            if (NB_PF(Q) && c == 0 && dc > 0) prefetch_edges<Q>(app_f, ctov_f, a.einfo, e0, min(NE, dc), rs, lane);
-                            if (NB_PF(Q) && c + 1 < cnt) {
-                                const int4 nx = wm.meta[c + 1];
-                                if (TileMeta::dc(nx) > 0) prefetch_edges<Q>(reinterpret_cast<float *>(reinterpret_cast<char *>(app) + (uint32_t)nx.y),
-                                                                            ctov + (uint32_t)nx.z - (size_t)TileMeta::e0(nx) * rs, a.einfo, TileMeta::e0(nx),
-                                                                            min(NE, TileMeta::dc(nx)), rs, lane);
-                            }
-                            gf16_phase1<CLOSED>(wm, gf, c, e0, dc, dcm, app_f, ctov_f, a.einfo, n_m, rs, lane, a.slow_counter);
+                            gf16_phase1<CLOSED>(wm, gf, c, e0, dc, dcm, app_f, ctov_f, n_m, rs, lane, a.slow_counter);
                         }
                         __syncwarp();
                         tile_elementary_steps<Q>(ls, wm.meta, cnt, dcm, wm.mask, lane, a.nb_oper);
@@ -845,7 +769,6 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                         }
                     } else {
                         tile_phase1<Q, CLOSED>(a, wm, gf, cnt, reinterpret_cast<const char *>(app), reinterpret_cast<const char *>(ctov), rl, pol_stream, pol_keep, minform, lane);
-                        if (NB_P3_PREFETCH && cnt > 0) prefetch_rows<Q>(reinterpret_cast<const char *>(app), wm.ew, wm.meta[0], lane);
                         tile_elementary_steps<Q>(wm.ls, wm.meta, cnt, dcm, wm.mask, lane, a.nb_oper);
                         tile_phase3<Q, CLOSED>(a, wm, gf, cnt, reinterpret_cast<char *>(app), reinterpret_cast<char *>(ctov), dec, rl, pol_stream, minform, decide, lane);
                     }
@@ -875,10 +798,10 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                                 for (int j = 0; j < VPL; j++) v[e][j] = __fsub_rn(v[e][j], cv[j]);
                             }
                             float llr[NE]; int sym[NE];
-                            uint32_t scra[NE], sela[NE];
+                            uint32_t scra[NE];
 #pragma unroll
-            for (int e = 0; e < NE; e++) { scra[e] = wm.scra(e); sela[e] = wm.sela(e); }
-            select_edges<Q, NE>(v, lane, scra, sela, n_m, llr, sym, a.slow_counter);
+                            for (int e = 0; e < NE; e++) scra[e] = wm.scra(e);
+                            select_edges<Q, NE>(v, lane, scra, n_m, llr, sym, a.slow_counter);
 #pragma unroll
                             for (int e = 0; e < NE; e++) {
                                 if (t + e < dc && lane < n_m) {
@@ -957,15 +880,13 @@ __global__ void __launch_bounds__(UNIT_NT) select_kernel(const float *rows, floa
     constexpr int VPL = QTraits<Q>::VPL;
     constexpr int UW = UNIT_NT / 32;
     __shared__ uint32_t scr_s[UW][QTraits<Q>::SCR_WORDS + 64];     /* + slack: a lane that popped the +inf row reads one row further */
-    __shared__ uint32_t sel_s[UW][36];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const uint32_t scr[1] = { smem_u32(scr_s[warp]) };
-    const uint32_t sel[1] = { smem_u32(sel_s[warp]) };
     for (int r = blockIdx.x * UW + warp; r < B; r += gridDim.x * UW) {
         float v[1][VPL];
         load_row<Q>(rows + (size_t)r * Q, lane, v[0]);
         float l[1]; int s[1];
-        select_edges<Q, 1>(v, lane, scr, sel, n_m, l, s, slow);
+        select_edges<Q, 1>(v, lane, scr, n_m, l, s, slow);
         if (lane < n_m) { llr[(size_t)r * n_m + lane] = l[0]; gf[(size_t)r * n_m + lane] = s[0]; }
         __syncwarp();
     }
@@ -1293,7 +1214,7 @@ static void plan_smem(KArgs &k, int nw, int cpw)
     k.lstride = align_up(5 * k.n_m, 4);
     if (((k.lstride / 4) & 1) == 0) k.lstride += 4;       /* odd number of words: consecutive lists start in different banks */
     const int s3 = NE * k.q * 4;                                             /* clean rows */
-    const int sq = NE * scr_words(k.q) * 4 + NE * 36 * 4;                     /* selection queues + winners */
+    const int sq = NE * scr_words(k.q) * 4 + NE * 36 * 4;                     /* selection queues + 36 unused words per edge */
     if (k.ecn == 0) {
         /* per-warp lists: U[cpw][dc_max] | R[cpw][L - dc_max] as one array, each list {n_m f32 | n_m u8}.  Scratch aliases them. */
         const int ub = cpw * k.dc_max * k.lstride, rb = cpw * (k.L - k.dc_max) * k.lstride;

@@ -317,8 +317,8 @@ template <int Q> __device__ __forceinline__ int warp_argmin(const float (&v)[QTr
  * a register network and parks them in shared memory ([rank][lane], row VPL = +inf); n_m+1 rounds of
  * one REDUX.MIN over the lane heads pop the global minimum, the owning lane stepping to its next row;
  * every lane then re-reads its head row, so the load needs no predicate and no copy.  The minimum comes
- * back warp-uniform, so lane r simply keeps the result of round r (NB_SEL_CAPTURE = 1: one compare + select, no
- * shared-memory traffic) or the winner stores it to sel[r] (NB_SEL_CAPTURE = 0).  The NEDG independent
+ * back warp-uniform, so lane r simply keeps the result of round r: one compare + select, no shared-memory
+ * traffic.  n_m = 20 and n_m = 16 run their rounds straight-line, other n_m a rolled loop.  The NEDG independent
  * REDUX chains are interleaved so that their latencies overlap.  The dropped low bits of the winners come
  * from the owning lane by two shuffles (each lane keeps the low bytes of its VPL values packed in one or two
  * registers), so no dense row is written for the read-back.  A result is accepted only if (a) no value was
@@ -327,32 +327,18 @@ template <int Q> __device__ __forceinline__ int warp_argmin(const float (&v)[QTr
  * place with full comparisons; otherwise that edge re-runs the exact scan (same semantics as the
  * reference loop).
  *
- * scr[e]: SCR_WORDS u32 of warp-private scratch (free on entry, free on return); sel[e]: 36 u32; both as shared-window addresses.
+ * scr[e]: SCR_WORDS u32 of warp-private scratch as a shared-window address (free on entry, free on return).
  * Result: lane k < n_m holds (out_llr[e], out_sym[e]) = k-th entry of edge e.
  */
-#ifndef NB_SEL_CAPTURE
-#define NB_SEL_CAPTURE 1
-#endif
-#ifndef NB_SEL_UNROLL
-#define NB_SEL_UNROLL 1        /* n_m = 20 and n_m = 16: all reduction rounds straight-line */
-#endif
-#ifndef NB_SEL_LOOKAHEAD
-#define NB_SEL_LOOKAHEAD 0     /* capture mode only; measured: no gain (226.7 vs 226.4 Mbit/s), one instruction more per round */
-#endif
-#if !NB_SEL_CAPTURE
-#undef NB_SEL_LOOKAHEAD
-#define NB_SEL_LOOKAHEAD 0
-#endif
 template <int Q, int NEDG>
 __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>::VPL], int lane, const uint32_t (&scr)[NEDG],
-                                             const uint32_t (&sel)[NEDG], int n_m, float (&out_llr)[NEDG], int (&out_sym)[NEDG],
-                                             unsigned *slow_counter)
+                                             int n_m, float (&out_llr)[NEDG], int (&out_sym)[NEDG], unsigned *slow_counter)
 {
     constexpr int VPL = QTraits<Q>::VPL;
     constexpr int LOGQ = QTraits<Q>::LOGQ;
     const bool active = (Q >= 32) || lane < Q;
     const int rounds = (n_m + 1 < Q) ? n_m + 1 : Q;
-    uint32_t head[NEDG], nk[NEDG], nxt[NEDG], selp[NEDG], mine[NEDG], lo[NEDG][2];
+    uint32_t head[NEDG], nxt[NEDG], mine[NEDG], lo[NEDG][2];
     bool bad[NEDG];
 #pragma unroll
     for (int e = 0; e < NEDG; e++) {
@@ -384,14 +370,7 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
         for (int j = 0; j < VPL; j++) sts_u32(col + 128 * j, key[j]);
         sts_u32(col + 128 * VPL, NB_KEY_INF);
         head[e] = key[0];
-#if NB_SEL_LOOKAHEAD
-        nk[e] = VPL > 1 ? key[VPL > 1 ? 1 : 0] : NB_KEY_INF;     /* the lane's next key is already in a register ... */
-        nxt[e] = col + 128;                              /* ... and this is its row */
-#else
-        nk[e] = 0;
         nxt[e] = col;                                   /* row of the lane's current head */
-#endif
-        selp[e] = sel[e];
         mine[e] = NB_KEY_INF;
     }
     if constexpr (Q == 16 && NEDG == 2) {
@@ -413,23 +392,6 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
         mine[1] = __shfl_sync(NB_FULL, x, 16 | (lane & 15));
     } else {
     /* no __syncwarp needed: every lane only reads back what it wrote itself */
-#if NB_SEL_CAPTURE && NB_SEL_LOOKAHEAD
-/* the winner takes its next key from a register and reloads the one behind it: the shared-memory latency is off the
- * REDUX -> compare -> REDUX chain (it only matters when the same lane wins twice in a row) */
-#define NB_SEL_ROUND(E, OFF)                                                                                   \
-    asm volatile("{\n\t"                                                                                        \
-                 ".reg .pred p, c;\n\t"                                                                         \
-                 ".reg .u32 m;\n\t"                                                                             \
-                 "redux.sync.min.u32 m, %0, 0xffffffff;\n\t"                                                    \
-                 "setp.eq.u32 p, %0, m;\n\t"                                                                    \
-                 "selp.u32 %0, %3, %0, p;\n\t"                                                                  \
-                 "@p add.u32 %1, %1, 128;\n\t"                                                                  \
-                 "ld.shared.u32 %3, [%1];\n\t"                                                                  \
-                 "setp.eq.u32 c, %4, " #OFF ";\n\t"                                                             \
-                 "selp.u32 %2, m, %2, c;\n\t"                                                                   \
-                 "}"                                                                                             \
-                 : "+r"(head[E]), "+r"(nxt[E]), "+r"(mine[E]), "+r"(nk[E]) : "r"(lr) : "memory")
-#elif NB_SEL_CAPTURE
 #define NB_SEL_ROUND(E, OFF)                                                                                   \
     asm volatile("{\n\t"                                                                                        \
                  ".reg .pred p, c;\n\t"                                                                         \
@@ -442,8 +404,6 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
                  "selp.u32 %2, m, %2, c;\n\t"                                                                   \
                  "}"                                                                                             \
                  : "+r"(head[E]), "+r"(nxt[E]), "+r"(mine[E]) : "r"(lr) : "memory")
-#endif
-#if NB_SEL_CAPTURE
 /* the last round only has to name the (n_m+1)-th key for the boundary test: nothing is popped */
 #define NB_SEL_PEEK(E)                                                                                          \
     asm volatile("{\n\t"                                                                                        \
@@ -457,7 +417,6 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
     const int full = rounds - 1;
     int r = 0;
     int lr = lane;                                    /* lane - r: lane r keeps the minimum of round r */
-#if NB_SEL_UNROLL && !NB_SEL_LOOKAHEAD
     /* the usual list lengths straight-line: the rolled loop below spends 13 of its 61 instructions per four rounds on
      * loop-carried register moves, the convergence check in front of the first REDUX and the counter */
 #define NB_SEL_ROUNDS4(A, B, C, D)                                      \
@@ -470,9 +429,8 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
         if (full == 20) { NB_SEL_ROUNDS4(16, 17, 18, 19) }
         r = full; lr = lane - full;
     }
-#endif
 #pragma unroll 1
-    for (; r + 4 <= full; r += 4) {                   /* n_m = 20 or 16 full rounds: no remainder */
+    for (; r + 4 <= full; r += 4) {
 #pragma unroll
         for (int e = 0; e < NEDG; e++) NB_SEL_ROUND(e, 0);
 #pragma unroll
@@ -491,53 +449,6 @@ __device__ __forceinline__ void select_edges(const float (&mvc)[NEDG][QTraits<Q>
     }
 #pragma unroll
     for (int e = 0; e < NEDG; e++) NB_SEL_PEEK(e);
-#else
-#define NB_SEL_ROUND(E, OFF)                                                                                   \
-    asm volatile("{\n\t"                                                                                        \
-                 ".reg .pred p;\n\t"                                                                            \
-                 ".reg .u32 m;\n\t"                                                                             \
-                 "redux.sync.min.u32 m, %0, 0xffffffff;\n\t"                                                    \
-                 "setp.eq.u32 p, %0, m;\n\t"                                                                    \
-                 "@p st.shared.u32 [%2+" #OFF "], %0;\n\t"                                                      \
-                 "@p add.u32 %1, %1, 128;\n\t"                                                                  \
-                 "ld.shared.u32 %0, [%1];\n\t"                                                                  \
-                 "}"                                                                                             \
-                 : "+r"(head[E]), "+r"(nxt[E]) : "r"(selp[E]) : "memory")
-#define NB_SEL_PEEK(E)                                                                                          \
-    asm volatile("{\n\t"                                                                                        \
-                 ".reg .pred p;\n\t"                                                                            \
-                 ".reg .u32 m;\n\t"                                                                             \
-                 "redux.sync.min.u32 m, %0, 0xffffffff;\n\t"                                                    \
-                 "setp.eq.u32 p, %0, m;\n\t"                                                                    \
-                 "@p st.shared.u32 [%1], %0;\n\t"                                                               \
-                 "}"                                                                                             \
-                 :: "r"(head[E]), "r"(selp[E]) : "memory")
-    const int full = rounds - 1;
-    int r = 0;
-#pragma unroll 1
-    for (; r + 4 <= full; r += 4) {
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) NB_SEL_ROUND(e, 0);
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) NB_SEL_ROUND(e, 4);
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) NB_SEL_ROUND(e, 8);
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) NB_SEL_ROUND(e, 12);
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) selp[e] += 16;
-    }
-#pragma unroll 1
-    for (; r < full; r++) {
-#pragma unroll
-        for (int e = 0; e < NEDG; e++) { NB_SEL_ROUND(e, 0); selp[e] += 4; }
-    }
-#pragma unroll
-    for (int e = 0; e < NEDG; e++) NB_SEL_PEEK(e);
-    __syncwarp();
-#pragma unroll
-    for (int e = 0; e < NEDG; e++) mine[e] = lds_u32(sel[e] + 4 * min(lane, rounds - 1));
-#endif
     }
     __syncwarp();
 #pragma unroll

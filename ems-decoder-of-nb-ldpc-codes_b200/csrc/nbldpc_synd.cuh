@@ -28,14 +28,6 @@
 #pragma once
 #include "nbldpc_device.cuh"
 
-#ifndef NB_SYND_UNROLL_A
-#define NB_SYND_UNROLL_A 2               /* configurations in flight per lane in the syndrome pass */
-#endif
-#ifndef NB_SYND_UNROLL_B
-#define NB_SYND_UNROLL_B 2               /* ... and in the scatter pass */
-#endif
-#define NB_STR2(x) #x
-#define NB_PRAGMA_UNROLL(n) _Pragma(NB_STR2(unroll n))
 #define NB_SYND_MAX 1024                 /* configurations per check node: 32 per lane, kept in registers */
 #define NB_SYND_CAND 32                  /* candidates per edge collected for the exact saturation level (more: bitwise search) */
 
@@ -162,7 +154,7 @@ __device__ __forceinline__ bool synd_prepare(const SyndMem &sm, int lane)
         uint32_t lb[4];
 #pragma unroll
         for (int j = 0; j < 4; j++) lb[j] = sm.lists + lds_u32(sm.perm + 4 * j) * sm.lstride;
-NB_PRAGMA_UNROLL(NB_SYND_UNROLL_A)
+#pragma unroll 2
         for (int i = lane; i < S; i += 32) {
             const uint32_t cw = lds_u32(sm.cfg + 4 * i), mem = lds_u8(sm.cfgmask + i);
             float llr = 0.0f;
@@ -257,7 +249,7 @@ NB_PRAGMA_UNROLL(NB_SYND_UNROLL_A)
             if (d < 4) sb0 |= b << (8 * d); else sb1 |= b << (8 * (d - 4));
         }
         __syncwarp();                                    /* the saturation histograms are about to be overwritten by the grouped keys */
-NB_PRAGMA_UNROLL(NB_SYND_UNROLL_B)
+#pragma unroll 2
         for (int i = lane; i < S; i += 32) {
             const uint32_t key = lds_u32(sm.keya + 4 * i), gf = lds_u8(sm.gfa + i), mem = lds_u8(sm.cfgmask + i);
             uint32_t pos;
