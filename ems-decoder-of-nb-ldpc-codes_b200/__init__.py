@@ -21,6 +21,7 @@ OK, EINVAL, EIO, ENOMEM, ECUDA, ESTATE, ERANK = 0, -1, -2, -3, -4, -5, -6
 ALIST_AUTO, ALIST_UBS, ALIST_KN, ALIST_FULL = 0, 1, 2, 3
 SOFT_NONE, SOFT_LIST, SOFT_BITS = 0, 1, 2
 MAP_APSK64, MAP_QAM = 1, 2
+FADING_SYMBOL, FADING_COMPONENT = 1, 2
 
 _ip = C.POINTER(C.c_int)
 _fp = C.POINTER(C.c_float)
@@ -74,6 +75,15 @@ def constellation(kind, q):
     return mod
 
 
+def rotate_constellation(mod, degrees):
+    """nbgpu_rotate_constellation: mod[q][2] rotated by `degrees` (computed in double, rounded once), e.g. for signal-space
+    diversity under NBGPU_FADING_COMPONENT."""
+    m = np.ascontiguousarray(mod, np.float32).reshape(-1, 2)
+    out = np.zeros_like(m)
+    _check(lib().nbgpu_rotate_constellation(m.shape[0], C.c_double(degrees), m.ctypes.data_as(_fp), out.ctypes.data_as(_fp)))
+    return out
+
+
 def lib():
     """The loaded C-ABI library.  Fails loudly when it has not been built."""
     global _lib
@@ -111,6 +121,11 @@ def lib():
         "nbgpu_channel_awgn_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
         "nbgpu_decode_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
         "nbgpu_upload_mapped": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
+        "nbgpu_rotate_constellation": (C.c_int, [C.c_int, C.c_double, _fp, _fp]),
+        "nbgpu_awgn_faded_noise": (C.c_int, [vp, C.POINTER(Rng), _ip, _fp, C.c_float, C.c_int, _fp]),
+        "nbgpu_channel_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
+        "nbgpu_decode_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
+        "nbgpu_upload_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
         "nbgpu_create": (C.c_int, [C.POINTER(vp), vp, C.POINTER(Params), C.c_int, C.c_int]),
         "nbgpu_destroy": (None, [vp]),
         "nbgpu_last_error": (C.c_char_p, [vp]),
@@ -137,6 +152,7 @@ def lib():
         "nbgpu_source_frames": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_frames_apsk64": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_frames_mapped": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
+        "nbgpu_source_frames_faded": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float, C.c_int]),
         "nbgpu_source_download": (C.c_int, [vp, _ip, _fp]),
         "nbgpu_source_results": (C.c_int, [vp, _ip, _ip, _ip]),
         "nbgpu_source_fixups": (C.c_long, [vp]),
@@ -254,6 +270,15 @@ class Code:
         _check(lib().nbgpu_awgn_mapped_noise(self.h, C.byref(self.rng), _i(nb), _f(m), C.c_float(ebn), _f(noisy)))
         return noisy
 
+    def noise_faded(self, nbin, mod, ebn, fading):
+        """nbgpu_awgn_faded_noise: one frame of the faded mapped channel on mod[q][2], rx[N][4] = (y_I, y_Q, rho_I, rho_Q);
+        fading = FADING_SYMBOL (5N draws) or FADING_COMPONENT (6N draws)."""
+        rx = np.zeros((self.N, 4), np.float32)
+        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
+        m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
+        _check(lib().nbgpu_awgn_faded_noise(self.h, C.byref(self.rng), _i(nb), _f(m), C.c_float(ebn), int(fading), _f(rx)))
+        return rx
+
     def accumulate_stats(self, codeword_bits, decide, synd, iters, stats):
         cb = np.ascontiguousarray(codeword_bits, np.int32)
         d = np.ascontiguousarray(decide, np.int32)
@@ -289,7 +314,7 @@ class Decoder:
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
         self.soft_k = 0
-        self.source_channel = None                            # "bpsk" | "apsk64" | "mapped": channel of the generated batch
+        self.source_channel = None                            # "bpsk" | "apsk64" | "mapped" | "faded": channel of the generated batch
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
@@ -348,6 +373,30 @@ class Decoder:
         _check(lib().nbgpu_upload_mapped(self.h, _f(noisy), C.c_float(sigma), noisy.shape[0]), self.h)
         self.B = noisy.shape[0]
 
+    def decode_faded(self, rx, sigma):
+        """nbgpu_decode_faded: frames received over the faded mapped channel, rx [B, N, 4] = (y_I, y_Q, rho_I, rho_Q), on the
+        bound constellation."""
+        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
+        B = rx.shape[0]
+        d, s, it = self._out(B)
+        _check(lib().nbgpu_decode_faded(self.h, _f(rx), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
+        self.B = B
+        return d, s, it
+
+    def channel_faded(self, rx, sigma, want_sorted=False):
+        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
+        B = rx.shape[0]
+        llr = np.zeros((B, self.code.N, self.code.q), np.float32)
+        il = np.zeros_like(llr) if want_sorted else None
+        ig = np.zeros(llr.shape, np.int32) if want_sorted else None
+        _check(lib().nbgpu_channel_faded(self.h, _f(rx), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
+        return (llr, il, ig) if want_sorted else llr
+
+    def upload_faded(self, rx, sigma):
+        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
+        _check(lib().nbgpu_upload_faded(self.h, _f(rx), C.c_float(sigma), rx.shape[0]), self.h)
+        self.B = rx.shape[0]
+
     def decode_noisy_into(self, noisy, sigma, out):
         """nbgpu_decode_noisy on caller-owned (e.g. pinned) buffers, no allocation: noisy [B,N,logq] f32, out = (decide, synd, iters)."""
         B = noisy.shape[0]
@@ -401,18 +450,25 @@ class Decoder:
         self._source(lib().nbgpu_source_frames_mapped, frame0, B, ebn, origin)
         self.source_channel = "mapped"
 
-    def _source(self, fn, frame0, B, ebn, origin):
+    def source_frames_faded(self, frame0, B, ebn, fading, origin=None):
+        """nbgpu_source_frames_faded: the same for the faded mapped channel on the bound constellation (fading = FADING_SYMBOL
+        or FADING_COMPONENT); source_download then returns rx [B, N, 4]."""
+        self._source(lib().nbgpu_source_frames_faded, frame0, B, ebn, origin, int(fading))
+        self.source_channel = "faded"
+
+    def _source(self, fn, frame0, B, ebn, origin, *extra):
         r = Rng()
         lib().nbgpu_rng_reference_default(C.byref(r))
         if origin is not None:
             r.x = origin
-        _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn)), self.h)
+        _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn), *extra), self.h)
         self.B = B
 
     def source_download(self, want_noisy=True):
-        """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped"""
+        """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped,
+        [B, N, 4] for faded"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        spf = 2 if self.source_channel in ("apsk64", "mapped") else self.code.logq
+        spf = 4 if self.source_channel == "faded" else 2 if self.source_channel in ("apsk64", "mapped") else self.code.logq
         noisy = np.zeros((self.B, self.code.N, spf), np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy

@@ -51,7 +51,7 @@ struct KArgs {
     int n_m, nb_oper, passes, early_stop, nb_iter_max;
     float offset;
     int F, nw, cpw, cap, nsteps, L;     /* frames per group, warps per CTA, check nodes per warp, items per step, steps, lists per node */
-    int B, input_kind, frame0;          /* frames of this launch; 0 = BPSK samples, 1 = dense LLR, 2 = mapped (I, Q) samples; batch index of its first frame */
+    int B, input_kind, frame0;          /* frames of this launch; 0 = BPSK samples, 1 = dense LLR, 2 = mapped (I, Q) samples, 3 = faded (I, Q, rho_I, rho_Q); batch index of its first frame */
     double den;                         /* 2.0 * (double)(float)(sigma*sigma), channel.c:73 */
     const int *step_ptr, *isolated;
     int n_isolated;
@@ -59,7 +59,7 @@ struct KArgs {
     const uint32_t *einfo;              /* [E] variable | coefficient << 20 | last-visit flag << 28 */
     const int *row_ptr, *col;
     const uint8_t *hval, *rotin, *rotout, *img, *inv;
-    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, input_kind 2 (set per launch) */
+    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, input_kind 2 and 3 (set per launch) */
     int gf_closed;
     const float *in;
     float *app; uint8_t *ctov; uint8_t *dec;
@@ -265,20 +265,27 @@ __device__ __forceinline__ void intake_variable(const float *noisy_n, double den
 /* LLR intake for one variable sent as one point of a q-point constellation (the mapped channel; channel.c:268-291 for
  * 64-APSK): for every symbol k, TMP[k] = (float)( (double)((I - mI)^2) / (2 sigma^2) + (double)((Q - mQ)^2) / (2 sigma^2) )
  * with (mI, mQ) = mod[binary image of k]; differences and squares in f32, divisions and the sum in f64, as the reference
- * evaluates them (a reciprocal multiply would round differently).  GF(16): lanes >= 16 hold no symbol. */
+ * evaluates them (a reciprocal multiply would round differently).  GF(16): lanes >= 16 hold no symbol.
+ * s = (I, Q, rho_I, rho_Q): the faded channel (input kind 3) scales the point by its amplitudes, I - rho_I * mI in f32
+ * (include/nbldpc_b200.h, NBGPU_FADING_SYMBOL); kind 2 passes rho = 1, and a product with 1.0f is exact. */
 template <int Q>
-__device__ __forceinline__ void intake_mapped(const float *noisy_n, double den, const float *mod, const uint8_t *img, int lane,
+__device__ __forceinline__ void intake_mapped(const float4 s, double den, const float *mod, const uint8_t *img, int lane,
                                               float (&v)[QTraits<Q>::VPL])
 {
-    const float y0 = noisy_n[0], y1 = noisy_n[1];
 #pragma unroll
     for (int j = 0; j < QTraits<Q>::VPL; j++) {
         if (Q < 32 && lane >= Q) { v[j] = 0.0f; continue; }
         const int som = img[QTraits<Q>::sym(lane, j)];
-        const float d0 = __fsub_rn(y0, mod[2 * som]), d1 = __fsub_rn(y1, mod[2 * som + 1]);
+        const float d0 = __fsub_rn(s.x, __fmul_rn(s.z, mod[2 * som])), d1 = __fsub_rn(s.y, __fmul_rn(s.w, mod[2 * som + 1]));
         const double a = __ddiv_rn((double)__fmul_rn(d0, d0), den), b = __ddiv_rn((double)__fmul_rn(d1, d1), den);
         v[j] = __double2float_rn(__dadd_rn(a, b));
     }
+}
+/* symbol r of a mapped (kind 2: [..][2], rho = 1) or faded (kind 3: [..][4], one 16-byte load) input as intake_mapped reads it */
+__device__ __forceinline__ float4 mapped_input(const float *in, int kind, size_t r)
+{
+    if (kind == 3) return *reinterpret_cast<const float4 *>(in + r * 4);
+    return make_float4(in[r * 2], in[r * 2 + 1], 1.0f, 1.0f);
 }
 
 __device__ __forceinline__ void load_gf_tables(unsigned char *smem, const KArgs &a, GFTab &gf)
@@ -702,7 +709,7 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
             float v[VPL];
             if (a.input_kind == 0) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
                                                       reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
-            else if (a.input_kind == 2) intake_mapped<Q>(a.in + ((size_t)(base + f) * N + n) * 2, a.den, a.mod, gf.img, lane, v);
+            else if (a.input_kind >= 2) intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
             else load_row<Q>(a.in + ((size_t)(base + f) * N + n) * Q, lane, v);
             store_row<Q>(app + ((size_t)f * N + n) * Q, lane, v);
         }
@@ -1051,7 +1058,7 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
     const long total = (long)B * a.N;
     for (long r = (long)blockIdx.x * UW + warp; r < total; r += (long)gridDim.x * UW) {
         float v[VPL];
-        if (kind == 2) intake_mapped<Q>(noisy + r * 2, a.den, a.mod, a.img, lane, v);
+        if (kind >= 2) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
         else intake_variable<Q>(noisy + r * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
         if (llr) store_row<Q>(llr + r * Q, lane, v);
         if (illr) {
@@ -1123,8 +1130,8 @@ struct nbgpu_ctx {
     unsigned *d_queue, *d_slow, *d_ready, *d_fault;
     unsigned *h_ready;                       /* pinned: cumulative frame counts of the input pieces of decode_host */
     int resident_B, resident_kind;
-    const float *resident_mod;               /* table of the resident batch (kind 2): d_mod or d_map */
-    int mapped_dropped;                      /* the resident mapped batch was dropped by nbgpu_set_constellation */
+    const float *resident_mod;               /* table of the resident batch (kind 2: d_mod or d_map; kind 3: d_map) */
+    int mapped_dropped;                      /* kind (2 mapped, 3 faded) of the resident batch nbgpu_set_constellation dropped, else 0 */
     /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
@@ -1132,7 +1139,7 @@ struct nbgpu_ctx {
     /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames / _apsk64 / _mapped */
     struct {
         int ready, nlevels, B;
-        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 mapped (64-APSK or bound table) */
+        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 mapped (64-APSK or bound table), 3 faded */
         int *d_level_ptr, *d_row_order, *d_ut_ptr, *d_ut_col, *d_perm, *d_bit_errors;
         uint8_t *d_ut_val, *d_piv, *d_mulimg, *d_divimg, *d_cw, *d_flag_img;
         unsigned *d_flag_count, *d_flags, *d_patch_idx;
@@ -1495,7 +1502,7 @@ static int ensure_input(nbgpu_ctx *c, size_t floats)
     return NBGPU_OK;
 }
 
-/* mod: the constellation of a kind-2 batch (d_mod or d_map), nullptr otherwise */
+/* mod: the constellation of a kind-2 or kind-3 batch (d_mod or d_map), nullptr otherwise */
 static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B, int kind, const float *mod)
 {
     if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
@@ -1547,6 +1554,14 @@ extern "C" int nbgpu_upload_mapped(nbgpu_ctx *c, const float *noisy, float sigma
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
     return upload_common(c, noisy, (size_t)c->N * 2, B, 2, c->d_map);
 }
+extern "C" int nbgpu_upload_faded(nbgpu_ctx *c, const float *rx, float sigma, int B)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    c->k.den = 2.0 * (double)(float)(sigma * sigma);
+    return upload_common(c, rx, (size_t)c->N * 4, B, 3, c->d_map);
+}
 
 extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
 {
@@ -1559,16 +1574,19 @@ extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
     CK(c, cudaMemcpyAsync(c->d_map, mod, 2 * (size_t)c->q * sizeof(float), cudaMemcpyHostToDevice, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
     memcpy(c->map_h, mod, 2 * (size_t)c->q * sizeof(float));
-    if (c->resident_B > 0 && c->resident_kind == 2 && c->resident_mod == c->d_map) {
+    if (c->resident_B > 0 && c->resident_kind >= 2 && c->resident_mod == c->d_map) {
         /* its samples were made for the old table: decoding them on the new one would be wrong */
-        c->resident_B = 0; c->mapped_dropped = 1; c->soft_made = NBGPU_SOFT_NONE; c->src.state = 0;
+        c->resident_B = 0; c->mapped_dropped = c->resident_kind; c->soft_made = NBGPU_SOFT_NONE; c->src.state = 0;
     }
     return NBGPU_OK;
 }
 
 extern "C" int nbgpu_run(nbgpu_ctx *c)
 {
-    if (c && c->resident_B < 1 && c->mapped_dropped) { ctx_err(c, "nbgpu_run: the mapped batch was dropped when nbgpu_set_constellation bound a new table"); return NBGPU_ESTATE; }
+    if (c && c->resident_B < 1 && c->mapped_dropped) {
+        ctx_err(c, "nbgpu_run: the %s batch was dropped when nbgpu_set_constellation bound a new table", c->mapped_dropped == 3 ? "faded" : "mapped");
+        return NBGPU_ESTATE;
+    }
     if (!c || c->resident_B < 1) { ctx_err(c, "nbgpu_run: no resident batch (call nbgpu_upload_* first)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     KArgs k = c->k;
@@ -1754,6 +1772,14 @@ extern "C" int nbgpu_decode_mapped(nbgpu_ctx *c, const float *noisy, float sigma
     c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
     return decode_host(c, noisy, (size_t)c->N * 2, 2, c->d_map, B, decide, synd, iters);
 }
+extern "C" int nbgpu_decode_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, int *decide, int *synd, int *iters)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    c->k.den = 2.0 * (double)(float)(sigma * sigma);
+    return decode_host(c, rx, (size_t)c->N * 4, 3, c->d_map, B, decide, synd, iters);
+}
 
 
 /* ------------------------------------------------------------------------------------------------
@@ -1843,11 +1869,12 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
     return NBGPU_OK;
 }
 
-/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]) and nbgpu_source_frames_apsk64 / _mapped (kind 2, mapped:
- * noisy[B][N][2] on the table mod_d, whose host copy is mod_h).  The channel fixes the draws per frame D, sigma, the noise
- * kernel and the host recomputation of a flagged sample; encoder, flag read-back and patch are shared. */
+/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]), nbgpu_source_frames_apsk64 / _mapped (kind 2, mapped:
+ * noisy[B][N][2] on the table mod_d, whose host copy is mod_h) and nbgpu_source_frames_faded (kind 3, rx[B][N][4] on the
+ * bound table, fading 1 or 2).  The channel fixes the draws per frame D, sigma, the noise kernel and the host recomputation
+ * of a flagged sample (faded: of a whole symbol); encoder, flag read-back and patch are shared. */
 static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind,
-                           const float *mod_d, const float *mod_h)
+                           int fading, const float *mod_d, const float *mod_h)
 {
     /* the frames are encoded with the code's tables but decoded and scored with the context's: only the context's own code
      * (by content, so that a copy loaded per thread or rank qualifies) is accepted, and the encoder tables built from it
@@ -1855,48 +1882,70 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     if (code_hash(code) != c->code_hash) { ctx_err(c, "nbgpu_source_frames: the code is not the one the decoder was created for"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
-    const int spf = kind == 2 ? 2 : c->logq;                    /* noisy samples per symbol */
-    if ((double)B * c->N * spf >= 2147483648.0) { ctx_err(c, "frame source: B*N*%s must stay below 2^31", kind == 2 ? "2" : "log2(q)"); return NBGPU_EINVAL; }
+    const int spf = kind == 3 ? 4 : kind == 2 ? 2 : c->logq;   /* noisy samples (faded: samples and amplitudes) per symbol */
+    if ((double)B * c->N * spf >= 2147483648.0) { ctx_err(c, "frame source: B*N*%s must stay below 2^31", kind == 3 ? "4" : kind == 2 ? "2" : "log2(q)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     int rc;
     if (!c->src.ready && (rc = source_setup(c, code))) { source_teardown(c); return rc; }
     if ((rc = ensure_input(c, (size_t)c->N * spf * B))) return rc;
     const uint64_t koff = (uint64_t)(c->N - c->M) * c->logq;   /* information-bit draws, tools.c:124-136 */
-    /* K log2 q information bits, then two draws per noisy sample (channel.c:56-57 per bit, channel.c:234-263 per I/Q) */
-    const uint64_t D = koff + 2 * (uint64_t)c->N * spf;
-    const float sigma = kind == 2 ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
+    /* K log2 q information bits, then two draws per noisy sample (channel.c:56-57 per bit, channel.c:234-263 per I/Q) and,
+     * faded, one amplitude draw (SYMBOL) or two (COMPONENT) per symbol */
+    const int S = kind == 3 ? 4 + fading : 2 * spf;             /* draws per symbol (BPSK: 2 log2 q) */
+    const uint64_t D = koff + (uint64_t)c->N * S;
+    const float sigma = kind >= 2 ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
     nbgpu_rng r = *origin;
     nbgpu_rng_skip(&r, frame0 * D);
     c->src.D = D;
     SrcArgs a = source_args(c, code, B);
     a.x0 = r.x; a.sigma = sigma; a.mod = mod_d;
+    if (kind == 3) a.flag_cap = SRC_FLAG_CAP / 4;               /* a flagged symbol takes four patch entries */
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
     const long long threads = (long long)B * c->N;
-    if (kind == 2) source_noise_mapped_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
-    else source_noise_kernel<<<(unsigned)((threads + 255) / 256), 256, 0, c->stream>>>(a);
+    const unsigned blocks = (unsigned)((threads + 255) / 256);
+    if (kind == 3 && fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
+    else if (kind == 3) source_noise_mapped_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
+    else if (kind == 2) source_noise_mapped_kernel<0><<<blocks, 256, 0, c->stream>>>(a);
+    else source_noise_kernel<<<blocks, 256, 0, c->stream>>>(a);
     CK(c, cudaGetLastError());
     c->launches += 2;
     unsigned nflag = 0;
     CK(c, cudaMemcpyAsync(&nflag, c->src.d_flag_count, sizeof nflag, cudaMemcpyDeviceToHost, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
-    if (nflag > SRC_FLAG_CAP) { ctx_err(c, "frame source: %u samples flagged for host recomputation (capacity %u); margin too wide", nflag, SRC_FLAG_CAP); return NBGPU_EINVAL; }
+    if (nflag > a.flag_cap) { ctx_err(c, "frame source: %u %s flagged for host recomputation (capacity %u); margin too wide", nflag, kind == 3 ? "symbols" : "samples", a.flag_cap); return NBGPU_EINVAL; }
     c->src.fixups = nflag;
     if (nflag) {
         /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
-         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in both channels. */
-        std::vector<unsigned> idx(nflag);
+         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in both channels.
+         * A faded flag is symbol n of the batch: its S draws, its four values. */
+        std::vector<unsigned> idx(nflag), pidx;
         std::vector<float> val(nflag);
-        std::vector<uint8_t> img(kind == 2 ? nflag : 0);
+        std::vector<uint8_t> img(kind >= 2 ? nflag : 0);
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (kind == 2) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
-        const uint64_t per = (uint64_t)c->N * spf;
-        for (unsigned i = 0; i < nflag; i++) {
-            const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
-            nbgpu_rng g; g.x = a.x0;
-            nbgpu_rng_skip(&g, f * D + koff + 2 * s);
-            const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-            val[i] = kind == 2 ? nbgpu_mapped_sample(sigma, mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+        if (kind >= 2) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
+        if (kind == 3) {
+            pidx.resize(4 * (size_t)nflag); val.resize(4 * (size_t)nflag);
+            for (unsigned i = 0; i < nflag; i++) {
+                const uint64_t f = idx[i] / c->N, n = idx[i] % c->N;
+                nbgpu_rng g; g.x = a.x0;
+                nbgpu_rng_skip(&g, f * D + koff + (uint64_t)S * n);
+                float dr[6];
+                for (int j = 0; j < S; j++) dr[j] = (float)nbgpu_rng_drand48(&g);
+                nbgpu_faded_sample(sigma, mod_h + 2 * img[i], dr, fading, &val[4 * (size_t)i]);
+                for (int j = 0; j < 4; j++) pidx[4 * (size_t)i + j] = 4 * idx[i] + j;
+            }
+            idx.swap(pidx);
+            nflag *= 4;
+        } else {
+            const uint64_t per = (uint64_t)c->N * spf;
+            for (unsigned i = 0; i < nflag; i++) {
+                const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
+                nbgpu_rng g; g.x = a.x0;
+                nbgpu_rng_skip(&g, f * D + koff + 2 * s);
+                const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
+                val[i] = kind == 2 ? nbgpu_mapped_sample(sigma, mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+            }
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
         CK(c, cudaMemcpyAsync(c->src.d_patch_val, val.data(), nflag * sizeof(float), cudaMemcpyHostToDevice, c->stream));
@@ -1914,7 +1963,7 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
 extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
     if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    return source_generate(c, code, origin, frame0, B, EbN, 0, nullptr, nullptr);
+    return source_generate(c, code, origin, frame0, B, EbN, 0, 0, nullptr, nullptr);
 }
 
 extern "C" int nbgpu_source_frames_apsk64(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
@@ -1923,7 +1972,7 @@ extern "C" int nbgpu_source_frames_apsk64(nbgpu_ctx *c, nbgpu_code *code, const 
     if (!apsk64_ok(c)) return NBGPU_EINVAL;
     float mod[128];
     nbgpu_apsk64_table(mod);
-    return source_generate(c, code, origin, frame0, B, EbN, 2, c->d_mod, mod);
+    return source_generate(c, code, origin, frame0, B, EbN, 2, 0, c->d_mod, mod);
 }
 
 extern "C" int nbgpu_source_frames_mapped(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
@@ -1931,7 +1980,23 @@ extern "C" int nbgpu_source_frames_mapped(nbgpu_ctx *c, nbgpu_code *code, const 
     if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     int rc = mapped_ok(c);
     if (rc) return rc;
-    return source_generate(c, code, origin, frame0, B, EbN, 2, c->d_map, c->map_h);
+    return source_generate(c, code, origin, frame0, B, EbN, 2, 0, c->d_map, c->map_h);
+}
+
+static int fading_ok(nbgpu_ctx *c, int fading)
+{
+    if (fading == NBGPU_FADING_SYMBOL || fading == NBGPU_FADING_COMPONENT) return 1;
+    ctx_err(c, "faded channel: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fading);
+    return 0;
+}
+
+extern "C" int nbgpu_source_frames_faded(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int fading)
+{
+    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    if (!fading_ok(c, fading)) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    return source_generate(c, code, origin, frame0, B, EbN, 3, fading, c->d_map, c->map_h);
 }
 
 extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixups : 0; }
@@ -1948,7 +2013,7 @@ extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
         for (size_t i = 0; i < cw.size(); i++) codeword[i] = c->inv_h[cw[i]];
     }
     if (noisy) {
-        const size_t spf = c->src.kind == 2 ? 2 : c->logq;
+        const size_t spf = c->src.kind == 3 ? 4 : c->src.kind == 2 ? 2 : c->logq;
         CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * spf * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
@@ -2197,7 +2262,7 @@ static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, 
 {
     if (!c || !noisy || B < 1 || ((illr == NULL) != (igf == NULL))) { ctx_err(c, "nbgpu_channel_awgn_*: bad argument"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
-    const int N = c->N, q = c->q, per = kind == 2 ? 2 : c->logq;
+    const int N = c->N, q = c->q, per = kind == 3 ? 4 : kind == 2 ? 2 : c->logq;
     DevBuf<float> dn, dl, dil; DevBuf<int> dig;
     CK(c, dn.alloc((size_t)B * N * per)); CK(c, dl.alloc((size_t)B * N * q));
     if (illr) { CK(c, dil.alloc((size_t)B * N * q)); CK(c, dig.alloc((size_t)B * N * q)); }
@@ -2235,4 +2300,11 @@ extern "C" int nbgpu_channel_awgn_mapped(nbgpu_ctx *c, const float *noisy, float
     int rc = mapped_ok(c);
     if (rc) return rc;
     return channel_common(c, noisy, sigma, B, llr, illr, igf, 2, c->d_map);
+}
+extern "C" int nbgpu_channel_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, float *llr, float *illr, int *igf)
+{
+    if (!c) return NBGPU_EINVAL;
+    int rc = mapped_ok(c);
+    if (rc) return rc;
+    return channel_common(c, rx, sigma, B, llr, illr, igf, 3, c->d_map);
 }

@@ -524,6 +524,54 @@ int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, 
     return NBGPU_OK;
 }
 
+int nbgpu_rotate_constellation(int q, double degrees, const float *mod, float *out)
+{
+    if (q != 16 && q != 64 && q != 256) { nbgpu_set_global_error("nbgpu_rotate_constellation: q = %d (16, 64 or 256)", q); return NBGPU_EINVAL; }
+    if (!mod || !out) { nbgpu_set_global_error("nbgpu_rotate_constellation: NULL table"); return NBGPU_EINVAL; }
+    if (!isfinite(degrees)) { nbgpu_set_global_error("nbgpu_rotate_constellation: degrees = %g is not finite", degrees); return NBGPU_EINVAL; }
+    const double t = degrees * (M_PI / 180.0), c = cos(t), s = sin(t);
+    for (int x = 0; x < q; x++) {
+        const double i = mod[2 * x], qq = mod[2 * x + 1];     /* both read before out (which may be mod) is written */
+        out[2 * x] = (float)(i * c - qq * s);
+        out[2 * x + 1] = (float)(i * s + qq * c);
+    }
+    return NBGPU_OK;
+}
+
+/* the faded channel's one symbol (include/nbldpc_b200.h, NBGPU_FADING_SYMBOL); also the host recomputation of the faded
+ * symbols the device source flags (nbldpc_source.cuh) */
+void nbgpu_faded_sample(float sigma, const float *m, const float *d, int fading, float *rx)
+{
+    const double pi = NB_PI;
+    const float rho_i = (float)sqrt(-log((double)d[4]));
+    const float rho_q = fading == NBGPU_FADING_COMPONENT ? (float)sqrt(-log((double)d[5])) : rho_i;
+    rx[0] = (float)((double)rho_i * (double)m[0] + sigma * sqrt(-2.0 * log(d[0])) * cos(2.0 * pi * d[1]));
+    rx[1] = (float)((double)rho_q * (double)m[1] + sigma * sqrt(-2.0 * log(d[2])) * cos(2.0 * pi * d[3]));
+    rx[2] = rho_i;
+    rx[3] = rho_q;
+}
+
+/* rx[N][4] of one frame of the faded mapped channel: per symbol u_I, v_I, u_Q, v_Q, w_I (, w_Q) */
+int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, int fading, float *rx)
+{
+    const float sigma = nbgpu_sigma_apsk64(EbN);
+    int n, b;
+    if (!c || !r || !mod || !rx) { nbgpu_set_global_error("nbgpu_awgn_faded_noise: NULL argument"); return NBGPU_EINVAL; }
+    if (fading != NBGPU_FADING_SYMBOL && fading != NBGPU_FADING_COMPONENT) {
+        nbgpu_set_global_error("nbgpu_awgn_faded_noise: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fading);
+        return NBGPU_EINVAL;
+    }
+    const int S = fading == NBGPU_FADING_COMPONENT ? 6 : 5;
+    for (n = 0; n < c->N; n++) {
+        int som = 0;
+        float d[6];
+        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
+        for (b = 0; b < S; b++) d[b] = draw_float(r);
+        nbgpu_faded_sample(sigma, mod + 2 * som, d, fading, rx + 4 * (size_t)n);
+    }
+    return NBGPU_OK;
+}
+
 /* noisy[N][2] over the 64-APSK table (nbgpu_apsk64_table) */
 int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
 {

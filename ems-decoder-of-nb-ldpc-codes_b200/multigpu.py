@@ -3,7 +3,8 @@
 Frames of a Monte-Carlo run are independent (SURVEY.md section 8e): frame f consumes the drand48 draws
 [f*D, (f+1)*D) with D = (K + 2N) * log2(q) (K*log2(q) information bits, tools.c:124-136, then two draws per
 transmitted bit, channel.c:56-57; D = K*log2(q) + 4N for a code sent one symbol per constellation point, 64-APSK or any
-mapped table, two draws for each of the I and Q samples of a symbol, channel.c:234-263), so every rank can generate its own frames by LCG jump-ahead.  There is no
+mapped table, two draws for each of the I and Q samples of a symbol, channel.c:234-263; D = K*log2(q) + 5N or + 6N under
+symbol or component Rayleigh fading, one or two amplitude draws more per symbol), so every rank can generate its own frames by LCG jump-ahead.  There is no
 collective on the decode path.  Results meet in ONE collective:
 
   * `allreduce_counters` -- sum of the int64 counters (throughput runs: frames, non-zero syndromes, iterations, ...);
@@ -16,9 +17,27 @@ torch is used for the process group only (NCCL on GPUs, gloo in the CPU tests).
 import numpy as np
 
 
-def draws_per_frame(code, channel="bpsk"):
+FADINGS = {"symbol": 1, "component": 2}                    # FADING_SYMBOL, FADING_COMPONENT of the library
+
+
+def _fading(channel, fading):
+    """fading=None | "symbol" | "component" -> 0, 1, 2; fading is a property of the mapped channel only"""
+    if fading is None:
+        return 0
+    if channel != "mapped":
+        raise ValueError("fading=%r needs channel='mapped', not %r" % (fading, channel))
+    if fading not in FADINGS:
+        raise ValueError("fading must be 'symbol' or 'component', not %r" % (fading,))
+    return FADINGS[fading]
+
+
+def draws_per_frame(code, channel="bpsk", fading=None):
     """drand48 draws one frame of the reference's main loop consumes: tools.c:124-136, then channel.c:56-57 ("bpsk",
-    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table)"""
+    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table);
+    fading="symbol" / "component" (mapped only): one / two Rayleigh amplitude draws more per symbol"""
+    fd = _fading(channel, fading)
+    if fd:
+        return code.K * code.logq + (4 + fd) * code.N
     if channel == "bpsk":
         return (code.K + 2 * code.N) * code.logq
     if channel in ("apsk64", "mapped"):
@@ -62,7 +81,7 @@ def gather_rows(rows):
 
 
 def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_err_frames=40, decoder=None, channel="bpsk",
-                constellation=None):
+                constellation=None, fading=None):
     """The reference's Monte-Carlo loop (NB_LDPC.c:250-511) sharded by frame block over `world` ranks.
 
     Either decode(noisy, sigma) -> (decide[B, N], synd[B], iters[B]) with frames made by the host source, or
@@ -71,10 +90,12 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     channel="bpsk" (ModelChannel_AWGN_BPSK): noisy[B, N, logq], e.g. Decoder.decode_noisy; "apsk64" (ModelChannel_AWGN_64,
     GF(64) codes): noisy[B, N, 2] with sigma_apsk64, e.g. Decoder.decode_apsk64, and Decoder.source_frames_apsk64; "mapped":
     the same on constellation=mod[q][2] (any field), e.g. Decoder.decode_mapped on a decoder with mod bound, and
-    Decoder.source_frames_mapped (the decoder gets mod bound here).
+    Decoder.source_frames_mapped (the decoder gets mod bound here).  fading="symbol" | "component" (channel="mapped" only):
+    the same under Rayleigh fading, frames rx[B, N, 4], e.g. Decoder.decode_faded, and Decoder.source_frames_faded.
     Returns on rank 0 the dict of the reference's statistics, None on the other ranks."""
     lo, hi = frame_range(frames, rank, world)
-    D = draws_per_frame(code, channel)
+    D = draws_per_frame(code, channel, fading)
+    fd = _fading(channel, fading)
     apsk = channel == "apsk64"
     mapped = channel == "mapped"
     if mapped and constellation is None:
@@ -94,8 +115,11 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     for b0 in range(lo, hi, batch):
         b1 = min(hi, b0 + batch)
         if decoder is not None:
-            src = decoder.source_frames_apsk64 if apsk else decoder.source_frames_mapped if mapped else decoder.source_frames
-            src(b0, b1 - b0, ebn)
+            if fd:
+                decoder.source_frames_faded(b0, b1 - b0, ebn, fd)
+            else:
+                src = decoder.source_frames_apsk64 if apsk else decoder.source_frames_mapped if mapped else decoder.source_frames
+                src(b0, b1 - b0, ebn)
             decoder.run()
             rows[b0 - lo:b1 - lo] = np.stack(decoder.source_results(), axis=1)
             continue
@@ -103,7 +127,9 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         for _ in range(b0, b1):
             _, nbin = code.random_codeword()
             bits.append(nbin)
-            if mapped:
+            if fd:
+                noisy.append(code.noise_faded(nbin, constellation, ebn, fd))
+            elif mapped:
                 noisy.append(code.noise_mapped(nbin, constellation, ebn))
             else:
                 noisy.append(code.noise_apsk64(nbin, ebn) if apsk else code.noise(nbin, ebn))

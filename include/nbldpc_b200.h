@@ -111,6 +111,32 @@ int nbgpu_constellation(int kind, int q, float *mod /*[q][2]*/);
 int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/,
                             const float *mod /*[q][2]*/, float EbN, float *noisy /*[N][2]*/);
 
+/* ---- Faded mapped channels: the mapped channel under Rayleigh fading with perfect channel state at the receiver ----
+ * Symbol n is received as y_c = rho_c * mod[img(s_n)][c] + sigma * n_c, c = I, Q, with a real Rayleigh amplitude rho_c,
+ * E[rho^2] = 1 (coherent detection with perfect CSI reduces complex fading to this form):
+ *   NBGPU_FADING_SYMBOL     one amplitude per symbol, rho_I = rho_Q;
+ *   NBGPU_FADING_COMPONENT  independent amplitudes for I and Q (signal-space diversity, for rotated constellations).
+ * Sigma and EbN as for every mapped call (nbgpu_sigma_apsk64); with E[rho^2] = 1 the argument is the average Es/N0.
+ * Received frame: rx[N][4] = (y_I, y_Q, rho_I, rho_Q) f32 per symbol ([B][N][4] for a batch).
+ * LLR of symbol k: LLR[k] = (float)((double)(d_I*d_I)/den + (double)(d_Q*d_Q)/den), d_c = y_c - rho_c*m_c (product and
+ *   difference in f32, round to nearest), den = 2*(double)(float)(sigma^2), (m_I, m_Q) = mod[img(k)].  With rho = 1 this is
+ *   the mapped channel's LLR bit for bit; rho = 0 (an erased symbol) gives a constant row.  rx is not validated.
+ * Stream: frame f owns the draws [f*D, (f+1)*D), D = K log2(q) + S*N, S = 5 (SYMBOL) or 6 (COMPONENT).  Symbol n reads its
+ *   draws from K log2(q) + S*n on, in the order u_I, v_I, u_Q, v_Q, w_I and (COMPONENT only) w_Q, each (float)drand48();
+ *   rho = (float)sqrt(-log((double)w)) (w = 1.0f gives rho = 0, a legal value);
+ *   y_c = (float)((double)rho_c*(double)m_c + sigma*sqrt(-2 ln u_c)*cos(2 PI v_c)), PI = 3.1415926536.
+ *
+ * nbgpu_rotate_constellation  out[x] = (m_I cos t - m_Q sin t, m_I sin t + m_Q cos t), t = degrees in radians, computed in
+ *                       double and rounded once; out may equal mod.  NBGPU_EINVAL for q not in {16, 64, 256}, a NULL
+ *                       pointer or non-finite degrees.
+ * nbgpu_awgn_faded_noise  rx[N][4] of one frame on the caller's drand48 stream (S*N draws); a bad fading value is
+ *                       NBGPU_EINVAL. */
+#define NBGPU_FADING_SYMBOL    1
+#define NBGPU_FADING_COMPONENT 2
+int nbgpu_rotate_constellation(int q, double degrees, const float *mod /*[q][2]*/, float *out /*[q][2], may equal mod*/);
+int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/,
+                           const float *mod /*[q][2]*/, float EbN, int fading, float *rx /*[N][4]*/);
+
 
 /* Configuration table of the syndrome-based check node: replaces build_config_table + sort_config_table
  * (syndrome_decoder.c:1542, 2285) and the truncation NB_LDPC.c:198-201.  Returns the number of
@@ -179,12 +205,18 @@ int nbgpu_channel_awgn_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, 
                               float *llr, float *illr, int *igf);
 int nbgpu_decode_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B,
                         int *decide, int *synd, int *iters);
+/* The faded mapped channel (see NBGPU_FADING_SYMBOL) on the bound table: as the *_mapped calls, with rx[B][N][4] =
+ * (y_I, y_Q, rho_I, rho_Q) in place of noisy[B][N][2].  NBGPU_ESTATE with no bound table; re-binding drops a resident faded
+ * batch as it drops a mapped one.  Soft output works on faded batches as on any other. */
+int nbgpu_channel_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B, float *llr, float *illr, int *igf);
+int nbgpu_decode_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B, int *decide, int *synd, int *iters);
 
 /* Same work split into stages so that a caller can keep inputs resident in HBM (bench.py "value"):
  * upload (H2D) -> run (kernel only, asynchronous on the ctx stream) -> download (D2H + sync). */
 int nbgpu_upload_noisy(nbgpu_ctx *ctx, const float *noisy, float sigma, int B);
 int nbgpu_upload_apsk64(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* 64-APSK samples, see below */
 int nbgpu_upload_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* mapped samples, bound table */
+int nbgpu_upload_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B);       /* faded samples + CSI, bound table */
 int nbgpu_upload_llr(nbgpu_ctx *ctx, const float *llr, int B);
 int nbgpu_run(nbgpu_ctx *ctx);                  /* decode the resident batch; returns after launch    */
 int nbgpu_sync(nbgpu_ctx *ctx);
@@ -229,8 +261,16 @@ int  nbgpu_source_frames_apsk64(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rn
  * samples bit-identical to nbgpu_random_codeword + nbgpu_awgn_mapped_noise with that table; the batch is resident as after
  * nbgpu_upload_mapped.  NBGPU_ESTATE with no bound table (context unchanged); the other refusals as above. */
 int  nbgpu_source_frames_mapped(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
+/* The same for the faded mapped channel (fading = NBGPU_FADING_SYMBOL or NBGPU_FADING_COMPONENT) on the bound table:
+ * D = K log2(q) + S*N draws per frame, rx bit-identical to nbgpu_random_codeword + nbgpu_awgn_faded_noise (a symbol whose
+ * rho or y could round differently on the device is recomputed whole by the host); the batch is resident as after
+ * nbgpu_upload_faded.  NBGPU_ESTATE with no bound table, NBGPU_EINVAL for a bad fading value (context unchanged); B*N*4
+ * must stay below 2^31; the other refusals as above. */
+int  nbgpu_source_frames_faded(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN,
+                               int fading);
 /* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq]
- * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 / _mapped */
+ * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 / _mapped, rx [B][N][4] after
+ * nbgpu_source_frames_faded */
 int  nbgpu_source_download(nbgpu_ctx *ctx, int *codeword, float *noisy);
 /* after nbgpu_run: information-bit errors of each frame (NB_LDPC.c:479-485), syndrome value, iteration count;
  * feed them to the frame-order statistics rule (NB_LDPC.c:474-507).  12 bytes per frame cross PCIe. */
@@ -259,8 +299,8 @@ int nbgpu_get_state(nbgpu_ctx *ctx, int frame, float *APP, float *CtoV);
 #define NBGPU_SOFT_NONE 0
 #define NBGPU_SOFT_LIST 1
 #define NBGPU_SOFT_BITS 2
-/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 / _mapped including their streamed
- * path, nbgpu_source_frames / _apsk64 / _mapped + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
+/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 / _mapped / _faded including their
+ * streamed path, nbgpu_source_frames / _apsk64 / _mapped / _faded + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
  * if that does not fit, after which ctx stays usable with soft output off.  A bad kind or k is NBGPU_EINVAL and leaves
  * the context as it was.  Invalidates the soft output of the last batch. */
 int nbgpu_set_soft_output(nbgpu_ctx *ctx, int kind, int k);
