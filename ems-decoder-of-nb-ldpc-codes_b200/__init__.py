@@ -248,36 +248,30 @@ class Code:
     def sigma(self, ebn):
         return float(lib().nbgpu_sigma(self.h, C.c_float(ebn)))
 
+    def _noise(self, fn, nbin, fps, *args):
+        out = np.zeros((self.N, fps), np.float32)
+        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
+        _check(fn(self.h, C.byref(self.rng), _i(nb), *args, _f(out)))
+        return out
+
     def noise(self, nbin, ebn):
         """channel.c:52-62 for one frame; nbin None = all-zero codeword."""
-        noisy = np.zeros((self.N, self.logq), np.float32)
-        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
-        _check(lib().nbgpu_awgn_bpsk_noise(self.h, C.byref(self.rng), _i(nb), C.c_float(ebn), _f(noisy)))
-        return noisy
+        return self._noise(lib().nbgpu_awgn_bpsk_noise, nbin, self.logq, C.c_float(ebn))
 
     def noise_apsk64(self, nbin, ebn):
         """channel.c:234-263 for one frame of a GF(64) code sent as 64-APSK symbols: noisy[N][2]."""
-        noisy = np.zeros((self.N, 2), np.float32)
-        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
-        _check(lib().nbgpu_awgn_apsk64_noise(self.h, C.byref(self.rng), _i(nb), C.c_float(ebn), _f(noisy)))
-        return noisy
+        return self._noise(lib().nbgpu_awgn_apsk64_noise, nbin, 2, C.c_float(ebn))
 
     def noise_mapped(self, nbin, mod, ebn):
         """channel.c:234-263 on the constellation mod[q][2] (by binary image) for one frame: noisy[N][2], sigma_apsk64(ebn)."""
-        noisy = np.zeros((self.N, 2), np.float32)
-        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
         m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
-        _check(lib().nbgpu_awgn_mapped_noise(self.h, C.byref(self.rng), _i(nb), _f(m), C.c_float(ebn), _f(noisy)))
-        return noisy
+        return self._noise(lib().nbgpu_awgn_mapped_noise, nbin, 2, _f(m), C.c_float(ebn))
 
     def noise_faded(self, nbin, mod, ebn, fading):
         """nbgpu_awgn_faded_noise: one frame of the faded mapped channel on mod[q][2], rx[N][4] = (y_I, y_Q, rho_I, rho_Q);
         fading = FADING_SYMBOL (5N draws) or FADING_COMPONENT (6N draws)."""
-        rx = np.zeros((self.N, 4), np.float32)
-        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
         m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
-        _check(lib().nbgpu_awgn_faded_noise(self.h, C.byref(self.rng), _i(nb), _f(m), C.c_float(ebn), int(fading), _f(rx)))
-        return rx
+        return self._noise(lib().nbgpu_awgn_faded_noise, nbin, 4, _f(m), C.c_float(ebn), int(fading))
 
     def accumulate_stats(self, codeword_bits, decide, synd, iters, stats):
         cb = np.ascontiguousarray(codeword_bits, np.int32)
@@ -314,36 +308,45 @@ class Decoder:
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
         self.soft_k = 0
-        self.source_channel = None                            # "bpsk" | "apsk64" | "mapped" | "faded": channel of the generated batch
+        self._source_fps = 0                                  # floats per symbol of the generated batch
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
 
-    def decode_noisy(self, noisy, sigma):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, self.code.logq)
-        B = noisy.shape[0]
+    # the per-channel calls: frames [B, N, fps] f32 with fps floats per symbol; sigma=None for dense LLRs
+    def _decode(self, fn, frames, fps, sigma=None):
+        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        B = x.shape[0]
         d, s, it = self._out(B)
-        _check(lib().nbgpu_decode_noisy(self.h, _f(noisy), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
+        sig = () if sigma is None else (C.c_float(sigma),)
+        _check(fn(self.h, _f(x), *sig, B, _i(d), _i(s), _i(it)), self.h)
         self.B = B
         return d, s, it
 
-    def decode_apsk64(self, noisy, sigma):
-        """nbgpu_decode_apsk64: frames of a GF(64) code received as 64-APSK samples [B, N, 2]."""
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
-        B = noisy.shape[0]
-        d, s, it = self._out(B)
-        _check(lib().nbgpu_decode_apsk64(self.h, _f(noisy), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
-        self.B = B
-        return d, s, it
-
-    def channel_apsk64(self, noisy, sigma, want_sorted=False):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
-        B = noisy.shape[0]
+    def _channel(self, fn, frames, fps, sigma, want_sorted):
+        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        B = x.shape[0]
         llr = np.zeros((B, self.code.N, self.code.q), np.float32)
         il = np.zeros_like(llr) if want_sorted else None
         ig = np.zeros(llr.shape, np.int32) if want_sorted else None
-        _check(lib().nbgpu_channel_awgn_apsk64(self.h, _f(noisy), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
+        _check(fn(self.h, _f(x), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
         return (llr, il, ig) if want_sorted else llr
+
+    def _upload(self, fn, frames, fps, sigma=None):
+        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        sig = () if sigma is None else (C.c_float(sigma),)
+        _check(fn(self.h, _f(x), *sig, x.shape[0]), self.h)
+        self.B = x.shape[0]                                   # only once the batch is resident: it sizes every download
+
+    def decode_noisy(self, noisy, sigma):
+        return self._decode(lib().nbgpu_decode_noisy, noisy, self.code.logq, sigma)
+
+    def decode_apsk64(self, noisy, sigma):
+        """nbgpu_decode_apsk64: frames of a GF(64) code received as 64-APSK samples [B, N, 2]."""
+        return self._decode(lib().nbgpu_decode_apsk64, noisy, 2, sigma)
+
+    def channel_apsk64(self, noisy, sigma, want_sorted=False):
+        return self._channel(lib().nbgpu_channel_awgn_apsk64, noisy, 2, sigma, want_sorted)
 
     def set_constellation(self, mod):
         """nbgpu_set_constellation: bind mod[q][2] (by binary image) to the *_mapped calls of this context."""
@@ -352,50 +355,24 @@ class Decoder:
 
     def decode_mapped(self, noisy, sigma):
         """nbgpu_decode_mapped: frames received as samples [B, N, 2] of the bound constellation."""
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
-        B = noisy.shape[0]
-        d, s, it = self._out(B)
-        _check(lib().nbgpu_decode_mapped(self.h, _f(noisy), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
-        self.B = B
-        return d, s, it
+        return self._decode(lib().nbgpu_decode_mapped, noisy, 2, sigma)
 
     def channel_mapped(self, noisy, sigma, want_sorted=False):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
-        B = noisy.shape[0]
-        llr = np.zeros((B, self.code.N, self.code.q), np.float32)
-        il = np.zeros_like(llr) if want_sorted else None
-        ig = np.zeros(llr.shape, np.int32) if want_sorted else None
-        _check(lib().nbgpu_channel_awgn_mapped(self.h, _f(noisy), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
-        return (llr, il, ig) if want_sorted else llr
+        return self._channel(lib().nbgpu_channel_awgn_mapped, noisy, 2, sigma, want_sorted)
 
     def upload_mapped(self, noisy, sigma):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, 2)
-        _check(lib().nbgpu_upload_mapped(self.h, _f(noisy), C.c_float(sigma), noisy.shape[0]), self.h)
-        self.B = noisy.shape[0]
+        self._upload(lib().nbgpu_upload_mapped, noisy, 2, sigma)
 
     def decode_faded(self, rx, sigma):
         """nbgpu_decode_faded: frames received over the faded mapped channel, rx [B, N, 4] = (y_I, y_Q, rho_I, rho_Q), on the
         bound constellation."""
-        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
-        B = rx.shape[0]
-        d, s, it = self._out(B)
-        _check(lib().nbgpu_decode_faded(self.h, _f(rx), C.c_float(sigma), B, _i(d), _i(s), _i(it)), self.h)
-        self.B = B
-        return d, s, it
+        return self._decode(lib().nbgpu_decode_faded, rx, 4, sigma)
 
     def channel_faded(self, rx, sigma, want_sorted=False):
-        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
-        B = rx.shape[0]
-        llr = np.zeros((B, self.code.N, self.code.q), np.float32)
-        il = np.zeros_like(llr) if want_sorted else None
-        ig = np.zeros(llr.shape, np.int32) if want_sorted else None
-        _check(lib().nbgpu_channel_faded(self.h, _f(rx), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
-        return (llr, il, ig) if want_sorted else llr
+        return self._channel(lib().nbgpu_channel_faded, rx, 4, sigma, want_sorted)
 
     def upload_faded(self, rx, sigma):
-        rx = np.ascontiguousarray(rx, np.float32).reshape(-1, self.code.N, 4)
-        _check(lib().nbgpu_upload_faded(self.h, _f(rx), C.c_float(sigma), rx.shape[0]), self.h)
-        self.B = rx.shape[0]
+        self._upload(lib().nbgpu_upload_faded, rx, 4, sigma)
 
     def decode_noisy_into(self, noisy, sigma, out):
         """nbgpu_decode_noisy on caller-owned (e.g. pinned) buffers, no allocation: noisy [B,N,logq] f32, out = (decide, synd, iters)."""
@@ -405,22 +382,13 @@ class Decoder:
         return out
 
     def decode_llr(self, llr):
-        llr = np.ascontiguousarray(llr, np.float32).reshape(-1, self.code.N, self.code.q)
-        B = llr.shape[0]
-        d, s, it = self._out(B)
-        _check(lib().nbgpu_decode_llr(self.h, _f(llr), B, _i(d), _i(s), _i(it)), self.h)
-        self.B = B
-        return d, s, it
+        return self._decode(lib().nbgpu_decode_llr, llr, self.code.q)
 
     def upload_noisy(self, noisy, sigma):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, self.code.logq)
-        _check(lib().nbgpu_upload_noisy(self.h, _f(noisy), C.c_float(sigma), noisy.shape[0]), self.h)
-        self.B = noisy.shape[0]                               # only once the batch is resident: it sizes every download
+        self._upload(lib().nbgpu_upload_noisy, noisy, self.code.logq, sigma)
 
     def upload_llr(self, llr):
-        llr = np.ascontiguousarray(llr, np.float32).reshape(-1, self.code.N, self.code.q)
-        _check(lib().nbgpu_upload_llr(self.h, _f(llr), llr.shape[0]), self.h)
-        self.B = llr.shape[0]
+        self._upload(lib().nbgpu_upload_llr, llr, self.code.q)
 
     def run(self):
         _check(lib().nbgpu_run(self.h), self.h)
@@ -436,40 +404,36 @@ class Decoder:
     def source_frames(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames: frames [frame0, frame0+B) of the reference's stream generated on the device and left resident
         (origin: drand48 state before frame 0 as an int, default = the reference's unseeded stream)."""
-        self._source(lib().nbgpu_source_frames, frame0, B, ebn, origin)
-        self.source_channel = "bpsk"
+        self._source(lib().nbgpu_source_frames, self.code.logq, frame0, B, ebn, origin)
 
     def source_frames_apsk64(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames_apsk64: the same for a GF(64) code sent as 64-APSK symbols (ModelChannel_AWGN_64); the batch is
         resident as after an upload of noisy[B, N, 2] samples."""
-        self._source(lib().nbgpu_source_frames_apsk64, frame0, B, ebn, origin)
-        self.source_channel = "apsk64"
+        self._source(lib().nbgpu_source_frames_apsk64, 2, frame0, B, ebn, origin)
 
     def source_frames_mapped(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames_mapped: the same for a code sent on the bound constellation; D = K log2(q) + 4N draws per frame."""
-        self._source(lib().nbgpu_source_frames_mapped, frame0, B, ebn, origin)
-        self.source_channel = "mapped"
+        self._source(lib().nbgpu_source_frames_mapped, 2, frame0, B, ebn, origin)
 
     def source_frames_faded(self, frame0, B, ebn, fading, origin=None):
         """nbgpu_source_frames_faded: the same for the faded mapped channel on the bound constellation (fading = FADING_SYMBOL
         or FADING_COMPONENT); source_download then returns rx [B, N, 4]."""
-        self._source(lib().nbgpu_source_frames_faded, frame0, B, ebn, origin, int(fading))
-        self.source_channel = "faded"
+        self._source(lib().nbgpu_source_frames_faded, 4, frame0, B, ebn, origin, int(fading))
 
-    def _source(self, fn, frame0, B, ebn, origin, *extra):
+    def _source(self, fn, fps, frame0, B, ebn, origin, *extra):
         r = Rng()
         lib().nbgpu_rng_reference_default(C.byref(r))
         if origin is not None:
             r.x = origin
         _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn), *extra), self.h)
         self.B = B
+        self._source_fps = fps
 
     def source_download(self, want_noisy=True):
         """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped,
         [B, N, 4] for faded"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        spf = 4 if self.source_channel == "faded" else 2 if self.source_channel in ("apsk64", "mapped") else self.code.logq
-        noisy = np.zeros((self.B, self.code.N, spf), np.float32) if want_noisy else None
+        noisy = np.zeros((self.B, self.code.N, self._source_fps), np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy
 
@@ -538,13 +502,7 @@ class Decoder:
         return llr
 
     def channel(self, noisy, sigma, want_sorted=False):
-        noisy = np.ascontiguousarray(noisy, np.float32).reshape(-1, self.code.N, self.code.logq)
-        B = noisy.shape[0]
-        llr = np.zeros((B, self.code.N, self.code.q), np.float32)
-        il = np.zeros_like(llr) if want_sorted else None
-        ig = np.zeros(llr.shape, np.int32) if want_sorted else None
-        _check(lib().nbgpu_channel_awgn_bpsk(self.h, _f(noisy), C.c_float(sigma), B, _f(llr), _f(il), _i(ig)), self.h)
-        return (llr, il, ig) if want_sorted else llr
+        return self._channel(lib().nbgpu_channel_awgn_bpsk, noisy, self.code.logq, sigma, want_sorted)
 
     def check_node(self, node, vllr, vgf):
         dc = int(self.code.row_deg[node])

@@ -46,12 +46,16 @@
 
 #define UNIT_NT 256       /* block size of the small unit-boundary kernels */
 
+/* what the intake reads per variable (KArgs::input_kind): BPSK samples [logq], a dense LLR row [q], mapped (I, Q) samples [2]
+ * or faded (I, Q, rho_I, rho_Q) [4]; the mapped and faded intakes read KArgs::mod */
+enum InputKind { INPUT_BPSK = 0, INPUT_LLR = 1, INPUT_MAPPED = 2, INPUT_FADED = 3 };
+
 struct KArgs {
     int N, M, E, q, logq, dc_max, dc_min;
     int n_m, nb_oper, passes, early_stop, nb_iter_max;
     float offset;
     int F, nw, cpw, cap, nsteps, L;     /* frames per group, warps per CTA, check nodes per warp, items per step, steps, lists per node */
-    int B, input_kind, frame0;          /* frames of this launch; 0 = BPSK samples, 1 = dense LLR, 2 = mapped (I, Q) samples, 3 = faded (I, Q, rho_I, rho_Q); batch index of its first frame */
+    int B, input_kind, frame0;          /* frames of this launch; InputKind; batch index of its first frame */
     double den;                         /* 2.0 * (double)(float)(sigma*sigma), channel.c:73 */
     const int *step_ptr, *isolated;
     int n_isolated;
@@ -59,7 +63,7 @@ struct KArgs {
     const uint32_t *einfo;              /* [E] variable | coefficient << 20 | last-visit flag << 28 */
     const int *row_ptr, *col;
     const uint8_t *hval, *rotin, *rotout, *img, *inv;
-    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, input_kind 2 and 3 (set per launch) */
+    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, INPUT_MAPPED and INPUT_FADED (set per launch) */
     int gf_closed;
     const float *in;
     float *app; uint8_t *ctov; uint8_t *dec;
@@ -266,8 +270,8 @@ __device__ __forceinline__ void intake_variable(const float *noisy_n, double den
  * 64-APSK): for every symbol k, TMP[k] = (float)( (double)((I - mI)^2) / (2 sigma^2) + (double)((Q - mQ)^2) / (2 sigma^2) )
  * with (mI, mQ) = mod[binary image of k]; differences and squares in f32, divisions and the sum in f64, as the reference
  * evaluates them (a reciprocal multiply would round differently).  GF(16): lanes >= 16 hold no symbol.
- * s = (I, Q, rho_I, rho_Q): the faded channel (input kind 3) scales the point by its amplitudes, I - rho_I * mI in f32
- * (include/nbldpc_b200.h, NBGPU_FADING_SYMBOL); kind 2 passes rho = 1, and a product with 1.0f is exact. */
+ * s = (I, Q, rho_I, rho_Q): the faded channel (INPUT_FADED) scales the point by its amplitudes, I - rho_I * mI in f32
+ * (include/nbldpc_b200.h, NBGPU_FADING_SYMBOL); INPUT_MAPPED passes rho = 1, and a product with 1.0f is exact. */
 template <int Q>
 __device__ __forceinline__ void intake_mapped(const float4 s, double den, const float *mod, const uint8_t *img, int lane,
                                               float (&v)[QTraits<Q>::VPL])
@@ -281,10 +285,11 @@ __device__ __forceinline__ void intake_mapped(const float4 s, double den, const 
         v[j] = __double2float_rn(__dadd_rn(a, b));
     }
 }
-/* symbol r of a mapped (kind 2: [..][2], rho = 1) or faded (kind 3: [..][4], one 16-byte load) input as intake_mapped reads it */
+/* symbol r of a mapped (INPUT_MAPPED: [..][2], rho = 1) or faded (INPUT_FADED: [..][4], one 16-byte load) input as intake_mapped
+ * reads it */
 __device__ __forceinline__ float4 mapped_input(const float *in, int kind, size_t r)
 {
-    if (kind == 3) return *reinterpret_cast<const float4 *>(in + r * 4);
+    if (kind == INPUT_FADED) return *reinterpret_cast<const float4 *>(in + r * 4);
     return make_float4(in[r * 2], in[r * 2 + 1], 1.0f, 1.0f);
 }
 
@@ -707,9 +712,9 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
         for (int w = warp; w < nf * N; w += nw) {
             const int f = w / N, n = w - f * N;
             float v[VPL];
-            if (a.input_kind == 0) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
-                                                      reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
-            else if (a.input_kind >= 2) intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
+            if (a.input_kind == INPUT_BPSK) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
+                                                               reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
+            else if (a.input_kind >= INPUT_MAPPED) intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
             else load_row<Q>(a.in + ((size_t)(base + f) * N + n) * Q, lane, v);
             store_row<Q>(app + ((size_t)f * N + n) * Q, lane, v);
         }
@@ -1058,7 +1063,7 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
     const long total = (long)B * a.N;
     for (long r = (long)blockIdx.x * UW + warp; r < total; r += (long)gridDim.x * UW) {
         float v[VPL];
-        if (kind >= 2) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
+        if (kind >= INPUT_MAPPED) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
         else intake_variable<Q>(noisy + r * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
         if (llr) store_row<Q>(llr + r * Q, lane, v);
         if (illr) {
@@ -1104,6 +1109,19 @@ static const void *checknode_fn(int q, int closed, int ecn)
 /* ------------------------------------------------------------------------------------------------
  * context
  * ---------------------------------------------------------------------------------------------- */
+/* A channel as the host code uses it, resolved once per call by channel_of(): the intake, the frame layout, how the frame
+ * source draws a symbol and which constellation both read. */
+enum ChannelId { CH_BPSK, CH_LLR, CH_APSK64, CH_MAPPED, CH_FADED };
+struct Channel {
+    int rc;                      /* NBGPU_OK, or the refusal of channel_of (the rest is then unset) */
+    int kind;                    /* InputKind */
+    int fps;                     /* floats per symbol of a frame: log2 q, q, 2 (I, Q) or 4 (I, Q, rho_I, rho_Q) */
+    int draws;                   /* frame source: drand48 draws per symbol after the information bits */
+    bool apsk_sigma;             /* sigma = nbgpu_sigma_apsk64(EbN) (every constellation), else nbgpu_sigma(code, EbN) */
+    const float *mod_d, *mod_h;  /* constellation [q][2] on the device and its host copy; nullptr for BPSK and LLR */
+    int fading;                  /* CH_FADED: NBGPU_FADING_SYMBOL or NBGPU_FADING_COMPONENT of the frame source */
+};
+
 struct nbgpu_ctx {
     int device;
     cudaStream_t stream, copy_stream;        /* kernels | host<->device copies of the chunked end-to-end path */
@@ -1122,6 +1140,7 @@ struct nbgpu_ctx {
     uint8_t *d_cfg; float *d_ctov_dense;
     uint8_t *d_hval, *d_rotin, *d_rotout, *d_img, *d_inv;
     float *d_mod;                            /* the 64-APSK table (q = 64), used by every *_apsk64 call */
+    float mod_h[128];                        /* host copy of the 64-APSK table, for the frame source's fix-up */
     float *d_map;                            /* the bound table of the mapped calls (nbgpu_set_constellation), NULL until bound */
     float map_h[512];                        /* host copy of the bound table, for the frame source's fix-up */
     float *d_app; uint8_t *d_ctov; uint8_t *d_dec;
@@ -1129,17 +1148,16 @@ struct nbgpu_ctx {
     int *d_decide, *d_synd, *d_iters, *d_frame_slot, *d_slot_frame;
     unsigned *d_queue, *d_slow, *d_ready, *d_fault;
     unsigned *h_ready;                       /* pinned: cumulative frame counts of the input pieces of decode_host */
-    int resident_B, resident_kind;
-    const float *resident_mod;               /* table of the resident batch (kind 2: d_mod or d_map; kind 3: d_map) */
-    int mapped_dropped;                      /* kind (2 mapped, 3 faded) of the resident batch nbgpu_set_constellation dropped, else 0 */
+    int resident_B;
+    Channel resident;                        /* channel of the batch in d_in (kept when nbgpu_set_constellation drops it) */
+    int mapped_dropped;                      /* InputKind (mapped, faded) of the resident batch nbgpu_set_constellation dropped, else 0 */
     /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
     int soft_made, soft_B, decoded;
-    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames / _apsk64 / _mapped */
+    /* device frame source (nbldpc_source.cuh), set up by the first nbgpu_source_frames* call */
     struct {
         int ready, nlevels, B;
-        int kind;                /* channel of the generated batch, as resident_kind: 0 BPSK, 2 mapped (64-APSK or bound table), 3 faded */
         int *d_level_ptr, *d_row_order, *d_ut_ptr, *d_ut_col, *d_perm, *d_bit_errors;
         uint8_t *d_ut_val, *d_piv, *d_mulimg, *d_divimg, *d_cw, *d_flag_img;
         unsigned *d_flag_count, *d_flags, *d_patch_idx;
@@ -1147,7 +1165,8 @@ struct nbgpu_ctx {
         uint64_t D;              /* draws per frame of the generated batch (depends on the channel) */
         double margin;
         long fixups;
-        int state;               /* 0: nothing generated; 1: batch generated, not decoded; 2: generated batch decoded */
+        int state;               /* 0: nothing generated, or d_in overwritten by an upload since; 1: batch generated, not decoded;
+                                    2: generated batch decoded */
     } src;
     long launches;
     float last_ms;
@@ -1420,9 +1439,8 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
         (rc = upload(c, &c->d_img, img)) || (rc = upload(c, &c->d_inv, inv))) { nbgpu_destroy(c); return rc; }
     if (p->ecn_kind == 1) { if ((rc = upload(c, &c->d_cfg, cfg8))) { nbgpu_destroy(c); return rc; } k.cfg = c->d_cfg; }
     if (q == 64) {                                       /* 64-APSK intake (ModelChannel_AWGN_64): the constellation, built on the host */
-        std::vector<float> mod(128);
-        nbgpu_apsk64_table(mod.data());
-        if ((rc = upload(c, &c->d_mod, mod))) { nbgpu_destroy(c); return rc; }
+        nbgpu_apsk64_table(c->mod_h);
+        if ((rc = upload(c, &c->d_mod, std::vector<float>(c->mod_h, c->mod_h + 128)))) { nbgpu_destroy(c); return rc; }
     }
     k.row_ptr = c->d_row_ptr; k.col = c->d_col; k.cninfo = c->d_cninfo; k.einfo = c->d_einfo; k.step_ptr = c->d_step_ptr; k.isolated = c->d_isolated;
     k.hval = c->d_hval; k.rotin = c->d_rotin; k.rotout = c->d_rotout; k.img = c->d_img; k.inv = c->d_inv;
@@ -1502,65 +1520,77 @@ static int ensure_input(nbgpu_ctx *c, size_t floats)
     return NBGPU_OK;
 }
 
-/* mod: the constellation of a kind-2 or kind-3 batch (d_mod or d_map), nullptr otherwise */
-static int upload_common(nbgpu_ctx *c, const float *src, size_t per_frame, int B, int kind, const float *mod)
+/* Channel `id` of context c.  Refusals: the 64-APSK channel on another field than GF(64) (NBGPU_EINVAL), a mapped or faded
+ * channel with no bound table (NBGPU_ESTATE), a fading value other than NBGPU_FADING_SYMBOL / _COMPONENT (NBGPU_EINVAL).
+ * fading only sets the frame source's draws: the faded intake reads the amplitudes from the frames. */
+static Channel channel_of(nbgpu_ctx *c, ChannelId id, int fading = NBGPU_FADING_SYMBOL)
 {
-    if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    Channel ch = {};
+    if (!c) { ctx_err(NULL, "NULL context"); ch.rc = NBGPU_EINVAL; }
+    else if (id == CH_APSK64 && c->q != 64) {
+        ctx_err(c, "64-APSK intake (ModelChannel_AWGN_64, channel.c:112) maps one GF(64) symbol to one constellation point: q = %d", c->q);
+        ch.rc = NBGPU_EINVAL;
+    } else if (id == CH_FADED && fading != NBGPU_FADING_SYMBOL && fading != NBGPU_FADING_COMPONENT) {
+        ctx_err(c, "faded channel: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fading);
+        ch.rc = NBGPU_EINVAL;
+    } else if ((id == CH_MAPPED || id == CH_FADED) && !c->d_map) {
+        ctx_err(c, "mapped channel: no constellation bound to this context (call nbgpu_set_constellation first)");
+        ch.rc = NBGPU_ESTATE;
+    } else if (id == CH_BPSK) ch = { NBGPU_OK, INPUT_BPSK, c->logq, 2 * c->logq };           /* two draws per code bit, channel.c:56-57 */
+    else if (id == CH_LLR) ch = { NBGPU_OK, INPUT_LLR, c->q };
+    else {      /* two draws per I/Q sample (channel.c:234-263); faded: one amplitude draw (SYMBOL) or two (COMPONENT) more */
+        const bool faded = id == CH_FADED, apsk = id == CH_APSK64;
+        ch = { NBGPU_OK, faded ? INPUT_FADED : INPUT_MAPPED, faded ? 4 : 2, faded ? 4 + fading : 4, true, apsk ? c->d_mod : c->d_map,
+               apsk ? c->mod_h : c->map_h, faded ? fading : 0 };
+    }
+    return ch;
+}
+
+static double den_of(float sigma) { return 2.0 * (double)(float)(sigma * sigma); }     /* 2.0*SQR(sigma), channel.c:73 / :280 */
+
+/* B frames of channel ch are now in d_in, uploaded by the caller or made by the frame source */
+static void set_resident(nbgpu_ctx *c, const Channel &ch, int B, float sigma, bool generated)
+{
+    c->k.den = den_of(sigma);
+    c->resident_B = B; c->resident = ch; c->mapped_dropped = 0;
+    c->src.state = generated ? 1 : 0;
+    if (generated) c->src.B = B;
+}
+
+static int upload_common(nbgpu_ctx *c, const Channel &ch, const float *src, float sigma, int B)
+{
+    if (ch.rc) return ch.rc;
+    if (!src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;                           /* even a rejected batch: the caller moved on from the last one */
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
-    int rc = ensure_input(c, per_frame * (size_t)B);          /* grows on demand: dense-LLR batches are q/log2(q) times larger */
+    const size_t per_frame = (size_t)c->N * ch.fps;
+    int rc = ensure_input(c, per_frame * B);                  /* grows on demand: dense-LLR batches are q/log2(q) times larger */
     if (rc) return rc;
     CK(c, cudaMemcpyAsync(c->d_in, src, per_frame * B * sizeof(float), cudaMemcpyHostToDevice, c->stream));
-    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod; c->mapped_dropped = 0; c->src.state = 0;
+    set_resident(c, ch, B, sigma, false);
     return NBGPU_OK;
 }
 
 extern "C" int nbgpu_upload_noisy(nbgpu_ctx *c, const float *noisy, float sigma, int B)
 {
-    if (!c) return NBGPU_EINVAL;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:73 */
-    return upload_common(c, noisy, (size_t)c->N * c->logq, B, 0, nullptr);
+    return upload_common(c, channel_of(c, CH_BPSK), noisy, sigma, B);
 }
 extern "C" int nbgpu_upload_llr(nbgpu_ctx *c, const float *llr, int B)
 {
-    if (!c) return NBGPU_EINVAL;
-    return upload_common(c, llr, (size_t)c->N * c->q, B, 1, nullptr);
-}
-static int apsk64_ok(nbgpu_ctx *c)
-{
-    if (c->q == 64) return 1;
-    ctx_err(c, "64-APSK intake (ModelChannel_AWGN_64, channel.c:112) maps one GF(64) symbol to one constellation point: q = %d", c->q);
-    return 0;
+    return upload_common(c, channel_of(c, CH_LLR), llr, 0.0f, B);
 }
 extern "C" int nbgpu_upload_apsk64(nbgpu_ctx *c, const float *noisy, float sigma, int B)
 {
-    if (!c) return NBGPU_EINVAL;
-    if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return upload_common(c, noisy, (size_t)c->N * 2, B, 2, c->d_mod);
-}
-static int mapped_ok(nbgpu_ctx *c)
-{
-    if (c->d_map) return NBGPU_OK;
-    ctx_err(c, "mapped channel: no constellation bound to this context (call nbgpu_set_constellation first)");
-    return NBGPU_ESTATE;
+    return upload_common(c, channel_of(c, CH_APSK64), noisy, sigma, B);
 }
 extern "C" int nbgpu_upload_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return upload_common(c, noisy, (size_t)c->N * 2, B, 2, c->d_map);
+    return upload_common(c, channel_of(c, CH_MAPPED), noisy, sigma, B);
 }
 extern "C" int nbgpu_upload_faded(nbgpu_ctx *c, const float *rx, float sigma, int B)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);
-    return upload_common(c, rx, (size_t)c->N * 4, B, 3, c->d_map);
+    return upload_common(c, channel_of(c, CH_FADED), rx, sigma, B);
 }
 
 extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
@@ -1574,9 +1604,9 @@ extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
     CK(c, cudaMemcpyAsync(c->d_map, mod, 2 * (size_t)c->q * sizeof(float), cudaMemcpyHostToDevice, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
     memcpy(c->map_h, mod, 2 * (size_t)c->q * sizeof(float));
-    if (c->resident_B > 0 && c->resident_kind >= 2 && c->resident_mod == c->d_map) {
-        /* its samples were made for the old table: decoding them on the new one would be wrong */
-        c->resident_B = 0; c->mapped_dropped = c->resident_kind; c->soft_made = NBGPU_SOFT_NONE; c->src.state = 0;
+    if (c->resident_B > 0 && c->resident.mod_d == c->d_map) {
+        /* its samples were made for the old table: decoding them on the new one would be wrong (they stay downloadable) */
+        c->resident_B = 0; c->mapped_dropped = c->resident.kind; c->soft_made = NBGPU_SOFT_NONE;
     }
     return NBGPU_OK;
 }
@@ -1584,13 +1614,13 @@ extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
 extern "C" int nbgpu_run(nbgpu_ctx *c)
 {
     if (c && c->resident_B < 1 && c->mapped_dropped) {
-        ctx_err(c, "nbgpu_run: the %s batch was dropped when nbgpu_set_constellation bound a new table", c->mapped_dropped == 3 ? "faded" : "mapped");
+        ctx_err(c, "nbgpu_run: the %s batch was dropped when nbgpu_set_constellation bound a new table", c->mapped_dropped == INPUT_FADED ? "faded" : "mapped");
         return NBGPU_ESTATE;
     }
     if (!c || c->resident_B < 1) { ctx_err(c, "nbgpu_run: no resident batch (call nbgpu_upload_* first)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     KArgs k = c->k;
-    k.B = c->resident_B; k.input_kind = c->resident_kind; k.in = c->d_in; k.mod = c->resident_mod;
+    k.B = c->resident_B; k.input_kind = c->resident.kind; k.in = c->d_in; k.mod = c->resident.mod_d;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     const int groups = (k.B + k.F - 1) / k.F;
     const int grid = std::min(c->grid, groups);
@@ -1688,21 +1718,23 @@ extern "C" int nbgpu_download(nbgpu_ctx *c, int *decide, int *synd, int *iters)
  * only the first groups ever wait and the H2D time disappears behind the kernel -- without cutting the batch into several
  * launches, whose starts and tails cost as much as the copies they hid (measured: 340 ms either way against 327.6 ms for the
  * kernel alone on config 5).  Small batches take the plain upload / run / download path (and keep their state readable). */
-static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kind, const float *mod, int B, int *decide, int *synd, int *iters)
+static int decode_host(nbgpu_ctx *c, const Channel &ch, const float *src, float sigma, int B, int *decide, int *synd, int *iters)
 {
-    if (!c || !src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    if (ch.rc) return ch.rc;
+    if (!src) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     const int wave = c->grid * c->k.F;
     if (B < 2 * wave || getenv("NBGPU_NO_CHUNKS")) {
-        int rc = upload_common(c, src, per_frame, B, kind, mod);
+        int rc = upload_common(c, ch, src, sigma, B);
         if (rc || (rc = nbgpu_run(c)) || (rc = nbgpu_download(c, decide, synd, iters))) return rc;
         return NBGPU_OK;
     }
     CK(c, cudaSetDevice(c->device));
-    int rc = ensure_input(c, per_frame * (size_t)B);
+    const size_t per_frame = (size_t)c->N * ch.fps;
+    int rc = ensure_input(c, per_frame * B);
     if (rc) return rc;
-    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod; c->mapped_dropped = 0; c->src.state = 0;
+    set_resident(c, ch, B, sigma, false);
     /* pieces: one wave first, the rest in up to 7 equal runs of whole waves */
     int lo[9], np = 1;
     {
@@ -1722,7 +1754,7 @@ static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kin
         CK(c, cudaMemcpyAsync(c->d_ready, c->h_ready + i, sizeof(unsigned), cudaMemcpyHostToDevice, c->copy_stream));
     }
     KArgs k = c->k;
-    k.B = B; k.input_kind = kind; k.in = c->d_in; k.mod = mod; k.ready = c->d_ready;
+    k.B = B; k.input_kind = ch.kind; k.in = c->d_in; k.mod = ch.mod_d; k.ready = c->d_ready;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     CK(c, cudaStreamWaitEvent(c->stream, c->ev_h2d[0], 0));   /* the counter starts at zero */
     CK(c, cudaEventRecord(c->ev0, c->stream));
@@ -1748,37 +1780,23 @@ static int decode_host(nbgpu_ctx *c, const float *src, size_t per_frame, int kin
 
 extern "C" int nbgpu_decode_noisy(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
 {
-    if (!c) return NBGPU_EINVAL;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:73 */
-    return decode_host(c, noisy, (size_t)c->N * c->logq, 0, nullptr, B, decide, synd, iters);
+    return decode_host(c, channel_of(c, CH_BPSK), noisy, sigma, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_llr(nbgpu_ctx *c, const float *llr, int B, int *decide, int *synd, int *iters)
 {
-    if (!c) return NBGPU_EINVAL;
-    return decode_host(c, llr, (size_t)c->N * c->q, 1, nullptr, B, decide, synd, iters);
+    return decode_host(c, channel_of(c, CH_LLR), llr, 0.0f, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_apsk64(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
 {
-    if (!c) return NBGPU_EINVAL;
-    if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return decode_host(c, noisy, (size_t)c->N * 2, 2, c->d_mod, B, decide, synd, iters);
+    return decode_host(c, channel_of(c, CH_APSK64), noisy, sigma, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);                      /* 2.0*SQR(sigma), channel.c:280 */
-    return decode_host(c, noisy, (size_t)c->N * 2, 2, c->d_map, B, decide, synd, iters);
+    return decode_host(c, channel_of(c, CH_MAPPED), noisy, sigma, B, decide, synd, iters);
 }
 extern "C" int nbgpu_decode_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, int *decide, int *synd, int *iters)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);
-    return decode_host(c, rx, (size_t)c->N * 4, 3, c->d_map, B, decide, synd, iters);
+    return decode_host(c, channel_of(c, CH_FADED), rx, sigma, B, decide, synd, iters);
 }
 
 
@@ -1869,51 +1887,50 @@ extern "C" int nbgpu_source_set_margin(nbgpu_ctx *c, double margin)
     return NBGPU_OK;
 }
 
-/* Body of nbgpu_source_frames (kind 0, BPSK: noisy[B][N][logq]), nbgpu_source_frames_apsk64 / _mapped (kind 2, mapped:
- * noisy[B][N][2] on the table mod_d, whose host copy is mod_h) and nbgpu_source_frames_faded (kind 3, rx[B][N][4] on the
- * bound table, fading 1 or 2).  The channel fixes the draws per frame D, sigma, the noise kernel and the host recomputation
- * of a flagged sample (faded: of a whole symbol); encoder, flag read-back and patch are shared. */
-static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int kind,
-                           int fading, const float *mod_d, const float *mod_h)
+/* Body of every nbgpu_source_frames* call: B frames of channel `id` (fading: CH_FADED only).  The channel fixes the draws per
+ * frame D, sigma, the noise kernel and the host recomputation of a flagged sample (faded: of a whole symbol); encoder, flag
+ * read-back and patch are shared. */
+static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, ChannelId id,
+                           int fading = NBGPU_FADING_SYMBOL)
 {
+    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
+    const Channel ch = channel_of(c, id, fading);
+    if (ch.rc) return ch.rc;
     /* the frames are encoded with the code's tables but decoded and scored with the context's: only the context's own code
      * (by content, so that a copy loaded per thread or rank qualifies) is accepted, and the encoder tables built from it
      * stay valid for every later call */
     if (code_hash(code) != c->code_hash) { ctx_err(c, "nbgpu_source_frames: the code is not the one the decoder was created for"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
-    const int spf = kind == 3 ? 4 : kind == 2 ? 2 : c->logq;   /* noisy samples (faded: samples and amplitudes) per symbol */
-    if ((double)B * c->N * spf >= 2147483648.0) { ctx_err(c, "frame source: B*N*%s must stay below 2^31", kind == 3 ? "4" : kind == 2 ? "2" : "log2(q)"); return NBGPU_EINVAL; }
+    if ((double)B * c->N * ch.fps >= 2147483648.0) { ctx_err(c, "frame source: B*N*%d must stay below 2^31", ch.fps); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     int rc;
     if (!c->src.ready && (rc = source_setup(c, code))) { source_teardown(c); return rc; }
-    if ((rc = ensure_input(c, (size_t)c->N * spf * B))) return rc;
+    if ((rc = ensure_input(c, (size_t)c->N * ch.fps * B))) return rc;
     const uint64_t koff = (uint64_t)(c->N - c->M) * c->logq;   /* information-bit draws, tools.c:124-136 */
-    /* K log2 q information bits, then two draws per noisy sample (channel.c:56-57 per bit, channel.c:234-263 per I/Q) and,
-     * faded, one amplitude draw (SYMBOL) or two (COMPONENT) per symbol */
-    const int S = kind == 3 ? 4 + fading : 2 * spf;             /* draws per symbol (BPSK: 2 log2 q) */
+    const int S = ch.draws;
     const uint64_t D = koff + (uint64_t)c->N * S;
-    const float sigma = kind >= 2 ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
+    const float sigma = ch.apsk_sigma ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
     nbgpu_rng r = *origin;
     nbgpu_rng_skip(&r, frame0 * D);
     c->src.D = D;
     SrcArgs a = source_args(c, code, B);
-    a.x0 = r.x; a.sigma = sigma; a.mod = mod_d;
-    if (kind == 3) a.flag_cap = SRC_FLAG_CAP / 4;               /* a flagged symbol takes four patch entries */
+    a.x0 = r.x; a.sigma = sigma; a.mod = ch.mod_d;
+    if (ch.kind == INPUT_FADED) a.flag_cap = SRC_FLAG_CAP / 4;  /* a flagged symbol takes four patch entries */
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
     const long long threads = (long long)B * c->N;
     const unsigned blocks = (unsigned)((threads + 255) / 256);
-    if (kind == 3 && fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
-    else if (kind == 3) source_noise_mapped_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
-    else if (kind == 2) source_noise_mapped_kernel<0><<<blocks, 256, 0, c->stream>>>(a);
+    if (ch.fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
+    else if (ch.fading == NBGPU_FADING_SYMBOL) source_noise_mapped_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
+    else if (ch.kind == INPUT_MAPPED) source_noise_mapped_kernel<0><<<blocks, 256, 0, c->stream>>>(a);
     else source_noise_kernel<<<blocks, 256, 0, c->stream>>>(a);
     CK(c, cudaGetLastError());
     c->launches += 2;
     unsigned nflag = 0;
     CK(c, cudaMemcpyAsync(&nflag, c->src.d_flag_count, sizeof nflag, cudaMemcpyDeviceToHost, c->stream));
     CK(c, cudaStreamSynchronize(c->stream));
-    if (nflag > a.flag_cap) { ctx_err(c, "frame source: %u %s flagged for host recomputation (capacity %u); margin too wide", nflag, kind == 3 ? "symbols" : "samples", a.flag_cap); return NBGPU_EINVAL; }
+    if (nflag > a.flag_cap) { ctx_err(c, "frame source: %u %s flagged for host recomputation (capacity %u); margin too wide", nflag, ch.kind == INPUT_FADED ? "symbols" : "samples", a.flag_cap); return NBGPU_EINVAL; }
     c->src.fixups = nflag;
     if (nflag) {
         /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
@@ -1921,10 +1938,10 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
          * A faded flag is symbol n of the batch: its S draws, its four values. */
         std::vector<unsigned> idx(nflag), pidx;
         std::vector<float> val(nflag);
-        std::vector<uint8_t> img(kind >= 2 ? nflag : 0);
+        std::vector<uint8_t> img(ch.kind >= INPUT_MAPPED ? nflag : 0);
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (kind >= 2) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
-        if (kind == 3) {
+        if (ch.kind >= INPUT_MAPPED) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
+        if (ch.kind == INPUT_FADED) {
             pidx.resize(4 * (size_t)nflag); val.resize(4 * (size_t)nflag);
             for (unsigned i = 0; i < nflag; i++) {
                 const uint64_t f = idx[i] / c->N, n = idx[i] % c->N;
@@ -1932,19 +1949,19 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
                 nbgpu_rng_skip(&g, f * D + koff + (uint64_t)S * n);
                 float dr[6];
                 for (int j = 0; j < S; j++) dr[j] = (float)nbgpu_rng_drand48(&g);
-                nbgpu_faded_sample(sigma, mod_h + 2 * img[i], dr, fading, &val[4 * (size_t)i]);
+                nbgpu_faded_sample(sigma, ch.mod_h + 2 * img[i], dr, ch.fading, &val[4 * (size_t)i]);
                 for (int j = 0; j < 4; j++) pidx[4 * (size_t)i + j] = 4 * idx[i] + j;
             }
             idx.swap(pidx);
             nflag *= 4;
         } else {
-            const uint64_t per = (uint64_t)c->N * spf;
+            const uint64_t per = (uint64_t)c->N * ch.fps;
             for (unsigned i = 0; i < nflag; i++) {
                 const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
                 nbgpu_rng g; g.x = a.x0;
                 nbgpu_rng_skip(&g, f * D + koff + 2 * s);
                 const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-                val[i] = kind == 2 ? nbgpu_mapped_sample(sigma, mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+                val[i] = ch.kind == INPUT_MAPPED ? nbgpu_mapped_sample(sigma, ch.mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
             }
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
@@ -1954,49 +1971,25 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         CK(c, cudaStreamSynchronize(c->stream));                 /* idx/val are stack-scoped */
         c->launches += 1;
     }
-    c->k.den = 2.0 * (double)(float)(sigma * sigma);            /* 2.0*SQR(sigma), channel.c:73 / channel.c:280 */
-    c->resident_B = B; c->resident_kind = kind; c->resident_mod = mod_d; c->mapped_dropped = 0;
-    c->src.B = B; c->src.kind = kind; c->src.state = 1;
+    set_resident(c, ch, B, sigma, true);
     return NBGPU_OK;
 }
 
 extern "C" int nbgpu_source_frames(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
-    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    return source_generate(c, code, origin, frame0, B, EbN, 0, 0, nullptr, nullptr);
+    return source_generate(c, code, origin, frame0, B, EbN, CH_BPSK);
 }
-
 extern "C" int nbgpu_source_frames_apsk64(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
-    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    float mod[128];
-    nbgpu_apsk64_table(mod);
-    return source_generate(c, code, origin, frame0, B, EbN, 2, 0, c->d_mod, mod);
+    return source_generate(c, code, origin, frame0, B, EbN, CH_APSK64);
 }
-
 extern "C" int nbgpu_source_frames_mapped(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
 {
-    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    return source_generate(c, code, origin, frame0, B, EbN, 2, 0, c->d_map, c->map_h);
+    return source_generate(c, code, origin, frame0, B, EbN, CH_MAPPED);
 }
-
-static int fading_ok(nbgpu_ctx *c, int fading)
-{
-    if (fading == NBGPU_FADING_SYMBOL || fading == NBGPU_FADING_COMPONENT) return 1;
-    ctx_err(c, "faded channel: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fading);
-    return 0;
-}
-
 extern "C" int nbgpu_source_frames_faded(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int fading)
 {
-    if (!c || !code || !origin) { ctx_err(c, "NULL argument"); return NBGPU_EINVAL; }
-    if (!fading_ok(c, fading)) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    return source_generate(c, code, origin, frame0, B, EbN, 3, fading, c->d_map, c->map_h);
+    return source_generate(c, code, origin, frame0, B, EbN, CH_FADED, fading);
 }
 
 extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixups : 0; }
@@ -2004,6 +1997,7 @@ extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixu
 extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
 {
     if (!c || !c->src.ready || c->src.B < 1) { ctx_err(c, "nbgpu_source_download: no generated batch"); return NBGPU_EINVAL; }
+    if (c->src.state == 0) { ctx_err(c, "nbgpu_source_download: the generated batch was replaced by an uploaded batch"); return NBGPU_ESTATE; }
     CK(c, cudaSetDevice(c->device));
     const int B = c->src.B;
     if (codeword) {
@@ -2013,8 +2007,7 @@ extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
         for (size_t i = 0; i < cw.size(); i++) codeword[i] = c->inv_h[cw[i]];
     }
     if (noisy) {
-        const size_t spf = c->src.kind == 3 ? 4 : c->src.kind == 2 ? 2 : c->logq;
-        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * spf * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * c->resident.fps * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
     return NBGPU_OK;
@@ -2258,18 +2251,19 @@ extern "C" int nbgpu_decision_syndrome(nbgpu_ctx *c, const float *app, int *deci
     return NBGPU_OK;
 }
 
-static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf, int kind, const float *mod)
+static int channel_common(nbgpu_ctx *c, const Channel &ch, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    if (!c || !noisy || B < 1 || ((illr == NULL) != (igf == NULL))) { ctx_err(c, "nbgpu_channel_awgn_*: bad argument"); return NBGPU_EINVAL; }
+    if (ch.rc) return ch.rc;
+    if (!noisy || B < 1 || ((illr == NULL) != (igf == NULL))) { ctx_err(c, "nbgpu_channel_awgn_*: bad argument"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
-    const int N = c->N, q = c->q, per = kind == 3 ? 4 : kind == 2 ? 2 : c->logq;
+    const int N = c->N, q = c->q, per = ch.fps, kind = ch.kind;
     DevBuf<float> dn, dl, dil; DevBuf<int> dig;
     CK(c, dn.alloc((size_t)B * N * per)); CK(c, dl.alloc((size_t)B * N * q));
     if (illr) { CK(c, dil.alloc((size_t)B * N * q)); CK(c, dig.alloc((size_t)B * N * q)); }
     CK(c, cudaMemcpyAsync(dn.p, noisy, (size_t)B * N * per * 4, cudaMemcpyHostToDevice, c->stream));
     KArgs k = c->k;
-    k.den = 2.0 * (double)(float)(sigma * sigma);
-    k.mod = mod;
+    k.den = den_of(sigma);
+    k.mod = ch.mod_d;
     const int grid = (int)std::min<long>(((long)B * N + UNIT_NT / 32 - 1) / (UNIT_NT / 32), 148 * 8);
     if (q == 16) channel_kernel<16><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
     else if (q == 64) channel_kernel<64><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
@@ -2286,25 +2280,17 @@ static int channel_common(nbgpu_ctx *c, const float *noisy, float sigma, int B, 
 }
 extern "C" int nbgpu_channel_awgn_bpsk(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    return channel_common(c, noisy, sigma, B, llr, illr, igf, 0, nullptr);
+    return channel_common(c, channel_of(c, CH_BPSK), noisy, sigma, B, llr, illr, igf);
 }
 extern "C" int nbgpu_channel_awgn_apsk64(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    if (!c) return NBGPU_EINVAL;
-    if (!apsk64_ok(c)) return NBGPU_EINVAL;
-    return channel_common(c, noisy, sigma, B, llr, illr, igf, 2, c->d_mod);
+    return channel_common(c, channel_of(c, CH_APSK64), noisy, sigma, B, llr, illr, igf);
 }
 extern "C" int nbgpu_channel_awgn_mapped(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    return channel_common(c, noisy, sigma, B, llr, illr, igf, 2, c->d_map);
+    return channel_common(c, channel_of(c, CH_MAPPED), noisy, sigma, B, llr, illr, igf);
 }
 extern "C" int nbgpu_channel_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, float *llr, float *illr, int *igf)
 {
-    if (!c) return NBGPU_EINVAL;
-    int rc = mapped_ok(c);
-    if (rc) return rc;
-    return channel_common(c, rx, sigma, B, llr, illr, igf, 3, c->d_map);
+    return channel_common(c, channel_of(c, CH_FADED), rx, sigma, B, llr, illr, igf);
 }

@@ -31,18 +31,38 @@ def _fading(channel, fading):
     return FADINGS[fading]
 
 
+def _sigma_apsk64(code, ebn):
+    from . import sigma_apsk64
+    return sigma_apsk64(ebn)
+
+
+# per channel: drand48 draws per symbol after the K*log2(q) information bits (fading adds 1 or 2), sigma(code, ebn), the host
+# noise of one frame (code, nbin, ebn, mod, fading) and the device source of a batch (decoder, frame0, B, ebn, fading)
+_CHANNELS = {
+    "bpsk": (lambda code: 2 * code.logq, lambda code, ebn: code.sigma(ebn),
+             lambda code, nbin, ebn, mod, fd: code.noise(nbin, ebn),
+             lambda d, frame0, B, ebn, fd: d.source_frames(frame0, B, ebn)),
+    "apsk64": (lambda code: 4, _sigma_apsk64,
+               lambda code, nbin, ebn, mod, fd: code.noise_apsk64(nbin, ebn),
+               lambda d, frame0, B, ebn, fd: d.source_frames_apsk64(frame0, B, ebn)),
+    "mapped": (lambda code: 4, _sigma_apsk64,
+               lambda code, nbin, ebn, mod, fd: code.noise_faded(nbin, mod, ebn, fd) if fd else code.noise_mapped(nbin, mod, ebn),
+               lambda d, frame0, B, ebn, fd: d.source_frames_faded(frame0, B, ebn, fd) if fd else d.source_frames_mapped(frame0, B, ebn)),
+}
+
+
+def _channel(channel):
+    if channel not in _CHANNELS:
+        raise ValueError("channel must be 'bpsk', 'apsk64' or 'mapped', not %r" % (channel,))
+    return _CHANNELS[channel]
+
+
 def draws_per_frame(code, channel="bpsk", fading=None):
     """drand48 draws one frame of the reference's main loop consumes: tools.c:124-136, then channel.c:56-57 ("bpsk",
     ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table);
     fading="symbol" / "component" (mapped only): one / two Rayleigh amplitude draws more per symbol"""
     fd = _fading(channel, fading)
-    if fd:
-        return code.K * code.logq + (4 + fd) * code.N
-    if channel == "bpsk":
-        return (code.K + 2 * code.N) * code.logq
-    if channel in ("apsk64", "mapped"):
-        return code.K * code.logq + 4 * code.N
-    raise ValueError("channel must be 'bpsk', 'apsk64' or 'mapped', not %r" % (channel,))
+    return code.K * code.logq + (_channel(channel)[0](code) + fd) * code.N
 
 
 def frame_range(total, rank, world):
@@ -96,30 +116,21 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     lo, hi = frame_range(frames, rank, world)
     D = draws_per_frame(code, channel, fading)
     fd = _fading(channel, fading)
-    apsk = channel == "apsk64"
-    mapped = channel == "mapped"
-    if mapped and constellation is None:
+    _, sigma_of, noise, source = _channel(channel)
+    if channel == "mapped" and constellation is None:
         raise ValueError("channel='mapped' needs constellation=mod[q][2]")
-    if mapped and decoder is not None:
+    if channel == "mapped" and decoder is not None:
         decoder.set_constellation(constellation)
     code.prepare_encoder()
     code.rng_default()
     code.rng_skip(lo * D)
-    if apsk or mapped:
-        from . import sigma_apsk64
-        sigma = sigma_apsk64(ebn)
-    else:
-        sigma = code.sigma(ebn)
+    sigma = sigma_of(code, ebn)
     bing = code.tables()[0]
     rows = np.zeros((hi - lo, 3), np.int64)
     for b0 in range(lo, hi, batch):
         b1 = min(hi, b0 + batch)
         if decoder is not None:
-            if fd:
-                decoder.source_frames_faded(b0, b1 - b0, ebn, fd)
-            else:
-                src = decoder.source_frames_apsk64 if apsk else decoder.source_frames_mapped if mapped else decoder.source_frames
-                src(b0, b1 - b0, ebn)
+            source(decoder, b0, b1 - b0, ebn, fd)
             decoder.run()
             rows[b0 - lo:b1 - lo] = np.stack(decoder.source_results(), axis=1)
             continue
@@ -127,12 +138,7 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         for _ in range(b0, b1):
             _, nbin = code.random_codeword()
             bits.append(nbin)
-            if fd:
-                noisy.append(code.noise_faded(nbin, constellation, ebn, fd))
-            elif mapped:
-                noisy.append(code.noise_mapped(nbin, constellation, ebn))
-            else:
-                noisy.append(code.noise_apsk64(nbin, ebn) if apsk else code.noise(nbin, ebn))
+            noisy.append(noise(code, nbin, ebn, constellation, fd))
         dec, synd, it = decode(np.stack(noisy), sigma)
         for i in range(b1 - b0):
             err = int((bing[dec[i, :code.K]] != bits[i][:code.K]).sum())                    # NB_LDPC.c:479-485

@@ -270,7 +270,8 @@ int  nbgpu_source_frames_faded(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng
                                int fading);
 /* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq]
  * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 / _mapped, rx [B][N][4] after
- * nbgpu_source_frames_faded */
+ * nbgpu_source_frames_faded; NBGPU_ESTATE once an upload or a decode call has replaced the batch (a batch dropped by
+ * nbgpu_set_constellation stays readable) */
 int  nbgpu_source_download(nbgpu_ctx *ctx, int *codeword, float *noisy);
 /* after nbgpu_run: information-bit errors of each frame (NB_LDPC.c:479-485), syndrome value, iteration count;
  * feed them to the frame-order statistics rule (NB_LDPC.c:474-507).  12 bytes per frame cross PCIe. */

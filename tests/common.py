@@ -1,12 +1,18 @@
-"""Shared helpers of the test-suite: fixture loading, matrix lookup, seeded frame generation."""
+"""Shared helpers of the test-suite: fixture loading, matrix lookup, seeded frame generation, the channels' host frames and
+the Monte-Carlo driver."""
 import glob
 import hashlib
+import importlib
 import os
+import subprocess
 
 import numpy as np
 import pytest
 
+import nbldpc
 import oracle_lib as ol
+
+multigpu = importlib.import_module("ems-decoder-of-nb-ldpc-codes_b200.multigpu")
 
 ROOT = ol.ROOT
 GOLDEN_DIR = os.path.join(ROOT, "tests", "golden")
@@ -56,6 +62,24 @@ def code_path(rel):
             write_alist_ubs(path, a)
         _STANDIN[rel] = path
     return _STANDIN[rel]
+
+
+_SYN = {}
+
+
+def mpath(rel):
+    """reference matrices, plus small synthetic GF(16) codes (the only GF(16) matrix of the reference is the 64800-bit one)"""
+    if not rel.startswith("synthetic/"):
+        return code_path(rel)
+    if rel not in _SYN:
+        import re
+        import tempfile
+        q, N, M, dc = [int(x) for x in re.match(r"synthetic/GF(\d+)_N(\d+)_M(\d+)_dc(\d+)", rel).groups()]
+        a = random_regular_code(np.random.default_rng(q + N + dc), N, M, q, dc)
+        path = os.path.join(tempfile.mkdtemp(prefix="nbldpc_syn_"), rel.split("/")[1])
+        write_alist_ubs(path, a)
+        _SYN[rel] = path
+    return _SYN[rel]
 
 
 def golden_names():
@@ -299,3 +323,88 @@ def write_alist_kn(path, a):
         f.write(" ".join(map(str, np.bincount(col, minlength=N))) + "\n" + " ".join(map(str, rd)) + "\n\n")
         for m in range(M):
             f.write("   ".join("%d %d" % (col[e] + 1, val[e] - 1) for e in range(rp[m], rp[m + 1])) + "\n")
+
+
+# ---- channels: host frames, device-source checks, the Monte-Carlo driver ------------------------------------------------
+EXE = os.path.join(os.path.dirname(nbldpc.LIB_PATH), "nbldpc_mc")
+CONSOLE = r"<(\d+)> FER=\s*(\d+)\s*/\s*(\d+)\s*=\s*[\d.]+\s*BER=\s*(\d+)\s*/\s*x\s*=\s*[\d.eE+-]+\s*avr_it=([\d.]+)"
+PI = 3.1415926536                                              # channel.c:18
+# one code per field; GF(16) has no matrix file, so a seeded random code stands in (mpath)
+CODES = {16: "synthetic/GF16_N24_M12_dc4", 64: "matrices/N96_K48_GF64", 256: "matrices/KN/N96_K48_GF256.txt"}
+ESN = {16: 10.0, 64: 15.0, 256: 23.0}                          # Es/N0 (dB) at which the QAM frames mix easy and hard ones
+FADING_NAMES = {nbldpc.FADING_SYMBOL: "symbol", nbldpc.FADING_COMPONENT: "component"}
+
+
+def field_code(q):
+    path = mpath(CODES[q])
+    return nbldpc.Code(path), path
+
+
+def seeded_table(q, seed=5):
+    """a table that is neither normalised nor symmetric, with two coincident points"""
+    mod = np.random.default_rng(seed).normal(0, 1.7, (q, 2)).astype(np.float32)
+    mod[3] = mod[1]
+    return mod
+
+
+def oracle_llr_mapped(o, noisy, mod, sigma):
+    """channel.c:266-291 on mod: f32 differences and squares, f64 divisions by 2 (float)(sigma^2) and sum, rounded to f32"""
+    img = (o.bingf.astype(np.int64) << np.arange(o.bingf.shape[1])).sum(1)
+    den = 2.0 * float(np.float32(sigma) * np.float32(sigma))
+    d0 = (noisy[:, 0:1].astype(np.float32) - mod[img, 0][None, :]).astype(np.float32)
+    d1 = (noisy[:, 1:2].astype(np.float32) - mod[img, 1][None, :]).astype(np.float32)
+    a = (d0 * d0).astype(np.float64) / den
+    b = (d1 * d1).astype(np.float64) / den
+    return (a + b).astype(np.float32)
+
+
+def host_frames(code, frame0, B, ebn, channel, mod=None, fading=None):
+    """frames [frame0, frame0 + B) of the host source: (codewords [B, N], bits [B, N, logq], frames) on channel "bpsk"
+    (noisy [B, N, logq]), "apsk64" (noisy [B, N, 2]) or "mapped" on mod (noisy [B, N, 2]; with fading = FADING_SYMBOL or
+    FADING_COMPONENT, rx [B, N, 4])"""
+    code.prepare_encoder()
+    code.rng_default()
+    code.rng_skip(frame0 * multigpu.draws_per_frame(code, channel, fading=FADING_NAMES.get(fading)))
+    cws, bits, noisy = [], [], []
+    for _ in range(B):
+        cw, nbin = code.random_codeword()
+        cws.append(cw); bits.append(nbin)
+        if fading:
+            noisy.append(code.noise_faded(nbin, mod, ebn, fading))
+        elif channel == "mapped":
+            noisy.append(code.noise_mapped(nbin, mod, ebn))
+        else:
+            noisy.append(code.noise_apsk64(nbin, ebn) if channel == "apsk64" else code.noise(nbin, ebn))
+    return np.stack(cws), np.stack(bits), np.stack(noisy)
+
+
+def same_stream(d, code, frame0, B, ebn, channel, mod=None, fading=None):
+    """the batch d generated equals host_frames, codewords and frames bit for bit"""
+    cw, _, noisy = host_frames(code, frame0, B, ebn, channel, mod, fading)
+    gcw, gnoisy = d.source_download()
+    assert gnoisy.shape == noisy.shape
+    return (gcw == cw).all() and gnoisy.tobytes() == noisy.tobytes()
+
+
+def soft(d, kind):
+    return d.soft_list() if kind == nbldpc.SOFT_LIST else (d.soft_bits(),)
+
+
+def waves(code, n_m, early=True, **kw):
+    """a batch of more than two waves of the decoder's geometry (one frame per CTA): streamed path and slot reuse"""
+    d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, early_stop=early, max_batch=1 << 14, frames_per_cta=1, **kw)
+    g = d.geometry()
+    d.close()
+    return 2 * g["grid"] * g["frames_per_cta"] + 37
+
+
+def run_driver(tmp_path, sub, path, ebn, n_m, source, channel, *tail, devices="0"):
+    """nbldpc_mc on 2000 frames of `path` in tmp_path/sub (channel, then the fading and degrees arguments in tail):
+    (console output, results-file lines without their time stamps)"""
+    d = tmp_path / sub
+    os.makedirs(d / "data")
+    r = subprocess.run([EXE, "2000", "10", path, ebn, str(n_m), "0.3", "25", "128", devices, "0", str(source), str(channel), *tail],
+                       cwd=d, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
+    assert r.returncode == 0, r.stdout[-2000:]
+    lines = list((d / "data").glob("results_*.txt"))[0].read_text().splitlines()
+    return r.stdout, [ln.split("time:")[0] for ln in lines]

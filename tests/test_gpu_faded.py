@@ -15,10 +15,8 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import matrix_path
-from test_gpu_mapped import CONSOLE, ESN, EXE, PI, _code, _host_frames, seeded_table
-
-multigpu = __import__("importlib").import_module("ems-decoder-of-nb-ldpc-codes_b200.multigpu")
+from common import (CONSOLE, ESN, EXE, FADING_NAMES, PI, field_code, host_frames, matrix_path, multigpu, run_driver, same_stream,
+                    seeded_table, soft, waves)
 
 gpu = pytest.mark.gpu
 KINDS = {"symbol": nbldpc.FADING_SYMBOL, "component": nbldpc.FADING_COMPONENT}
@@ -60,44 +58,10 @@ def oracle_llr_faded(o, rx, mod, sigma):
     return (a + b).astype(np.float32)
 
 
-def _faded_frames(code, frame0, B, ebn, mod, fading):
-    code.prepare_encoder()
-    code.rng_default()
-    code.rng_skip(frame0 * multigpu.draws_per_frame(code, "mapped", fading=_name(fading)))
-    cws, rxs = [], []
-    for _ in range(B):
-        cw, nbin = code.random_codeword()
-        cws.append(cw)
-        rxs.append(code.noise_faded(nbin, mod, ebn, fading))
-    return np.stack(cws), np.stack(rxs)
-
-
-def _name(fading):
-    return {v: k for k, v in KINDS.items()}[fading]
-
-
-def _same_faded_stream(d, code, frame0, B, ebn, mod, fading):
-    cw, rx = _faded_frames(code, frame0, B, ebn, mod, fading)
-    gcw, grx = d.source_download()
-    assert grx.shape == rx.shape == (B, code.N, 4)
-    return (gcw == cw).all() and grx.tobytes() == rx.tobytes()
-
-
-def _waves(code, n_m, early=True, **kw):
-    d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, early_stop=early, max_batch=1 << 14, frames_per_cta=1, **kw)
-    g = d.geometry()
-    d.close()
-    return 2 * g["grid"] * g["frames_per_cta"] + 37                 # more than two waves: streamed path and slot reuse
-
-
-def _soft(d, kind):
-    return d.soft_list() if kind == nbldpc.SOFT_LIST else (d.soft_bits(),)
-
-
 # ---- CPU ---------------------------------------------------------------------------------------------------------------
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_host_faded_noise_equals_the_oracle(q):
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     nbin = np.random.default_rng(q + 1).integers(0, 2, (code.N, code.logq)).astype(np.int32)
     for mod in (nbldpc.constellation(nbldpc.MAP_QAM, q), seeded_table(q)):
@@ -134,7 +98,7 @@ def test_host_faded_noise_equals_the_oracle(q):
 
 
 def test_rayleigh_amplitudes_have_unit_mean_power():
-    code, _ = _code(256)
+    code, _ = field_code(256)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, 256)
     code.rng_default()
     rho = np.concatenate([code.noise_faded(None, mod, 20.0, nbldpc.FADING_COMPONENT)[:, 2:].ravel() for _ in range(4200)])
@@ -147,12 +111,12 @@ def test_rayleigh_amplitudes_have_unit_mean_power():
 
 @pytest.mark.parametrize("fading", ["symbol", "component"])
 def test_draws_per_frame_faded_skips_whole_frames(fading):
-    code, _ = _code(256)
+    code, _ = field_code(256)
     fd = KINDS[fading]
     mod = nbldpc.constellation(nbldpc.MAP_QAM, 256)
     D = multigpu.draws_per_frame(code, "mapped", fading=fading)
     assert D == code.K * 8 + S[fd] * code.N
-    _, rx = _faded_frames(code, 0, 7, 25.0, mod, fd)
+    _, _, rx = host_frames(code, 0, 7, 25.0, "mapped", mod, fd)
     for f in (1, 3, 6):
         code.rng_default(); code.rng_skip(f * D)
         _, nb = code.random_codeword()
@@ -160,7 +124,7 @@ def test_draws_per_frame_faded_skips_whole_frames(fading):
 
 
 def test_fading_is_a_property_of_the_mapped_channel_only():
-    code, _ = _code(64)
+    code, _ = field_code(64)
     for ch in ("bpsk", "apsk64"):
         with pytest.raises(ValueError):
             multigpu.draws_per_frame(code, ch, fading="symbol")
@@ -238,7 +202,7 @@ def test_c_driver_refuses_fading_without_a_constellation_before_any_device(tmp_p
 @gpu
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_channel_faded_equals_the_oracle(q):
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     B = 6
     d = nbldpc.Decoder(code, min(20, q), 25, 10, 0.3, max_batch=B)
@@ -246,7 +210,7 @@ def test_channel_faded_equals_the_oracle(q):
     for mod in (nbldpc.rotate_constellation(nbldpc.constellation(nbldpc.MAP_QAM, q), 11.0), seeded_table(q)):
         d.set_constellation(mod)
         for fading in (nbldpc.FADING_SYMBOL, nbldpc.FADING_COMPONENT):
-            _, rx = _faded_frames(code, 5, B, FADE_ESN[q] - 4, mod, fading)
+            _, _, rx = host_frames(code, 5, B, FADE_ESN[q] - 4, "mapped", mod, fading)
             # channel state the stream never makes: erased (0), negative, large, and -0
             n = rx.shape[0] * rx.shape[1]
             flat = rx.reshape(n, 4)
@@ -272,22 +236,22 @@ def test_channel_faded_equals_the_oracle(q):
 def test_faded_intake_with_unit_amplitudes_is_the_mapped_intake(q):
     """rho = 1: decode_faded equals decode_mapped bit for bit (decisions, syndromes, iterations, LIST and BITS soft output),
     streamed and through upload_faded + run; channel_faded equals channel_mapped"""
-    code, _ = _code(q)
+    code, _ = field_code(q)
     n_m = 16 if q == 16 else 20
-    B = _waves(code, n_m)
+    B = waves(code, n_m)
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=B, frames_per_cta=1)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
     d.set_constellation(mod)
-    _, _, noisy = _host_frames(code, 0, B, ESN[q], mod)
+    _, _, noisy = host_frames(code, 0, B, ESN[q], "mapped", mod)
     rx = np.concatenate([noisy, np.ones_like(noisy)], axis=2)
     sigma = nbldpc.sigma_apsk64(ESN[q])
     for kind, k in ((nbldpc.SOFT_LIST, 4), (nbldpc.SOFT_BITS, 0)):
         d.set_soft_output(kind, k)
-        ref = d.decode_mapped(noisy, sigma); rsoft = _soft(d, kind)
-        got = d.decode_faded(rx, sigma); gsoft = _soft(d, kind)
+        ref = d.decode_mapped(noisy, sigma); rsoft = soft(d, kind)
+        got = d.decode_faded(rx, sigma); gsoft = soft(d, kind)
         assert all((x == y).all() for x, y in zip(got, ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(gsoft, rsoft))
         d.upload_faded(rx, sigma); d.run()
-        assert all((x == y).all() for x, y in zip(d.download(), ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(_soft(d, kind), rsoft))
+        assert all((x == y).all() for x, y in zip(d.download(), ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(soft(d, kind), rsoft))
     assert len(set(ref[2].tolist())) > 1
     a = d.channel_mapped(noisy[:3], sigma, want_sorted=True)
     b = d.channel_faded(rx[:3], sigma, want_sorted=True)
@@ -302,19 +266,19 @@ def test_faded_intake_with_unit_amplitudes_is_the_mapped_intake(q):
 def test_decode_faded_equals_the_oracle(q, early, ecn, fading, erase):
     """decode_faded (streamed) and upload_faded + run on batches of more than two waves, frame for frame against the oracle's
     decode loop on oracle_llr_faded; L-Bubble and the syndrome-based check node; one case with ~10 % erased symbols"""
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     n_m = 16 if q == 16 else 20
     kw = dict(ecn_kind=1, d1=n_m - 1, d2=min(15, n_m - 1), d3=5, cfg_trunc=1000, n_cv=25) if ecn else {}
     cfg = o.build_config_table(int(code.row_deg[0]), n_m - 1, min(15, n_m - 1), 5, 1000) if ecn else None
-    B = _waves(code, n_m, early, **kw)
+    B = waves(code, n_m, early, **kw)
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, early_stop=early, max_batch=B, frames_per_cta=1, **kw)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
     if fading == nbldpc.FADING_COMPONENT:
         mod = nbldpc.rotate_constellation(mod, SSD_DEGREES)
     d.set_constellation(mod)
     ebn = FADE_ESN[q]
-    _, rx = _faded_frames(code, 60, B, ebn, mod, fading)
+    _, _, rx = host_frames(code, 60, B, ebn, "mapped", mod, fading)
     if erase:
         er = np.random.default_rng(3).random(rx.shape[:2]) < 0.1
         rx[er, 2:] = 0.0
@@ -333,31 +297,31 @@ def test_decode_faded_equals_the_oracle(q, early, ecn, fading, erase):
 @gpu
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_generated_faded_frames_equal_the_host_stream(q):
-    code, _ = _code(q)
+    code, _ = field_code(q)
     B = 200
     d = nbldpc.Decoder(code, min(20, q), 25, 10, 0.3, max_batch=B)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
     d.set_constellation(mod)
     for fading in (nbldpc.FADING_SYMBOL, nbldpc.FADING_COMPONENT):
-        D = multigpu.draws_per_frame(code, "mapped", fading=_name(fading))
+        D = multigpu.draws_per_frame(code, "mapped", fading=FADING_NAMES[fading])
         far = (1 << 32) // D + 1000
         for frame0 in (0, 12345, far):
             d.source_frames_faded(frame0, B, FADE_ESN[q], fading)
-            assert _same_faded_stream(d, code, frame0, B, FADE_ESN[q], mod, fading), (fading, frame0)
+            assert same_stream(d, code, frame0, B, FADE_ESN[q], "mapped", mod, fading), (fading, frame0)
         # the widest margin flags many symbols; each is recomputed whole and the stream is unchanged
         base = d.source_fixups()
         d.source_set_margin(2.0 ** -20)
         d.source_frames_faded(7, B, FADE_ESN[q] - 5, fading)
         n = d.source_fixups()
         assert n > max(100, 50 * base) and n > 0.5 * B * code.N, (n, base)
-        assert _same_faded_stream(d, code, 7, B, FADE_ESN[q] - 5, mod, fading)
+        assert same_stream(d, code, 7, B, FADE_ESN[q] - 5, "mapped", mod, fading)
         d.source_set_margin(2.0 ** -46)
     d.close()
 
 
 @gpu
 def test_faded_state_rules():
-    code, _ = _code(64)
+    code, _ = field_code(64)
     B = 32
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=B)
     qam, apsk = nbldpc.constellation(nbldpc.MAP_QAM, 64), nbldpc.apsk64_table()
@@ -375,13 +339,13 @@ def test_faded_state_rules():
         with pytest.raises(nbldpc.NbgpuError) as e:
             d.source_frames_faded(3, B, 20.0, bad)
         assert e.value.code == nbldpc.EINVAL
-    assert _same_faded_stream(d, code, 3, B, 20.0, qam, nbldpc.FADING_SYMBOL)
+    assert same_stream(d, code, 3, B, 20.0, "mapped", qam, nbldpc.FADING_SYMBOL)
     d.run()
     d.source_results()
     # re-binding drops the resident faded batch, generated or uploaded ...
     d.set_soft_output(nbldpc.SOFT_BITS)
     for make in (lambda: d.source_frames_faded(3, B, 20.0, nbldpc.FADING_COMPONENT),
-                 lambda: d.upload_faded(_faded_frames(code, 3, B, 20.0, qam, nbldpc.FADING_SYMBOL)[1], 0.1)):
+                 lambda: d.upload_faded(host_frames(code, 3, B, 20.0, "mapped", qam, nbldpc.FADING_SYMBOL)[2], 0.1)):
         make(); d.run(); d.soft_bits()
         d.set_constellation(qam)
         with pytest.raises(nbldpc.NbgpuError) as e:
@@ -401,7 +365,7 @@ def test_faded_state_rules():
     assert all((x == y).all() for x, y in zip(d.source_results(), ref))
     # BPSK, LLR, 64-APSK, mapped and faded batches alternate on one context
     d.set_constellation(qam)
-    _, _, mn = _host_frames(code, 11, B, 14.0, qam)
+    _, _, mn = host_frames(code, 11, B, 14.0, "mapped", qam)
     llr = d.channel_mapped(mn, nbldpc.sigma_apsk64(14.0))
     rm = d.decode_mapped(mn, nbldpc.sigma_apsk64(14.0))
     for _ in range(2):
@@ -415,7 +379,7 @@ def test_faded_state_rules():
         assert (d.download()[0] == rm[0]).all()
         for fading in (nbldpc.FADING_SYMBOL, nbldpc.FADING_COMPONENT):
             d.source_frames_faded(11, B, 20.0, fading)
-            assert _same_faded_stream(d, code, 11, B, 20.0, qam, fading)
+            assert same_stream(d, code, 11, B, 20.0, "mapped", qam, fading)
             d.run()
             d.source_results()
     d.close()
@@ -424,59 +388,49 @@ def test_faded_state_rules():
 @gpu
 @pytest.mark.parametrize("q,fading", [(16, nbldpc.FADING_SYMBOL), (256, nbldpc.FADING_COMPONENT)])
 def test_soft_output_of_generated_faded_batch_equals_host_frames(q, fading):
-    code, _ = _code(q)
+    code, _ = field_code(q)
     B, ebn = 48, FADE_ESN[q]
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
-    _, rx = _faded_frames(code, 20, B, ebn, mod, fading)
+    _, _, rx = host_frames(code, 20, B, ebn, "mapped", mod, fading)
     sigma = nbldpc.sigma_apsk64(ebn)
     d = nbldpc.Decoder(code, 16, 25, 10, 0.3, max_batch=B)
     d.set_constellation(mod)
     for kind, k in ((nbldpc.SOFT_LIST, 4), (nbldpc.SOFT_BITS, 0)):
         d.set_soft_output(kind, k)
         d.decode_faded(rx, sigma)
-        ref = _soft(d, kind)
+        ref = soft(d, kind)
         d.source_frames_faded(20, B, ebn, fading)
         d.run()
-        assert all(x.tobytes() == y.tobytes() for x, y in zip(_soft(d, kind), ref)), kind
+        assert all(x.tobytes() == y.tobytes() for x, y in zip(soft(d, kind), ref)), kind
     d.close()
-
-
-def _driver(tmp_path, sub, path, ebn, n_m, source, fading, degrees, devices="0"):
-    d = tmp_path / sub
-    os.makedirs(d / "data")
-    r = subprocess.run([EXE, "2000", "10", path, ebn, str(n_m), "0.3", "25", "128", devices, "0", str(source), "2", str(fading), degrees],
-                       cwd=d, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:]
-    lines = list((d / "data").glob("results_*.txt"))[0].read_text().splitlines()
-    return r.stdout, [ln.split("time:")[0] for ln in lines]
 
 
 @gpu
 @pytest.mark.parametrize("q,fading,degrees", [(16, 1, "0"), (256, 2, "3.576")])
 def test_c_driver_faded_sources_contexts_and_monte_carlo_agree(tmp_path, q, fading, degrees):
-    code, path = _code(q)
+    code, path = field_code(q)
     esn, n_m = FADE_ESN[q], (16 if q == 16 else 20)
-    out1, file1 = _driver(tmp_path, "device", path, "%.1f" % esn, n_m, 1, fading, degrees)
-    out0, file0 = _driver(tmp_path, "host", path, "%.1f" % esn, n_m, 0, fading, degrees)
-    out2, file2 = _driver(tmp_path, "two_contexts", path, "%.1f" % esn, n_m, 1, fading, degrees, "0,0")
+    out1, file1 = run_driver(tmp_path, "device", path, "%.1f" % esn, n_m, 1, 2, str(fading), degrees)
+    out0, file0 = run_driver(tmp_path, "host", path, "%.1f" % esn, n_m, 0, 2, str(fading), degrees)
+    out2, file2 = run_driver(tmp_path, "two_contexts", path, "%.1f" % esn, n_m, 1, 2, str(fading), degrees, devices="0,0")
     last = [re.findall(CONSOLE, o)[-1] for o in (out1, out0, out2)]
     assert last[0] == last[1] == last[2], last
     assert file1 == file0 == file2 and len(file1) == 1, (file1, file0, file2)
     mod = nbldpc.rotate_constellation(nbldpc.constellation(nbldpc.MAP_QAM, q), float(degrees))
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=128)
     d.set_constellation(mod)
-    kw = dict(batch=128, channel="mapped", constellation=mod, fading=_name(fading))
+    kw = dict(batch=128, channel="mapped", constellation=mod, fading=FADING_NAMES[fading])
     for st in (multigpu.monte_carlo(code, 2000, esn, decode=d.decode_faded, **kw), multigpu.monte_carlo(code, 2000, esn, decoder=d, **kw)):
         assert (st["undetected"], st["err_frames"], st["frames"], st["bit_errors"], "%.2f" % (st["sum_it"] / st["frames"])) == \
             (int(last[0][0]), int(last[0][1]), int(last[0][2]), int(last[0][3]), last[0][4]), st
     d.close()
     # a two-point sweep equals its single points
     lo = esn - 2
-    out, lines = _driver(tmp_path, "sweep", path, "%.1f:%.1f:2" % (lo, lo + 2), n_m, 1, fading, degrees)
+    out, lines = run_driver(tmp_path, "sweep", path, "%.1f:%.1f:2" % (lo, lo + 2), n_m, 1, 2, str(fading), degrees)
     blocks = out.split("---- Eb/No = ")[1:]
     assert len(blocks) == 2 and len(lines) == 2
     for i in range(2):
-        o1, l1 = _driver(tmp_path, "single%d" % i, path, "%.1f" % (lo + 2 * i), n_m, 1, fading, degrees)
+        o1, l1 = run_driver(tmp_path, "single%d" % i, path, "%.1f" % (lo + 2 * i), n_m, 1, 2, str(fading), degrees)
         assert re.findall(CONSOLE, o1)[-1] == re.findall(CONSOLE, blocks[i])[-1] and l1 == [lines[i]], (i, l1, lines[i])
 
 
@@ -484,7 +438,7 @@ def test_c_driver_faded_sources_contexts_and_monte_carlo_agree(tmp_path, q, fadi
 def test_rayleigh_fading_costs_frames_that_awgn_does_not():
     """on the fixed stream: at the lowest Es/N0 of a 1 dB grid where 256-QAM over AWGN decodes every one of 384 frames, symbol
     fading loses many (on this short code both channels are error-free a few dB higher, so the point is found from below)"""
-    code, _ = _code(256)
+    code, _ = field_code(256)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, 256)
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=128)
     first = 16.0

@@ -11,8 +11,8 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import LABELLINGS, code_arrays, is_closed, labelled_tables, oracle_frames, oracle_with_tables, product_frames
-from test_gpu_mapped import ESN, oracle_llr_mapped
+from common import (ESN, LABELLINGS, code_arrays, is_closed, labelled_tables, oracle_frames, oracle_llr_mapped, oracle_with_tables,
+                    product_frames)
 from test_gpu_parity import _lists, mpath
 from test_gpu_soft_output import ref_bits, ref_list, wave_of
 from test_gpu_source import _host_frames

@@ -1,8 +1,8 @@
 """The mapped channel: one GF(q) symbol sent as one point of a q-point constellation mod[q][2] (nbgpu_constellation,
 nbgpu_set_constellation and the *_mapped calls), for GF(16), GF(64) and GF(256).  64-APSK is the mapped channel on the
 64-APSK table, so with that table every mapped call reproduces its *_apsk64 counterpart bit for bit; with Gray square QAM
-and other tables the results are checked against `oracle_noise_mapped` / `oracle_llr_mapped` below, the table-taking forms
-of the oracle's 64-APSK noise and LLR, which the CPU tests pin to the oracle's own 64-APSK functions on the APSK table."""
+and other tables the results are checked against `oracle_noise_mapped` below and `common.oracle_llr_mapped`, the table-taking
+forms of the oracle's 64-APSK noise and LLR, which the CPU tests pin to the oracle's own 64-APSK functions on the APSK table."""
 import ctypes as C
 import math
 import os
@@ -14,18 +14,10 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import code_path, matrix_path
-from test_gpu_parity import mpath
-
-multigpu = __import__("importlib").import_module("ems-decoder-of-nb-ldpc-codes_b200.multigpu")
+from common import (CONSOLE, ESN, EXE, PI, field_code, host_frames, matrix_path, multigpu, oracle_llr_mapped, run_driver,
+                    same_stream, seeded_table, soft, waves)
 
 gpu = pytest.mark.gpu
-EXE = os.path.join(os.path.dirname(nbldpc.LIB_PATH), "nbldpc_mc")
-CONSOLE = r"<(\d+)> FER=\s*(\d+)\s*/\s*(\d+)\s*=\s*[\d.]+\s*BER=\s*(\d+)\s*/\s*x\s*=\s*[\d.eE+-]+\s*avr_it=([\d.]+)"
-PI = 3.1415926536                                              # channel.c:18
-# one code per field; GF(16) has no matrix file, so a seeded random code stands in (test_gpu_parity.mpath)
-CODES = {16: "synthetic/GF16_N24_M12_dc4", 64: "matrices/N96_K48_GF64", 256: "matrices/KN/N96_K48_GF256.txt"}
-ESN = {16: 10.0, 64: 15.0, 256: 23.0}                          # Es/N0 (dB) at which the QAM frames mix easy and hard ones
 
 
 # ---- the oracle's mapped channel (the 64-APSK functions of oracle/nbldpc_oracle.c with the table as an argument) ----------
@@ -53,48 +45,6 @@ def oracle_noise_mapped(o, nbin, mod, ebn):
             u = float(np.float32(o.drand48())); v = float(np.float32(o.drand48()))
             noisy[n, c] = np.float32(float(mod[som, c]) + sigma * math.sqrt(-2.0 * math.log(u)) * math.cos(2.0 * PI * v))
     return noisy
-
-
-def oracle_llr_mapped(o, noisy, mod, sigma):
-    """channel.c:266-291 on mod: f32 differences and squares, f64 divisions by 2 (float)(sigma^2) and sum, rounded to f32"""
-    img = (o.bingf.astype(np.int64) << np.arange(o.bingf.shape[1])).sum(1)
-    den = 2.0 * float(np.float32(sigma) * np.float32(sigma))
-    d0 = (noisy[:, 0:1].astype(np.float32) - mod[img, 0][None, :]).astype(np.float32)
-    d1 = (noisy[:, 1:2].astype(np.float32) - mod[img, 1][None, :]).astype(np.float32)
-    a = (d0 * d0).astype(np.float64) / den
-    b = (d1 * d1).astype(np.float64) / den
-    return (a + b).astype(np.float32)
-
-
-def seeded_table(q, seed=5):
-    """a table that is neither normalised nor symmetric, with two coincident points"""
-    mod = np.random.default_rng(seed).normal(0, 1.7, (q, 2)).astype(np.float32)
-    mod[3] = mod[1]
-    return mod
-
-
-def _host_frames(code, frame0, B, ebn, mod):
-    code.prepare_encoder()
-    code.rng_default()
-    code.rng_skip(frame0 * multigpu.draws_per_frame(code, "mapped"))
-    cws, bits, noisy = [], [], []
-    for _ in range(B):
-        cw, nbin = code.random_codeword()
-        cws.append(cw); bits.append(nbin)
-        noisy.append(code.noise_mapped(nbin, mod, ebn))
-    return np.stack(cws), np.stack(bits), np.stack(noisy)
-
-
-def _same_stream(d, code, frame0, B, ebn, mod):
-    cw, _, noisy = _host_frames(code, frame0, B, ebn, mod)
-    gcw, gnoisy = d.source_download()
-    assert gnoisy.shape == noisy.shape
-    return (gcw == cw).all() and gnoisy.tobytes() == noisy.tobytes()
-
-
-def _code(q):
-    path = mpath(CODES[q])
-    return nbldpc.Code(path), path
 
 
 # ---- CPU ---------------------------------------------------------------------------------------------------------------
@@ -147,7 +97,7 @@ def test_oracle_mapped_forms_are_the_oracle_apsk64_functions():
 
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_host_mapped_noise_equals_apsk64_and_the_oracle(q):
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     nbin = np.random.default_rng(q).integers(0, 2, (code.N, code.logq)).astype(np.int32)
     tables = [nbldpc.constellation(nbldpc.MAP_QAM, q), seeded_table(q)]
@@ -178,11 +128,11 @@ def test_host_mapped_noise_equals_apsk64_and_the_oracle(q):
 
 
 def test_draws_per_frame_mapped_skips_whole_frames():
-    code, _ = _code(256)
+    code, _ = field_code(256)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, 256)
     D = multigpu.draws_per_frame(code, "mapped")
     assert D == code.K * 8 + 4 * code.N
-    _, _, noisy = _host_frames(code, 0, 7, 20.0, mod)
+    _, _, noisy = host_frames(code, 0, 7, 20.0, "mapped", mod)
     for f in (1, 3, 6):
         code.rng_default(); code.rng_skip(f * D)
         _, nb = code.random_codeword()
@@ -215,14 +165,14 @@ def test_mapped_abi_without_a_gpu():
 @gpu
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_channel_mapped_equals_the_oracle(q):
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     B = 6
     d = nbldpc.Decoder(code, min(20, q), 25, 10, 0.3, max_batch=B)
     tables = [nbldpc.constellation(nbldpc.MAP_QAM, q), seeded_table(q)] + ([nbldpc.apsk64_table()] if q == 64 else [])
     for mod in tables:
         d.set_constellation(mod)
-        _, _, noisy = _host_frames(code, 3, B, ESN[q] - 3, mod)
+        _, _, noisy = host_frames(code, 3, B, ESN[q] - 3, "mapped", mod)
         sigma = nbldpc.sigma_apsk64(ESN[q] - 3)
         llr, il, ig = d.channel_mapped(noisy, sigma, want_sorted=True)
         for f in range(B):
@@ -236,30 +186,23 @@ def test_channel_mapped_equals_the_oracle(q):
     d.close(); o.close()
 
 
-def _soft(d, kind):
-    return d.soft_list() if kind == nbldpc.SOFT_LIST else (d.soft_bits(),)
-
-
 @gpu
 @pytest.mark.parametrize("early", [True, False])
 def test_decode_mapped_with_the_apsk_table_equals_decode_apsk64(early):
-    code, _ = _code(64)
+    code, _ = field_code(64)
     mod = nbldpc.apsk64_table()
-    d = nbldpc.Decoder(code, 20, 25, 10, 0.3, early_stop=early, max_batch=1 << 14, frames_per_cta=1)
-    g = d.geometry()
-    B = 2 * g["grid"] * g["frames_per_cta"] + 37              # more than two waves: streamed path and slot reuse
-    d.close()
+    B = waves(code, 20, early)
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, early_stop=early, max_batch=B, frames_per_cta=1)
     d.set_constellation(mod)
-    _, _, noisy = _host_frames(code, 0, B, 8.0, mod)
+    _, _, noisy = host_frames(code, 0, B, 8.0, "mapped", mod)
     sigma = nbldpc.sigma_apsk64(8.0)
     for kind, k in ((nbldpc.SOFT_LIST, 4), (nbldpc.SOFT_BITS, 0)):
         d.set_soft_output(kind, k)
-        ref = d.decode_apsk64(noisy, sigma); rsoft = _soft(d, kind)
-        got = d.decode_mapped(noisy, sigma); gsoft = _soft(d, kind)
+        ref = d.decode_apsk64(noisy, sigma); rsoft = soft(d, kind)
+        got = d.decode_mapped(noisy, sigma); gsoft = soft(d, kind)
         assert all((x == y).all() for x, y in zip(got, ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(gsoft, rsoft))
         d.upload_mapped(noisy, sigma); d.run()
-        assert all((x == y).all() for x, y in zip(d.download(), ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(_soft(d, kind), rsoft))
+        assert all((x == y).all() for x, y in zip(d.download(), ref)) and all(x.tobytes() == y.tobytes() for x, y in zip(soft(d, kind), rsoft))
     if early:
         assert len(set(ref[2].tolist())) > 1
     d.close()
@@ -270,20 +213,17 @@ def test_decode_mapped_with_the_apsk_table_equals_decode_apsk64(early):
 def test_decode_mapped_qam_equals_the_oracle(q, early, ecn):
     """decode_mapped (streamed) and upload_mapped + run (resident) on batches of more than two waves, frame for frame
     against the oracle's decode loop on the oracle's mapped LLRs; L-Bubble and the syndrome-based check node"""
-    code, path = _code(q)
+    code, path = field_code(q)
     o = ol.Oracle(path, code.dialect)
     n_m = 16 if q == 16 else 20
     kw = dict(ecn_kind=1, d1=n_m - 1, d2=min(15, n_m - 1), d3=5, cfg_trunc=1000, n_cv=25) if ecn else {}
     cfg = o.build_config_table(int(code.row_deg[0]), n_m - 1, min(15, n_m - 1), 5, 1000) if ecn else None
-    d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, early_stop=early, max_batch=1 << 14, frames_per_cta=1, **kw)
-    g = d.geometry()
-    B = 2 * g["grid"] * g["frames_per_cta"] + 37
-    d.close()
+    B = waves(code, n_m, early, **kw)
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, early_stop=early, max_batch=B, frames_per_cta=1, **kw)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
     d.set_constellation(mod)
     ebn = ESN[q]
-    _, _, noisy = _host_frames(code, 40, B, ebn, mod)
+    _, _, noisy = host_frames(code, 40, B, ebn, "mapped", mod)
     sigma = nbldpc.sigma_apsk64(ebn)
     dec, synd, it = d.decode_mapped(noisy, sigma)
     d.upload_mapped(noisy, sigma); d.run()
@@ -306,7 +246,7 @@ def _far(code):
 @gpu
 @pytest.mark.parametrize("q", [16, 64, 256])
 def test_generated_mapped_frames_equal_the_host_stream(q):
-    code, _ = _code(q)
+    code, _ = field_code(q)
     B = 200
     d = nbldpc.Decoder(code, min(20, q), 25, 10, 0.3, max_batch=B)
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
@@ -314,7 +254,7 @@ def test_generated_mapped_frames_equal_the_host_stream(q):
     for frame0 in (0, 12345, _far(code)):
         for ebn in (ESN[q] - 3, ESN[q]):
             d.source_frames_mapped(frame0, B, ebn)
-            assert _same_stream(d, code, frame0, B, ebn, mod), (frame0, ebn)
+            assert same_stream(d, code, frame0, B, ebn, "mapped", mod), (frame0, ebn)
     if q == 64:                                                # the APSK table bound: the 64-APSK stream
         d.set_constellation(nbldpc.apsk64_table())
         for frame0 in (0, _far(code)):
@@ -328,25 +268,25 @@ def test_generated_mapped_frames_equal_the_host_stream(q):
 
 @gpu
 def test_flagged_mapped_samples_are_recomputed_with_the_batch_table():
-    code, _ = _code(256)
+    code, _ = field_code(256)
     B, ebn = 64, 20.0
     mod = nbldpc.constellation(nbldpc.MAP_QAM, 256)
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=B)
     d.set_constellation(mod)
     d.source_frames_mapped(7, B, ebn)
     base = d.source_fixups()
-    assert _same_stream(d, code, 7, B, ebn, mod)
+    assert same_stream(d, code, 7, B, ebn, "mapped", mod)
     d.source_set_margin(2.0 ** -20)
     d.source_frames_mapped(7, B, ebn)
     n = d.source_fixups()
     assert n > max(100, 50 * base) and n > 0.6 * B * code.N * 2, (n, base)
-    assert _same_stream(d, code, 7, B, ebn, mod)
+    assert same_stream(d, code, 7, B, ebn, "mapped", mod)
     d.close()
 
 
 @gpu
 def test_mapped_state_rules():
-    code, _ = _code(64)
+    code, _ = field_code(64)
     B = 32
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=B)
     qam, apsk = nbldpc.constellation(nbldpc.MAP_QAM, 64), nbldpc.apsk64_table()
@@ -369,7 +309,7 @@ def test_mapped_state_rules():
     d.source_frames_mapped(3, B, 14.0)
     with pytest.raises(nbldpc.NbgpuError):
         d.set_constellation(np.full((64, 2), -np.inf, np.float32))
-    assert _same_stream(d, code, 3, B, 14.0, qam)
+    assert same_stream(d, code, 3, B, 14.0, "mapped", qam)
     d.run()
     d.source_results()
     # re-binding drops the resident mapped batch ...
@@ -400,9 +340,9 @@ def test_mapped_state_rules():
         _, a = d.source_download()
         assert a.shape == (B, code.N, 2)
         d.source_frames_mapped(11, B, 14.0)
-        assert _same_stream(d, code, 11, B, 14.0, qam)
+        assert same_stream(d, code, 11, B, 14.0, "mapped", qam)
     # with QAM bound, decode_apsk64 still uses the APSK table
-    _, _, an = _host_frames(code, 0, B, 8.0, apsk)
+    _, _, an = host_frames(code, 0, B, 8.0, "mapped", apsk)
     sigma = nbldpc.sigma_apsk64(8.0)
     r1 = d.decode_apsk64(an, sigma)
     d.set_constellation(apsk)
@@ -415,43 +355,56 @@ def test_mapped_state_rules():
 
 
 @gpu
+def test_source_download_refuses_a_generated_batch_an_upload_replaced():
+    """an upload or a decode overwrites the generated samples: nbgpu_source_download refuses (NBGPU_ESTATE) instead of returning
+    the old codewords beside the new samples; a batch that nbgpu_set_constellation dropped keeps its samples"""
+    code, _ = field_code(64)
+    B = 16
+    d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=B)
+    qam = nbldpc.constellation(nbldpc.MAP_QAM, 64)
+    d.set_constellation(qam)
+    for replace in (lambda: d.upload_noisy(np.zeros((B, code.N, code.logq), np.float32), 0.5),
+                    lambda: d.decode_mapped(np.zeros((B, code.N, 2), np.float32), 0.5),
+                    lambda: d.decode_llr(np.zeros((B, code.N, code.q), np.float32))):
+        d.source_frames(3, B, 3.0)
+        replace()
+        with pytest.raises(nbldpc.NbgpuError) as e:
+            d.source_download()
+        assert e.value.code == nbldpc.ESTATE
+    d.source_frames_mapped(3, B, 14.0)
+    d.set_constellation(qam)
+    assert same_stream(d, code, 3, B, 14.0, "mapped", qam)
+    d.close()
+
+
+@gpu
 @pytest.mark.parametrize("q", [16, 256])
 def test_soft_output_of_generated_mapped_batch_equals_host_frames(q):
-    code, _ = _code(q)
+    code, _ = field_code(q)
     B, ebn = 48, ESN[q]
     mod = nbldpc.constellation(nbldpc.MAP_QAM, q)
-    _, _, noisy = _host_frames(code, 20, B, ebn, mod)
+    _, _, noisy = host_frames(code, 20, B, ebn, "mapped", mod)
     sigma = nbldpc.sigma_apsk64(ebn)
     d = nbldpc.Decoder(code, 16, 25, 10, 0.3, max_batch=B)
     d.set_constellation(mod)
     for kind, k in ((nbldpc.SOFT_LIST, 4), (nbldpc.SOFT_BITS, 0)):
         d.set_soft_output(kind, k)
         d.decode_mapped(noisy, sigma)
-        ref = _soft(d, kind)
+        ref = soft(d, kind)
         d.source_frames_mapped(20, B, ebn)
         d.run()
-        assert all(x.tobytes() == y.tobytes() for x, y in zip(_soft(d, kind), ref)), kind
+        assert all(x.tobytes() == y.tobytes() for x, y in zip(soft(d, kind), ref)), kind
     d.close()
-
-
-def _driver(tmp_path, sub, path, ebn, source, devices="0"):
-    d = tmp_path / sub
-    os.makedirs(d / "data")
-    r = subprocess.run([EXE, "2000", "10", path, ebn, "16", "0.3", "25", "128", devices, "0", str(source), "2"],
-                       cwd=d, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:]
-    lines = list((d / "data").glob("results_*.txt"))[0].read_text().splitlines()
-    return r.stdout, [ln.split("time:")[0] for ln in lines]
 
 
 @gpu
 @pytest.mark.parametrize("q", [16, 256])
 def test_c_driver_qam_sources_contexts_and_monte_carlo_agree(tmp_path, q):
-    code, path = _code(q)
+    code, path = field_code(q)
     ebn = "%.1f" % ESN[q]
-    out1, file1 = _driver(tmp_path, "device", path, ebn, 1)
-    out0, file0 = _driver(tmp_path, "host", path, ebn, 0)
-    out2, file2 = _driver(tmp_path, "two_contexts", path, ebn, 1, "0,0")
+    out1, file1 = run_driver(tmp_path, "device", path, ebn, 16, 1, 2)
+    out0, file0 = run_driver(tmp_path, "host", path, ebn, 16, 0, 2)
+    out2, file2 = run_driver(tmp_path, "two_contexts", path, ebn, 16, 1, 2, devices="0,0")
     last = [re.findall(CONSOLE, o)[-1] for o in (out1, out0, out2)]
     assert last[0] == last[1] == last[2], last
     assert file1 == file0 == file2 and len(file1) == 1, (file1, file0, file2)
@@ -465,9 +418,9 @@ def test_c_driver_qam_sources_contexts_and_monte_carlo_agree(tmp_path, q):
     d.close()
     # an Es/N0 sweep equals its single points
     lo = ESN[q] - 1
-    out, lines = _driver(tmp_path, "sweep", path, "%.1f:%.1f:1" % (lo, lo + 1), 1)
+    out, lines = run_driver(tmp_path, "sweep", path, "%.1f:%.1f:1" % (lo, lo + 1), 16, 1, 2)
     blocks = out.split("---- Eb/No = ")[1:]
     assert len(blocks) == 2 and len(lines) == 2
     for i in range(2):
-        o1, l1 = _driver(tmp_path, "single%d" % i, path, "%.1f" % (lo + i), 1)
+        o1, l1 = run_driver(tmp_path, "single%d" % i, path, "%.1f" % (lo + i), 16, 1, 2)
         assert re.findall(CONSOLE, o1)[-1] == re.findall(CONSOLE, blocks[i])[-1] and l1 == [lines[i]], (i, l1, lines[i])

@@ -8,28 +8,12 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import (Golden, code_path, golden_names, matrix_path, oracle_frames, product_frames, random_regular_code, sha,
+from common import (Golden, code_path, golden_names, matrix_path, mpath, oracle_frames, product_frames, random_regular_code, sha,
                     write_alist_ubs)
 
 pytestmark = pytest.mark.gpu
 
 Q_CODES = {16: "synthetic/GF16_N32_M8_dc8", 64: "matrices/N96_K48_GF64", 256: "matrices/KN/N96_K48_GF256.txt"}
-_SYN = {}
-
-
-def mpath(rel):
-    """reference matrices, plus small synthetic GF(16) codes (the only GF(16) matrix of the reference is the 64800-bit one)"""
-    if not rel.startswith("synthetic/"):
-        return code_path(rel)
-    if rel not in _SYN:
-        import re
-        import tempfile
-        q, N, M, dc = [int(x) for x in re.match(r"synthetic/GF(\d+)_N(\d+)_M(\d+)_dc(\d+)", rel).groups()]
-        a = random_regular_code(np.random.default_rng(q + N + dc), N, M, q, dc)
-        path = os.path.join(tempfile.mkdtemp(prefix="nbldpc_syn_"), rel.split("/")[1])
-        write_alist_ubs(path, a)
-        _SYN[rel] = path
-    return _SYN[rel]
 
 
 def _dec(rel, n_m, nb_oper=25, nb_iter_max=10, offset=0.3, **kw):

@@ -11,32 +11,9 @@ import pytest
 
 import nbldpc
 import oracle_lib as ol
-from common import code_path, matrix_path
-
-multigpu = __import__("importlib").import_module("ems-decoder-of-nb-ldpc-codes_b200.multigpu")
+from common import CONSOLE, EXE, code_path, host_frames, matrix_path, multigpu, run_driver, same_stream
 
 gpu = pytest.mark.gpu
-EXE = os.path.join(os.path.dirname(nbldpc.LIB_PATH), "nbldpc_mc")
-CONSOLE = r"<(\d+)> FER=\s*(\d+)\s*/\s*(\d+)\s*=\s*[\d.]+\s*BER=\s*(\d+)\s*/\s*x\s*=\s*[\d.eE+-]+\s*avr_it=([\d.]+)"
-
-
-def _host_frames(code, frame0, B, ebn, channel="apsk64"):
-    code.prepare_encoder()
-    code.rng_default()
-    code.rng_skip(frame0 * multigpu.draws_per_frame(code, channel))
-    cws, bits, noisy = [], [], []
-    for _ in range(B):
-        cw, nbin = code.random_codeword()
-        cws.append(cw); bits.append(nbin)
-        noisy.append(code.noise_apsk64(nbin, ebn) if channel == "apsk64" else code.noise(nbin, ebn))
-    return np.stack(cws), np.stack(bits), np.stack(noisy)
-
-
-def _same_stream(d, code, frame0, B, ebn, channel="apsk64"):
-    cw, _, noisy = _host_frames(code, frame0, B, ebn, channel)
-    gcw, gnoisy = d.source_download()
-    assert gnoisy.shape == noisy.shape
-    return (gcw == cw).all() and gnoisy.tobytes() == noisy.tobytes()
 
 
 # ---- CPU ---------------------------------------------------------------------------------------------------------------
@@ -46,7 +23,7 @@ def test_draws_per_frame_apsk64_skips_whole_frames():
     D = multigpu.draws_per_frame(code, "apsk64")
     assert D == 6 * code.K + 4 * code.N
     ebn = 7.0
-    cw, _, noisy = _host_frames(code, 0, 9, ebn)
+    cw, _, noisy = host_frames(code, 0, 9, ebn, "apsk64")
     for f in (1, 4, 8):
         code.rng_default()
         code.rng_skip(f * D)
@@ -79,7 +56,7 @@ def test_generated_apsk64_frames_equal_the_host_stream(rel):
     for frame0 in (0, 12345, far):
         for ebn in (6.0, 9.5):
             d.source_frames_apsk64(frame0, B, ebn)
-            assert _same_stream(d, code, frame0, B, ebn), (frame0, ebn)
+            assert same_stream(d, code, frame0, B, ebn, "apsk64"), (frame0, ebn)
     d.close()
 
 
@@ -91,12 +68,12 @@ def test_flagged_apsk64_samples_are_recomputed_by_the_host():
     d = nbldpc.Decoder(code, 16, 25, 10, 0.3, max_batch=B)
     d.source_frames_apsk64(7, B, ebn)
     base = d.source_fixups()
-    assert _same_stream(d, code, 7, B, ebn)
+    assert same_stream(d, code, 7, B, ebn, "apsk64")
     d.source_set_margin(2.0 ** -20)
     d.source_frames_apsk64(7, B, ebn)
     n = d.source_fixups()
     assert n > max(100, 50 * base) and n > 0.6 * B * code.N * 2, (n, base)   # > 60 %: both I and Q samples were flagged
-    assert _same_stream(d, code, 7, B, ebn)
+    assert same_stream(d, code, 7, B, ebn, "apsk64")
     d.close()
 
 
@@ -124,7 +101,7 @@ def test_apsk64_results_equal_the_host_driven_run(rel, ebn):
     iters = set()
     for f0 in range(0, frames, batch):
         B = min(batch, frames - f0)
-        cw, bits, noisy = _host_frames(code, f0, B, ebn)
+        cw, bits, noisy = host_frames(code, f0, B, ebn, "apsk64")
         dec, synd, it = d.decode_apsk64(noisy, sigma)
         err = np.array([(bing[dec[i, :code.K]] != bits[i][:code.K]).sum() for i in range(B)])
         d.source_frames_apsk64(f0, B, ebn)
@@ -150,11 +127,11 @@ def test_bpsk_and_apsk64_batches_alternate_on_one_context():
     B = 64
     d = nbldpc.Decoder(code, 20, 25, 10, 0.3, max_batch=B)
     d.source_frames(5, B, 3.0)
-    assert _same_stream(d, code, 5, B, 3.0, "bpsk")
+    assert same_stream(d, code, 5, B, 3.0, "bpsk")
     d.source_frames_apsk64(5, B, 8.0)
-    assert _same_stream(d, code, 5, B, 8.0)
+    assert same_stream(d, code, 5, B, 8.0, "apsk64")
     d.source_frames(900, B, 2.5)
-    assert _same_stream(d, code, 900, B, 2.5, "bpsk")
+    assert same_stream(d, code, 900, B, 2.5, "bpsk")
     # a later upload replaces the generated batch
     d.source_frames_apsk64(70, B, 8.0)
     d.run()
@@ -168,7 +145,7 @@ def test_bpsk_and_apsk64_batches_alternate_on_one_context():
         d.source_frames_apsk64(0, B + 1, 8.0)
     assert e.value.code == nbldpc.EINVAL
     d.source_frames_apsk64(11, B, 8.5)
-    assert _same_stream(d, code, 11, B, 8.5)
+    assert same_stream(d, code, 11, B, 8.5, "apsk64")
     d.close()
     # another field than GF(64): refused with the intake's wording, the context still generates BPSK frames
     c256 = nbldpc.Code(matrix_path("matrices/KN/N96_K48_GF256.txt"))
@@ -177,7 +154,7 @@ def test_bpsk_and_apsk64_batches_alternate_on_one_context():
         d.source_frames_apsk64(0, 8, 8.0)
     assert e.value.code == nbldpc.EINVAL and "q = 256" in str(e.value)
     d.source_frames(3, 8, 3.0)
-    assert _same_stream(d, c256, 3, 8, 3.0, "bpsk")
+    assert same_stream(d, c256, 3, 8, 3.0, "bpsk")
     d.close()
 
 
@@ -185,7 +162,7 @@ def test_bpsk_and_apsk64_batches_alternate_on_one_context():
 def test_soft_output_of_generated_apsk64_batch_equals_host_frames():
     code = nbldpc.Code(code_path("matrices/N96_K48_GF64"))
     B, ebn, n_m = 48, 8.0, 16
-    _, _, noisy = _host_frames(code, 20, B, ebn)
+    _, _, noisy = host_frames(code, 20, B, ebn, "apsk64")
     sigma = nbldpc.sigma_apsk64(ebn)
     d = nbldpc.Decoder(code, n_m, 25, 10, 0.3, max_batch=B)
     for kind, k in ((nbldpc.SOFT_LIST, 4), (nbldpc.SOFT_BITS, 0)):
@@ -200,13 +177,7 @@ def test_soft_output_of_generated_apsk64_batch_equals_host_frames():
 
 
 def _driver(tmp_path, sub, ebn, source, devices="0"):
-    d = tmp_path / sub
-    os.makedirs(d / "data")
-    r = subprocess.run([EXE, "2000", "10", code_path("matrices/N96_K48_GF64"), ebn, "20", "0.3", "25", "128", devices, "0", str(source), "1"],
-                       cwd=d, stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-2000:]
-    lines = list((d / "data").glob("results_*.txt"))[0].read_text().splitlines()
-    return r.stdout, [ln.split("time:")[0] for ln in lines]
+    return run_driver(tmp_path, sub, code_path("matrices/N96_K48_GF64"), ebn, 20, source, 1, devices=devices)
 
 
 @gpu
