@@ -75,6 +75,28 @@ def constellation(kind, q):
     return mod
 
 
+def split_qam(q, points):
+    """nbgpu_split_qam: the Gray square QAM table mod[M][2], M = 2^(log2(q)/points), by sub-image, of the split channel: (16, 2),
+    (64, 3) and (256, 4) give QPSK, (256, 2) gives 16-QAM; other pairs are refused (bind your own table)."""
+    M = 1 << ((q.bit_length() - 1) // points) if points > 0 else 0
+    mod = np.zeros((max(M, 1), 2), np.float32)
+    _check(lib().nbgpu_split_qam(q, points, mod.ctypes.data_as(_fp)))
+    return mod
+
+
+def _split_table(logq, mod, points):
+    """mod as the [M][2] f32 table the split calls read, M = 2^(logq / points): a table of another size is a ValueError (the
+    library reads exactly 2M floats).  For a points value the library refuses (NBGPU_EINVAL) it reads none, and mod passes
+    through flattened."""
+    m = np.ascontiguousarray(mod, np.float32)
+    if points < 2 or logq % points:
+        return m.reshape(-1, 2)
+    M = 1 << (logq // points)
+    if m.size != 2 * M:
+        raise ValueError("split table for %d points per GF(%d) symbol must be [%d][2], not %s" % (points, 1 << logq, M, m.shape))
+    return m.reshape(M, 2)
+
+
 def rotate_constellation(mod, degrees):
     """nbgpu_rotate_constellation: mod[q][2] rotated by `degrees` (computed in double, rounded once), e.g. for signal-space
     diversity under NBGPU_FADING_COMPONENT."""
@@ -126,6 +148,12 @@ def lib():
         "nbgpu_channel_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
         "nbgpu_decode_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
         "nbgpu_upload_faded": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
+        "nbgpu_split_qam": (C.c_int, [C.c_int, C.c_int, _fp]),
+        "nbgpu_awgn_split_noise": (C.c_int, [vp, C.POINTER(Rng), _ip, C.c_int, _fp, C.c_float, _fp]),
+        "nbgpu_set_split_constellation": (C.c_int, [vp, C.c_int, _fp]),
+        "nbgpu_channel_split": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
+        "nbgpu_decode_split": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
+        "nbgpu_upload_split": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
         "nbgpu_create": (C.c_int, [C.POINTER(vp), vp, C.POINTER(Params), C.c_int, C.c_int]),
         "nbgpu_destroy": (None, [vp]),
         "nbgpu_last_error": (C.c_char_p, [vp]),
@@ -153,6 +181,7 @@ def lib():
         "nbgpu_source_frames_apsk64": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_frames_mapped": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_frames_faded": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float, C.c_int]),
+        "nbgpu_source_frames_split": (C.c_int, [vp, vp, C.POINTER(Rng), C.c_uint64, C.c_int, C.c_float]),
         "nbgpu_source_download": (C.c_int, [vp, _ip, _fp]),
         "nbgpu_source_results": (C.c_int, [vp, _ip, _ip, _ip]),
         "nbgpu_source_fixups": (C.c_long, [vp]),
@@ -273,6 +302,13 @@ class Code:
         m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
         return self._noise(lib().nbgpu_awgn_faded_noise, nbin, 4, _f(m), C.c_float(ebn), int(fading))
 
+    def noise_split(self, nbin, mod, points, ebn):
+        """nbgpu_awgn_split_noise: one frame of the split channel, each symbol sent as `points` points of mod[M][2] (by
+        sub-image), noisy[N][points][2]; 4*N*points draws, sigma_apsk64(ebn)."""
+        m = _split_table(self.logq, mod, int(points))
+        out = self._noise(lib().nbgpu_awgn_split_noise, nbin, 2 * points, C.c_int(points), _f(m), C.c_float(ebn))
+        return out.reshape(self.N, points, 2)
+
     def accumulate_stats(self, codeword_bits, decide, synd, iters, stats):
         cb = np.ascontiguousarray(codeword_bits, np.int32)
         d = np.ascontiguousarray(decide, np.int32)
@@ -308,7 +344,8 @@ class Decoder:
         _check(lib().nbgpu_create(C.byref(self.h), code.h, C.byref(self.p), device, max_batch))
         self.B = 0
         self.soft_k = 0
-        self._source_fps = 0                                  # floats per symbol of the generated batch
+        self._source_shape = ()                               # shape of one symbol of the generated batch
+        self.split_points = 0                                 # points per symbol of the bound split table
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
@@ -374,6 +411,31 @@ class Decoder:
     def upload_faded(self, rx, sigma):
         self._upload(lib().nbgpu_upload_faded, rx, 4, sigma)
 
+    def set_split_constellation(self, mod, points):
+        """nbgpu_set_split_constellation: bind mod[M][2] (by sub-image), M = 2^(log2(q)/points), to the *_split calls."""
+        m = _split_table(self.code.logq, mod, int(points))
+        _check(lib().nbgpu_set_split_constellation(self.h, int(points), _f(m)), self.h)
+        self.split_points = int(points)
+
+    def _split_frames(self, noisy):
+        """(frames, floats per symbol) of a split call: frames must be [B, N, P, 2] for the bound P.  Nothing bound: the library
+        refuses the call (NBGPU_ESTATE)."""
+        x = np.asarray(noisy)
+        P = self.split_points
+        if P and (x.ndim != 4 or x.shape[1:] != (self.code.N, P, 2)):
+            raise ValueError("split frames must be [B, %d, %d, 2] for the bound table, not %s" % (self.code.N, P, x.shape))
+        return x, 2 * max(P, 1)
+
+    def decode_split(self, noisy, sigma):
+        """nbgpu_decode_split: frames received as samples [B, N, P, 2] of the bound split table."""
+        return self._decode(lib().nbgpu_decode_split, *self._split_frames(noisy), sigma)
+
+    def channel_split(self, noisy, sigma, want_sorted=False):
+        return self._channel(lib().nbgpu_channel_split, *self._split_frames(noisy), sigma, want_sorted)
+
+    def upload_split(self, noisy, sigma):
+        self._upload(lib().nbgpu_upload_split, *self._split_frames(noisy), sigma)
+
     def decode_noisy_into(self, noisy, sigma, out):
         """nbgpu_decode_noisy on caller-owned (e.g. pinned) buffers, no allocation: noisy [B,N,logq] f32, out = (decide, synd, iters)."""
         B = noisy.shape[0]
@@ -404,36 +466,41 @@ class Decoder:
     def source_frames(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames: frames [frame0, frame0+B) of the reference's stream generated on the device and left resident
         (origin: drand48 state before frame 0 as an int, default = the reference's unseeded stream)."""
-        self._source(lib().nbgpu_source_frames, self.code.logq, frame0, B, ebn, origin)
+        self._source(lib().nbgpu_source_frames, (self.code.logq,), frame0, B, ebn, origin)
 
     def source_frames_apsk64(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames_apsk64: the same for a GF(64) code sent as 64-APSK symbols (ModelChannel_AWGN_64); the batch is
         resident as after an upload of noisy[B, N, 2] samples."""
-        self._source(lib().nbgpu_source_frames_apsk64, 2, frame0, B, ebn, origin)
+        self._source(lib().nbgpu_source_frames_apsk64, (2,), frame0, B, ebn, origin)
 
     def source_frames_mapped(self, frame0, B, ebn, origin=None):
         """nbgpu_source_frames_mapped: the same for a code sent on the bound constellation; D = K log2(q) + 4N draws per frame."""
-        self._source(lib().nbgpu_source_frames_mapped, 2, frame0, B, ebn, origin)
+        self._source(lib().nbgpu_source_frames_mapped, (2,), frame0, B, ebn, origin)
 
     def source_frames_faded(self, frame0, B, ebn, fading, origin=None):
         """nbgpu_source_frames_faded: the same for the faded mapped channel on the bound constellation (fading = FADING_SYMBOL
         or FADING_COMPONENT); source_download then returns rx [B, N, 4]."""
-        self._source(lib().nbgpu_source_frames_faded, 4, frame0, B, ebn, origin, int(fading))
+        self._source(lib().nbgpu_source_frames_faded, (4,), frame0, B, ebn, origin, int(fading))
 
-    def _source(self, fn, fps, frame0, B, ebn, origin, *extra):
+    def source_frames_split(self, frame0, B, ebn, origin=None):
+        """nbgpu_source_frames_split: the same for the split channel on the bound split table; D = K log2(q) + 4NP draws per
+        frame; source_download then returns noisy [B, N, P, 2]."""
+        self._source(lib().nbgpu_source_frames_split, (self.split_points, 2), frame0, B, ebn, origin)
+
+    def _source(self, fn, shape, frame0, B, ebn, origin, *extra):
         r = Rng()
         lib().nbgpu_rng_reference_default(C.byref(r))
         if origin is not None:
             r.x = origin
         _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn), *extra), self.h)
         self.B = B
-        self._source_fps = fps
+        self._source_shape = shape
 
     def source_download(self, want_noisy=True):
         """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped,
-        [B, N, 4] for faded"""
+        [B, N, 4] for faded, [B, N, P, 2] for split"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        noisy = np.zeros((self.B, self.code.N, self._source_fps), np.float32) if want_noisy else None
+        noisy = np.zeros((self.B, self.code.N) + self._source_shape, np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy
 

@@ -46,9 +46,9 @@
 
 #define UNIT_NT 256       /* block size of the small unit-boundary kernels */
 
-/* what the intake reads per variable (KArgs::input_kind): BPSK samples [logq], a dense LLR row [q], mapped (I, Q) samples [2]
- * or faded (I, Q, rho_I, rho_Q) [4]; the mapped and faded intakes read KArgs::mod */
-enum InputKind { INPUT_BPSK = 0, INPUT_LLR = 1, INPUT_MAPPED = 2, INPUT_FADED = 3 };
+/* what the intake reads per variable (KArgs::input_kind): BPSK samples [logq], a dense LLR row [q], mapped (I, Q) samples [2],
+ * faded (I, Q, rho_I, rho_Q) [4] or split (I, Q) samples of P points [P][2]; the mapped, faded and split intakes read KArgs::mod */
+enum InputKind { INPUT_BPSK = 0, INPUT_LLR = 1, INPUT_MAPPED = 2, INPUT_FADED = 3, INPUT_SPLIT = 4 };
 
 struct KArgs {
     int N, M, E, q, logq, dc_max, dc_min;
@@ -63,7 +63,7 @@ struct KArgs {
     const uint32_t *einfo;              /* [E] variable | coefficient << 20 | last-visit flag << 28 */
     const int *row_ptr, *col;
     const uint8_t *hval, *rotin, *rotout, *img, *inv;
-    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, INPUT_MAPPED and INPUT_FADED (set per launch) */
+    const float *mod;                   /* [q][2] constellation of the launch's batch by binary image, INPUT_MAPPED and INPUT_FADED; [M][2] by sub-image, INPUT_SPLIT (set per launch) */
     int gf_closed;
     const float *in;
     float *app; uint8_t *ctov; uint8_t *dec;
@@ -91,6 +91,8 @@ struct KArgs {
     /* soft output (nbgpu_set_soft_output), read by decode_kernel<..., SOFT = true> only.  Kept at the end of the struct so
      * that the fields above keep their parameter offsets in every kernel. */
     int soft_kind, soft_k;              /* NBGPU_SOFT_LIST with k symbols per variable, or NBGPU_SOFT_BITS (k = 0)  */
+    int split_p;                        /* INPUT_SPLIT: points per symbol (set per launch).  In the alignment gap in front of
+                                           soft_llr: KArgs keeps its size, so the parameters behind it keep their offsets too */
     float *soft_llr;                    /* [B][N][k] (LIST) or [B][N][logq] (BITS)                                  */
     uint8_t *soft_sym;                  /* [B][N][k] symbols (LIST)                                                 */
 };
@@ -284,6 +286,33 @@ __device__ __forceinline__ void intake_mapped(const float4 s, double den, const 
         const double a = __ddiv_rn((double)__fmul_rn(d0, d0), den), b = __ddiv_rn((double)__fmul_rn(d1, d1), den);
         v[j] = __double2float_rn(__dadd_rn(a, b));
     }
+}
+/* LLR intake for one variable of the split channel (include/nbldpc_b200.h, nbgpu_split_qam): P points of M = 2^m points each,
+ * pts = the variable's [P][2] samples.  Lane l < P*M computes t_{l/M}[l%M] = (double)(dI^2)/den + (double)(dQ^2)/den (f32
+ * differences and squares, f64 divisions and sum) into t (32 doubles of warp scratch); then every symbol adds its P entries in
+ * f64, j = 0 ... P-1, and rounds once.  2*P*M <= 64 f64 divisions per variable instead of the mapped intake's 2q. */
+template <int Q>
+__device__ __forceinline__ void intake_split(const float *pts, int P, double den, const float *mod, const uint8_t *img, int lane,
+                                             double *t, float (&v)[QTraits<Q>::VPL])
+{
+    /* opaque: m and mask are computed here instead of being hoisted into the callers' loops (channel_kernel<16>: 47 -> 40 registers) */
+    asm volatile("" : "+r"(P));
+    const int m = QTraits<Q>::LOGQ / P, mask = (1 << m) - 1;
+    if (lane < P << m) {
+        const int x = lane & mask, j = lane >> m;
+        const float dI = __fsub_rn(pts[2 * j], mod[2 * x]), dQ = __fsub_rn(pts[2 * j + 1], mod[2 * x + 1]);
+        t[lane] = __dadd_rn(__ddiv_rn((double)__fmul_rn(dI, dI), den), __ddiv_rn((double)__fmul_rn(dQ, dQ), den));
+    }
+    __syncwarp();
+#pragma unroll
+    for (int k = 0; k < QTraits<Q>::VPL; k++) {
+        if (Q < 32 && lane >= Q) { v[k] = 0.0f; continue; }
+        const int im = img[QTraits<Q>::sym(lane, k)];
+        double s = t[im & mask];
+        for (int j = 1; j < P; j++) s = __dadd_rn(s, t[(j << m) | ((im >> (j * m)) & mask)]);
+        v[k] = __double2float_rn(s);
+    }
+    __syncwarp();
 }
 /* symbol r of a mapped (INPUT_MAPPED: [..][2], rho = 1) or faded (INPUT_FADED: [..][4], one 16-byte load) input as intake_mapped
  * reads it */
@@ -714,7 +743,11 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
             float v[VPL];
             if (a.input_kind == INPUT_BPSK) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
                                                                reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
-            else if (a.input_kind >= INPUT_MAPPED) intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
+            else if (a.input_kind == INPUT_MAPPED || a.input_kind == INPUT_FADED)
+                intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
+            else if (a.input_kind == INPUT_SPLIT)       /* scratch: 32 doubles, within the phase-1 scratch of plan_smem */
+                intake_split<Q>(a.in + ((size_t)(base + f) * N + n) * (2 * a.split_p), a.split_p, a.den, a.mod, gf.img, lane,
+                                reinterpret_cast<double *>(wm.scr(0)), v);
             else load_row<Q>(a.in + ((size_t)(base + f) * N + n) * Q, lane, v);
             store_row<Q>(app + ((size_t)f * N + n) * Q, lane, v);
         }
@@ -1057,13 +1090,14 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
 {
     constexpr int VPL = QTraits<Q>::VPL;
     constexpr int UW = UNIT_NT / 32;
-    __shared__ double ts[UW][16];
+    __shared__ double ts[UW][32];
     __shared__ float rows[UW][Q];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long total = (long)B * a.N;
     for (long r = (long)blockIdx.x * UW + warp; r < total; r += (long)gridDim.x * UW) {
         float v[VPL];
-        if (kind >= INPUT_MAPPED) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
+        if (kind == INPUT_MAPPED || kind == INPUT_FADED) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
+        else if (kind == INPUT_SPLIT) intake_split<Q>(noisy + r * (2 * a.split_p), a.split_p, a.den, a.mod, a.img, lane, ts[warp], v);
         else intake_variable<Q>(noisy + r * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
         if (llr) store_row<Q>(llr + r * Q, lane, v);
         if (illr) {
@@ -1111,15 +1145,16 @@ static const void *checknode_fn(int q, int closed, int ecn)
  * ---------------------------------------------------------------------------------------------- */
 /* A channel as the host code uses it, resolved once per call by channel_of(): the intake, the frame layout, how the frame
  * source draws a symbol and which constellation both read. */
-enum ChannelId { CH_BPSK, CH_LLR, CH_APSK64, CH_MAPPED, CH_FADED };
+enum ChannelId { CH_BPSK, CH_LLR, CH_APSK64, CH_MAPPED, CH_FADED, CH_SPLIT };
 struct Channel {
     int rc;                      /* NBGPU_OK, or the refusal of channel_of (the rest is then unset) */
     int kind;                    /* InputKind */
-    int fps;                     /* floats per symbol of a frame: log2 q, q, 2 (I, Q) or 4 (I, Q, rho_I, rho_Q) */
+    int fps;                     /* floats per symbol of a frame: log2 q, q, 2 (I, Q), 4 (I, Q, rho_I, rho_Q) or 2P (split) */
     int draws;                   /* frame source: drand48 draws per symbol after the information bits */
     bool apsk_sigma;             /* sigma = nbgpu_sigma_apsk64(EbN) (every constellation), else nbgpu_sigma(code, EbN) */
-    const float *mod_d, *mod_h;  /* constellation [q][2] on the device and its host copy; nullptr for BPSK and LLR */
+    const float *mod_d, *mod_h;  /* constellation [q][2] ([M][2] split) on the device and its host copy; nullptr for BPSK and LLR */
     int fading;                  /* CH_FADED: NBGPU_FADING_SYMBOL or NBGPU_FADING_COMPONENT of the frame source */
+    int points;                  /* CH_SPLIT: points per symbol (KArgs::split_p) */
 };
 
 struct nbgpu_ctx {
@@ -1143,6 +1178,9 @@ struct nbgpu_ctx {
     float mod_h[128];                        /* host copy of the 64-APSK table, for the frame source's fix-up */
     float *d_map;                            /* the bound table of the mapped calls (nbgpu_set_constellation), NULL until bound */
     float map_h[512];                        /* host copy of the bound table, for the frame source's fix-up */
+    float *d_split;                          /* the split table (nbgpu_set_split_constellation), [M][2] with M <= 16; NULL until bound */
+    float split_h[32];                       /* its host copy */
+    int split_p;                             /* its points per symbol */
     float *d_app; uint8_t *d_ctov; uint8_t *d_dec;
     float *d_in; size_t in_capacity;
     int *d_decide, *d_synd, *d_iters, *d_frame_slot, *d_slot_frame;
@@ -1150,7 +1188,7 @@ struct nbgpu_ctx {
     unsigned *h_ready;                       /* pinned: cumulative frame counts of the input pieces of decode_host */
     int resident_B;
     Channel resident;                        /* channel of the batch in d_in (kept when nbgpu_set_constellation drops it) */
-    int mapped_dropped;                      /* InputKind (mapped, faded) of the resident batch nbgpu_set_constellation dropped, else 0 */
+    int mapped_dropped;                      /* InputKind (mapped, faded, split) of the resident batch that re-binding its table dropped, else 0 */
     /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
@@ -1494,7 +1532,7 @@ extern "C" void nbgpu_destroy(nbgpu_ctx *c)
     if (!c) return;
     cudaSetDevice(c->device);
     void *bufs[] = { c->d_cfg, c->d_ctov_dense, c->d_row_ptr, c->d_col, c->d_cninfo, c->d_einfo, c->d_step_ptr, c->d_isolated, c->d_hval, c->d_rotin,
-                     c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_map, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
+                     c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_map, c->d_split, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
                      c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue, c->k.soft_llr, c->k.soft_sym };
     for (void *b : bufs) if (b) cudaFree(b);
     if (c->h_ready) cudaFreeHost(c->h_ready);
@@ -1521,7 +1559,7 @@ static int ensure_input(nbgpu_ctx *c, size_t floats)
 }
 
 /* Channel `id` of context c.  Refusals: the 64-APSK channel on another field than GF(64) (NBGPU_EINVAL), a mapped or faded
- * channel with no bound table (NBGPU_ESTATE), a fading value other than NBGPU_FADING_SYMBOL / _COMPONENT (NBGPU_EINVAL).
+ * channel with no bound table or a split channel with no split table (NBGPU_ESTATE), a fading value other than NBGPU_FADING_SYMBOL / _COMPONENT (NBGPU_EINVAL).
  * fading only sets the frame source's draws: the faded intake reads the amplitudes from the frames. */
 static Channel channel_of(nbgpu_ctx *c, ChannelId id, int fading = NBGPU_FADING_SYMBOL)
 {
@@ -1536,6 +1574,11 @@ static Channel channel_of(nbgpu_ctx *c, ChannelId id, int fading = NBGPU_FADING_
     } else if ((id == CH_MAPPED || id == CH_FADED) && !c->d_map) {
         ctx_err(c, "mapped channel: no constellation bound to this context (call nbgpu_set_constellation first)");
         ch.rc = NBGPU_ESTATE;
+    } else if (id == CH_SPLIT && !c->d_split) {
+        ctx_err(c, "split channel: no split constellation bound to this context (call nbgpu_set_split_constellation first)");
+        ch.rc = NBGPU_ESTATE;
+    } else if (id == CH_SPLIT) {      /* the mapped channel's two draws per I/Q sample, over P points per symbol */
+        ch = { NBGPU_OK, INPUT_SPLIT, 2 * c->split_p, 4 * c->split_p, true, c->d_split, c->split_h, 0, c->split_p };
     } else if (id == CH_BPSK) ch = { NBGPU_OK, INPUT_BPSK, c->logq, 2 * c->logq };           /* two draws per code bit, channel.c:56-57 */
     else if (id == CH_LLR) ch = { NBGPU_OK, INPUT_LLR, c->q };
     else {      /* two draws per I/Q sample (channel.c:234-263); faded: one amplitude draw (SYMBOL) or two (COMPONENT) more */
@@ -1592,6 +1635,10 @@ extern "C" int nbgpu_upload_faded(nbgpu_ctx *c, const float *rx, float sigma, in
 {
     return upload_common(c, channel_of(c, CH_FADED), rx, sigma, B);
 }
+extern "C" int nbgpu_upload_split(nbgpu_ctx *c, const float *noisy, float sigma, int B)
+{
+    return upload_common(c, channel_of(c, CH_SPLIT), noisy, sigma, B);
+}
 
 extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
 {
@@ -1611,8 +1658,36 @@ extern "C" int nbgpu_set_constellation(nbgpu_ctx *c, const float *mod)
     return NBGPU_OK;
 }
 
+extern "C" int nbgpu_set_split_constellation(nbgpu_ctx *c, int points, const float *mod)
+{
+    if (!c || !mod) { ctx_err(c, "nbgpu_set_split_constellation: NULL argument"); return NBGPU_EINVAL; }
+    if (!nbgpu_split_points_ok(c->logq, points)) {
+        ctx_err(c, "nbgpu_set_split_constellation: %d points per GF(%d) symbol (need P >= 2 dividing log2 q = %d)", points, c->q, c->logq);
+        return NBGPU_EINVAL;
+    }
+    const int M = 1 << (c->logq / points);
+    for (int i = 0; i < 2 * M; i++)
+        if (!std::isfinite(mod[i])) { ctx_err(c, "nbgpu_set_split_constellation: mod[%d][%d] = %g is not finite", i / 2, i % 2, (double)mod[i]); return NBGPU_EINVAL; }
+    CK(c, cudaSetDevice(c->device));
+    if (!c->d_split) CK(c, cudaMalloc((void **)&c->d_split, sizeof c->split_h));
+    /* stream order: a launch in flight still reads the old table */
+    CK(c, cudaMemcpyAsync(c->d_split, mod, 2 * (size_t)M * sizeof(float), cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
+    memcpy(c->split_h, mod, 2 * (size_t)M * sizeof(float));
+    c->split_p = points;
+    if (c->resident_B > 0 && c->resident.mod_d == c->d_split) {
+        /* made for the old table (or another P): dropped, as nbgpu_set_constellation drops a mapped batch */
+        c->resident_B = 0; c->mapped_dropped = c->resident.kind; c->soft_made = NBGPU_SOFT_NONE;
+    }
+    return NBGPU_OK;
+}
+
 extern "C" int nbgpu_run(nbgpu_ctx *c)
 {
+    if (c && c->resident_B < 1 && c->mapped_dropped == INPUT_SPLIT) {
+        ctx_err(c, "nbgpu_run: the split batch was dropped when nbgpu_set_split_constellation bound a new table");
+        return NBGPU_ESTATE;
+    }
     if (c && c->resident_B < 1 && c->mapped_dropped) {
         ctx_err(c, "nbgpu_run: the %s batch was dropped when nbgpu_set_constellation bound a new table", c->mapped_dropped == INPUT_FADED ? "faded" : "mapped");
         return NBGPU_ESTATE;
@@ -1620,7 +1695,7 @@ extern "C" int nbgpu_run(nbgpu_ctx *c)
     if (!c || c->resident_B < 1) { ctx_err(c, "nbgpu_run: no resident batch (call nbgpu_upload_* first)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     KArgs k = c->k;
-    k.B = c->resident_B; k.input_kind = c->resident.kind; k.in = c->d_in; k.mod = c->resident.mod_d;
+    k.B = c->resident_B; k.input_kind = c->resident.kind; k.in = c->d_in; k.mod = c->resident.mod_d; k.split_p = c->resident.points;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     const int groups = (k.B + k.F - 1) / k.F;
     const int grid = std::min(c->grid, groups);
@@ -1754,7 +1829,7 @@ static int decode_host(nbgpu_ctx *c, const Channel &ch, const float *src, float 
         CK(c, cudaMemcpyAsync(c->d_ready, c->h_ready + i, sizeof(unsigned), cudaMemcpyHostToDevice, c->copy_stream));
     }
     KArgs k = c->k;
-    k.B = B; k.input_kind = ch.kind; k.in = c->d_in; k.mod = ch.mod_d; k.ready = c->d_ready;
+    k.B = B; k.input_kind = ch.kind; k.in = c->d_in; k.mod = ch.mod_d; k.split_p = ch.points; k.ready = c->d_ready;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     CK(c, cudaStreamWaitEvent(c->stream, c->ev_h2d[0], 0));   /* the counter starts at zero */
     CK(c, cudaEventRecord(c->ev0, c->stream));
@@ -1797,6 +1872,10 @@ extern "C" int nbgpu_decode_mapped(nbgpu_ctx *c, const float *noisy, float sigma
 extern "C" int nbgpu_decode_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, int *decide, int *synd, int *iters)
 {
     return decode_host(c, channel_of(c, CH_FADED), rx, sigma, B, decide, synd, iters);
+}
+extern "C" int nbgpu_decode_split(nbgpu_ctx *c, const float *noisy, float sigma, int B, int *decide, int *synd, int *iters)
+{
+    return decode_host(c, channel_of(c, CH_SPLIT), noisy, sigma, B, decide, synd, iters);
 }
 
 
@@ -1915,13 +1994,14 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     nbgpu_rng_skip(&r, frame0 * D);
     c->src.D = D;
     SrcArgs a = source_args(c, code, B);
-    a.x0 = r.x; a.sigma = sigma; a.mod = ch.mod_d;
+    a.x0 = r.x; a.sigma = sigma; a.mod = ch.mod_d; a.points = ch.points;
     if (ch.kind == INPUT_FADED) a.flag_cap = SRC_FLAG_CAP / 4;  /* a flagged symbol takes four patch entries */
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
-    const long long threads = (long long)B * c->N;
+    const long long threads = (long long)B * c->N * (ch.kind == INPUT_SPLIT ? ch.points : 1);       /* symbols, or split points */
     const unsigned blocks = (unsigned)((threads + 255) / 256);
-    if (ch.fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
+    if (ch.kind == INPUT_SPLIT) source_noise_mapped_kernel<SRC_SPLIT><<<blocks, 256, 0, c->stream>>>(a);
+    else if (ch.fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
     else if (ch.fading == NBGPU_FADING_SYMBOL) source_noise_mapped_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
     else if (ch.kind == INPUT_MAPPED) source_noise_mapped_kernel<0><<<blocks, 256, 0, c->stream>>>(a);
     else source_noise_kernel<<<blocks, 256, 0, c->stream>>>(a);
@@ -1934,13 +2014,15 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     c->src.fixups = nflag;
     if (nflag) {
         /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
-         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in both channels.
+         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in the BPSK, mapped and
+         * split channels (a split flag carries the point's sub-image and mod_h is the split table).
          * A faded flag is symbol n of the batch: its S draws, its four values. */
         std::vector<unsigned> idx(nflag), pidx;
         std::vector<float> val(nflag);
-        std::vector<uint8_t> img(ch.kind >= INPUT_MAPPED ? nflag : 0);
+        const bool table = ch.kind != INPUT_BPSK;           /* mapped, faded, split: the flag carries the point's image */
+        std::vector<uint8_t> img(table ? nflag : 0);
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (ch.kind >= INPUT_MAPPED) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
+        if (table) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
         if (ch.kind == INPUT_FADED) {
             pidx.resize(4 * (size_t)nflag); val.resize(4 * (size_t)nflag);
             for (unsigned i = 0; i < nflag; i++) {
@@ -1961,7 +2043,7 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
                 nbgpu_rng g; g.x = a.x0;
                 nbgpu_rng_skip(&g, f * D + koff + 2 * s);
                 const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-                val[i] = ch.kind == INPUT_MAPPED ? nbgpu_mapped_sample(sigma, ch.mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+                val[i] = ch.kind != INPUT_BPSK ? nbgpu_mapped_sample(sigma, ch.mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
             }
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
@@ -1990,6 +2072,10 @@ extern "C" int nbgpu_source_frames_mapped(nbgpu_ctx *c, nbgpu_code *code, const 
 extern "C" int nbgpu_source_frames_faded(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN, int fading)
 {
     return source_generate(c, code, origin, frame0, B, EbN, CH_FADED, fading);
+}
+extern "C" int nbgpu_source_frames_split(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN)
+{
+    return source_generate(c, code, origin, frame0, B, EbN, CH_SPLIT);
 }
 
 extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixups : 0; }
@@ -2263,7 +2349,7 @@ static int channel_common(nbgpu_ctx *c, const Channel &ch, const float *noisy, f
     CK(c, cudaMemcpyAsync(dn.p, noisy, (size_t)B * N * per * 4, cudaMemcpyHostToDevice, c->stream));
     KArgs k = c->k;
     k.den = den_of(sigma);
-    k.mod = ch.mod_d;
+    k.mod = ch.mod_d; k.split_p = ch.points;
     const int grid = (int)std::min<long>(((long)B * N + UNIT_NT / 32 - 1) / (UNIT_NT / 32), 148 * 8);
     if (q == 16) channel_kernel<16><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
     else if (q == 64) channel_kernel<64><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
@@ -2293,4 +2379,8 @@ extern "C" int nbgpu_channel_awgn_mapped(nbgpu_ctx *c, const float *noisy, float
 extern "C" int nbgpu_channel_faded(nbgpu_ctx *c, const float *rx, float sigma, int B, float *llr, float *illr, int *igf)
 {
     return channel_common(c, channel_of(c, CH_FADED), rx, sigma, B, llr, illr, igf);
+}
+extern "C" int nbgpu_channel_split(nbgpu_ctx *c, const float *noisy, float sigma, int B, float *llr, float *illr, int *igf)
+{
+    return channel_common(c, channel_of(c, CH_SPLIT), noisy, sigma, B, llr, illr, igf);
 }

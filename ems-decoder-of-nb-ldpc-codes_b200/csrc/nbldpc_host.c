@@ -485,6 +485,20 @@ float nbgpu_mapped_sample(float sigma, float point, float u, float v)
     return (float)(point + sigma * sqrt(-2.0 * log(u)) * cos(2.0 * pi * v));
 }
 
+/* Gray-labelled square M-QAM, M = 2^(2m), m bits per axis: mod[M][2] of average power 1 (include/nbldpc_b200.h, NBGPU_MAP_QAM) */
+static void gray_qam(int m, float *mod)
+{
+    const int L = 1 << m, M = L * L;
+    const double scale = sqrt(2.0 * (M - 1) / 3.0);             /* average power 1 */
+    for (int x = 0; x < M; x++)
+        for (int c = 0; c < 2; c++) {
+            const int g = (x >> (c * m)) & (L - 1);                 /* I: bits [0, m), Q: bits [m, 2m) */
+            int level = g;
+            for (int s = g >> 1; s; s >>= 1) level ^= s;            /* inverse binary-reflected Gray code */
+            mod[2 * x + c] = (float)((double)(2 * level - (L - 1)) / scale);
+        }
+}
+
 int nbgpu_constellation(int kind, int q, float *mod)
 {
     if (!mod) { nbgpu_set_global_error("nbgpu_constellation: NULL table"); return NBGPU_EINVAL; }
@@ -494,15 +508,25 @@ int nbgpu_constellation(int kind, int q, float *mod)
     }
     if (kind != NBGPU_MAP_QAM) { nbgpu_set_global_error("nbgpu_constellation: unknown kind %d (NBGPU_MAP_APSK64 = %d, NBGPU_MAP_QAM = %d)", kind, NBGPU_MAP_APSK64, NBGPU_MAP_QAM); return NBGPU_EINVAL; }
     if (q != 16 && q != 64 && q != 256) { nbgpu_set_global_error("nbgpu_constellation: square QAM for q = 16, 64 or 256, not %d", q); return NBGPU_EINVAL; }
-    const int m = q == 16 ? 2 : q == 64 ? 3 : 4, L = 1 << m;
-    const double scale = sqrt(2.0 * (q - 1) / 3.0);             /* average power 1 */
-    for (int x = 0; x < q; x++)
-        for (int c = 0; c < 2; c++) {
-            const int g = (x >> (c * m)) & (L - 1);                 /* I: bits [0, m), Q: bits [m, 2m) */
-            int level = g;
-            for (int s = g >> 1; s; s >>= 1) level ^= s;            /* inverse binary-reflected Gray code */
-            mod[2 * x + c] = (float)((double)(2 * level - (L - 1)) / scale);
-        }
+    gray_qam(q == 16 ? 2 : q == 64 ? 3 : 4, mod);
+    return NBGPU_OK;
+}
+
+int nbgpu_split_points_ok(int logq, int points)
+{
+    return points >= 2 && points <= logq && logq % points == 0;
+}
+
+int nbgpu_split_qam(int q, int points, float *mod)
+{
+    const int logq = q == 16 ? 4 : q == 64 ? 6 : q == 256 ? 8 : 0;
+    if (!mod) { nbgpu_set_global_error("nbgpu_split_qam: NULL table"); return NBGPU_EINVAL; }
+    if (!logq || !nbgpu_split_points_ok(logq, points) || (logq / points) % 2) {
+        nbgpu_set_global_error("nbgpu_split_qam: no square QAM for GF(%d) over %d points per symbol (built in: (16, 2), (64, 3), "
+                               "(256, 2), (256, 4); for other pairs bind your own table)", q, points);
+        return NBGPU_EINVAL;
+    }
+    gray_qam(logq / points / 2, mod);
     return NBGPU_OK;
 }
 
@@ -568,6 +592,32 @@ int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, c
         for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
         for (b = 0; b < S; b++) d[b] = draw_float(r);
         nbgpu_faded_sample(sigma, mod + 2 * som, d, fading, rx + 4 * (size_t)n);
+    }
+    return NBGPU_OK;
+}
+
+/* noisy[N][P][2] of one frame of the split channel: point j of symbol n is mod[sub-image j], u, v for I then u, v for Q */
+int nbgpu_awgn_split_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int points, const float *mod, float EbN, float *noisy)
+{
+    const float sigma = nbgpu_sigma_apsk64(EbN);
+    int n, b, j;
+    if (!c || !r || !mod || !noisy) { nbgpu_set_global_error("nbgpu_awgn_split_noise: NULL argument"); return NBGPU_EINVAL; }
+    if (!nbgpu_split_points_ok(c->logq, points)) {
+        nbgpu_set_global_error("nbgpu_awgn_split_noise: %d points per GF(%d) symbol (need P >= 2 dividing log2 q = %d)", points, c->q, c->logq);
+        return NBGPU_EINVAL;
+    }
+    const int m = c->logq / points;
+    for (n = 0; n < c->N; n++) {
+        int som = 0;
+        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
+        for (j = 0; j < points; j++) {
+            const int sub = (som >> (j * m)) & ((1 << m) - 1);
+            for (b = 0; b < 2; b++) {
+                float u = draw_float(r);
+                float v = draw_float(r);
+                noisy[2 * ((size_t)n * points + j) + b] = nbgpu_mapped_sample(sigma, mod[2 * sub + b], u, v);
+            }
+        }
     }
     return NBGPU_OK;
 }

@@ -43,6 +43,8 @@ float nbgpu_noise_sample(float sigma, float u, float v, int bit);          /* ch
 float nbgpu_mapped_sample(float sigma, float point, float u, float v);    /* channel.c:234-263, one I or Q sample of any table */
 /* one faded symbol: draws d[] = u_I, v_I, u_Q, v_Q, w_I (, w_Q) of the stream, point m[2] -> rx[4] = (y_I, y_Q, rho_I, rho_Q) */
 void nbgpu_faded_sample(float sigma, const float *m, const float *d, int fading, float *rx);
+/* split channel: 1 if `points` points per GF(q) symbol is allowed (P >= 2 dividing log2 q), else 0 */
+int nbgpu_split_points_ok(int logq, int points);
 
 /* syndrome_ems configuration table (syndrome_decoder.c:1542, 1661, 2285); returns malloc'd [size*dc] */
 int *nbgpu_build_config_table(int dc, int d1, int d2, int d3, int trunc, int *size_out);

@@ -10,8 +10,8 @@
  *   the error count         NB_LDPC.c:479-485 information-bit errors of the decided word
  *
  * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q for BPSK, K log2 q + 4N for a mapped
- * channel (two draws per noisy sample) and K log2 q + 5N or + 6N for a faded one (one or two amplitude draws more per
- * symbol), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of
+ * channel (two draws per noisy sample), K log2 q + 5N or + 6N for a faded one (one or two amplitude draws more per
+ * symbol) and K log2 q + 4NP for the split channel (P points per symbol), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of
  * the affine map in constant memory).  D is a property of the batch: one context may alternate the channels.
  *
  * Exactness.  Everything except log() and cos() is IEEE arithmetic that the device reproduces bit for bit (explicit
@@ -56,8 +56,11 @@ struct SrcArgs {
     const int *decide;           /* [B][N] */
     int *bit_errors;             /* [B] */
     const float *mod;            /* [q][2] constellation of a mapped batch by binary image (the decoder's intake table) */
-    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged mapped sample (q <= 256) */
+    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged mapped sample (q <= 256); split: of the point */
+    int points;                  /* split channel: points per symbol (source_noise_mapped_kernel<SRC_SPLIT>) */
 };
+
+#define SRC_SPLIT 3              /* source_noise_mapped_kernel<SRC_SPLIT>: the split channel */
 
 __device__ __forceinline__ uint64_t src_skip(uint64_t x, uint64_t n)
 {
@@ -153,10 +156,35 @@ __device__ __forceinline__ bool src_ambiguous(double y, double t, double margin)
  * FADING = NBGPU_FADING_SYMBOL / _COMPONENT: the faded mapped channel (include/nbldpc_b200.h), 5 or 6 draws per symbol
  * (u_I, v_I, u_Q, v_Q, w_I, w_Q), rho = (float)sqrt(-log(w)), y = rho * point + noise with the product exact in f64, written
  * as rx[B][N][4] = (y_I, y_Q, rho_I, rho_Q) in one 16-byte store.  An ambiguous rho or y flags the whole symbol (its y values
- * used that rho): the flag holds the symbol's index, and the host recomputes all four values. */
+ * used that rho): the flag holds the symbol's index, and the host recomputes all four values.
+ * FADING = SRC_SPLIT: the split channel (include/nbldpc_b200.h, nbgpu_split_qam), the mapped channel over the B*N*P points of
+ * the batch: one thread per point p = n*P + j, its 4 draws from K log2 q + 4p on, the point mod[sub-image j of symbol n],
+ * written as noisy[B][N][P][2]; a flagged sample records the sub-image, so the host fix-up is the mapped channel's. */
 template <int FADING>
 __global__ void __launch_bounds__(256) source_noise_mapped_kernel(SrcArgs a)
 {
+    if constexpr (FADING == SRC_SPLIT) {
+        const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;          /* point of the batch */
+        const long long per = (long long)a.N * a.points;
+        if (id >= (long long)a.B * per) return;
+        const int f = (int)(id / per), p = (int)(id % per), m = a.logq / a.points;
+        uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)p * 4);
+        const int sub = (a.cw[(size_t)f * a.N + p / a.points] >> ((p % a.points) * m)) & ((1 << m) - 1);
+        const double sigma = (double)a.sigma;
+        float *out = a.noisy + (size_t)id * 2;
+        for (int c = 0; c < 2; c++) {
+            const float u = src_draw(x);
+            const float v = src_draw(x);
+            const double t = src_noise_term(sigma, u, v);
+            const double y = __dadd_rn((double)a.mod[2 * sub + c], t);
+            if (src_ambiguous(y, t, a.margin)) {
+                const unsigned slot = atomicAdd(a.flag_count, 1u);
+                if (slot < a.flag_cap) { a.flags[slot] = (unsigned)(id * 2 + c); a.flag_img[slot] = (uint8_t)sub; }
+            }
+            out[c] = __double2float_rn(y);
+        }
+        return;
+    }
     constexpr int S = FADING == 0 ? 4 : FADING == 1 ? 5 : 6;                    /* draws per symbol */
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= (long long)a.B * a.N) return;

@@ -4,7 +4,8 @@ Frames of a Monte-Carlo run are independent (SURVEY.md section 8e): frame f cons
 [f*D, (f+1)*D) with D = (K + 2N) * log2(q) (K*log2(q) information bits, tools.c:124-136, then two draws per
 transmitted bit, channel.c:56-57; D = K*log2(q) + 4N for a code sent one symbol per constellation point, 64-APSK or any
 mapped table, two draws for each of the I and Q samples of a symbol, channel.c:234-263; D = K*log2(q) + 5N or + 6N under
-symbol or component Rayleigh fading, one or two amplitude draws more per symbol), so every rank can generate its own frames by LCG jump-ahead.  There is no
+symbol or component Rayleigh fading, one or two amplitude draws more per symbol; D = K*log2(q) + 4NP for the split channel,
+P points per symbol), so every rank can generate its own frames by LCG jump-ahead.  There is no
 collective on the decode path.  Results meet in ONE collective:
 
   * `allreduce_counters` -- sum of the int64 counters (throughput runs: frames, non-zero syndromes, iterations, ...);
@@ -20,12 +21,19 @@ import numpy as np
 FADINGS = {"symbol": 1, "component": 2}                    # FADING_SYMBOL, FADING_COMPONENT of the library
 
 
-def _fading(channel, fading):
-    """fading=None | "symbol" | "component" -> 0, 1, 2; fading is a property of the mapped channel only"""
+def _extra(channel, fading, points):
+    """the channel's own parameter: fading=None | "symbol" | "component" -> 0, 1, 2 for "mapped"; points P for "split" (required);
+    0 otherwise.  fading belongs to the mapped channel only, points to the split channel only."""
+    if points is not None and channel != "split":
+        raise ValueError("points=%r needs channel='split', not %r" % (points, channel))
+    if fading is not None and channel != "mapped":
+        raise ValueError("fading=%r needs channel='mapped', not %r" % (fading, channel))
+    if channel == "split":
+        if points is None:
+            raise ValueError("channel='split' needs points=P")
+        return int(points)
     if fading is None:
         return 0
-    if channel != "mapped":
-        raise ValueError("fading=%r needs channel='mapped', not %r" % (fading, channel))
     if fading not in FADINGS:
         raise ValueError("fading must be 'symbol' or 'component', not %r" % (fading,))
     return FADINGS[fading]
@@ -36,33 +44,38 @@ def _sigma_apsk64(code, ebn):
     return sigma_apsk64(ebn)
 
 
-# per channel: drand48 draws per symbol after the K*log2(q) information bits (fading adds 1 or 2), sigma(code, ebn), the host
-# noise of one frame (code, nbin, ebn, mod, fading) and the device source of a batch (decoder, frame0, B, ebn, fading)
+# per channel, with x = the channel's own parameter (_extra: fading of "mapped", points of "split"): drand48 draws per symbol
+# after the K*log2(q) information bits (code, x), sigma(code, ebn), the host noise of one frame (code, nbin, ebn, mod, x) and
+# the device source of a batch (decoder, frame0, B, ebn, x)
 _CHANNELS = {
-    "bpsk": (lambda code: 2 * code.logq, lambda code, ebn: code.sigma(ebn),
-             lambda code, nbin, ebn, mod, fd: code.noise(nbin, ebn),
-             lambda d, frame0, B, ebn, fd: d.source_frames(frame0, B, ebn)),
-    "apsk64": (lambda code: 4, _sigma_apsk64,
-               lambda code, nbin, ebn, mod, fd: code.noise_apsk64(nbin, ebn),
-               lambda d, frame0, B, ebn, fd: d.source_frames_apsk64(frame0, B, ebn)),
-    "mapped": (lambda code: 4, _sigma_apsk64,
-               lambda code, nbin, ebn, mod, fd: code.noise_faded(nbin, mod, ebn, fd) if fd else code.noise_mapped(nbin, mod, ebn),
-               lambda d, frame0, B, ebn, fd: d.source_frames_faded(frame0, B, ebn, fd) if fd else d.source_frames_mapped(frame0, B, ebn)),
+    "bpsk": (lambda code, x: 2 * code.logq, lambda code, ebn: code.sigma(ebn),
+             lambda code, nbin, ebn, mod, x: code.noise(nbin, ebn),
+             lambda d, frame0, B, ebn, x: d.source_frames(frame0, B, ebn)),
+    "apsk64": (lambda code, x: 4, _sigma_apsk64,
+               lambda code, nbin, ebn, mod, x: code.noise_apsk64(nbin, ebn),
+               lambda d, frame0, B, ebn, x: d.source_frames_apsk64(frame0, B, ebn)),
+    "mapped": (lambda code, x: 4 + x, _sigma_apsk64,
+               lambda code, nbin, ebn, mod, x: code.noise_faded(nbin, mod, ebn, x) if x else code.noise_mapped(nbin, mod, ebn),
+               lambda d, frame0, B, ebn, x: d.source_frames_faded(frame0, B, ebn, x) if x else d.source_frames_mapped(frame0, B, ebn)),
+    "split": (lambda code, x: 4 * x, _sigma_apsk64,
+              lambda code, nbin, ebn, mod, x: code.noise_split(nbin, mod, x, ebn),
+              lambda d, frame0, B, ebn, x: d.source_frames_split(frame0, B, ebn)),
 }
 
 
 def _channel(channel):
     if channel not in _CHANNELS:
-        raise ValueError("channel must be 'bpsk', 'apsk64' or 'mapped', not %r" % (channel,))
+        raise ValueError("channel must be 'bpsk', 'apsk64', 'mapped' or 'split', not %r" % (channel,))
     return _CHANNELS[channel]
 
 
-def draws_per_frame(code, channel="bpsk", fading=None):
+def draws_per_frame(code, channel="bpsk", fading=None, points=None):
     """drand48 draws one frame of the reference's main loop consumes: tools.c:124-136, then channel.c:56-57 ("bpsk",
-    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table);
-    fading="symbol" / "component" (mapped only): one / two Rayleigh amplitude draws more per symbol"""
-    fd = _fading(channel, fading)
-    return code.K * code.logq + (_channel(channel)[0](code) + fd) * code.N
+    ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table;
+    "split", the same over points=P points per symbol); fading="symbol" / "component" (mapped only): one / two Rayleigh
+    amplitude draws more per symbol"""
+    x = _extra(channel, fading, points)
+    return code.K * code.logq + _channel(channel)[0](code, x) * code.N
 
 
 def frame_range(total, rank, world):
@@ -101,7 +114,7 @@ def gather_rows(rows):
 
 
 def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_err_frames=40, decoder=None, channel="bpsk",
-                constellation=None, fading=None):
+                constellation=None, fading=None, points=None):
     """The reference's Monte-Carlo loop (NB_LDPC.c:250-511) sharded by frame block over `world` ranks.
 
     Either decode(noisy, sigma) -> (decide[B, N], synd[B], iters[B]) with frames made by the host source, or
@@ -112,15 +125,20 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     the same on constellation=mod[q][2] (any field), e.g. Decoder.decode_mapped on a decoder with mod bound, and
     Decoder.source_frames_mapped (the decoder gets mod bound here).  fading="symbol" | "component" (channel="mapped" only):
     the same under Rayleigh fading, frames rx[B, N, 4], e.g. Decoder.decode_faded, and Decoder.source_frames_faded.
+    channel="split", points=P: every symbol sent as P points of constellation=mod[M][2] (e.g. split_qam(q, P)), frames
+    noisy[B, N, P, 2], e.g. Decoder.decode_split on a decoder with the table bound, and Decoder.source_frames_split (the decoder
+    gets the table bound here).
     Returns on rank 0 the dict of the reference's statistics, None on the other ranks."""
     lo, hi = frame_range(frames, rank, world)
-    D = draws_per_frame(code, channel, fading)
-    fd = _fading(channel, fading)
+    D = draws_per_frame(code, channel, fading, points)
+    x = _extra(channel, fading, points)
     _, sigma_of, noise, source = _channel(channel)
-    if channel == "mapped" and constellation is None:
-        raise ValueError("channel='mapped' needs constellation=mod[q][2]")
+    if channel in ("mapped", "split") and constellation is None:
+        raise ValueError("channel=%r needs constellation=mod" % (channel,))
     if channel == "mapped" and decoder is not None:
         decoder.set_constellation(constellation)
+    if channel == "split" and decoder is not None:
+        decoder.set_split_constellation(constellation, x)
     code.prepare_encoder()
     code.rng_default()
     code.rng_skip(lo * D)
@@ -130,7 +148,7 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     for b0 in range(lo, hi, batch):
         b1 = min(hi, b0 + batch)
         if decoder is not None:
-            source(decoder, b0, b1 - b0, ebn, fd)
+            source(decoder, b0, b1 - b0, ebn, x)
             decoder.run()
             rows[b0 - lo:b1 - lo] = np.stack(decoder.source_results(), axis=1)
             continue
@@ -138,7 +156,7 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         for _ in range(b0, b1):
             _, nbin = code.random_codeword()
             bits.append(nbin)
-            noisy.append(noise(code, nbin, ebn, constellation, fd))
+            noisy.append(noise(code, nbin, ebn, constellation, x))
         dec, synd, it = decode(np.stack(noisy), sigma)
         for i in range(b1 - b0):
             err = int((bing[dec[i, :code.K]] != bits[i][:code.K]).sum())                    # NB_LDPC.c:479-485

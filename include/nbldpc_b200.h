@@ -137,6 +137,30 @@ int nbgpu_rotate_constellation(int q, double degrees, const float *mod /*[q][2]*
 int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/,
                            const float *mod /*[q][2]*/, float EbN, int fading, float *rx /*[N][4]*/);
 
+/* ---- Split channel: one GF(q) symbol sent as P points of a smaller constellation (e.g. GF(256) over 16-QAM or QPSK) ----
+ * P points per symbol, P >= 2 dividing log2(q): q = 16: P in {2, 4}; q = 64: {2, 3, 6}; q = 256: {2, 4, 8}.  Each point
+ * carries m = log2(q)/P bits; the table is mod[M][2], M = 2^m, indexed by the point's m-bit sub-image (P*M <= 32).
+ *   Point j of symbol n carries image bits [j*m, (j+1)*m) (LSB first): sub_j = (img(s_n) >> (j*m)) & (M-1), sent as
+ *   mod[sub_j].  Symbol n is sent as points n*P ... n*P+P-1 (no interleaving across symbols).
+ *   Frame: noisy[N][P][2] (I, Q per point), [B][N][P][2] for a batch.
+ * Sigma and EbN as for every mapped call (nbgpu_sigma_apsk64); for a unit-power table the argument is Es/N0 per POINT.
+ * LLR of symbol k: t_j[x] = (double)(dI*dI)/den + (double)(dQ*dQ)/den with dI = y_{j,I} - mod[x][0], dQ = y_{j,Q} - mod[x][1]
+ *   (differences and squares in f32, round to nearest; divisions and the addition in f64), den = 2*(double)(float)(sigma^2);
+ *   LLR[k] = (float)(((t_0[sub_0] + t_1[sub_1]) + t_2[sub_2]) + ...): summed in f64 for j = 0 ... P-1, rounded to f32 once.
+ * Stream: frame f owns the draws [f*D, (f+1)*D), D = K log2(q) + 4*N*P.  Point p = n*P + j reads its draws from
+ *   K log2(q) + 4p on, in the order u_I, v_I, u_Q, v_Q, each (float)drand48(); y = (float)(point + sigma*sqrt(-2 ln u)*cos(2 PI v))
+ *   as for the mapped channel: the mapped stream over N*P points.
+ *
+ * nbgpu_split_qam     writes mod[M][2] for the pairs with an even m: Gray square M-QAM by the closed form of NBGPU_MAP_QAM with
+ *                     q replaced by M: (16, 2), (64, 3) and (256, 4) give QPSK, (256, 2) gives 16-QAM (bit for bit
+ *                     nbgpu_constellation(NBGPU_MAP_QAM, 16)).  Any other pair (odd m has no built-in table: bind your own) or
+ *                     a NULL table is NBGPU_EINVAL with a message, and the buffer is left untouched.
+ * nbgpu_awgn_split_noise  noisy[N][P][2] of one frame on the caller's drand48 stream (4*N*P draws); NBGPU_EINVAL for a bad P
+ *                     or a NULL argument. */
+int nbgpu_split_qam(int q, int points, float *mod /*[M][2]*/);
+int nbgpu_awgn_split_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/, int points,
+                           const float *mod /*[M][2]*/, float EbN, float *noisy /*[N][P][2]*/);
+
 
 /* Configuration table of the syndrome-based check node: replaces build_config_table + sort_config_table
  * (syndrome_decoder.c:1542, 2285) and the truncation NB_LDPC.c:198-201.  Returns the number of
@@ -210,6 +234,16 @@ int nbgpu_decode_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float 
  * batch as it drops a mapped one.  Soft output works on faded batches as on any other. */
 int nbgpu_channel_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B, float *llr, float *illr, int *igf);
 int nbgpu_decode_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B, int *decide, int *synd, int *iters);
+/* The split channel (see nbgpu_split_qam): nbgpu_set_split_constellation copies a caller's mod[M][2], M = 2^(log2(q)/points),
+ * into the context's split table, a binding of its own beside the one of nbgpu_set_constellation (NBGPU_EINVAL for a bad
+ * points, NULL or a non-finite value, context unchanged; none is bound after nbgpu_create).  The *_split calls work as their
+ * *_mapped counterparts with noisy[B][N][P][2] in place of noisy[B][N][2], including the streamed path of nbgpu_decode_split,
+ * soft output, and nbgpu_source_download returning noisy[B][N][P][2].  NBGPU_ESTATE with no split table bound.  Re-binding the split table drops a resident split batch (nbgpu_run returns NBGPU_ESTATE; its soft output and
+ * source results are gone) and leaves mapped, faded, BPSK and LLR batches alone; nbgpu_set_constellation does not drop a
+ * split batch. */
+int nbgpu_set_split_constellation(nbgpu_ctx *ctx, int points, const float *mod /*[M][2]*/);
+int nbgpu_channel_split(nbgpu_ctx *ctx, const float *noisy /*[B][N][P][2]*/, float sigma, int B, float *llr, float *illr, int *igf);
+int nbgpu_decode_split(nbgpu_ctx *ctx, const float *noisy /*[B][N][P][2]*/, float sigma, int B, int *decide, int *synd, int *iters);
 
 /* Same work split into stages so that a caller can keep inputs resident in HBM (bench.py "value"):
  * upload (H2D) -> run (kernel only, asynchronous on the ctx stream) -> download (D2H + sync). */
@@ -217,6 +251,7 @@ int nbgpu_upload_noisy(nbgpu_ctx *ctx, const float *noisy, float sigma, int B);
 int nbgpu_upload_apsk64(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* 64-APSK samples, see below */
 int nbgpu_upload_mapped(nbgpu_ctx *ctx, const float *noisy /*[B][N][2]*/, float sigma, int B);   /* mapped samples, bound table */
 int nbgpu_upload_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigma, int B);       /* faded samples + CSI, bound table */
+int nbgpu_upload_split(nbgpu_ctx *ctx, const float *noisy /*[B][N][P][2]*/, float sigma, int B); /* split samples, split table */
 int nbgpu_upload_llr(nbgpu_ctx *ctx, const float *llr, int B);
 int nbgpu_run(nbgpu_ctx *ctx);                  /* decode the resident batch; returns after launch    */
 int nbgpu_sync(nbgpu_ctx *ctx);
@@ -268,10 +303,15 @@ int  nbgpu_source_frames_mapped(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rn
  * must stay below 2^31; the other refusals as above. */
 int  nbgpu_source_frames_faded(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN,
                                int fading);
+/* The same for the split channel on the split table (nbgpu_set_split_constellation): D = K log2(q) + 4*N*P draws per frame,
+ * samples bit-identical to nbgpu_random_codeword + nbgpu_awgn_split_noise with that table; the batch is resident as after
+ * nbgpu_upload_split.  NBGPU_ESTATE with no split table bound (context unchanged); B*N*2P must stay below 2^31; the other
+ * refusals as above. */
+int  nbgpu_source_frames_split(nbgpu_ctx *ctx, nbgpu_code *code, const nbgpu_rng *origin, uint64_t frame0, int B, float EbN);
 /* what the source produced (either may be NULL): codeword symbols [B][N] (CodeWord of tools.c:258), noisy [B][N][logq]
  * after nbgpu_source_frames, noisy [B][N][2] (I, Q) after nbgpu_source_frames_apsk64 / _mapped, rx [B][N][4] after
- * nbgpu_source_frames_faded; NBGPU_ESTATE once an upload or a decode call has replaced the batch (a batch dropped by
- * nbgpu_set_constellation stays readable) */
+ * nbgpu_source_frames_faded, noisy [B][N][P][2] after nbgpu_source_frames_split; NBGPU_ESTATE once an upload or a decode
+ * call has replaced the batch (a batch dropped by nbgpu_set_constellation or nbgpu_set_split_constellation stays readable) */
 int  nbgpu_source_download(nbgpu_ctx *ctx, int *codeword, float *noisy);
 /* after nbgpu_run: information-bit errors of each frame (NB_LDPC.c:479-485), syndrome value, iteration count;
  * feed them to the frame-order statistics rule (NB_LDPC.c:474-507).  12 bytes per frame cross PCIe. */
@@ -300,8 +340,8 @@ int nbgpu_get_state(nbgpu_ctx *ctx, int frame, float *APP, float *CtoV);
 #define NBGPU_SOFT_NONE 0
 #define NBGPU_SOFT_LIST 1
 #define NBGPU_SOFT_BITS 2
-/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 / _mapped / _faded including their
- * streamed path, nbgpu_source_frames / _apsk64 / _mapped / _faded + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
+/* Arms every later decode launch of ctx (nbgpu_run, nbgpu_decode_noisy / _llr / _apsk64 / _mapped / _faded / _split including
+ * their streamed path, nbgpu_source_frames / _apsk64 / _mapped / _faded / _split + nbgpu_run) and allocates max_batch frames of output on the device: NBGPU_ENOMEM (with a message)
  * if that does not fit, after which ctx stays usable with soft output off.  A bad kind or k is NBGPU_EINVAL and leaves
  * the context as it was.  Invalidates the soft output of the last batch. */
 int nbgpu_set_soft_output(nbgpu_ctx *ctx, int kind, int k);
