@@ -1149,13 +1149,15 @@ enum ChannelId { CH_BPSK, CH_LLR, CH_APSK64, CH_MAPPED, CH_FADED, CH_SPLIT };
 struct Channel {
     int rc;                      /* NBGPU_OK, or the refusal of channel_of (the rest is then unset) */
     int kind;                    /* InputKind */
-    int fps;                     /* floats per symbol of a frame: log2 q, q, 2 (I, Q), 4 (I, Q, rho_I, rho_Q) or 2P (split) */
-    int draws;                   /* frame source: drand48 draws per symbol after the information bits */
+    int fps;                     /* floats per symbol of a frame: q (LLR), 4 (faded: I, Q, rho_I, rho_Q), else points * dims */
+    int draws;                   /* frame source: drand48 draws per symbol after the information bits (BPSK, mapped, split: 2 * fps) */
     bool apsk_sigma;             /* sigma = nbgpu_sigma_apsk64(EbN) (every constellation), else nbgpu_sigma(code, EbN) */
-    const float *mod_d, *mod_h;  /* constellation [q][2] ([M][2] split) on the device and its host copy; nullptr for BPSK and LLR */
+    const float *mod_d;          /* constellation [q][2] ([M][2] split) on the device; nullptr for BPSK and LLR */
+    const float *mod_h;          /* its host copy ([2][1] = {+1, -1} for BPSK), indexed [sub-image][dims] by the fix-up */
     int fading;                  /* CH_FADED: NBGPU_FADING_SYMBOL or NBGPU_FADING_COMPONENT of the frame source */
-    int points;                  /* CH_SPLIT: points per symbol (KArgs::split_p) */
+    int points, dims;            /* BPSK, mapped, split: a symbol is `points` points of `dims` coordinates (source_awgn_kernel) */
 };
+static int split_p(const Channel &ch) { return ch.kind == INPUT_SPLIT ? ch.points : 0; }    /* KArgs::split_p */
 
 struct nbgpu_ctx {
     int device;
@@ -1577,14 +1579,16 @@ static Channel channel_of(nbgpu_ctx *c, ChannelId id, int fading = NBGPU_FADING_
     } else if (id == CH_SPLIT && !c->d_split) {
         ctx_err(c, "split channel: no split constellation bound to this context (call nbgpu_set_split_constellation first)");
         ch.rc = NBGPU_ESTATE;
-    } else if (id == CH_SPLIT) {      /* the mapped channel's two draws per I/Q sample, over P points per symbol */
-        ch = { NBGPU_OK, INPUT_SPLIT, 2 * c->split_p, 4 * c->split_p, true, c->d_split, c->split_h, 0, c->split_p };
-    } else if (id == CH_BPSK) ch = { NBGPU_OK, INPUT_BPSK, c->logq, 2 * c->logq };           /* two draws per code bit, channel.c:56-57 */
-    else if (id == CH_LLR) ch = { NBGPU_OK, INPUT_LLR, c->q };
-    else {      /* two draws per I/Q sample (channel.c:234-263); faded: one amplitude draw (SYMBOL) or two (COMPONENT) more */
-        const bool faded = id == CH_FADED, apsk = id == CH_APSK64;
-        ch = { NBGPU_OK, faded ? INPUT_FADED : INPUT_MAPPED, faded ? 4 : 2, faded ? 4 + fading : 4, true, apsk ? c->d_mod : c->d_map,
-               apsk ? c->mod_h : c->map_h, faded ? fading : 0 };
+    } else if (id == CH_LLR) ch = { NBGPU_OK, INPUT_LLR, c->q };
+    else if (id == CH_FADED)          /* the mapped draws, then one amplitude draw (SYMBOL) or two (COMPONENT) */
+        ch = { NBGPU_OK, INPUT_FADED, 4, 4 + fading, true, c->d_map, c->map_h, fading };
+    else {                            /* two draws per sample: channel.c:56-57 (BPSK, one point per bit), channel.c:234-263 */
+        static const float bpsk[2] = { 1.0f, -1.0f };
+        if (id == CH_BPSK) ch = { NBGPU_OK, INPUT_BPSK, 0, 0, false, nullptr, bpsk, 0, c->logq, 1 };
+        else if (id == CH_SPLIT) ch = { NBGPU_OK, INPUT_SPLIT, 0, 0, true, c->d_split, c->split_h, 0, c->split_p, 2 };
+        else ch = { NBGPU_OK, INPUT_MAPPED, 0, 0, true, id == CH_APSK64 ? c->d_mod : c->d_map, id == CH_APSK64 ? c->mod_h : c->map_h, 0, 1, 2 };
+        ch.fps = ch.points * ch.dims;
+        ch.draws = 2 * ch.fps;
     }
     return ch;
 }
@@ -1695,7 +1699,7 @@ extern "C" int nbgpu_run(nbgpu_ctx *c)
     if (!c || c->resident_B < 1) { ctx_err(c, "nbgpu_run: no resident batch (call nbgpu_upload_* first)"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     KArgs k = c->k;
-    k.B = c->resident_B; k.input_kind = c->resident.kind; k.in = c->d_in; k.mod = c->resident.mod_d; k.split_p = c->resident.points;
+    k.B = c->resident_B; k.input_kind = c->resident.kind; k.in = c->d_in; k.mod = c->resident.mod_d; k.split_p = split_p(c->resident);
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     const int groups = (k.B + k.F - 1) / k.F;
     const int grid = std::min(c->grid, groups);
@@ -1829,7 +1833,7 @@ static int decode_host(nbgpu_ctx *c, const Channel &ch, const float *src, float 
         CK(c, cudaMemcpyAsync(c->d_ready, c->h_ready + i, sizeof(unsigned), cudaMemcpyHostToDevice, c->copy_stream));
     }
     KArgs k = c->k;
-    k.B = B; k.input_kind = ch.kind; k.in = c->d_in; k.mod = ch.mod_d; k.split_p = ch.points; k.ready = c->d_ready;
+    k.B = B; k.input_kind = ch.kind; k.in = c->d_in; k.mod = ch.mod_d; k.split_p = split_p(ch); k.ready = c->d_ready;
     CK(c, cudaMemsetAsync(c->d_queue, 0, sizeof(unsigned), c->stream));
     CK(c, cudaStreamWaitEvent(c->stream, c->ev_h2d[0], 0));   /* the counter starts at zero */
     CK(c, cudaEventRecord(c->ev0, c->stream));
@@ -1998,13 +2002,11 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     if (ch.kind == INPUT_FADED) a.flag_cap = SRC_FLAG_CAP / 4;  /* a flagged symbol takes four patch entries */
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
-    const long long threads = (long long)B * c->N * (ch.kind == INPUT_SPLIT ? ch.points : 1);       /* symbols, or split points */
-    const unsigned blocks = (unsigned)((threads + 255) / 256);
-    if (ch.kind == INPUT_SPLIT) source_noise_mapped_kernel<SRC_SPLIT><<<blocks, 256, 0, c->stream>>>(a);
-    else if (ch.fading == NBGPU_FADING_COMPONENT) source_noise_mapped_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
-    else if (ch.fading == NBGPU_FADING_SYMBOL) source_noise_mapped_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
-    else if (ch.kind == INPUT_MAPPED) source_noise_mapped_kernel<0><<<blocks, 256, 0, c->stream>>>(a);
-    else source_noise_kernel<<<blocks, 256, 0, c->stream>>>(a);
+    const unsigned blocks = (unsigned)(((long long)B * c->N + 255) / 256);                        /* one thread per symbol */
+    if (ch.fading == NBGPU_FADING_COMPONENT) source_faded_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
+    else if (ch.fading == NBGPU_FADING_SYMBOL) source_faded_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
+    else if (ch.dims == 2) source_awgn_kernel<2><<<blocks, 256, 0, c->stream>>>(a);
+    else source_awgn_kernel<1><<<blocks, 256, 0, c->stream>>>(a);
     CK(c, cudaGetLastError());
     c->launches += 2;
     unsigned nflag = 0;
@@ -2014,15 +2016,14 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     c->src.fixups = nflag;
     if (nflag) {
         /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
-         * channel.c:234-263).  Sample s of a frame reads the draws 2s, 2s+1 after the information bits in the BPSK, mapped and
-         * split channels (a split flag carries the point's sub-image and mod_h is the split table).
-         * A faded flag is symbol n of the batch: its S draws, its four values. */
+         * channel.c:234-263).  In the BPSK, mapped and split channels a flag is sample s of a frame, which reads the draws
+         * 2s, 2s+1 after the information bits, and the sub-image of its point.  A faded flag is symbol n of the batch and its
+         * image: its S draws, its four values. */
         std::vector<unsigned> idx(nflag), pidx;
         std::vector<float> val(nflag);
-        const bool table = ch.kind != INPUT_BPSK;           /* mapped, faded, split: the flag carries the point's image */
-        std::vector<uint8_t> img(table ? nflag : 0);
+        std::vector<uint8_t> img(nflag);
         CK(c, cudaMemcpy(idx.data(), c->src.d_flags, nflag * sizeof(unsigned), cudaMemcpyDeviceToHost));
-        if (table) CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
+        CK(c, cudaMemcpy(img.data(), c->src.d_flag_img, nflag, cudaMemcpyDeviceToHost));
         if (ch.kind == INPUT_FADED) {
             pidx.resize(4 * (size_t)nflag); val.resize(4 * (size_t)nflag);
             for (unsigned i = 0; i < nflag; i++) {
@@ -2039,11 +2040,11 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         } else {
             const uint64_t per = (uint64_t)c->N * ch.fps;
             for (unsigned i = 0; i < nflag; i++) {
-                const uint64_t id = idx[i] & 0x7fffffffu, f = id / per, s = id % per;
+                const uint64_t f = idx[i] / per, s = idx[i] % per;
                 nbgpu_rng g; g.x = a.x0;
                 nbgpu_rng_skip(&g, f * D + koff + 2 * s);
                 const float u = (float)nbgpu_rng_drand48(&g), v = (float)nbgpu_rng_drand48(&g);
-                val[i] = ch.kind != INPUT_BPSK ? nbgpu_mapped_sample(sigma, ch.mod_h[2 * img[i] + (s & 1)], u, v) : nbgpu_noise_sample(sigma, u, v, (int)(idx[i] >> 31));
+                val[i] = nbgpu_mapped_sample(sigma, ch.mod_h[ch.dims * img[i] + s % ch.dims], u, v);
             }
         }
         CK(c, cudaMemcpyAsync(c->src.d_patch_idx, idx.data(), nflag * sizeof(unsigned), cudaMemcpyHostToDevice, c->stream));
@@ -2349,7 +2350,7 @@ static int channel_common(nbgpu_ctx *c, const Channel &ch, const float *noisy, f
     CK(c, cudaMemcpyAsync(dn.p, noisy, (size_t)B * N * per * 4, cudaMemcpyHostToDevice, c->stream));
     KArgs k = c->k;
     k.den = den_of(sigma);
-    k.mod = ch.mod_d; k.split_p = ch.points;
+    k.mod = ch.mod_d; k.split_p = split_p(ch);
     const int grid = (int)std::min<long>(((long)B * N + UNIT_NT / 32 - 1) / (UNIT_NT / 32), 148 * 8);
     if (q == 16) channel_kernel<16><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);
     else if (q == 64) channel_kernel<64><<<grid, UNIT_NT, 0, c->stream>>>(k, dn.p, dl.p, illr ? dil.p : nullptr, illr ? dig.p : nullptr, B, kind);

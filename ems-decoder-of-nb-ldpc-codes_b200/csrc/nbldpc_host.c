@@ -422,24 +422,33 @@ float nbgpu_sigma(const nbgpu_code *c, float EbN)
     return (float)sqrt(1.0 / (2.0 * c->rate * pow(10, EbN / 10.0)));                    /* channel.c:51 */
 }
 
-/* one sample of channel.c:59; also the host recomputation of the samples the device source flags (nbldpc_source.cuh) */
-float nbgpu_noise_sample(float sigma, float u, float v, int bit)
+/* noisy[N][points][dims] of one frame: symbol n (binary image nbin[n][0..logq), LSB first) is sent as `points` points of
+ * m = logq / points bits, point j as mod[sub-image j] = mod[(img >> j*m) & (2^m - 1)], each coordinate plus Box-Muller
+ * noise from two draws in stream order: channel.c:52-62 (BPSK: one point per bit, dims = 1, mod = {+1, -1}) and
+ * channel.c:234-263 (mapped: one point, dims = 2; split: P points, dims = 2) */
+static void awgn_points(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int points, int dims, const float *mod, float sigma,
+                        float *noisy)
 {
-    const double pi = 3.1415926536;                                                     /* channel.c:18 */
-    const int s = 1 - 2 * bit;
-    return (float)(s + sigma * sqrt(-2.0 * log(u)) * cos(2.0 * pi * v));
+    const int m = c->logq / points;
+    int n, b, j;
+    for (n = 0; n < c->N; n++) {
+        int som = 0;
+        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
+        for (j = 0; j < points; j++) {
+            const int sub = (som >> (j * m)) & ((1 << m) - 1);
+            for (b = 0; b < dims; b++) {
+                float u = draw_float(r);
+                float v = draw_float(r);
+                *noisy++ = nbgpu_mapped_sample(sigma, mod[dims * sub + b], u, v);
+            }
+        }
+    }
 }
 
 int nbgpu_awgn_bpsk_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
 {
-    const float sigma = nbgpu_sigma(c, EbN);
-    const int cnt = c->N * c->logq;
-    int i;
-    for (i = 0; i < cnt; i++) {
-        float u = draw_float(r);
-        float v = draw_float(r);
-        noisy[i] = nbgpu_noise_sample(sigma, u, v, nbin ? nbin[i] : 0);
-    }
+    static const float bpsk[2] = { 1.0f, -1.0f };                                       /* channel.c:59: 1 - 2*bit */
+    awgn_points(c, r, nbin, c->logq, 1, bpsk, nbgpu_sigma(c, EbN), noisy);
     return NBGPU_OK;
 }
 
@@ -477,8 +486,8 @@ float nbgpu_sigma_apsk64(float EbN)
 {
     return (float)sqrt(1.0 / (2.0 * pow(10, EbN / 10.0)));      /* channel.c:232 (no code rate here) */
 }
-/* one sample of channel.c:234-263 (point = I or Q coordinate of the symbol's constellation point), for any table; also the
- * host recomputation of the mapped samples the device source flags (nbldpc_source.cuh) */
+/* one sample of channel.c:59 (point = 1 - 2*bit) or channel.c:234-263 (point = I or Q coordinate of a constellation point),
+ * for any table; also the host recomputation of the samples the device source flags (nbldpc_source.cuh) */
 float nbgpu_mapped_sample(float sigma, float point, float u, float v)
 {
     const double pi = NB_PI;
@@ -530,21 +539,11 @@ int nbgpu_split_qam(int q, int points, float *mod)
     return NBGPU_OK;
 }
 
-/* noisy[N][2]: the point mod[img] of symbol n (binary image nbin[n][0..logq), LSB first) plus Box-Muller noise, channel.c:234-263 */
+/* noisy[N][2]: the point mod[img] of symbol n plus Box-Muller noise, channel.c:234-263 */
 int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, float *noisy)
 {
-    const float sigma = nbgpu_sigma_apsk64(EbN);
-    int n, b;
     if (!c || !r || !mod || !noisy) { nbgpu_set_global_error("nbgpu_awgn_mapped_noise: NULL argument"); return NBGPU_EINVAL; }
-    for (n = 0; n < c->N; n++) {
-        int som = 0;
-        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
-        for (b = 0; b < 2; b++) {
-            float u = draw_float(r);
-            float v = draw_float(r);
-            noisy[2 * n + b] = nbgpu_mapped_sample(sigma, mod[2 * som + b], u, v);
-        }
-    }
+    awgn_points(c, r, nbin, 1, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
     return NBGPU_OK;
 }
 
@@ -599,26 +598,12 @@ int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, c
 /* noisy[N][P][2] of one frame of the split channel: point j of symbol n is mod[sub-image j], u, v for I then u, v for Q */
 int nbgpu_awgn_split_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int points, const float *mod, float EbN, float *noisy)
 {
-    const float sigma = nbgpu_sigma_apsk64(EbN);
-    int n, b, j;
     if (!c || !r || !mod || !noisy) { nbgpu_set_global_error("nbgpu_awgn_split_noise: NULL argument"); return NBGPU_EINVAL; }
     if (!nbgpu_split_points_ok(c->logq, points)) {
         nbgpu_set_global_error("nbgpu_awgn_split_noise: %d points per GF(%d) symbol (need P >= 2 dividing log2 q = %d)", points, c->q, c->logq);
         return NBGPU_EINVAL;
     }
-    const int m = c->logq / points;
-    for (n = 0; n < c->N; n++) {
-        int som = 0;
-        for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
-        for (j = 0; j < points; j++) {
-            const int sub = (som >> (j * m)) & ((1 << m) - 1);
-            for (b = 0; b < 2; b++) {
-                float u = draw_float(r);
-                float v = draw_float(r);
-                noisy[2 * ((size_t)n * points + j) + b] = nbgpu_mapped_sample(sigma, mod[2 * sub + b], u, v);
-            }
-        }
-    }
+    awgn_points(c, r, nbin, points, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
     return NBGPU_OK;
 }
 

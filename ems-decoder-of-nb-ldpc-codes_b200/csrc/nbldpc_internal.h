@@ -39,8 +39,9 @@ void nbgpu_free_schedule(nbgpu_schedule *s);
 void nbgpu_set_global_error(const char *fmt, ...);
 const char *nbgpu_get_global_error(void);
 
-float nbgpu_noise_sample(float sigma, float u, float v, int bit);          /* channel.c:59, one sample */
-float nbgpu_mapped_sample(float sigma, float point, float u, float v);    /* channel.c:234-263, one I or Q sample of any table */
+/* one noisy sample, (float)(point + sigma*sqrt(-2 ln u)*cos(2 PI v)): channel.c:59 (point = 1 - 2*bit) or channel.c:234-263
+ * (point = an I or Q coordinate of any table) */
+float nbgpu_mapped_sample(float sigma, float point, float u, float v);
 /* one faded symbol: draws d[] = u_I, v_I, u_Q, v_Q, w_I (, w_Q) of the stream, point m[2] -> rx[4] = (y_I, y_Q, rho_I, rho_Q) */
 void nbgpu_faded_sample(float sigma, const float *m, const float *d, int fading, float *rx);
 /* split channel: 1 if `points` points per GF(q) symbol is allowed (P >= 2 dividing log2 q), else 0 */

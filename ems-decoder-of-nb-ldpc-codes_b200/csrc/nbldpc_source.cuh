@@ -9,18 +9,20 @@
  *                                             or, for the mapped channel of any field, on the context's bound table
  *   the error count         NB_LDPC.c:479-485 information-bit errors of the decided word
  *
- * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), D = (K + 2N) log2 q for BPSK, K log2 q + 4N for a mapped
- * channel (two draws per noisy sample), K log2 q + 5N or + 6N for a faded one (one or two amplitude draws more per
- * symbol) and K log2 q + 4NP for the split channel (P points per symbol), so every thread reaches its own draws by LCG jump-ahead (48 precomputed powers of
- * the affine map in constant memory).  D is a property of the batch: one context may alternate the channels.
+ * Frame f of the stream owns the drand48 draws [f*D, (f+1)*D), so every thread reaches its own draws by LCG jump-ahead (48
+ * precomputed powers of the affine map in constant memory).  D is a property of the batch: one context may alternate the
+ * channels.  The BPSK, mapped and split channels send a symbol as P points of DIMS coordinates and take two draws per
+ * coordinate: D = K log2 q + 2*N*P*DIMS, with (P, DIMS) = (log2 q, 1) for BPSK, (1, 2) for a mapped channel and (P, 2) for
+ * the split one (source_awgn_kernel).  A faded channel takes K log2 q + 5N or + 6N (one or two amplitude draws more per
+ * symbol; source_faded_kernel).
  *
  * Exactness.  Everything except log() and cos() is IEEE arithmetic that the device reproduces bit for bit (explicit
  * __dmul_rn/__dadd_rn so that nothing is contracted into an FMA).  The device's log/cos may differ from glibc's by a
  * few ulp of a double, which changes the f32 sample only when the f64 value sits within that distance of an f32
  * rounding boundary.  Such samples (about one in 10^6) are FLAGGED by a margin test that is ~8x wider than the
- * documented error bounds, and recomputed by the host with glibc (nbgpu_noise_sample / nbgpu_mapped_sample /
- * nbgpu_faded_sample, nbldpc_host.c) before the decoder reads them.  tests/test_gpu_source.py, test_gpu_source_apsk64.py,
- * test_gpu_mapped.py and test_gpu_faded.py check the stream against the host source sample by sample.
+ * documented error bounds, and recomputed by the host with glibc (nbgpu_mapped_sample / nbgpu_faded_sample,
+ * nbldpc_host.c) before the decoder reads them.  tests/test_gpu_source.py, test_gpu_source_apsk64.py, test_gpu_mapped.py,
+ * test_gpu_split.py and test_gpu_faded.py check the stream against the host source sample by sample.
  *
  * GF arithmetic of the encoder runs on binary images (addition = XOR): mulimg[h][x] = img(h * sym(x)),
  * divimg[p][x] = img(sym(x) / p), both built on the host from the code's tables.
@@ -56,11 +58,10 @@ struct SrcArgs {
     const int *decide;           /* [B][N] */
     int *bit_errors;             /* [B] */
     const float *mod;            /* [q][2] constellation of a mapped batch by binary image (the decoder's intake table) */
-    uint8_t *flag_img;           /* [flag_cap] binary image of the symbol of each flagged mapped sample (q <= 256); split: of the point */
-    int points;                  /* split channel: points per symbol (source_noise_mapped_kernel<SRC_SPLIT>) */
+    uint8_t *flag_img;           /* [flag_cap] sub-image of the point of each flagged sample (the bit for BPSK; the symbol's
+                                    image for the mapped and faded channels, q <= 256) */
+    int points;                  /* source_awgn_kernel: points per symbol, P */
 };
-
-#define SRC_SPLIT 3              /* source_noise_mapped_kernel<SRC_SPLIT>: the split channel */
 
 __device__ __forceinline__ uint64_t src_skip(uint64_t x, uint64_t n)
 {
@@ -106,139 +107,94 @@ __global__ void __launch_bounds__(256) source_encode_kernel(SrcArgs a)
     for (int n = tid; n < a.N; n += blockDim.x) cw[a.perm[n]] = ns[n];          /* tools.c:257-258 */
 }
 
-/* One thread per codeword symbol: its 2*logq draws, log2 q noisy samples. */
-__global__ void __launch_bounds__(256) source_noise_kernel(SrcArgs a)
-{
-    const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= (long long)a.B * a.N) return;
-    const int f = (int)(id / a.N), n = (int)(id % a.N);
-    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * 2 * a.logq);
-    const int sym = a.cw[id];
-    const double sigma = (double)a.sigma;
-    float *out = a.noisy + (size_t)id * a.logq;
-    for (int l = 0; l < a.logq; l++) {
-        const float u = src_draw(x);
-        const float v = src_draw(x);
-        const int bit = (sym >> l) & 1;
-        const double r = sqrt(-2.0 * log((double)u));
-        const double c = cos(__dmul_rn(2.0 * 3.1415926536, (double)v));          /* PI of channel.c:18 */
-        const double t = __dmul_rn(__dmul_rn(sigma, r), c);
-        const double y = __dadd_rn((double)(1 - 2 * bit), t);                    /* channel.c:59 */
-        const float yf = __double2float_rn(y);
-        const double d = a.margin * (fabs(t) + fabs(y));
-        if (!(__double2float_rn(y + d) == __double2float_rn(y - d))) {            /* also true for inf/NaN */
-            const unsigned slot = atomicAdd(a.flag_count, 1u);
-            if (slot < a.flag_cap) a.flags[slot] = (unsigned)(id * a.logq + l) | ((unsigned)bit << 31);
-        }
-        out[l] = yf;
-    }
-}
-
-/* Box-Muller noise of one I or Q sample, sigma*sqrt(-2 ln u)*cos(2 pi v) (channel.c:234-263) */
+/* Box-Muller noise of one sample, sigma*sqrt(-2 ln u)*cos(2 pi v) (channel.c:59, channel.c:234-263) */
 __device__ __forceinline__ double src_noise_term(double sigma, float u, float v)
 {
     const double r = sqrt(-2.0 * log((double)u));
     const double cs = cos(__dmul_rn(2.0 * 3.1415926536, (double)v));             /* PI of channel.c:18 */
     return __dmul_rn(__dmul_rn(sigma, r), cs);
 }
-/* the f32 rounding of y = point + t could depend on the last bits of the device's log/cos (the margin test of
- * source_noise_kernel; also true for inf/NaN) */
+/* the f32 rounding of y = point + t could depend on the last bits of the device's log/cos (also true for inf/NaN) */
 __device__ __forceinline__ bool src_ambiguous(double y, double t, double margin)
 {
     const double d = margin * (fabs(t) + fabs(y));
     return !(__double2float_rn(y + d) == __double2float_rn(y - d));
 }
 
-/* Mapped channel (ModelChannel_AWGN_64, channel.c:234-263, on any q-point table): one thread per codeword symbol, its 4
- * draws (u, v for I, then u, v for Q), the symbol's constellation point plus noise, written as noisy[B][N][2] (the layout
- * of nbgpu_upload_apsk64 / _mapped).  Same arithmetic and margin test as source_noise_kernel; a flagged sample records its
- * symbol's image for the host.
- * FADING = NBGPU_FADING_SYMBOL / _COMPONENT: the faded mapped channel (include/nbldpc_b200.h), 5 or 6 draws per symbol
- * (u_I, v_I, u_Q, v_Q, w_I, w_Q), rho = (float)sqrt(-log(w)), y = rho * point + noise with the product exact in f64, written
- * as rx[B][N][4] = (y_I, y_Q, rho_I, rho_Q) in one 16-byte store.  An ambiguous rho or y flags the whole symbol (its y values
- * used that rho): the flag holds the symbol's index, and the host recomputes all four values.
- * FADING = SRC_SPLIT: the split channel (include/nbldpc_b200.h, nbgpu_split_qam), the mapped channel over the B*N*P points of
- * the batch: one thread per point p = n*P + j, its 4 draws from K log2 q + 4p on, the point mod[sub-image j of symbol n],
- * written as noisy[B][N][P][2]; a flagged sample records the sub-image, so the host fix-up is the mapped channel's. */
-template <int FADING>
-__global__ void __launch_bounds__(256) source_noise_mapped_kernel(SrcArgs a)
+/* BPSK, mapped and split channels: one thread per codeword symbol, sent as P = a.points points of m = log2 q / P bits each;
+ * point j is the sub-image (sym >> j*m) & (2^m - 1).  DIMS = 1: BPSK (P = log2 q), the point is 1 - 2*bit and no table is
+ * read.  DIMS = 2: the mapped channel (P = 1) or the split one (P >= 2), the point is (mod[sub][0], mod[sub][1]).  Every
+ * coordinate takes two draws, in stream order from K log2 q + 2*P*DIMS*n on, and is written as noisy[B][N][P][DIMS].  A flag
+ * records the sample index and the point's sub-image, so the host recomputes any flagged sample as the same expression. */
+template <int DIMS>
+__global__ void __launch_bounds__(256) source_awgn_kernel(SrcArgs a)
 {
-    if constexpr (FADING == SRC_SPLIT) {
-        const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;          /* point of the batch */
-        const long long per = (long long)a.N * a.points;
-        if (id >= (long long)a.B * per) return;
-        const int f = (int)(id / per), p = (int)(id % per), m = a.logq / a.points;
-        uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)p * 4);
-        const int sub = (a.cw[(size_t)f * a.N + p / a.points] >> ((p % a.points) * m)) & ((1 << m) - 1);
-        const double sigma = (double)a.sigma;
-        float *out = a.noisy + (size_t)id * 2;
-        for (int c = 0; c < 2; c++) {
-            const float u = src_draw(x);
-            const float v = src_draw(x);
-            const double t = src_noise_term(sigma, u, v);
-            const double y = __dadd_rn((double)a.mod[2 * sub + c], t);
-            if (src_ambiguous(y, t, a.margin)) {
-                const unsigned slot = atomicAdd(a.flag_count, 1u);
-                if (slot < a.flag_cap) { a.flags[slot] = (unsigned)(id * 2 + c); a.flag_img[slot] = (uint8_t)sub; }
-            }
-            out[c] = __double2float_rn(y);
+    const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (id >= (long long)a.B * a.N) return;
+    const int f = (int)(id / a.N), n = (int)(id % a.N), P = a.points, m = a.logq / P, fps = P * DIMS;
+    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * 2 * fps);
+    const int sym = a.cw[id];
+    const double sigma = (double)a.sigma;
+    for (int k = 0; k < fps; k++) {                                             /* coordinate c of point j, in stream order */
+        const int j = k / DIMS, c = k % DIMS, sub = (sym >> (j * m)) & ((1 << m) - 1);
+        const float u = src_draw(x);
+        const float v = src_draw(x);
+        const double t = src_noise_term(sigma, u, v);
+        const double y = __dadd_rn(DIMS == 1 ? (double)(1 - 2 * sub) : (double)a.mod[2 * sub + c], t);   /* channel.c:59 / :234-263 */
+        const unsigned s = (unsigned)id * fps + k;                               /* sample index: B*N*fps < 2^31 */
+        if (src_ambiguous(y, t, a.margin)) {
+            const unsigned slot = atomicAdd(a.flag_count, 1u);
+            if (slot < a.flag_cap) { a.flags[slot] = s; a.flag_img[slot] = (uint8_t)sub; }
         }
-        return;
+        a.noisy[s] = __double2float_rn(y);
     }
-    constexpr int S = FADING == 0 ? 4 : FADING == 1 ? 5 : 6;                    /* draws per symbol */
+}
+
+/* The faded mapped channel (include/nbldpc_b200.h): one thread per codeword symbol, FADING = NBGPU_FADING_SYMBOL / _COMPONENT,
+ * 5 or 6 draws per symbol (u_I, v_I, u_Q, v_Q, w_I, w_Q), rho = (float)sqrt(-log(w)), y = rho * point + noise with the product
+ * exact in f64, written as rx[B][N][4] = (y_I, y_Q, rho_I, rho_Q) in one 16-byte store.  An ambiguous rho or y flags the whole
+ * symbol (its y values used that rho): the flag holds the symbol's index, and the host recomputes all four values. */
+template <int FADING>
+__global__ void __launch_bounds__(256) source_faded_kernel(SrcArgs a)
+{
+    constexpr int S = FADING == 1 ? 5 : 6;                                      /* draws per symbol */
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (id >= (long long)a.B * a.N) return;
     const int f = (int)(id / a.N), n = (int)(id % a.N);
     uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * S);
     const int som = a.cw[id];
     const double sigma = (double)a.sigma;
-    if constexpr (FADING == 0) {
-        float *out = a.noisy + (size_t)id * 2;
-        for (int c = 0; c < 2; c++) {
-            const float u = src_draw(x);
-            const float v = src_draw(x);
-            const double t = src_noise_term(sigma, u, v);
-            const double y = __dadd_rn((double)a.mod[2 * som + c], t);           /* point + noise, channel.c:234-263 */
-            const float yf = __double2float_rn(y);
-            if (src_ambiguous(y, t, a.margin)) {
-                const unsigned slot = atomicAdd(a.flag_count, 1u);
-                if (slot < a.flag_cap) { a.flags[slot] = (unsigned)(id * 2 + c); a.flag_img[slot] = (uint8_t)som; }
-            }
-            out[c] = yf;
-        }
-    } else {
-        float d[S];
+    float d[S];
 #pragma unroll
-        for (int i = 0; i < S; i++) d[i] = src_draw(x);
-        float rho[2], y[2];
-        bool amb = false;
+    for (int i = 0; i < S; i++) d[i] = src_draw(x);
+    float rho[2], y[2];
+    bool amb = false;
 #pragma unroll
-        for (int c = 0; c < S - 4; c++) {
-            const double r = sqrt(-log((double)d[4 + c]));
-            const double e = a.margin * r;
-            rho[c] = __double2float_rn(r);
-            amb |= !(__double2float_rn(r + e) == __double2float_rn(r - e));
-        }
-        if constexpr (FADING == 1) rho[1] = rho[0];
-#pragma unroll
-        for (int c = 0; c < 2; c++) {
-            const double t = src_noise_term(sigma, d[2 * c], d[2 * c + 1]);
-            const double yd = __dadd_rn(__dmul_rn((double)rho[c], (double)a.mod[2 * som + c]), t);    /* the product is exact */
-            y[c] = __double2float_rn(yd);
-            amb |= src_ambiguous(yd, t, a.margin);
-        }
-        if (amb) {
-            const unsigned slot = atomicAdd(a.flag_count, 1u);
-            if (slot < a.flag_cap) { a.flags[slot] = (unsigned)id; a.flag_img[slot] = (uint8_t)som; }
-        }
-        *reinterpret_cast<float4 *>(a.noisy + (size_t)id * 4) = make_float4(y[0], y[1], rho[0], rho[1]);
+    for (int c = 0; c < S - 4; c++) {
+        const double r = sqrt(-log((double)d[4 + c]));
+        const double e = a.margin * r;
+        rho[c] = __double2float_rn(r);
+        amb |= !(__double2float_rn(r + e) == __double2float_rn(r - e));
     }
+    if constexpr (FADING == 1) rho[1] = rho[0];
+#pragma unroll
+    for (int c = 0; c < 2; c++) {
+        const double t = src_noise_term(sigma, d[2 * c], d[2 * c + 1]);
+        const double yd = __dadd_rn(__dmul_rn((double)rho[c], (double)a.mod[2 * som + c]), t);    /* the product is exact */
+        y[c] = __double2float_rn(yd);
+        amb |= src_ambiguous(yd, t, a.margin);
+    }
+    if (amb) {
+        const unsigned slot = atomicAdd(a.flag_count, 1u);
+        if (slot < a.flag_cap) { a.flags[slot] = (unsigned)id; a.flag_img[slot] = (uint8_t)som; }
+    }
+    *reinterpret_cast<float4 *>(a.noisy + (size_t)id * 4) = make_float4(y[0], y[1], rho[0], rho[1]);
 }
 
 __global__ void source_patch_kernel(float *noisy, const unsigned *idx, const float *val, int n)
 {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) noisy[idx[i] & 0x7fffffffu] = val[i];
+    if (i < n) noisy[idx[i]] = val[i];
 }
 
 /* One CTA per frame: information-bit errors of the decided word (NB_LDPC.c:479-485: the first K symbols). */
