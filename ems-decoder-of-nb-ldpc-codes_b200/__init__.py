@@ -22,6 +22,7 @@ ALIST_AUTO, ALIST_UBS, ALIST_KN, ALIST_FULL = 0, 1, 2, 3
 SOFT_NONE, SOFT_LIST, SOFT_BITS = 0, 1, 2
 MAP_APSK64, MAP_QAM = 1, 2
 FADING_SYMBOL, FADING_COMPONENT = 1, 2
+CHANNEL_BPSK, CHANNEL_MAPPED, CHANNEL_FADED, CHANNEL_SPLIT = 0, 1, 2, 3      # nbgpu_awgn_punctured_noise
 
 _ip = C.POINTER(C.c_int)
 _fp = C.POINTER(C.c_float)
@@ -97,6 +98,18 @@ def _split_table(logq, mod, points):
     return m.reshape(M, 2)
 
 
+def _pattern(vars):
+    """a puncturing pattern as the int32 array the library reads; the library checks range and duplicates.  Values an int32
+    cannot hold, or non-integers, are a ValueError (they must not wrap into a valid index)."""
+    v = np.asarray(() if vars is None else vars).reshape(-1)
+    if v.size and not np.issubdtype(v.dtype, np.integer):
+        raise ValueError("puncturing pattern must hold variable indices (integers), not %s" % v.dtype)
+    v = v.astype(np.int64)
+    if v.size and (v.min() < -2**31 or v.max() >= 2**31):
+        raise ValueError("puncturing pattern: index outside the int32 range")
+    return np.ascontiguousarray(v, np.int32)
+
+
 def rotate_constellation(mod, degrees):
     """nbgpu_rotate_constellation: mod[q][2] rotated by `degrees` (computed in double, rounded once), e.g. for signal-space
     diversity under NBGPU_FADING_COMPONENT."""
@@ -154,6 +167,9 @@ def lib():
         "nbgpu_channel_split": (C.c_int, [vp, _fp, C.c_float, C.c_int, _fp, _fp, _ip]),
         "nbgpu_decode_split": (C.c_int, [vp, _fp, C.c_float, C.c_int, _ip, _ip, _ip]),
         "nbgpu_upload_split": (C.c_int, [vp, _fp, C.c_float, C.c_int]),
+        "nbgpu_sigma_punctured": (C.c_float, [vp, C.c_int, C.c_float]),
+        "nbgpu_awgn_punctured_noise": (C.c_int, [vp, C.POINTER(Rng), _ip, C.c_int, C.c_int, _fp, C.c_float, C.c_int, _ip, _fp]),
+        "nbgpu_set_puncturing": (C.c_int, [vp, C.c_int, _ip]),
         "nbgpu_create": (C.c_int, [C.POINTER(vp), vp, C.POINTER(Params), C.c_int, C.c_int]),
         "nbgpu_destroy": (None, [vp]),
         "nbgpu_last_error": (C.c_char_p, [vp]),
@@ -274,8 +290,15 @@ class Code:
         _check(lib().nbgpu_random_codeword(self.h, C.byref(self.rng), _i(cw), _i(nbin)))
         return cw, nbin
 
-    def sigma(self, ebn):
-        return float(lib().nbgpu_sigma(self.h, C.c_float(ebn)))
+    def sigma(self, ebn, punctured=None):
+        """channel.c:51; punctured = variable indices never sent: sigma at the rate (N - M) / (N - p) of the transmitted word."""
+        if punctured is None:
+            return float(lib().nbgpu_sigma(self.h, C.c_float(ebn)))
+        p = _pattern(punctured).size
+        s = float(lib().nbgpu_sigma_punctured(self.h, p, C.c_float(ebn)))
+        if s != s:
+            _check(EINVAL)
+        return s
 
     def _noise(self, fn, nbin, fps, *args):
         out = np.zeros((self.N, fps), np.float32)
@@ -283,29 +306,53 @@ class Code:
         _check(fn(self.h, C.byref(self.rng), _i(nb), *args, _f(out)))
         return out
 
-    def noise(self, nbin, ebn):
-        """channel.c:52-62 for one frame; nbin None = all-zero codeword."""
+    def _punctured_noise(self, punctured, nbin, fps, channel, arg, mod, ebn):
+        """nbgpu_awgn_punctured_noise: the compact frame [N - p, fps] of the transmitted symbols"""
+        v = _pattern(punctured)
+        out = np.zeros((max(self.N - v.size, 0), fps), np.float32)
+        nb = np.ascontiguousarray(nbin, np.int32) if nbin is not None else None
+        _check(lib().nbgpu_awgn_punctured_noise(self.h, C.byref(self.rng), _i(nb), channel, int(arg), _f(mod), C.c_float(ebn),
+                                                v.size, _i(v), _f(out)))
+        return out
+
+    def noise(self, nbin, ebn, punctured=None):
+        """channel.c:52-62 for one frame; nbin None = all-zero codeword.  punctured = variable indices never sent: the frame is
+        then [N - p, logq] (transmitted symbols in variable order) at sigma(ebn, punctured)."""
+        if punctured is not None:
+            return self._punctured_noise(punctured, nbin, self.logq, CHANNEL_BPSK, 0, None, ebn)
         return self._noise(lib().nbgpu_awgn_bpsk_noise, nbin, self.logq, C.c_float(ebn))
 
-    def noise_apsk64(self, nbin, ebn):
-        """channel.c:234-263 for one frame of a GF(64) code sent as 64-APSK symbols: noisy[N][2]."""
+    def noise_apsk64(self, nbin, ebn, punctured=None):
+        """channel.c:234-263 for one frame of a GF(64) code sent as 64-APSK symbols: noisy[N][2] ([N - p][2] punctured)."""
+        if punctured is not None:
+            if self.q != 64:
+                raise ValueError("64-APSK maps one GF(64) symbol to one constellation point (q = %d)" % self.q)
+            return self.noise_mapped(nbin, apsk64_table(), ebn, punctured)
         return self._noise(lib().nbgpu_awgn_apsk64_noise, nbin, 2, C.c_float(ebn))
 
-    def noise_mapped(self, nbin, mod, ebn):
-        """channel.c:234-263 on the constellation mod[q][2] (by binary image) for one frame: noisy[N][2], sigma_apsk64(ebn)."""
+    def noise_mapped(self, nbin, mod, ebn, punctured=None):
+        """channel.c:234-263 on the constellation mod[q][2] (by binary image) for one frame: noisy[N][2], sigma_apsk64(ebn)
+        ([N - p][2] punctured)."""
         m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
+        if punctured is not None:
+            return self._punctured_noise(punctured, nbin, 2, CHANNEL_MAPPED, 0, m, ebn)
         return self._noise(lib().nbgpu_awgn_mapped_noise, nbin, 2, _f(m), C.c_float(ebn))
 
-    def noise_faded(self, nbin, mod, ebn, fading):
+    def noise_faded(self, nbin, mod, ebn, fading, punctured=None):
         """nbgpu_awgn_faded_noise: one frame of the faded mapped channel on mod[q][2], rx[N][4] = (y_I, y_Q, rho_I, rho_Q);
-        fading = FADING_SYMBOL (5N draws) or FADING_COMPONENT (6N draws)."""
+        fading = FADING_SYMBOL (5N draws) or FADING_COMPONENT (6N draws) ([N - p][4] punctured)."""
         m = np.ascontiguousarray(mod, np.float32).reshape(self.q, 2)
+        if punctured is not None:
+            return self._punctured_noise(punctured, nbin, 4, CHANNEL_FADED, int(fading), m, ebn)
         return self._noise(lib().nbgpu_awgn_faded_noise, nbin, 4, _f(m), C.c_float(ebn), int(fading))
 
-    def noise_split(self, nbin, mod, points, ebn):
+    def noise_split(self, nbin, mod, points, ebn, punctured=None):
         """nbgpu_awgn_split_noise: one frame of the split channel, each symbol sent as `points` points of mod[M][2] (by
-        sub-image), noisy[N][points][2]; 4*N*points draws, sigma_apsk64(ebn)."""
+        sub-image), noisy[N][points][2]; 4*N*points draws, sigma_apsk64(ebn) ([N - p][points][2] punctured)."""
         m = _split_table(self.logq, mod, int(points))
+        if punctured is not None:
+            out = self._punctured_noise(punctured, nbin, 2 * points, CHANNEL_SPLIT, int(points), m, ebn)
+            return out.reshape(-1, points, 2)
         out = self._noise(lib().nbgpu_awgn_split_noise, nbin, 2 * points, C.c_int(points), _f(m), C.c_float(ebn))
         return out.reshape(self.N, points, 2)
 
@@ -345,14 +392,35 @@ class Decoder:
         self.B = 0
         self.soft_k = 0
         self._source_shape = ()                               # shape of one symbol of the generated batch
+        self._source_nt = code.N                              # symbols per frame of the generated batch
         self.split_points = 0                                 # points per symbol of the bound split table
+        self.punctured = np.zeros(0, np.int32)                # the bound puncturing pattern (set_puncturing)
+        self.nt = code.N                                      # transmitted symbols per frame: N - p
+
+    def set_puncturing(self, vars):
+        """nbgpu_set_puncturing: variables `vars` (distinct, in [0, N), any order; empty = none) are never sent.  Every frame
+        this context takes or returns is then [B, N - p, ...], transmitted symbols in variable order; decisions, LLR rows and
+        soft output still cover all N variables.  Drops the resident batch."""
+        v = _pattern(vars)
+        _check(lib().nbgpu_set_puncturing(self.h, v.size, _i(v) if v.size else None), self.h)
+        self.punctured = v.copy()
+        self.nt = self.code.N - v.size
+
+    def _frames(self, frames, fps):
+        """frames as [B, nt, fps] f32; while a pattern is bound anything but [B, N - p, ...] of fps floats per symbol is a
+        ValueError (another layout would be read as other frames)"""
+        x = np.ascontiguousarray(frames, np.float32)
+        if self.nt != self.code.N and (x.ndim < 2 or x.shape[1] != self.nt or int(np.prod(x.shape[2:])) != fps):
+            raise ValueError("frames must be [B, %d, ...] with %d floats per symbol (%d of %d variables punctured), not %s"
+                             % (self.nt, fps, self.code.N - self.nt, self.code.N, x.shape))
+        return x.reshape(-1, self.nt, fps)
 
     def _out(self, B):
         return (np.zeros((B, self.code.N), np.int32), np.zeros(B, np.int32), np.zeros(B, np.int32))
 
     # the per-channel calls: frames [B, N, fps] f32 with fps floats per symbol; sigma=None for dense LLRs
     def _decode(self, fn, frames, fps, sigma=None):
-        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        x = self._frames(frames, fps)
         B = x.shape[0]
         d, s, it = self._out(B)
         sig = () if sigma is None else (C.c_float(sigma),)
@@ -361,7 +429,7 @@ class Decoder:
         return d, s, it
 
     def _channel(self, fn, frames, fps, sigma, want_sorted):
-        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        x = self._frames(frames, fps)
         B = x.shape[0]
         llr = np.zeros((B, self.code.N, self.code.q), np.float32)
         il = np.zeros_like(llr) if want_sorted else None
@@ -370,7 +438,7 @@ class Decoder:
         return (llr, il, ig) if want_sorted else llr
 
     def _upload(self, fn, frames, fps, sigma=None):
-        x = np.ascontiguousarray(frames, np.float32).reshape(-1, self.code.N, fps)
+        x = self._frames(frames, fps)
         sig = () if sigma is None else (C.c_float(sigma),)
         _check(fn(self.h, _f(x), *sig, x.shape[0]), self.h)
         self.B = x.shape[0]                                   # only once the batch is resident: it sizes every download
@@ -422,8 +490,8 @@ class Decoder:
         refuses the call (NBGPU_ESTATE)."""
         x = np.asarray(noisy)
         P = self.split_points
-        if P and (x.ndim != 4 or x.shape[1:] != (self.code.N, P, 2)):
-            raise ValueError("split frames must be [B, %d, %d, 2] for the bound table, not %s" % (self.code.N, P, x.shape))
+        if P and (x.ndim != 4 or x.shape[1:] != (self.nt, P, 2)):
+            raise ValueError("split frames must be [B, %d, %d, 2] for the bound table, not %s" % (self.nt, P, x.shape))
         return x, 2 * max(P, 1)
 
     def decode_split(self, noisy, sigma):
@@ -495,12 +563,13 @@ class Decoder:
         _check(fn(self.h, self.code.h, C.byref(r), frame0, B, C.c_float(ebn), *extra), self.h)
         self.B = B
         self._source_shape = shape
+        self._source_nt = self.nt
 
     def source_download(self, want_noisy=True):
         """(codeword [B, N], noisy) of the generated batch: noisy is [B, N, logq] for BPSK, [B, N, 2] for 64-APSK and mapped,
-        [B, N, 4] for faded, [B, N, P, 2] for split"""
+        [B, N, 4] for faded, [B, N, P, 2] for split; [B, N - p, ...] under a puncturing pattern"""
         cw = np.zeros((self.B, self.code.N), np.int32)
-        noisy = np.zeros((self.B, self.code.N) + self._source_shape, np.float32) if want_noisy else None
+        noisy = np.zeros((self.B, self._source_nt) + self._source_shape, np.float32) if want_noisy else None
         _check(lib().nbgpu_source_download(self.h, _i(cw), _f(noisy)), self.h)
         return cw, noisy
 

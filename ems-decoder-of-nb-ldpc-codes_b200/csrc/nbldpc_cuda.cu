@@ -95,6 +95,11 @@ struct KArgs {
                                            soft_llr: KArgs keeps its size, so the parameters behind it keep their offsets too */
     float *soft_llr;                    /* [B][N][k] (LIST) or [B][N][logq] (BITS)                                  */
     uint8_t *soft_sym;                  /* [B][N][k] symbols (LIST)                                                 */
+    /* puncturing (nbgpu_set_puncturing), read by the frame initialisation and channel_kernel: pmap[n] = compact index of
+     * variable n in the input frames [B][nt][..], -1 = punctured (intake row all 0.0f); nullptr with nt = N when no pattern
+     * is bound.  Behind every other field, so that those keep their parameter offsets in every kernel. */
+    const int *pmap;
+    int nt;
 };
 
 /* Lists of a warp's tile in shared memory, by 32-bit shared-window address: one array of cpw * L lists, the input lists
@@ -740,15 +745,19 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
         /* ---------------- frame initialisation: NB_LDPC.c:273-288 + channel.c:66-76 ---------------- */
         for (int w = warp; w < nf * N; w += nw) {
             const int f = w / N, n = w - f * N;
+            const int t = a.pmap ? a.pmap[n] : n;        /* the variable's symbol in the input frame; -1: punctured */
+            const size_t r = (size_t)(base + f) * a.nt + t;
             float v[VPL];
-            if (a.input_kind == INPUT_BPSK) intake_variable<Q>(a.in + ((size_t)(base + f) * N + n) * a.logq, a.den, gf.img, lane,
-                                                               reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
+            if (t < 0) {
+#pragma unroll
+                for (int j = 0; j < VPL; j++) v[j] = 0.0f;
+            } else if (a.input_kind == INPUT_BPSK) intake_variable<Q>(a.in + r * a.logq, a.den, gf.img, lane,
+                                                                      reinterpret_cast<double *>(wm.scr(0)), reinterpret_cast<float *>(wm.scr(0)) + 32, v);
             else if (a.input_kind == INPUT_MAPPED || a.input_kind == INPUT_FADED)
-                intake_mapped<Q>(mapped_input(a.in, a.input_kind, (size_t)(base + f) * N + n), a.den, a.mod, gf.img, lane, v);
+                intake_mapped<Q>(mapped_input(a.in, a.input_kind, r), a.den, a.mod, gf.img, lane, v);
             else if (a.input_kind == INPUT_SPLIT)       /* scratch: 32 doubles, within the phase-1 scratch of plan_smem */
-                intake_split<Q>(a.in + ((size_t)(base + f) * N + n) * (2 * a.split_p), a.split_p, a.den, a.mod, gf.img, lane,
-                                reinterpret_cast<double *>(wm.scr(0)), v);
-            else load_row<Q>(a.in + ((size_t)(base + f) * N + n) * Q, lane, v);
+                intake_split<Q>(a.in + r * (2 * a.split_p), a.split_p, a.den, a.mod, gf.img, lane, reinterpret_cast<double *>(wm.scr(0)), v);
+            else load_row<Q>(a.in + r * Q, lane, v);
             store_row<Q>(app + ((size_t)f * N + n) * Q, lane, v);
         }
         if constexpr (ECN == 0) {
@@ -1096,9 +1105,15 @@ __global__ void __launch_bounds__(UNIT_NT) channel_kernel(const KArgs a, const f
     const long total = (long)B * a.N;
     for (long r = (long)blockIdx.x * UW + warp; r < total; r += (long)gridDim.x * UW) {
         float v[VPL];
-        if (kind == INPUT_MAPPED || kind == INPUT_FADED) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)r), a.den, a.mod, a.img, lane, v);
-        else if (kind == INPUT_SPLIT) intake_split<Q>(noisy + r * (2 * a.split_p), a.split_p, a.den, a.mod, a.img, lane, ts[warp], v);
-        else intake_variable<Q>(noisy + r * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
+        long ri = r;                                    /* output row r = f * N + n reads input symbol f * nt + pmap[n] */
+        int t = 0;
+        if (a.pmap) { const long f = r / a.N; t = a.pmap[r - f * a.N]; ri = f * a.nt + t; }
+        if (t < 0) {
+#pragma unroll
+            for (int j = 0; j < VPL; j++) v[j] = 0.0f;
+        } else if (kind == INPUT_MAPPED || kind == INPUT_FADED) intake_mapped<Q>(mapped_input(noisy, kind, (size_t)ri), a.den, a.mod, a.img, lane, v);
+        else if (kind == INPUT_SPLIT) intake_split<Q>(noisy + ri * (2 * a.split_p), a.split_p, a.den, a.mod, a.img, lane, ts[warp], v);
+        else intake_variable<Q>(noisy + ri * a.logq, a.den, a.img, lane, ts[warp], rows[warp], v);
         if (llr) store_row<Q>(llr + r * Q, lane, v);
         if (illr) {
             /* full stable sort = q rounds of the exact scan (channel.c:78-91) */
@@ -1191,6 +1206,8 @@ struct nbgpu_ctx {
     int resident_B;
     Channel resident;                        /* channel of the batch in d_in (kept when nbgpu_set_constellation drops it) */
     int mapped_dropped;                      /* InputKind (mapped, faded, split) of the resident batch that re-binding its table dropped, else 0 */
+    int *d_punct;                            /* puncturing pattern (nbgpu_set_puncturing): k.pmap [N], then the transmitted variables [k.nt] */
+    int punct_dropped;                       /* 1: binding a pattern dropped the resident or generated batch */
     /* soft output: the armed kind and the device buffers live in k.soft_*; soft_made = the kind the last decode launch
      * produced for its soft_B frames (NBGPU_SOFT_NONE once re-armed or a new batch replaced it); decoded = a decode
      * kernel was launched at least once */
@@ -1522,6 +1539,7 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     k.out_decide = c->d_decide; k.out_synd = c->d_synd; k.out_iters = c->d_iters;
     k.frame_slot = c->d_frame_slot; k.slot_frame = c->d_slot_frame; k.queue = c->d_queue; k.slow_counter = c->d_slow;
     k.ready = nullptr; k.fault = c->d_fault;
+    k.pmap = nullptr; k.nt = N;
     /* the memsets above ran on the legacy stream, the kernels run on c->stream (non-blocking): order them once, here */
     CKF(cudaDeviceSynchronize());
 #undef CKF
@@ -1535,7 +1553,7 @@ extern "C" void nbgpu_destroy(nbgpu_ctx *c)
     cudaSetDevice(c->device);
     void *bufs[] = { c->d_cfg, c->d_ctov_dense, c->d_row_ptr, c->d_col, c->d_cninfo, c->d_einfo, c->d_step_ptr, c->d_isolated, c->d_hval, c->d_rotin,
                      c->d_rotout, c->d_img, c->d_inv, c->d_mod, c->d_map, c->d_split, c->d_app, c->d_ctov, c->d_dec, c->d_in, c->d_decide, c->d_synd,
-                     c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue, c->k.soft_llr, c->k.soft_sym };
+                     c->d_iters, c->d_frame_slot, c->d_slot_frame, c->d_queue, c->k.soft_llr, c->k.soft_sym, c->d_punct };
     for (void *b : bufs) if (b) cudaFree(b);
     if (c->h_ready) cudaFreeHost(c->h_ready);
     source_teardown(c);
@@ -1599,7 +1617,7 @@ static double den_of(float sigma) { return 2.0 * (double)(float)(sigma * sigma);
 static void set_resident(nbgpu_ctx *c, const Channel &ch, int B, float sigma, bool generated)
 {
     c->k.den = den_of(sigma);
-    c->resident_B = B; c->resident = ch; c->mapped_dropped = 0;
+    c->resident_B = B; c->resident = ch; c->mapped_dropped = 0; c->punct_dropped = 0;
     c->src.state = generated ? 1 : 0;
     if (generated) c->src.B = B;
 }
@@ -1611,7 +1629,7 @@ static int upload_common(nbgpu_ctx *c, const Channel &ch, const float *src, floa
     c->soft_made = NBGPU_SOFT_NONE;                           /* even a rejected batch: the caller moved on from the last one */
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
-    const size_t per_frame = (size_t)c->N * ch.fps;
+    const size_t per_frame = (size_t)c->k.nt * ch.fps;        /* transmitted symbols only */
     int rc = ensure_input(c, per_frame * B);                  /* grows on demand: dense-LLR batches are q/log2(q) times larger */
     if (rc) return rc;
     CK(c, cudaMemcpyAsync(c->d_in, src, per_frame * B * sizeof(float), cudaMemcpyHostToDevice, c->stream));
@@ -1686,8 +1704,35 @@ extern "C" int nbgpu_set_split_constellation(nbgpu_ctx *c, int points, const flo
     return NBGPU_OK;
 }
 
+extern "C" int nbgpu_set_puncturing(nbgpu_ctx *c, int p, const int *vars)
+{
+    if (!c) { ctx_err(NULL, "nbgpu_set_puncturing: NULL context"); return NBGPU_EINVAL; }
+    const int N = c->N;
+    std::vector<int> map(2 * (size_t)N);
+    const int nt = nbgpu_puncture_map(N, p, vars, map.data());
+    if (nt < 0) { ctx_err(c, "nbgpu_set_puncturing: %s", nbgpu_get_global_error()); return nt; }
+    for (int n = 0; n < N; n++) if (map[n] >= 0) map[N + map[n]] = n;
+    CK(c, cudaSetDevice(c->device));
+    if (p > 0) {
+        if (!c->d_punct) CK(c, cudaMalloc((void **)&c->d_punct, 2 * (size_t)N * sizeof(int)));
+        /* stream order: a launch in flight still reads the old pattern */
+        CK(c, cudaMemcpyAsync(c->d_punct, map.data(), ((size_t)N + nt) * sizeof(int), cudaMemcpyHostToDevice, c->stream));
+        CK(c, cudaStreamSynchronize(c->stream));
+    }
+    c->k.pmap = p > 0 ? c->d_punct : nullptr;
+    c->k.nt = nt;
+    /* frames of the old layout: neither decodable nor downloadable under the new one */
+    if (c->resident_B > 0 || c->src.state || c->mapped_dropped) c->punct_dropped = 1;
+    c->resident_B = 0; c->mapped_dropped = 0; c->soft_made = NBGPU_SOFT_NONE;
+    return NBGPU_OK;
+}
+
 extern "C" int nbgpu_run(nbgpu_ctx *c)
 {
+    if (c && c->resident_B < 1 && c->punct_dropped) {
+        ctx_err(c, "nbgpu_run: the batch was dropped when nbgpu_set_puncturing bound a new pattern");
+        return NBGPU_ESTATE;
+    }
     if (c && c->resident_B < 1 && c->mapped_dropped == INPUT_SPLIT) {
         ctx_err(c, "nbgpu_run: the split batch was dropped when nbgpu_set_split_constellation bound a new table");
         return NBGPU_ESTATE;
@@ -1810,7 +1855,7 @@ static int decode_host(nbgpu_ctx *c, const Channel &ch, const float *src, float 
         return NBGPU_OK;
     }
     CK(c, cudaSetDevice(c->device));
-    const size_t per_frame = (size_t)c->N * ch.fps;
+    const size_t per_frame = (size_t)c->k.nt * ch.fps;        /* transmitted symbols only */
     int rc = ensure_input(c, per_frame * B);
     if (rc) return rc;
     set_resident(c, ch, B, sigma, false);
@@ -1959,6 +2004,7 @@ static SrcArgs source_args(nbgpu_ctx *c, const nbgpu_code *code, int B)
     a.flag_count = c->src.d_flag_count; a.flags = c->src.d_flags; a.flag_cap = SRC_FLAG_CAP;
     a.decide = c->d_decide; a.bit_errors = c->src.d_bit_errors;
     a.flag_img = c->src.d_flag_img;
+    a.Nt = c->k.nt; a.tvar = c->k.pmap ? c->d_punct + c->N : nullptr;
     (void)code;
     return a;
 }
@@ -1985,15 +2031,20 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     if (code_hash(code) != c->code_hash) { ctx_err(c, "nbgpu_source_frames: the code is not the one the decoder was created for"); return NBGPU_EINVAL; }
     c->soft_made = NBGPU_SOFT_NONE;
     if (B < 1 || B > c->max_batch) { ctx_err(c, "B=%d outside 1..max_batch=%d", B, c->max_batch); return NBGPU_EINVAL; }
-    if ((double)B * c->N * ch.fps >= 2147483648.0) { ctx_err(c, "frame source: B*N*%d must stay below 2^31", ch.fps); return NBGPU_EINVAL; }
+    const int Nt = c->k.nt;                                   /* transmitted symbols (N without a puncturing pattern) */
+    if ((double)B * Nt * ch.fps >= 2147483648.0) {
+        if (Nt == c->N) ctx_err(c, "frame source: B*N*%d must stay below 2^31", ch.fps);
+        else ctx_err(c, "frame source: B*Nt*%d must stay below 2^31 (Nt = %d transmitted symbols)", ch.fps, Nt);
+        return NBGPU_EINVAL;
+    }
     CK(c, cudaSetDevice(c->device));
     int rc;
     if (!c->src.ready && (rc = source_setup(c, code))) { source_teardown(c); return rc; }
-    if ((rc = ensure_input(c, (size_t)c->N * ch.fps * B))) return rc;
+    if ((rc = ensure_input(c, (size_t)Nt * ch.fps * B))) return rc;
     const uint64_t koff = (uint64_t)(c->N - c->M) * c->logq;   /* information-bit draws, tools.c:124-136 */
     const int S = ch.draws;
-    const uint64_t D = koff + (uint64_t)c->N * S;
-    const float sigma = ch.apsk_sigma ? nbgpu_sigma_apsk64(EbN) : nbgpu_sigma(code, EbN);
+    const uint64_t D = koff + (uint64_t)Nt * S;
+    const float sigma = ch.apsk_sigma ? nbgpu_sigma_apsk64(EbN) : Nt < c->N ? nbgpu_sigma_punctured(code, c->N - Nt, EbN) : nbgpu_sigma(code, EbN);
     nbgpu_rng r = *origin;
     nbgpu_rng_skip(&r, frame0 * D);
     c->src.D = D;
@@ -2002,7 +2053,7 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
     if (ch.kind == INPUT_FADED) a.flag_cap = SRC_FLAG_CAP / 4;  /* a flagged symbol takes four patch entries */
     CK(c, cudaMemsetAsync(c->src.d_flag_count, 0, sizeof(unsigned), c->stream));
     source_encode_kernel<<<B, 256, c->N, c->stream>>>(a);
-    const unsigned blocks = (unsigned)(((long long)B * c->N + 255) / 256);                        /* one thread per symbol */
+    const unsigned blocks = (unsigned)(((long long)B * Nt + 255) / 256);              /* one thread per transmitted symbol */
     if (ch.fading == NBGPU_FADING_COMPONENT) source_faded_kernel<NBGPU_FADING_COMPONENT><<<blocks, 256, 0, c->stream>>>(a);
     else if (ch.fading == NBGPU_FADING_SYMBOL) source_faded_kernel<NBGPU_FADING_SYMBOL><<<blocks, 256, 0, c->stream>>>(a);
     else if (ch.dims == 2) source_awgn_kernel<2><<<blocks, 256, 0, c->stream>>>(a);
@@ -2018,7 +2069,7 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         /* samples whose f32 rounding could depend on the last bits of log/cos: recompute with the host's libm (channel.c:59,
          * channel.c:234-263).  In the BPSK, mapped and split channels a flag is sample s of a frame, which reads the draws
          * 2s, 2s+1 after the information bits, and the sub-image of its point.  A faded flag is symbol n of the batch and its
-         * image: its S draws, its four values. */
+         * image: its S draws, its four values.  Under puncturing, s and n count transmitted symbols only. */
         std::vector<unsigned> idx(nflag), pidx;
         std::vector<float> val(nflag);
         std::vector<uint8_t> img(nflag);
@@ -2027,9 +2078,9 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
         if (ch.kind == INPUT_FADED) {
             pidx.resize(4 * (size_t)nflag); val.resize(4 * (size_t)nflag);
             for (unsigned i = 0; i < nflag; i++) {
-                const uint64_t f = idx[i] / c->N, n = idx[i] % c->N;
+                const uint64_t f = idx[i] / Nt, t = idx[i] % Nt;
                 nbgpu_rng g; g.x = a.x0;
-                nbgpu_rng_skip(&g, f * D + koff + (uint64_t)S * n);
+                nbgpu_rng_skip(&g, f * D + koff + (uint64_t)S * t);
                 float dr[6];
                 for (int j = 0; j < S; j++) dr[j] = (float)nbgpu_rng_drand48(&g);
                 nbgpu_faded_sample(sigma, ch.mod_h + 2 * img[i], dr, ch.fading, &val[4 * (size_t)i]);
@@ -2038,7 +2089,7 @@ static int source_generate(nbgpu_ctx *c, nbgpu_code *code, const nbgpu_rng *orig
             idx.swap(pidx);
             nflag *= 4;
         } else {
-            const uint64_t per = (uint64_t)c->N * ch.fps;
+            const uint64_t per = (uint64_t)Nt * ch.fps;
             for (unsigned i = 0; i < nflag; i++) {
                 const uint64_t f = idx[i] / per, s = idx[i] % per;
                 nbgpu_rng g; g.x = a.x0;
@@ -2084,6 +2135,7 @@ extern "C" long nbgpu_source_fixups(const nbgpu_ctx *c) { return c ? c->src.fixu
 extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
 {
     if (!c || !c->src.ready || c->src.B < 1) { ctx_err(c, "nbgpu_source_download: no generated batch"); return NBGPU_EINVAL; }
+    if (c->punct_dropped) { ctx_err(c, "nbgpu_source_download: the generated batch was dropped when nbgpu_set_puncturing bound a new pattern"); return NBGPU_ESTATE; }
     if (c->src.state == 0) { ctx_err(c, "nbgpu_source_download: the generated batch was replaced by an uploaded batch"); return NBGPU_ESTATE; }
     CK(c, cudaSetDevice(c->device));
     const int B = c->src.B;
@@ -2094,7 +2146,7 @@ extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
         for (size_t i = 0; i < cw.size(); i++) codeword[i] = c->inv_h[cw[i]];
     }
     if (noisy) {
-        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->N * c->resident.fps * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+        CK(c, cudaMemcpyAsync(noisy, c->d_in, (size_t)B * c->k.nt * c->resident.fps * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
         CK(c, cudaStreamSynchronize(c->stream));
     }
     return NBGPU_OK;
@@ -2102,6 +2154,10 @@ extern "C" int nbgpu_source_download(nbgpu_ctx *c, int *codeword, float *noisy)
 
 extern "C" int nbgpu_source_results(nbgpu_ctx *c, int *bit_errors, int *synd, int *iters)
 {
+    if (c && c->src.B > 0 && c->punct_dropped) {
+        ctx_err(c, "nbgpu_source_results: the generated batch was dropped when nbgpu_set_puncturing bound a new pattern");
+        return NBGPU_ESTATE;
+    }
     if (!c || !c->src.ready || c->src.B < 1 || c->resident_B != c->src.B) { ctx_err(c, "nbgpu_source_results: no generated batch"); return NBGPU_EINVAL; }
     if (c->src.state != 2) { ctx_err(c, "nbgpu_source_results: the generated batch %s", c->src.state == 1 ? "has not been decoded (call nbgpu_run)" : "was replaced by an uploaded batch"); return NBGPU_ESTATE; }
     CK(c, cudaSetDevice(c->device));
@@ -2344,10 +2400,11 @@ static int channel_common(nbgpu_ctx *c, const Channel &ch, const float *noisy, f
     if (!noisy || B < 1 || ((illr == NULL) != (igf == NULL))) { ctx_err(c, "nbgpu_channel_awgn_*: bad argument"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     const int N = c->N, q = c->q, per = ch.fps, kind = ch.kind;
+    const size_t in_floats = (size_t)B * c->k.nt * per;       /* transmitted symbols only; the rows cover all N variables */
     DevBuf<float> dn, dl, dil; DevBuf<int> dig;
-    CK(c, dn.alloc((size_t)B * N * per)); CK(c, dl.alloc((size_t)B * N * q));
+    CK(c, dn.alloc(in_floats)); CK(c, dl.alloc((size_t)B * N * q));
     if (illr) { CK(c, dil.alloc((size_t)B * N * q)); CK(c, dig.alloc((size_t)B * N * q)); }
-    CK(c, cudaMemcpyAsync(dn.p, noisy, (size_t)B * N * per * 4, cudaMemcpyHostToDevice, c->stream));
+    CK(c, cudaMemcpyAsync(dn.p, noisy, in_floats * 4, cudaMemcpyHostToDevice, c->stream));
     KArgs k = c->k;
     k.den = den_of(sigma);
     k.mod = ch.mod_d; k.split_p = split_p(ch);

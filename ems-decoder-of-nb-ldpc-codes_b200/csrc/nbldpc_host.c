@@ -422,16 +422,18 @@ float nbgpu_sigma(const nbgpu_code *c, float EbN)
     return (float)sqrt(1.0 / (2.0 * c->rate * pow(10, EbN / 10.0)));                    /* channel.c:51 */
 }
 
-/* noisy[N][points][dims] of one frame: symbol n (binary image nbin[n][0..logq), LSB first) is sent as `points` points of
- * m = logq / points bits, point j as mod[sub-image j] = mod[(img >> j*m) & (2^m - 1)], each coordinate plus Box-Muller
- * noise from two draws in stream order: channel.c:52-62 (BPSK: one point per bit, dims = 1, mod = {+1, -1}) and
- * channel.c:234-263 (mapped: one point, dims = 2; split: P points, dims = 2) */
-static void awgn_points(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int points, int dims, const float *mod, float sigma,
-                        float *noisy)
+/* noisy[nt][points][dims] of one frame: transmitted symbol t, variable n = tx[t] (tx = NULL: n = t, every symbol sent) with
+ * binary image nbin[n][0..logq) (LSB first), is sent as `points` points of m = logq / points bits, point j as
+ * mod[sub-image j] = mod[(img >> j*m) & (2^m - 1)], each coordinate plus Box-Muller noise from two draws in stream order:
+ * channel.c:52-62 (BPSK: one point per bit, dims = 1, mod = {+1, -1}) and channel.c:234-263 (mapped: one point, dims = 2;
+ * split: P points, dims = 2) */
+static void awgn_points(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const int *tx, int nt, int points, int dims,
+                        const float *mod, float sigma, float *noisy)
 {
     const int m = c->logq / points;
-    int n, b, j;
-    for (n = 0; n < c->N; n++) {
+    int t, b, j;
+    for (t = 0; t < nt; t++) {
+        const int n = tx ? tx[t] : t;
         int som = 0;
         for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
         for (j = 0; j < points; j++) {
@@ -445,10 +447,11 @@ static void awgn_points(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int 
     }
 }
 
+static const float bpsk_points[2] = { 1.0f, -1.0f };                                   /* channel.c:59: 1 - 2*bit */
+
 int nbgpu_awgn_bpsk_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, float EbN, float *noisy)
 {
-    static const float bpsk[2] = { 1.0f, -1.0f };                                       /* channel.c:59: 1 - 2*bit */
-    awgn_points(c, r, nbin, c->logq, 1, bpsk, nbgpu_sigma(c, EbN), noisy);
+    awgn_points(c, r, nbin, NULL, c->N, c->logq, 1, bpsk_points, nbgpu_sigma(c, EbN), noisy);
     return NBGPU_OK;
 }
 
@@ -543,7 +546,7 @@ int nbgpu_split_qam(int q, int points, float *mod)
 int nbgpu_awgn_mapped_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, float *noisy)
 {
     if (!c || !r || !mod || !noisy) { nbgpu_set_global_error("nbgpu_awgn_mapped_noise: NULL argument"); return NBGPU_EINVAL; }
-    awgn_points(c, r, nbin, 1, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
+    awgn_points(c, r, nbin, NULL, c->N, 1, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
     return NBGPU_OK;
 }
 
@@ -574,24 +577,35 @@ void nbgpu_faded_sample(float sigma, const float *m, const float *d, int fading,
     rx[3] = rho_q;
 }
 
-/* rx[N][4] of one frame of the faded mapped channel: per symbol u_I, v_I, u_Q, v_Q, w_I (, w_Q) */
-int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, int fading, float *rx)
+/* rx[nt][4] of one frame of the faded mapped channel, transmitted symbols as in awgn_points: per symbol u_I, v_I, u_Q, v_Q,
+ * w_I (, w_Q) */
+static void faded_points(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const int *tx, int nt, const float *mod, float sigma,
+                         int fading, float *rx)
 {
-    const float sigma = nbgpu_sigma_apsk64(EbN);
-    int n, b;
-    if (!c || !r || !mod || !rx) { nbgpu_set_global_error("nbgpu_awgn_faded_noise: NULL argument"); return NBGPU_EINVAL; }
-    if (fading != NBGPU_FADING_SYMBOL && fading != NBGPU_FADING_COMPONENT) {
-        nbgpu_set_global_error("nbgpu_awgn_faded_noise: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fading);
-        return NBGPU_EINVAL;
-    }
     const int S = fading == NBGPU_FADING_COMPONENT ? 6 : 5;
-    for (n = 0; n < c->N; n++) {
+    int t, b;
+    for (t = 0; t < nt; t++) {
+        const int n = tx ? tx[t] : t;
         int som = 0;
         float d[6];
         for (b = 0; b < c->logq; b++) som += (nbin ? nbin[n * c->logq + b] : 0) << b;
         for (b = 0; b < S; b++) d[b] = draw_float(r);
-        nbgpu_faded_sample(sigma, mod + 2 * som, d, fading, rx + 4 * (size_t)n);
+        nbgpu_faded_sample(sigma, mod + 2 * som, d, fading, rx + 4 * (size_t)t);
     }
+}
+
+static int fading_ok(const char *fn, int fading)
+{
+    if (fading == NBGPU_FADING_SYMBOL || fading == NBGPU_FADING_COMPONENT) return 1;
+    nbgpu_set_global_error("%s: fading %d (NBGPU_FADING_SYMBOL = 1, NBGPU_FADING_COMPONENT = 2)", fn, fading);
+    return 0;
+}
+
+int nbgpu_awgn_faded_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, const float *mod, float EbN, int fading, float *rx)
+{
+    if (!c || !r || !mod || !rx) { nbgpu_set_global_error("nbgpu_awgn_faded_noise: NULL argument"); return NBGPU_EINVAL; }
+    if (!fading_ok("nbgpu_awgn_faded_noise", fading)) return NBGPU_EINVAL;
+    faded_points(c, r, nbin, NULL, c->N, mod, nbgpu_sigma_apsk64(EbN), fading, rx);
     return NBGPU_OK;
 }
 
@@ -603,7 +617,7 @@ int nbgpu_awgn_split_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, i
         nbgpu_set_global_error("nbgpu_awgn_split_noise: %d points per GF(%d) symbol (need P >= 2 dividing log2 q = %d)", points, c->q, c->logq);
         return NBGPU_EINVAL;
     }
-    awgn_points(c, r, nbin, points, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
+    awgn_points(c, r, nbin, NULL, c->N, points, 2, mod, nbgpu_sigma_apsk64(EbN), noisy);
     return NBGPU_OK;
 }
 
@@ -616,6 +630,62 @@ int nbgpu_awgn_apsk64_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, 
     nbgpu_apsk64_table(mod);
     return nbgpu_awgn_mapped_noise(c, r, nbin, mod, EbN, noisy);
 }
+
+/* ---- Puncturing (include/nbldpc_b200.h, nbgpu_set_puncturing) ---- */
+int nbgpu_puncture_map(int N, int p, const int *vars, int *map)
+{
+    int i, n, nt = 0;
+    if (p < 0 || p >= N || (p > 0 && !vars)) {
+        nbgpu_set_global_error("puncturing pattern: p = %d of N = %d variables (0 <= p <= N-1, and a list for p > 0)", p, N);
+        return NBGPU_EINVAL;
+    }
+    for (n = 0; n < N; n++) map[n] = 0;
+    for (i = 0; i < p; i++) {
+        if (vars[i] < 0 || vars[i] >= N) { nbgpu_set_global_error("puncturing pattern: variable %d outside [0, %d)", vars[i], N); return NBGPU_EINVAL; }
+        if (map[vars[i]]) { nbgpu_set_global_error("puncturing pattern: variable %d listed twice", vars[i]); return NBGPU_EINVAL; }
+        map[vars[i]] = -1;
+    }
+    for (n = 0; n < N; n++) map[n] = map[n] ? -1 : nt++;
+    return nt;
+}
+
+float nbgpu_sigma_punctured(const nbgpu_code *c, int p, float EbN)
+{
+    if (p < 0 || p >= c->N) { nbgpu_set_global_error("nbgpu_sigma_punctured: p = %d of N = %d variables", p, c->N); return NAN; }
+    const float rate_p = (float)(c->N - c->M) / (c->N - p);                            /* init.c:167 over N - p symbols */
+    return (float)sqrt(1.0 / (2.0 * rate_p * pow(10, EbN / 10.0)));                     /* channel.c:51 */
+}
+
+int nbgpu_awgn_punctured_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin, int channel, int arg, const float *mod,
+                               float EbN, int p, const int *vars, float *noisy)
+{
+    if (!c || !r || !noisy || (channel != NBGPU_CHANNEL_BPSK && !mod)) {
+        nbgpu_set_global_error("nbgpu_awgn_punctured_noise: NULL argument");
+        return NBGPU_EINVAL;
+    }
+    if (channel < NBGPU_CHANNEL_BPSK || channel > NBGPU_CHANNEL_SPLIT) {
+        nbgpu_set_global_error("nbgpu_awgn_punctured_noise: channel %d (NBGPU_CHANNEL_BPSK .. NBGPU_CHANNEL_SPLIT = 0 .. 3)", channel);
+        return NBGPU_EINVAL;
+    }
+    if (channel == NBGPU_CHANNEL_FADED && !fading_ok("nbgpu_awgn_punctured_noise", arg)) return NBGPU_EINVAL;
+    if (channel == NBGPU_CHANNEL_SPLIT && !nbgpu_split_points_ok(c->logq, arg)) {
+        nbgpu_set_global_error("nbgpu_awgn_punctured_noise: %d points per GF(%d) symbol (need P >= 2 dividing log2 q = %d)", arg, c->q, c->logq);
+        return NBGPU_EINVAL;
+    }
+    int *map = malloc(sizeof(int) * 2 * (size_t)c->N), *tx = map + c->N;
+    if (!map) { nbgpu_set_global_error("nbgpu_awgn_punctured_noise: out of memory"); return NBGPU_ENOMEM; }
+    const int nt = nbgpu_puncture_map(c->N, p, vars, map);
+    if (nt < 0) { free(map); return nt; }
+    for (int n = 0; n < c->N; n++) if (map[n] >= 0) tx[map[n]] = n;
+    const float sigma = channel == NBGPU_CHANNEL_BPSK ? nbgpu_sigma_punctured(c, p, EbN) : nbgpu_sigma_apsk64(EbN);
+    if (channel == NBGPU_CHANNEL_BPSK) awgn_points(c, r, nbin, tx, nt, c->logq, 1, bpsk_points, sigma, noisy);
+    else if (channel == NBGPU_CHANNEL_MAPPED) awgn_points(c, r, nbin, tx, nt, 1, 2, mod, sigma, noisy);
+    else if (channel == NBGPU_CHANNEL_SPLIT) awgn_points(c, r, nbin, tx, nt, arg, 2, mod, sigma, noisy);
+    else faded_points(c, r, nbin, tx, nt, mod, sigma, arg, noisy);
+    free(map);
+    return NBGPU_OK;
+}
+
 
 /* NB_LDPC.c:474-507 */
 int nbgpu_accumulate_stats(const nbgpu_code *c, const int *codeword_bits, const int *decide,

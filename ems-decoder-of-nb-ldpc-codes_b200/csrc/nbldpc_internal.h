@@ -46,6 +46,9 @@ float nbgpu_mapped_sample(float sigma, float point, float u, float v);
 void nbgpu_faded_sample(float sigma, const float *m, const float *d, int fading, float *rx);
 /* split channel: 1 if `points` points per GF(q) symbol is allowed (P >= 2 dividing log2 q), else 0 */
 int nbgpu_split_points_ok(int logq, int points);
+/* puncturing pattern of p variables of N: map[N] = compact index of each variable in the frames, -1 = punctured.  Returns
+ * Nt = N - p, or NBGPU_EINVAL with the message of nbgpu_set_puncturing (map then partly written) */
+int nbgpu_puncture_map(int N, int p, const int *vars, int *map);
 
 /* syndrome_ems configuration table (syndrome_decoder.c:1542, 1661, 2285); returns malloc'd [size*dc] */
 int *nbgpu_build_config_table(int dc, int d1, int d2, int d3, int trunc, int *size_out);

@@ -61,6 +61,8 @@ struct SrcArgs {
     uint8_t *flag_img;           /* [flag_cap] sub-image of the point of each flagged sample (the bit for BPSK; the symbol's
                                     image for the mapped and faded channels, q <= 256) */
     int points;                  /* source_awgn_kernel: points per symbol, P */
+    int Nt;                      /* transmitted symbols per frame: N, or N - p under a puncturing pattern */
+    const int *tvar;             /* [Nt] variable of each transmitted symbol, nullptr = every symbol (Nt = N) */
 };
 
 __device__ __forceinline__ uint64_t src_skip(uint64_t x, uint64_t n)
@@ -130,10 +132,10 @@ template <int DIMS>
 __global__ void __launch_bounds__(256) source_awgn_kernel(SrcArgs a)
 {
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= (long long)a.B * a.N) return;
-    const int f = (int)(id / a.N), n = (int)(id % a.N), P = a.points, m = a.logq / P, fps = P * DIMS;
-    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * 2 * fps);
-    const int sym = a.cw[id];
+    if (id >= (long long)a.B * a.Nt) return;
+    const int f = (int)(id / a.Nt), t = (int)(id % a.Nt), P = a.points, m = a.logq / P, fps = P * DIMS;
+    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)t * 2 * fps);
+    const int sym = a.cw[(size_t)f * a.N + (a.tvar ? a.tvar[t] : t)];
     const double sigma = (double)a.sigma;
     for (int k = 0; k < fps; k++) {                                             /* coordinate c of point j, in stream order */
         const int j = k / DIMS, c = k % DIMS, sub = (sym >> (j * m)) & ((1 << m) - 1);
@@ -141,7 +143,7 @@ __global__ void __launch_bounds__(256) source_awgn_kernel(SrcArgs a)
         const float v = src_draw(x);
         const double t = src_noise_term(sigma, u, v);
         const double y = __dadd_rn(DIMS == 1 ? (double)(1 - 2 * sub) : (double)a.mod[2 * sub + c], t);   /* channel.c:59 / :234-263 */
-        const unsigned s = (unsigned)id * fps + k;                               /* sample index: B*N*fps < 2^31 */
+        const unsigned s = (unsigned)id * fps + k;                               /* sample index: B*Nt*fps < 2^31 */
         if (src_ambiguous(y, t, a.margin)) {
             const unsigned slot = atomicAdd(a.flag_count, 1u);
             if (slot < a.flag_cap) { a.flags[slot] = s; a.flag_img[slot] = (uint8_t)sub; }
@@ -159,10 +161,10 @@ __global__ void __launch_bounds__(256) source_faded_kernel(SrcArgs a)
 {
     constexpr int S = FADING == 1 ? 5 : 6;                                      /* draws per symbol */
     const long long id = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (id >= (long long)a.B * a.N) return;
-    const int f = (int)(id / a.N), n = (int)(id % a.N);
-    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)n * S);
-    const int som = a.cw[id];
+    if (id >= (long long)a.B * a.Nt) return;
+    const int f = (int)(id / a.Nt), t = (int)(id % a.Nt);
+    uint64_t x = src_skip(a.x0, (uint64_t)f * a.D + (uint64_t)a.K * a.logq + (uint64_t)t * S);
+    const int som = a.cw[(size_t)f * a.N + (a.tvar ? a.tvar[t] : t)];
     const double sigma = (double)a.sigma;
     float d[S];
 #pragma unroll

@@ -5,7 +5,8 @@ Frames of a Monte-Carlo run are independent (SURVEY.md section 8e): frame f cons
 transmitted bit, channel.c:56-57; D = K*log2(q) + 4N for a code sent one symbol per constellation point, 64-APSK or any
 mapped table, two draws for each of the I and Q samples of a symbol, channel.c:234-263; D = K*log2(q) + 5N or + 6N under
 symbol or component Rayleigh fading, one or two amplitude draws more per symbol; D = K*log2(q) + 4NP for the split channel,
-P points per symbol), so every rank can generate its own frames by LCG jump-ahead.  There is no
+P points per symbol).  Under a puncturing pattern of p variables only the N - p transmitted symbols draw: N becomes N - p in
+the second term.  So every rank can generate its own frames by LCG jump-ahead.  There is no
 collective on the decode path.  Results meet in ONE collective:
 
   * `allreduce_counters` -- sum of the int64 counters (throughput runs: frames, non-zero syndromes, iterations, ...);
@@ -39,26 +40,27 @@ def _extra(channel, fading, points):
     return FADINGS[fading]
 
 
-def _sigma_apsk64(code, ebn):
+def _sigma_apsk64(code, ebn, punctured=None):
     from . import sigma_apsk64
     return sigma_apsk64(ebn)
 
 
-# per channel, with x = the channel's own parameter (_extra: fading of "mapped", points of "split"): drand48 draws per symbol
-# after the K*log2(q) information bits (code, x), sigma(code, ebn), the host noise of one frame (code, nbin, ebn, mod, x) and
-# the device source of a batch (decoder, frame0, B, ebn, x)
+# per channel, with x = the channel's own parameter (_extra: fading of "mapped", points of "split") and pv = the puncturing
+# pattern (None = none): drand48 draws per symbol after the K*log2(q) information bits (code, x), sigma(code, ebn, pv), the host
+# noise of one frame (code, nbin, ebn, mod, x, pv) and the device source of a batch (decoder, frame0, B, ebn, x)
 _CHANNELS = {
-    "bpsk": (lambda code, x: 2 * code.logq, lambda code, ebn: code.sigma(ebn),
-             lambda code, nbin, ebn, mod, x: code.noise(nbin, ebn),
+    "bpsk": (lambda code, x: 2 * code.logq, lambda code, ebn, pv: code.sigma(ebn, punctured=pv),
+             lambda code, nbin, ebn, mod, x, pv: code.noise(nbin, ebn, punctured=pv),
              lambda d, frame0, B, ebn, x: d.source_frames(frame0, B, ebn)),
     "apsk64": (lambda code, x: 4, _sigma_apsk64,
-               lambda code, nbin, ebn, mod, x: code.noise_apsk64(nbin, ebn),
+               lambda code, nbin, ebn, mod, x, pv: code.noise_apsk64(nbin, ebn, punctured=pv),
                lambda d, frame0, B, ebn, x: d.source_frames_apsk64(frame0, B, ebn)),
     "mapped": (lambda code, x: 4 + x, _sigma_apsk64,
-               lambda code, nbin, ebn, mod, x: code.noise_faded(nbin, mod, ebn, x) if x else code.noise_mapped(nbin, mod, ebn),
+               lambda code, nbin, ebn, mod, x, pv: (code.noise_faded(nbin, mod, ebn, x, punctured=pv) if x
+                                                    else code.noise_mapped(nbin, mod, ebn, punctured=pv)),
                lambda d, frame0, B, ebn, x: d.source_frames_faded(frame0, B, ebn, x) if x else d.source_frames_mapped(frame0, B, ebn)),
     "split": (lambda code, x: 4 * x, _sigma_apsk64,
-              lambda code, nbin, ebn, mod, x: code.noise_split(nbin, mod, x, ebn),
+              lambda code, nbin, ebn, mod, x, pv: code.noise_split(nbin, mod, x, ebn, punctured=pv),
               lambda d, frame0, B, ebn, x: d.source_frames_split(frame0, B, ebn)),
 }
 
@@ -69,13 +71,24 @@ def _channel(channel):
     return _CHANNELS[channel]
 
 
-def draws_per_frame(code, channel="bpsk", fading=None, points=None):
+def _npunct(code, punctured):
+    """p of a puncturing pattern (None = 0); a pattern the library would refuse is a ValueError here too"""
+    if punctured is None:
+        return 0
+    v = np.asarray(punctured).reshape(-1)
+    if v.size and (not np.issubdtype(v.dtype, np.integer) or v.min() < 0 or v.max() >= code.N or np.unique(v).size != v.size
+                   or v.size >= code.N):
+        raise ValueError("puncturing pattern must be p < N = %d distinct variable indices in [0, N)" % code.N)
+    return v.size
+
+
+def draws_per_frame(code, channel="bpsk", fading=None, points=None, punctured=None):
     """drand48 draws one frame of the reference's main loop consumes: tools.c:124-136, then channel.c:56-57 ("bpsk",
     ModelChannel_AWGN_BPSK) or channel.c:234-263 ("apsk64", ModelChannel_AWGN_64; "mapped", the same on any q-point table;
     "split", the same over points=P points per symbol); fading="symbol" / "component" (mapped only): one / two Rayleigh
-    amplitude draws more per symbol"""
+    amplitude draws more per symbol; punctured = variable indices never sent: those symbols draw nothing"""
     x = _extra(channel, fading, points)
-    return code.K * code.logq + _channel(channel)[0](code, x) * code.N
+    return code.K * code.logq + _channel(channel)[0](code, x) * (code.N - _npunct(code, punctured))
 
 
 def frame_range(total, rank, world):
@@ -114,7 +127,7 @@ def gather_rows(rows):
 
 
 def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_err_frames=40, decoder=None, channel="bpsk",
-                constellation=None, fading=None, points=None):
+                constellation=None, fading=None, points=None, punctured=None):
     """The reference's Monte-Carlo loop (NB_LDPC.c:250-511) sharded by frame block over `world` ranks.
 
     Either decode(noisy, sigma) -> (decide[B, N], synd[B], iters[B]) with frames made by the host source, or
@@ -128,9 +141,11 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
     channel="split", points=P: every symbol sent as P points of constellation=mod[M][2] (e.g. split_qam(q, P)), frames
     noisy[B, N, P, 2], e.g. Decoder.decode_split on a decoder with the table bound, and Decoder.source_frames_split (the decoder
     gets the table bound here).
+    punctured = variable indices never sent (any channel): frames hold the N - p transmitted symbols, [B, N - p, ...], and the
+    decoder gets the pattern bound here; BPSK sigma is taken at the rate of the transmitted word (Code.sigma).
     Returns on rank 0 the dict of the reference's statistics, None on the other ranks."""
     lo, hi = frame_range(frames, rank, world)
-    D = draws_per_frame(code, channel, fading, points)
+    D = draws_per_frame(code, channel, fading, points, punctured)
     x = _extra(channel, fading, points)
     _, sigma_of, noise, source = _channel(channel)
     if channel in ("mapped", "split") and constellation is None:
@@ -139,10 +154,12 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         decoder.set_constellation(constellation)
     if channel == "split" and decoder is not None:
         decoder.set_split_constellation(constellation, x)
+    if decoder is not None and (punctured is not None or decoder.nt != code.N):
+        decoder.set_puncturing(() if punctured is None else punctured)
     code.prepare_encoder()
     code.rng_default()
     code.rng_skip(lo * D)
-    sigma = sigma_of(code, ebn)
+    sigma = sigma_of(code, ebn, punctured)
     bing = code.tables()[0]
     rows = np.zeros((hi - lo, 3), np.int64)
     for b0 in range(lo, hi, batch):
@@ -156,7 +173,7 @@ def monte_carlo(code, frames, ebn, decode=None, batch=256, rank=0, world=1, max_
         for _ in range(b0, b1):
             _, nbin = code.random_codeword()
             bits.append(nbin)
-            noisy.append(noise(code, nbin, ebn, constellation, x))
+            noisy.append(noise(code, nbin, ebn, constellation, x, punctured))
         dec, synd, it = decode(np.stack(noisy), sigma)
         for i in range(b1 - b0):
             err = int((bing[dec[i, :code.K]] != bits[i][:code.K]).sum())                    # NB_LDPC.c:479-485

@@ -161,6 +161,41 @@ int nbgpu_split_qam(int q, int points, float *mod /*[M][2]*/);
 int nbgpu_awgn_split_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/, int points,
                            const float *mod /*[M][2]*/, float EbN, float *noisy /*[N][P][2]*/);
 
+/* ---- Puncturing: variables of the code that are never sent (rate matching) ----
+ * Pattern: p distinct variable indices in [0, N), in any order, 0 <= p <= N-1.  Nt = N - p variables are transmitted and keep
+ *   their order: compact index t is the t-th unpunctured variable.
+ * Frames: while a pattern is bound to a context (nbgpu_set_puncturing), every call of it that takes or returns frames uses
+ *   compact frames [B][Nt][fps] with the channel's floats per symbol fps (logq BPSK, q dense LLR, 2 64-APSK and mapped, 4
+ *   faded, 2P split): upload, decode (the streamed path included), channel, frame source and nbgpu_source_download, which
+ *   returns noisy [B][Nt][fps] and codewords [B][N].  The frame source's limit B*Nt*fps < 2^31 replaces B*N*fps.
+ * Intake: a punctured variable's intake row is all 0.0f (no information); transmitted rows are computed exactly as without a
+ *   pattern.  A punctured decode is therefore bit for bit nbgpu_decode_llr on the expanded llr[B][N][q] with zero rows there.
+ *   nbgpu_channel_* return llr[B][N][q] with zero rows at punctured variables; their sorted intrinsics are all 0.0f in GF
+ *   order (the stable sort).  An isolated punctured variable (no check node) decides symbol 0.
+ * Stream: frame f owns the draws [f*D, (f+1)*D), D = K log2(q) + S*Nt, with the channel's draws per symbol S (2 log2(q) BPSK,
+ *   4 64-APSK and mapped, 5 or 6 faded, 4P split).  The information bits are drawn as without a pattern, then each transmitted
+ *   symbol in compact order takes its S draws; punctured symbols draw nothing.  This is the unpunctured stream with the
+ *   punctured symbols' draws removed; p = 0 is the unpunctured stream.
+ * Sigma: BPSK takes the rate of the transmitted word, rate_p = (float)(N - M) / (N - p) (init.c:167 over Nt symbols), and
+ *   sigma = (float)sqrt(1 / (2 rate_p 10^(EbN/10))) as nbgpu_sigma (nbgpu_sigma_punctured; p = 0 gives nbgpu_sigma).  The
+ *   constellation channels keep Es/N0 (nbgpu_sigma_apsk64) and do not depend on the rate.
+ * Scoring: bit errors are counted over the first K symbols of the full decided word (NB_LDPC.c:479-485); decisions and soft
+ *   output cover all N variables.
+ *
+ * nbgpu_sigma_punctured       sigma of the punctured BPSK channel; NaN (with a message) for p outside [0, N).
+ * nbgpu_awgn_punctured_noise  the compact frame noisy[Nt][fps] of one channel on the caller's drand48 stream (S*Nt draws), with
+ *                             channel = NBGPU_CHANNEL_BPSK (mod unused), _MAPPED (mod[q][2]; 64-APSK is the mapped channel on
+ *                             nbgpu_apsk64_table), _FADED (arg = fading) or _SPLIT (mod[M][2], arg = points).  NBGPU_EINVAL for
+ *                             a bad channel, fading or points, a NULL argument or a pattern nbgpu_set_puncturing refuses.  With
+ *                             p = 0 it equals the channel's own noise call. */
+#define NBGPU_CHANNEL_BPSK   0
+#define NBGPU_CHANNEL_MAPPED 1
+#define NBGPU_CHANNEL_FADED  2
+#define NBGPU_CHANNEL_SPLIT  3
+float nbgpu_sigma_punctured(const nbgpu_code *c, int p, float EbN);
+int nbgpu_awgn_punctured_noise(const nbgpu_code *c, nbgpu_rng *r, const int *nbin /*[N][logq] or NULL = all-zero word*/, int channel,
+                               int arg, const float *mod, float EbN, int p, const int *vars /*[p]*/, float *noisy /*[N-p][fps]*/);
+
 
 /* Configuration table of the syndrome-based check node: replaces build_config_table + sort_config_table
  * (syndrome_decoder.c:1542, 2285) and the truncation NB_LDPC.c:198-201.  Returns the number of
@@ -244,6 +279,12 @@ int nbgpu_decode_faded(nbgpu_ctx *ctx, const float *rx /*[B][N][4]*/, float sigm
 int nbgpu_set_split_constellation(nbgpu_ctx *ctx, int points, const float *mod /*[M][2]*/);
 int nbgpu_channel_split(nbgpu_ctx *ctx, const float *noisy /*[B][N][P][2]*/, float sigma, int B, float *llr, float *illr, int *igf);
 int nbgpu_decode_split(nbgpu_ctx *ctx, const float *noisy /*[B][N][P][2]*/, float sigma, int B, int *decide, int *synd, int *iters);
+/* Puncturing (semantics in "Puncturing" above): binds the pattern vars[p] to the context; p = 0 unbinds (vars may
+ * then be NULL).  NBGPU_EINVAL, context unchanged, for NULL vars with p > 0, p < 0, p >= N, an index outside [0, N) or a
+ * duplicate.  Binding any pattern (re-binding and unbinding included) drops the resident batch: nbgpu_run returns NBGPU_ESTATE
+ * and names the reason, and the soft output, nbgpu_source_results and nbgpu_source_download return NBGPU_ESTATE until a new
+ * batch is uploaded or generated.  The constellation bindings are independent of the pattern. */
+int nbgpu_set_puncturing(nbgpu_ctx *ctx, int p, const int *vars /*[p]*/);
 
 /* Same work split into stages so that a caller can keep inputs resident in HBM (bench.py "value"):
  * upload (H2D) -> run (kernel only, asynchronous on the ctx stream) -> download (D2H + sync). */
