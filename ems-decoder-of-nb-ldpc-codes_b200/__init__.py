@@ -203,6 +203,7 @@ def lib():
         "nbgpu_source_fixups": (C.c_long, [vp]),
         "nbgpu_source_set_margin": (C.c_int, [vp, C.c_double]),
         "nbgpu_check_node": (C.c_int, [vp, C.c_int, _fp, _ip, _fp, _ip, C.c_int]),
+        "nbgpu_check_node_dense": (C.c_int, [vp, C.c_int, _fp, _fp, C.c_int]),
         "nbgpu_elementary_step": (C.c_int, [vp, _fp, _fp, _ip, _ip, _fp, _ip, C.c_int]),
         "nbgpu_select_nm": (C.c_int, [vp, _fp, _fp, _ip, C.c_int]),
         "nbgpu_decision_syndrome": (C.c_int, [vp, _fp, _ip, _ip, C.c_int]),
@@ -649,6 +650,14 @@ class Decoder:
         cg = np.zeros((B, dc, self.code.q), np.int32)
         _check(lib().nbgpu_check_node(self.h, node, _f(vllr), _i(vgf), _f(cl), _i(cg), B), self.h)
         return cl, cg
+
+    def check_node_dense(self, node, mvc):
+        """nbgpu_check_node_dense: the sum-product node (ecn_kind=2) on B sets of dense rows, mvc [B, dc, q] -> CtoV [B, dc, q]"""
+        dc = int(self.code.row_deg[node])
+        mvc = np.ascontiguousarray(mvc, np.float32).reshape(-1, dc, self.code.q)
+        ctov = np.zeros(mvc.shape, np.float32)
+        _check(lib().nbgpu_check_node_dense(self.h, node, _f(mvc), _f(ctov), mvc.shape[0]), self.h)
+        return ctov
 
     def elementary_step(self, in1, in2, idx1, idx2):
         n_m = self.p.n_m

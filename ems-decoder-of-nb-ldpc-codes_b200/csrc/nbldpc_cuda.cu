@@ -16,7 +16,8 @@
  *   phase 3  warp per edge, NE edges interleaved:  Mvc again (parked in the APP row by phase 1), saturation + offset +
  *            expansion to the dense q-vector (bubble_decoder.c:231-281), CtoV store, APP = Mcv + Mvc
  *            (NB_LDPC.c:415-450), fused Decision (tools.c:312)
- * With ecn = 1 the tile is processed one check node at a time through the syndrome-based node (nbldpc_synd.cuh).
+ * With ecn = 1 the tile is processed one check node at a time through the syndrome-based node (nbldpc_synd.cuh), with
+ * ecn = 2 through the sum-product node (nbldpc_spa.cuh).
  *
  * The kernel is bound by the shared/global wavefront pipe of the SM (l1tex data stage), not by HBM or issue slots
  * (ncu, profiles/): every design choice below trades wavefronts for ALU work -- conflict-free 128-bit row moves,
@@ -25,10 +26,11 @@
  * HBM layout per resident frame (slot): APP[N][q] f32 (row = 4q bytes, one coalesced warp access);
  * CtoV as one lossless record per edge {llr[n_m] f32, sat f32, stp i32, sym[n_m] u8} -- a dense CtoV
  * row is "stp explicit (symbol, LLR) pairs + one constant" (bubble_decoder.c:262-270); decisions u8.
- * The syndrome-based node stores CtoV as dense rows instead.
+ * The syndrome-based and sum-product nodes store CtoV as dense rows instead.
  */
 #include "nbldpc_device.cuh"
 #include "nbldpc_synd.cuh"
+#include "nbldpc_spa.cuh"
 #include "nbldpc_source.cuh"
 #include "nbldpc_internal.h"
 #include <cmath>
@@ -40,7 +42,8 @@
 #include <vector>
 
 #define NT_MAX 384         /* threads per CTA (upper bound; the plan may use fewer warps) */
-#define NT_SYND 256        /* syndrome check node: at most 8 warps per CTA (its shared memory allows 7 at 945 configurations), 128 registers */
+#define NT_SYND 256        /* syndrome and sum-product check nodes: at most 8 warps per CTA (shared memory allows 7 at 945 configurations,
+                              6 for a dc = 16 GF(256) sum-product code), 128 registers */
 #define CTAS_PER_SM 2      /* resident CTAs per SM the decode kernel is compiled for (register cap 65536 / (NT_MAX * CTAS_PER_SM)) */
 #define NE 2               /* edges interleaved per warp in phases 1 and 3 */
 
@@ -347,6 +350,14 @@ __device__ __forceinline__ SyndMem make_synd_mem(unsigned char *smem, const KArg
     sm.cfg = smem_u32(smem + a.off_cfg); sm.cfgmask = sm.cfg + (uint32_t)(a.S * a.dc_max);
     sm.lstride = a.lstride; sm.n_m = a.n_m; sm.dc = a.dc_max; sm.S = a.S; sm.n_cv = a.n_cv;
     return sm;
+}
+/* the sum-product node's rows in a warp's list area: U rows at wb_U, the permutation row at sw_rows (plan_smem) */
+__device__ __forceinline__ SpaMem make_spa_mem(unsigned char *smem, const KArgs &a, int warp)
+{
+    const uint32_t wb = smem_u32(smem + a.off_wb + warp * a.wb_bytes);
+    SpaMem sp;
+    sp.urow = wb + a.wb_U; sp.prow = wb + a.sw_rows;
+    return sp;
 }
 __device__ __forceinline__ void load_cfg_table(unsigned char *smem, const KArgs &a)
 {
@@ -717,8 +728,8 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
     uint8_t *ctov = a.ctov + blockIdx.x * F * frame_ctov;
     uint8_t *dec = a.dec + (size_t)blockIdx.x * F * N;
     const size_t frame_dense = (size_t)a.E * Q;
-    float *ctov_d = ECN == 1 ? a.ctov_dense + blockIdx.x * F * frame_dense : nullptr;
-    const uint32_t rec_bytes = ECN == 1 ? (uint32_t)(Q * 4) : (uint32_t)rs;      /* bytes of CtoV state per edge */
+    float *ctov_d = ECN != 0 ? a.ctov_dense + blockIdx.x * F * frame_dense : nullptr;
+    const uint32_t rec_bytes = ECN != 0 ? (uint32_t)(Q * 4) : (uint32_t)rs;      /* bytes of CtoV state per edge */
 
     for (;;) {
         __syncthreads();
@@ -826,7 +837,7 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                         tile_elementary_steps<Q>(wm.ls, wm.meta, cnt, dcm, wm.mask, lane, a.nb_oper);
                         tile_phase3<Q, CLOSED>(a, wm, gf, cnt, reinterpret_cast<char *>(app), reinterpret_cast<char *>(ctov), dec, rl, pol_stream, minform, decide, lane);
                     }
-                } else {
+                } else if constexpr (ECN == 1) {
                     /* ---------------- syndrome-based check node: one node at a time per warp ---------------- */
                     const SyndMem sm = make_synd_mem(smem, a, warp);
                     for (int c = 0; c < cnt; c++) {
@@ -888,6 +899,50 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                                 if (lane == 0) dec_f[var] = (uint8_t)dd;
                             }
                             __syncwarp();
+                        }
+                    }
+                } else {
+                    /* ---------------- sum-product check node: one node at a time per warp ---------------- */
+                    const SpaMem sp = make_spa_mem(smem, a, warp);
+                    for (int c = 0; c < cnt; c++) {
+                        const int4 mt = wm.meta[c];
+                        const int dc = TileMeta::dc(mt);
+                        if (dc == 0) continue;
+                        float *app_f = reinterpret_cast<float *>(reinterpret_cast<char *>(app) + (uint32_t)mt.y);
+                        float *cd0 = reinterpret_cast<float *>(reinterpret_cast<char *>(ctov_d) + (uint32_t)mt.z);     /* dense CtoV row of the node's edge 0 */
+                        uint8_t *dec_f = dec + (uint32_t)mt.w;
+                        /* Mvc = APP - CtoV (NB_LDPC.c:334), parked in the APP row for the update below; then into the check domain */
+                        for (int t = 0; t < dc; t++) {
+                            const uint32_t ei = wm.ew[c * dcm + t];
+                            float *arow = app_f + (size_t)((ei & 0xfffffu) * (uint32_t)Q);
+                            float v[VPL], cv[VPL];
+                            load_row<Q>(arow, lane, v);
+                            load_row<Q>(cd0 + (size_t)((uint32_t)t * (uint32_t)Q), lane, cv);
+#pragma unroll
+                            for (int j = 0; j < VPL; j++) v[j] = __fsub_rn(v[j], cv[j]);
+                            store_row<Q>(arow, lane, v);
+                            spa_in<Q, CLOSED>(sp, t, v, (ei >> 20) & 0xff, gf, lane);
+                        }
+                        spa_bwd<Q>(sp, dc, cd0, lane);
+                        float fwd[VPL];
+#pragma unroll
+                        for (int j = 0; j < VPL; j++) fwd[j] = 1.0f;
+                        for (int t = 0; t < dc; t++) {
+                            const uint32_t ei = wm.ew[c * dcm + t];
+                            const uint32_t var = ei & 0xfffffu;
+                            float *cdrow = cd0 + (size_t)((uint32_t)t * (uint32_t)Q);
+                            float *arow = app_f + (size_t)(var * (uint32_t)Q);
+                            float mcv[VPL], v[VPL];
+                            spa_out<Q, CLOSED>(sp, t, cdrow, fwd, (ei >> 20) & 0xff, gf, lane, mcv);
+                            load_row<Q>(arow, lane, v);                       /* the parked Mvc */
+#pragma unroll
+                            for (int j = 0; j < VPL; j++) v[j] = __fadd_rn(mcv[j], v[j]);     /* NB_LDPC.c:448 */
+                            store_row<Q>(cdrow, lane, mcv);                   /* NB_LDPC.c:438 */
+                            store_row<Q>(arow, lane, v);
+                            if (decide && (ei >> 28)) {
+                                const int dd = warp_argmin<Q>(v, lane);
+                                if (lane == 0) dec_f[var] = (uint8_t)dd;
+                            }
                         }
                     }
                 }
@@ -1055,6 +1110,39 @@ __global__ void __launch_bounds__(NT_MAX, 1) checknode_synd_kernel(const KArgs a
     }
 }
 
+/* one check node (sum-product ECN) for B input sets, one warp per set: steps 2-7 of the node (include/nbldpc_b200.h) from
+ * mvc[b][t][.] (symbol order) to ctov[b][t][.], through the decoder's spa_in / spa_bwd / spa_out; the output rows are the
+ * backward-product scratch, as the dense CtoV rows are in the decoder */
+template <int Q, bool CLOSED>
+__global__ void __launch_bounds__(NT_SYND, 1) checknode_spa_kernel(const KArgs a, int node, const float *mvc, float *ctov, int B)
+{
+    constexpr int VPL = QTraits<Q>::VPL;
+    extern __shared__ __align__(16) unsigned char smem[];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nw = blockDim.x >> 5;
+    GFTab gf;
+    load_gf_tables(smem, a, gf);
+    __syncthreads();
+    const SpaMem sp = make_spa_mem(smem, a, warp);
+    const int e0 = a.row_ptr[node], dc = a.row_ptr[node + 1] - e0;
+    for (int b = blockIdx.x * nw + warp; b < B; b += gridDim.x * nw) {
+        float *out = ctov + (size_t)b * dc * Q;
+        for (int t = 0; t < dc; t++) {
+            float v[VPL];
+            load_row<Q>(mvc + ((size_t)b * dc + t) * Q, lane, v);
+            spa_in<Q, CLOSED>(sp, t, v, a.hval[e0 + t], gf, lane);
+        }
+        spa_bwd<Q>(sp, dc, out, lane);
+        float fwd[VPL];
+#pragma unroll
+        for (int j = 0; j < VPL; j++) fwd[j] = 1.0f;
+        for (int t = 0; t < dc; t++) {
+            float cv[VPL];
+            spa_out<Q, CLOSED>(sp, t, out + (size_t)t * Q, fwd, a.hval[e0 + t], gf, lane, cv);
+            store_row<Q>(out + (size_t)t * Q, lane, cv);
+        }
+    }
+}
+
 /* Decision + Syndrom on dense APP[B][N][q] */
 template <int Q>
 __global__ void __launch_bounds__(UNIT_NT) decision_kernel(const KArgs a, const float *app, int *decide, int B)
@@ -1142,11 +1230,16 @@ template <int ECN, bool SOFT> static const void *decode_fn_e(int q, int closed)
 static const void *decode_fn(int q, int closed, int ecn, bool soft)
 {
     if (q != 16 && q != 64 && q != 256) return nullptr;
+    if (ecn == 2) return soft ? decode_fn_e<2, true>(q, closed) : decode_fn_e<2, false>(q, closed);
     if (soft) return ecn ? decode_fn_e<1, true>(q, closed) : decode_fn_e<0, true>(q, closed);
     return ecn ? decode_fn_e<1, false>(q, closed) : decode_fn_e<0, false>(q, closed);
 }
 static const void *checknode_fn(int q, int closed, int ecn)
 {
+    if (ecn == 2) {
+        if (closed) return q == 16 ? (const void *)checknode_spa_kernel<16, true> : q == 64 ? (const void *)checknode_spa_kernel<64, true> : (const void *)checknode_spa_kernel<256, true>;
+        return q == 16 ? (const void *)checknode_spa_kernel<16, false> : q == 64 ? (const void *)checknode_spa_kernel<64, false> : (const void *)checknode_spa_kernel<256, false>;
+    }
     if (ecn) {
         if (closed) return q == 16 ? (const void *)checknode_synd_kernel<16, true> : q == 64 ? (const void *)checknode_synd_kernel<64, true> : (const void *)checknode_synd_kernel<256, true>;
         return q == 16 ? (const void *)checknode_synd_kernel<16, false> : q == 64 ? (const void *)checknode_synd_kernel<64, false> : (const void *)checknode_synd_kernel<256, false>;
@@ -1307,6 +1400,12 @@ static void plan_smem(KArgs &k, int nw, int cpw)
         if (s3 <= ub && k.dc_min >= 3) k.wb_scr3 = 0;      /* phase-3 rows over the input lists, dead after phase 2 ... */
         else { k.wb_scr3 = align_up(total, 16); total = k.wb_scr3 + s3; }   /* ... unless they do not fit, or degree 2: the output lists ARE input lists */
         k.wb_bytes = align_up(total, 16);
+    } else if (k.ecn == 2) {
+        /* sum-product check node, per warp: U rows [dc_max][q] (the intake and the soft output's selection use the same bytes as
+         * scratch, before and after the passes) | permutation row [q] */
+        k.wb_U = 0; k.wb_R = 0; k.wb_scr1 = 0; k.wb_scr3 = 0;
+        k.sw_rows = align_up(std::max(k.dc_max * k.q * 4, sq), 16);
+        k.wb_bytes = align_up(k.sw_rows + k.q * 4, 16);
     } else {
         /* syndrome check node: CTA-wide configuration table, then per warp: lists | grouped keys (aliased by the selection scratch of
          * phase 1, dead once the node's lists are written) | grouped configuration indices | histograms / output rows | group starts | perm */
@@ -1335,7 +1434,7 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     *out = NULL;
     if (!code || !p) { ctx_err(NULL, "nbgpu_create: NULL argument"); return NBGPU_EINVAL; }
     if (code->q != 16 && code->q != 64 && code->q != 256) { ctx_err(NULL, "GF(%d): kernels exist for GF(16), GF(64) and GF(256) only (init.c:431-435)", code->q); return NBGPU_EINVAL; }
-    if (p->ecn_kind != 0 && p->ecn_kind != 1) { ctx_err(NULL, "ecn_kind %d unknown (0 = CheckPassLogEMS, 1 = syndrome_ems)", p->ecn_kind); return NBGPU_EINVAL; }
+    if (p->ecn_kind < 0 || p->ecn_kind > 2) { ctx_err(NULL, "ecn_kind %d unknown (0 = CheckPassLogEMS, 1 = syndrome_ems, 2 = sum-product)", p->ecn_kind); return NBGPU_EINVAL; }
     if (p->n_m < 5 || p->n_m > 32 || p->n_m > code->q) { ctx_err(NULL, "n_m=%d unsupported: need 5 <= n_m <= min(q,32) (ElementaryStep reads row 4, bubble_decoder.c:457)", p->n_m); return NBGPU_EINVAL; }
     if (p->nb_iter_max < 2) { ctx_err(NULL, "nb_iter_max must be >= 2 (nb_iter_max-1 passes are run, NB_LDPC.c:314)"); return NBGPU_EINVAL; }
     if (p->nb_oper < 1) { ctx_err(NULL, "nb_oper must be >= 1"); return NBGPU_EINVAL; }
@@ -1420,8 +1519,8 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     k.F = 1;
     int nw = getenv("NBGPU_WARPS") ? atoi(getenv("NBGPU_WARPS")) : NT_MAX / 32, cpw = getenv("NBGPU_CPW") ? atoi(getenv("NBGPU_CPW")) : 8;
     /* the register budget is what limits residency: keep all NT_MAX/32 warps and shrink the tile before dropping warps */
-    if (p->ecn_kind == 1 && !getenv("NBGPU_CPW")) cpw = 4;       /* nodes of a tile are processed one after the other: no shared-memory cost */
-    nw = std::max(1, std::min(nw, (p->ecn_kind == 1 ? NT_SYND : NT_MAX) / 32)); cpw = std::max(1, std::min(cpw, 32));
+    if (p->ecn_kind != 0 && !getenv("NBGPU_CPW")) cpw = 4;       /* nodes of a tile are processed one after the other: no shared-memory cost */
+    nw = std::max(1, std::min(nw, (p->ecn_kind != 0 ? NT_SYND : NT_MAX) / 32)); cpw = std::max(1, std::min(cpw, 32));
     if (p->cns_per_step > 0) cpw = std::max(1, std::min(cpw, (p->cns_per_step + nw - 1) / nw));
     if (p->ecn_kind == 0 && !getenv("NBGPU_WARPS") && !getenv("NBGPU_CPW") && p->cns_per_step <= 0) {
         /* Pick (warps, nodes per warp) among the plans that fit.  Cost of one tile in instructions: phases 1/3 grow with the
@@ -1448,7 +1547,7 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     for (;;) {
         plan_smem(k, nw, cpw);
         if (k.smem_bytes <= budget) break;
-        if (p->ecn_kind == 1) { if (nw > 1) nw--; else break; }
+        if (p->ecn_kind != 0) { if (nw > 1) nw--; else break; }
         else if (cpw > 4) cpw--; else if (nw > 8) nw -= 2; else if (cpw > 1) cpw--; else if (nw > 1) nw--; else break;
     }
     if (k.smem_bytes > 227 * 1024) { ctx_err(c, "decoder working set does not fit in shared memory (%d bytes for one warp)", k.smem_bytes); nbgpu_destroy(c); return NBGPU_EINVAL; }
@@ -1521,8 +1620,8 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     c->nslots = c->grid * k.F;
 
     CKF(cudaMalloc((void **)&c->d_app, (size_t)c->nslots * N * q * sizeof(float)));
-    CKF(cudaMalloc((void **)&c->d_ctov, (p->ecn_kind == 1 ? 0 : (size_t)c->nslots * E * k.rec_stride) + 512));
-    if (p->ecn_kind == 1) CKF(cudaMalloc((void **)&c->d_ctov_dense, (size_t)c->nslots * E * q * sizeof(float)));
+    CKF(cudaMalloc((void **)&c->d_ctov, (p->ecn_kind != 0 ? 0 : (size_t)c->nslots * E * k.rec_stride) + 512));
+    if (p->ecn_kind != 0) CKF(cudaMalloc((void **)&c->d_ctov_dense, (size_t)c->nslots * E * q * sizeof(float)));
     CKF(cudaMalloc((void **)&c->d_dec, (size_t)c->nslots * N));
     CKF(cudaMemset(c->d_dec, 0, (size_t)c->nslots * N));
     CKF(cudaMalloc((void **)&c->d_decide, (size_t)max_batch * N * sizeof(int)));
@@ -2185,7 +2284,7 @@ extern "C" int nbgpu_get_state(nbgpu_ctx *c, int frame, float *APP, float *CtoV)
     if (owner != frame) { ctx_err(c, "state of frame %d was overwritten by frame %d (batch larger than the resident slots)", frame, owner); return NBGPU_ESTATE; }
     const int N = c->N, q = c->q, E = c->E, n_m = c->p.n_m, rs = c->k.rec_stride;
     if (APP) CK(c, cudaMemcpy(APP, c->d_app + (size_t)slot * N * q, (size_t)N * q * sizeof(float), cudaMemcpyDeviceToHost));
-    if (CtoV && c->k.ecn == 1) {
+    if (CtoV && c->k.ecn != 0) {
         CK(c, cudaMemcpy(CtoV, c->d_ctov_dense + (size_t)slot * E * q, (size_t)E * q * sizeof(float), cudaMemcpyDeviceToHost));
     } else if (CtoV) {
         std::vector<uint8_t> rec((size_t)E * rs);
@@ -2351,6 +2450,7 @@ extern "C" int nbgpu_elementary_step(nbgpu_ctx *c, const float *in1, const float
 extern "C" int nbgpu_check_node(nbgpu_ctx *c, int node, const float *vllr, const int *vgf, float *cllr, int *cgf, int B)
 {
     if (!c || !vllr || !vgf || !cllr || !cgf || B < 1 || node < 0 || node >= c->M) { ctx_err(c, "nbgpu_check_node: bad argument"); return NBGPU_EINVAL; }
+    if (c->k.ecn == 2) { ctx_err(c, "nbgpu_check_node: the sum-product check node (ecn_kind = 2) takes dense rows, not n_m lists: use nbgpu_check_node_dense"); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     const int dc = c->row_ptr_h[node + 1] - c->row_ptr_h[node], n_m = c->p.n_m, q = c->q;
     DevBuf<float> dvl, dcl; DevBuf<int> dvg, dcg;
@@ -2369,6 +2469,29 @@ extern "C" int nbgpu_check_node(nbgpu_ctx *c, int node, const float *vllr, const
     CK(c, cudaStreamSynchronize(c->stream));
     CK(c, cudaMemcpy(cllr, dcl.p, (size_t)B * dc * q * 4, cudaMemcpyDeviceToHost));
     CK(c, cudaMemcpy(cgf, dcg.p, (size_t)B * dc * q * 4, cudaMemcpyDeviceToHost));
+    return NBGPU_OK;
+}
+
+extern "C" int nbgpu_check_node_dense(nbgpu_ctx *c, int node, const float *mvc, float *ctov, int B)
+{
+    if (!c || !mvc || !ctov || B < 1 || node < 0 || node >= c->M) { ctx_err(c, "nbgpu_check_node_dense: bad argument"); return NBGPU_EINVAL; }
+    if (c->k.ecn != 2) { ctx_err(c, "nbgpu_check_node_dense: the context's check node is ecn_kind %d; dense rows are the sum-product node's (ecn_kind = 2)", c->k.ecn); return NBGPU_EINVAL; }
+    CK(c, cudaSetDevice(c->device));
+    const int dc = c->row_ptr_h[node + 1] - c->row_ptr_h[node], q = c->q;
+    const size_t n = (size_t)B * dc * q;
+    DevBuf<float> din, dout;
+    CK(c, din.alloc(n)); CK(c, dout.alloc(n));
+    CK(c, cudaMemcpyAsync(din.p, mvc, n * 4, cudaMemcpyHostToDevice, c->stream));
+    const int grid = std::min((B + c->k.nw - 1) / c->k.nw, 148);
+    {
+        const float *a1 = din.p; float *a2 = dout.p;
+        void *args[] = { (void *)&c->k, (void *)&node, (void *)&a1, (void *)&a2, (void *)&B };
+        CK(c, cudaLaunchKernel(checknode_fn(q, c->k.gf_closed, 2), dim3(grid), dim3(c->k.nw * 32), args, c->k.smem_bytes, c->stream));
+    }
+    CK(c, cudaGetLastError());
+    c->launches++;
+    CK(c, cudaMemcpyAsync(ctov, dout.p, n * 4, cudaMemcpyDeviceToHost, c->stream));
+    CK(c, cudaStreamSynchronize(c->stream));
     return NBGPU_OK;
 }
 

@@ -205,12 +205,35 @@ int nbgpu_config_table(int dc, int d1, int d2, int d3, int trunc, int *table, in
 /* ------------------------------------------------------------------------------------------------
  * Device side
  * ---------------------------------------------------------------------------------------------- */
+/* The sum-product check node (ecn_kind = 2).  The schedule, CtoV initialisation (all 0), Decision, Syndrom, early
+ * termination, iteration counts and statistics are those of the other two kinds; only the check-node update differs.
+ * Limits: q in {16, 64, 256}, check degrees 2 ... 16, irregular rows included.  For check node m with edges e = 0 ... dc-1
+ * in file order, variable v_e and coefficient h_e, all arithmetic in IEEE f32 rounded to nearest, one operation at a time:
+ *   1. Mvc_e[x] = APP[v_e][x] - CtoV_e[x].
+ *   2. mu_e = min_x Mvc_e[x];  p_e[x] = 0 where Mvc_e[x] >= 1e5 and Mvc_e[x] > mu_e ("absent"), else E(mu_e - Mvc_e[x]).
+ *      So max_x p_e[x] = 1.
+ *   3. Into the check domain: u_e[img(MULGF[x][h_e])] = p_e[x]  (img = binary image).
+ *   4. U_e = WHT(u_e): stage s = 0 ... log2 q - 1 pairs the indices i < j that differ in bit s only and writes
+ *      (u[i] + u[j], u[i] - u[j]).  Then r_e = 1 / U_e[0] (one division) and U_e[k] = U_e[k] * r_e for every k.
+ *   5. T_e[k] = fwd_e[k] * bwd_e[k] with fwd_0 = 1, fwd_{e+1} = fwd_e * U_e, bwd_{dc-1} = 1, bwd_{e-1} = bwd_e * U_e.
+ *   6. t_e = WHT(T_e) with the same stages, no 1/q factor.  c_max = max_k t_e[k].
+ *   7. c_e[x] = max(t_e[img(MULGF[x][h_e])], c_max * tau) with tau = 2^-20, and CtoV_e[x] = L(c_max) - L(c_e[x]),
+ *      which lies in [0, 20 ln 2].  The exact t_e is q times a probability vector, so c_max >= 1; measured against a
+ *      float64 brute force, the round-off of the transforms stays below 2^-24 c_max, so values under tau c_max carry
+ *      round-off of 1/16 of themselves or more.
+ *   8. APP[v_e][x] = Mvc_e[x] + CtoV_e[x].
+ * E and L are the library's f32 exp and log (csrc/nbldpc_spa_math.h): explicit range reduction and a fixed polynomial,
+ * so that every build gives the same bits.  E: d < -87 gives 0, else largest error 1.22 ulp over [-87, 0].  L: largest
+ * error 1.97 ulp over [2^-24, 2^9].  Both bounds come from an exhaustive check over every float of those domains
+ * (scripts/check_spa_math.c). */
 typedef struct {
     int   n_m;          /* decoder.nbMax, argv[5]; 5 <= n_m <= min(q,32)                          */
     int   nb_oper;      /* NbOper, argv[7]: max pops per ElementaryStep                            */
     int   nb_iter_max;  /* NbIterMax, argv[2] (>= 2)                                               */
     float offset;       /* argv[6]                                                                 */
-    int   ecn_kind;     /* 0 = CheckPassLogEMS (L-Bubble F/B), 1 = syndrome_ems                    */
+    int   ecn_kind;     /* 0 = CheckPassLogEMS (L-Bubble F/B), 1 = syndrome_ems, 2 = sum-product
+                           (q-ary belief propagation, below; n_m, nb_oper and offset are validated as
+                           for the other kinds but not used)                                        */
     int   early_stop;   /* 1 = stop a frame at the first zero syndrome (NB_LDPC.c:470); 0 = always
                            run nb_iter_max-1 passes (fixed-iteration throughput mode)               */
     /* syndrome_ems only (NB_LDPC.c:185-201, commented out there; see DESIGN.md "Syndrome path").
@@ -399,6 +422,10 @@ int nbgpu_download_soft_bits(nbgpu_ctx *ctx, float *llr);
  * decoder->M_CtoV_LLR/GF after it. */
 int nbgpu_check_node(nbgpu_ctx *ctx, int node, const float *vllr, const int *vgf,
                      float *cllr, int *cgf, int B);
+/* Steps 2-7 of the sum-product node (ecn_kind = 2) of check node `node` for B input sets: mvc[B][dc][q] -> ctov[B][dc][q],
+ * both in symbol order, through the decoder's own device functions.  NBGPU_EINVAL on a context of another ecn_kind;
+ * nbgpu_check_node is NBGPU_EINVAL on an ecn_kind = 2 context. */
+int nbgpu_check_node_dense(nbgpu_ctx *ctx, int node, const float *mvc, float *ctov, int B);
 /* ElementaryStep (bubble_decoder.h:28) for B independent pairs of n_m-lists (symbols, -1 = absent) */
 int nbgpu_elementary_step(nbgpu_ctx *ctx, const float *in1, const float *in2, const int *idx1,
                           const int *idx2, float *out, int *idxout, int B);
