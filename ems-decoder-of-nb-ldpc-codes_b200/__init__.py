@@ -380,7 +380,10 @@ class Code:
 
 
 class Decoder:
-    """nbgpu_ctx: the decode path NB_LDPC.c:266-474 for batches of frames on one B200."""
+    """nbgpu_ctx: the decode path NB_LDPC.c:266-474 for batches of frames on one B200.
+
+    ecn_kind selects the check node: 0 = CheckPassLogEMS (L-Bubble), 1 = syndrome_ems, 2 = sum-product (belief propagation),
+    4 = Min-Max; for 2 and 4, n_m, nb_oper and offset are validated but not used (include/nbldpc_b200.h)."""
 
     def __init__(self, code, n_m, nb_oper, nb_iter_max, offset, early_stop=True, ecn_kind=0, device=0,
                  max_batch=1, d1=0, d2=0, d3=0, cfg_trunc=0, n_cv=0, border=0, frames_per_cta=0, cns_per_step=0):
@@ -652,7 +655,8 @@ class Decoder:
         return cl, cg
 
     def check_node_dense(self, node, mvc):
-        """nbgpu_check_node_dense: the sum-product node (ecn_kind=2) on B sets of dense rows, mvc [B, dc, q] -> CtoV [B, dc, q]"""
+        """nbgpu_check_node_dense: the context's dense node, sum-product (ecn_kind=2) or Min-Max (ecn_kind=4), on B sets of dense
+        rows, mvc [B, dc, q] -> CtoV [B, dc, q]"""
         dc = int(self.code.row_deg[node])
         mvc = np.ascontiguousarray(mvc, np.float32).reshape(-1, dc, self.code.q)
         ctov = np.zeros(mvc.shape, np.float32)

@@ -17,7 +17,7 @@
  *            expansion to the dense q-vector (bubble_decoder.c:231-281), CtoV store, APP = Mcv + Mvc
  *            (NB_LDPC.c:415-450), fused Decision (tools.c:312)
  * With ecn = 1 the tile is processed one check node at a time through the syndrome-based node (nbldpc_synd.cuh), with
- * ecn = 2 through the sum-product node (nbldpc_spa.cuh).
+ * ecn = 2 through the sum-product node (nbldpc_spa.cuh), with ecn = 4 through the Min-Max node (nbldpc_minmax.cuh).
  *
  * The kernel is bound by the shared/global wavefront pipe of the SM (l1tex data stage), not by HBM or issue slots
  * (ncu, profiles/): every design choice below trades wavefronts for ALU work -- conflict-free 128-bit row moves,
@@ -26,11 +26,12 @@
  * HBM layout per resident frame (slot): APP[N][q] f32 (row = 4q bytes, one coalesced warp access);
  * CtoV as one lossless record per edge {llr[n_m] f32, sat f32, stp i32, sym[n_m] u8} -- a dense CtoV
  * row is "stp explicit (symbol, LLR) pairs + one constant" (bubble_decoder.c:262-270); decisions u8.
- * The syndrome-based and sum-product nodes store CtoV as dense rows instead.
+ * The syndrome-based, sum-product and Min-Max nodes store CtoV as dense rows instead.
  */
 #include "nbldpc_device.cuh"
 #include "nbldpc_synd.cuh"
 #include "nbldpc_spa.cuh"
+#include "nbldpc_minmax.cuh"
 #include "nbldpc_source.cuh"
 #include "nbldpc_internal.h"
 #include <cmath>
@@ -42,7 +43,7 @@
 #include <vector>
 
 #define NT_MAX 384         /* threads per CTA (upper bound; the plan may use fewer warps) */
-#define NT_SYND 256        /* syndrome and sum-product check nodes: at most 8 warps per CTA (shared memory allows 7 at 945 configurations,
+#define NT_SYND 256        /* syndrome, sum-product and Min-Max check nodes: at most 8 warps per CTA (shared memory allows 7 at 945 configurations,
                               6 for a dc = 16 GF(256) sum-product code), 128 registers */
 #define CTAS_PER_SM 2      /* resident CTAs per SM the decode kernel is compiled for (register cap 65536 / (NT_MAX * CTAS_PER_SM)) */
 #define NE 2               /* edges interleaved per warp in phases 1 and 3 */
@@ -351,7 +352,7 @@ __device__ __forceinline__ SyndMem make_synd_mem(unsigned char *smem, const KArg
     sm.lstride = a.lstride; sm.n_m = a.n_m; sm.dc = a.dc_max; sm.S = a.S; sm.n_cv = a.n_cv;
     return sm;
 }
-/* the sum-product node's rows in a warp's list area: U rows at wb_U, the permutation row at sw_rows (plan_smem) */
+/* the dense nodes' rows (sum-product, Min-Max) in a warp's list area: U rows at wb_U, the permutation row at sw_rows (plan_smem) */
 __device__ __forceinline__ SpaMem make_spa_mem(unsigned char *smem, const KArgs &a, int warp)
 {
     const uint32_t wb = smem_u32(smem + a.off_wb + warp * a.wb_bytes);
@@ -902,7 +903,7 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                         }
                     }
                 } else {
-                    /* ---------------- sum-product check node: one node at a time per warp ---------------- */
+                    /* ---------------- dense-row check nodes (sum-product, Min-Max): one node at a time per warp ---------------- */
                     const SpaMem sp = make_spa_mem(smem, a, warp);
                     for (int c = 0; c < cnt; c++) {
                         const int4 mt = wm.meta[c];
@@ -921,9 +922,11 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
 #pragma unroll
                             for (int j = 0; j < VPL; j++) v[j] = __fsub_rn(v[j], cv[j]);
                             store_row<Q>(arow, lane, v);
-                            spa_in<Q, CLOSED>(sp, t, v, (ei >> 20) & 0xff, gf, lane);
+                            if constexpr (ECN == 2) spa_in<Q, CLOSED>(sp, t, v, (ei >> 20) & 0xff, gf, lane);
+                            else mm_in<Q, CLOSED>(sp, t, v, (ei >> 20) & 0xff, gf, lane);
                         }
-                        spa_bwd<Q>(sp, dc, cd0, lane);
+                        if constexpr (ECN == 2) spa_bwd<Q>(sp, dc, cd0, lane);
+                        else mm_bwd<Q>(sp, dc, cd0, lane);
                         float fwd[VPL];
 #pragma unroll
                         for (int j = 0; j < VPL; j++) fwd[j] = 1.0f;
@@ -933,7 +936,8 @@ __global__ void __launch_bounds__(ECN ? NT_SYND : NT_MAX, CTAS_PER_SM) decode_ke
                             float *cdrow = cd0 + (size_t)((uint32_t)t * (uint32_t)Q);
                             float *arow = app_f + (size_t)(var * (uint32_t)Q);
                             float mcv[VPL], v[VPL];
-                            spa_out<Q, CLOSED>(sp, t, cdrow, fwd, (ei >> 20) & 0xff, gf, lane, mcv);
+                            if constexpr (ECN == 2) spa_out<Q, CLOSED>(sp, t, cdrow, fwd, (ei >> 20) & 0xff, gf, lane, mcv);
+                            else mm_out<Q, CLOSED>(sp, t, dc, cdrow, fwd, (ei >> 20) & 0xff, gf, lane, mcv);
                             load_row<Q>(arow, lane, v);                       /* the parked Mvc */
 #pragma unroll
                             for (int j = 0; j < VPL; j++) v[j] = __fadd_rn(mcv[j], v[j]);     /* NB_LDPC.c:448 */
@@ -1110,11 +1114,11 @@ __global__ void __launch_bounds__(NT_MAX, 1) checknode_synd_kernel(const KArgs a
     }
 }
 
-/* one check node (sum-product ECN) for B input sets, one warp per set: steps 2-7 of the node (include/nbldpc_b200.h) from
- * mvc[b][t][.] (symbol order) to ctov[b][t][.], through the decoder's spa_in / spa_bwd / spa_out; the output rows are the
- * backward-product scratch, as the dense CtoV rows are in the decoder */
-template <int Q, bool CLOSED>
-__global__ void __launch_bounds__(NT_SYND, 1) checknode_spa_kernel(const KArgs a, int node, const float *mvc, float *ctov, int B)
+/* one check node (dense ECN: 2 = sum-product, 4 = Min-Max) for B input sets, one warp per set: the node's steps after Mvc
+ * (include/nbldpc_b200.h) from mvc[b][t][.] (symbol order) to ctov[b][t][.], through the decoder's spa_* / mm_* functions;
+ * the output rows are the backward-partial scratch, as the dense CtoV rows are in the decoder */
+template <int Q, bool CLOSED, int ECN>
+__global__ void __launch_bounds__(NT_SYND, 1) checknode_dense_kernel(const KArgs a, int node, const float *mvc, float *ctov, int B)
 {
     constexpr int VPL = QTraits<Q>::VPL;
     extern __shared__ __align__(16) unsigned char smem[];
@@ -1129,15 +1133,18 @@ __global__ void __launch_bounds__(NT_SYND, 1) checknode_spa_kernel(const KArgs a
         for (int t = 0; t < dc; t++) {
             float v[VPL];
             load_row<Q>(mvc + ((size_t)b * dc + t) * Q, lane, v);
-            spa_in<Q, CLOSED>(sp, t, v, a.hval[e0 + t], gf, lane);
+            if constexpr (ECN == 2) spa_in<Q, CLOSED>(sp, t, v, a.hval[e0 + t], gf, lane);
+            else mm_in<Q, CLOSED>(sp, t, v, a.hval[e0 + t], gf, lane);
         }
-        spa_bwd<Q>(sp, dc, out, lane);
+        if constexpr (ECN == 2) spa_bwd<Q>(sp, dc, out, lane);
+        else mm_bwd<Q>(sp, dc, out, lane);
         float fwd[VPL];
 #pragma unroll
         for (int j = 0; j < VPL; j++) fwd[j] = 1.0f;
         for (int t = 0; t < dc; t++) {
             float cv[VPL];
-            spa_out<Q, CLOSED>(sp, t, out + (size_t)t * Q, fwd, a.hval[e0 + t], gf, lane, cv);
+            if constexpr (ECN == 2) spa_out<Q, CLOSED>(sp, t, out + (size_t)t * Q, fwd, a.hval[e0 + t], gf, lane, cv);
+            else mm_out<Q, CLOSED>(sp, t, dc, out + (size_t)t * Q, fwd, a.hval[e0 + t], gf, lane, cv);
             store_row<Q>(out + (size_t)t * Q, lane, cv);
         }
     }
@@ -1231,15 +1238,19 @@ static const void *decode_fn(int q, int closed, int ecn, bool soft)
 {
     if (q != 16 && q != 64 && q != 256) return nullptr;
     if (ecn == 2) return soft ? decode_fn_e<2, true>(q, closed) : decode_fn_e<2, false>(q, closed);
+    if (ecn == 4) return soft ? decode_fn_e<4, true>(q, closed) : decode_fn_e<4, false>(q, closed);
     if (soft) return ecn ? decode_fn_e<1, true>(q, closed) : decode_fn_e<0, true>(q, closed);
     return ecn ? decode_fn_e<1, false>(q, closed) : decode_fn_e<0, false>(q, closed);
 }
+template <int ECN> static const void *checknode_dense_fn(int q, int closed)
+{
+    if (closed) return q == 16 ? (const void *)checknode_dense_kernel<16, true, ECN> : q == 64 ? (const void *)checknode_dense_kernel<64, true, ECN> : (const void *)checknode_dense_kernel<256, true, ECN>;
+    return q == 16 ? (const void *)checknode_dense_kernel<16, false, ECN> : q == 64 ? (const void *)checknode_dense_kernel<64, false, ECN> : (const void *)checknode_dense_kernel<256, false, ECN>;
+}
 static const void *checknode_fn(int q, int closed, int ecn)
 {
-    if (ecn == 2) {
-        if (closed) return q == 16 ? (const void *)checknode_spa_kernel<16, true> : q == 64 ? (const void *)checknode_spa_kernel<64, true> : (const void *)checknode_spa_kernel<256, true>;
-        return q == 16 ? (const void *)checknode_spa_kernel<16, false> : q == 64 ? (const void *)checknode_spa_kernel<64, false> : (const void *)checknode_spa_kernel<256, false>;
-    }
+    if (ecn == 2) return checknode_dense_fn<2>(q, closed);
+    if (ecn == 4) return checknode_dense_fn<4>(q, closed);
     if (ecn) {
         if (closed) return q == 16 ? (const void *)checknode_synd_kernel<16, true> : q == 64 ? (const void *)checknode_synd_kernel<64, true> : (const void *)checknode_synd_kernel<256, true>;
         return q == 16 ? (const void *)checknode_synd_kernel<16, false> : q == 64 ? (const void *)checknode_synd_kernel<64, false> : (const void *)checknode_synd_kernel<256, false>;
@@ -1400,9 +1411,10 @@ static void plan_smem(KArgs &k, int nw, int cpw)
         if (s3 <= ub && k.dc_min >= 3) k.wb_scr3 = 0;      /* phase-3 rows over the input lists, dead after phase 2 ... */
         else { k.wb_scr3 = align_up(total, 16); total = k.wb_scr3 + s3; }   /* ... unless they do not fit, or degree 2: the output lists ARE input lists */
         k.wb_bytes = align_up(total, 16);
-    } else if (k.ecn == 2) {
-        /* sum-product check node, per warp: U rows [dc_max][q] (the intake and the soft output's selection use the same bytes as
-         * scratch, before and after the passes) | permutation row [q] */
+    } else if (k.ecn == 2 || k.ecn == 4) {
+        /* sum-product and Min-Max check nodes, per warp: U rows [dc_max][q] (the intake and the soft output's selection use the same
+         * bytes as scratch, before and after the passes) | permutation row [q] (Min-Max: also the row operand of a convolution;
+         * its rows enter the check domain straight into the U rows) */
         k.wb_U = 0; k.wb_R = 0; k.wb_scr1 = 0; k.wb_scr3 = 0;
         k.sw_rows = align_up(std::max(k.dc_max * k.q * 4, sq), 16);
         k.wb_bytes = align_up(k.sw_rows + k.q * 4, 16);
@@ -1434,7 +1446,7 @@ extern "C" int nbgpu_create(nbgpu_ctx **out, const nbgpu_code *code, const nbgpu
     *out = NULL;
     if (!code || !p) { ctx_err(NULL, "nbgpu_create: NULL argument"); return NBGPU_EINVAL; }
     if (code->q != 16 && code->q != 64 && code->q != 256) { ctx_err(NULL, "GF(%d): kernels exist for GF(16), GF(64) and GF(256) only (init.c:431-435)", code->q); return NBGPU_EINVAL; }
-    if (p->ecn_kind < 0 || p->ecn_kind > 2) { ctx_err(NULL, "ecn_kind %d unknown (0 = CheckPassLogEMS, 1 = syndrome_ems, 2 = sum-product)", p->ecn_kind); return NBGPU_EINVAL; }
+    if (p->ecn_kind < 0 || p->ecn_kind > 4 || p->ecn_kind == 3) { ctx_err(NULL, "ecn_kind %d unknown (0 = CheckPassLogEMS, 1 = syndrome_ems, 2 = sum-product, 4 = Min-Max)", p->ecn_kind); return NBGPU_EINVAL; }
     if (p->n_m < 5 || p->n_m > 32 || p->n_m > code->q) { ctx_err(NULL, "n_m=%d unsupported: need 5 <= n_m <= min(q,32) (ElementaryStep reads row 4, bubble_decoder.c:457)", p->n_m); return NBGPU_EINVAL; }
     if (p->nb_iter_max < 2) { ctx_err(NULL, "nb_iter_max must be >= 2 (nb_iter_max-1 passes are run, NB_LDPC.c:314)"); return NBGPU_EINVAL; }
     if (p->nb_oper < 1) { ctx_err(NULL, "nb_oper must be >= 1"); return NBGPU_EINVAL; }
@@ -2450,7 +2462,7 @@ extern "C" int nbgpu_elementary_step(nbgpu_ctx *c, const float *in1, const float
 extern "C" int nbgpu_check_node(nbgpu_ctx *c, int node, const float *vllr, const int *vgf, float *cllr, int *cgf, int B)
 {
     if (!c || !vllr || !vgf || !cllr || !cgf || B < 1 || node < 0 || node >= c->M) { ctx_err(c, "nbgpu_check_node: bad argument"); return NBGPU_EINVAL; }
-    if (c->k.ecn == 2) { ctx_err(c, "nbgpu_check_node: the sum-product check node (ecn_kind = 2) takes dense rows, not n_m lists: use nbgpu_check_node_dense"); return NBGPU_EINVAL; }
+    if (c->k.ecn == 2 || c->k.ecn == 4) { ctx_err(c, "nbgpu_check_node: the %s check node (ecn_kind = %d) takes dense rows, not n_m lists: use nbgpu_check_node_dense", c->k.ecn == 2 ? "sum-product" : "Min-Max", c->k.ecn); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     const int dc = c->row_ptr_h[node + 1] - c->row_ptr_h[node], n_m = c->p.n_m, q = c->q;
     DevBuf<float> dvl, dcl; DevBuf<int> dvg, dcg;
@@ -2475,7 +2487,7 @@ extern "C" int nbgpu_check_node(nbgpu_ctx *c, int node, const float *vllr, const
 extern "C" int nbgpu_check_node_dense(nbgpu_ctx *c, int node, const float *mvc, float *ctov, int B)
 {
     if (!c || !mvc || !ctov || B < 1 || node < 0 || node >= c->M) { ctx_err(c, "nbgpu_check_node_dense: bad argument"); return NBGPU_EINVAL; }
-    if (c->k.ecn != 2) { ctx_err(c, "nbgpu_check_node_dense: the context's check node is ecn_kind %d; dense rows are the sum-product node's (ecn_kind = 2)", c->k.ecn); return NBGPU_EINVAL; }
+    if (c->k.ecn != 2 && c->k.ecn != 4) { ctx_err(c, "nbgpu_check_node_dense: the context's check node is ecn_kind %d; dense rows are the sum-product node's (ecn_kind = 2) and the Min-Max node's (ecn_kind = 4)", c->k.ecn); return NBGPU_EINVAL; }
     CK(c, cudaSetDevice(c->device));
     const int dc = c->row_ptr_h[node + 1] - c->row_ptr_h[node], q = c->q;
     const size_t n = (size_t)B * dc * q;
@@ -2486,7 +2498,7 @@ extern "C" int nbgpu_check_node_dense(nbgpu_ctx *c, int node, const float *mvc, 
     {
         const float *a1 = din.p; float *a2 = dout.p;
         void *args[] = { (void *)&c->k, (void *)&node, (void *)&a1, (void *)&a2, (void *)&B };
-        CK(c, cudaLaunchKernel(checknode_fn(q, c->k.gf_closed, 2), dim3(grid), dim3(c->k.nw * 32), args, c->k.smem_bytes, c->stream));
+        CK(c, cudaLaunchKernel(checknode_fn(q, c->k.gf_closed, c->k.ecn), dim3(grid), dim3(c->k.nw * 32), args, c->k.smem_bytes, c->stream));
     }
     CK(c, cudaGetLastError());
     c->launches++;

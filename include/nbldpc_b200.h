@@ -226,14 +226,31 @@ int nbgpu_config_table(int dc, int d1, int d2, int d3, int trunc, int *table, in
  * so that every build gives the same bits.  E: d < -87 gives 0, else largest error 1.22 ulp over [-87, 0].  L: largest
  * error 1.97 ulp over [2^-24, 2^9].  Both bounds come from an exhaustive check over every float of those domains
  * (scripts/check_spa_math.c). */
+/* The Min-Max check node (ecn_kind = 4; Savin, 2008).  Schedule, CtoV initialisation, Decision, Syndrom, early termination,
+ * iteration counts, statistics and limits are those of the sum-product node.  For check node m with edges e = 0 ... dc-1 in
+ * file order, variable v_e and coefficient h_e, all arithmetic in IEEE f32 rounded to nearest, one operation at a time:
+ *   1. Mvc_e[x] = APP[v_e][x] - CtoV_e[x].
+ *   2. mu_e = min_x Mvc_e[x];  w_e[x] = Mvc_e[x] - mu_e.  So w_e >= 0, and w_e = 0 at the minimum.  Values >= 1e5 get no
+ *      special case: a large value loses every max/min on its own.
+ *   3. Into the check domain: u_e[img(MULGF[x][h_e])] = w_e[x].
+ *   4. With the min-max convolution over XOR of binary images, (A (*) B)[z] = min_a max(A[a], B[a ^ z]):
+ *      t_e = (*) of u_j over j != e, i.e. t_e[z] is the least, over the configurations (y_j), j != e, with XOR y_j = z, of
+ *      max_j u_j[y_j].  For dc = 2, t_0 = u_1 and t_1 = u_0.  (*) is associative and commutative and every result is one of
+ *      its inputs, so any order of evaluation gives the same bits; the kernel relies on that (forward and backward partials,
+ *      pruned candidates).
+ *   5. Back to the variable domain: CtoV_e[x] = t_e[img(MULGF[x][h_e])].  So min_x CtoV_e[x] = 0, and CtoV_e takes only values
+ *      of the w rows.
+ *   6. APP[v_e][x] = Mvc_e[x] + CtoV_e[x], with Mvc the value of step 1.
+ * n_m, nb_oper and offset are validated as for the other kinds and not used. */
 typedef struct {
     int   n_m;          /* decoder.nbMax, argv[5]; 5 <= n_m <= min(q,32)                          */
     int   nb_oper;      /* NbOper, argv[7]: max pops per ElementaryStep                            */
     int   nb_iter_max;  /* NbIterMax, argv[2] (>= 2)                                               */
     float offset;       /* argv[6]                                                                 */
     int   ecn_kind;     /* 0 = CheckPassLogEMS (L-Bubble F/B), 1 = syndrome_ems, 2 = sum-product
-                           (q-ary belief propagation, below; n_m, nb_oper and offset are validated as
-                           for the other kinds but not used)                                        */
+                           (q-ary belief propagation, above), 4 = Min-Max (above); for 2 and 4,
+                           n_m, nb_oper and offset are validated as for the other kinds but not
+                           used.  3 is not assigned.                                                */
     int   early_stop;   /* 1 = stop a frame at the first zero syndrome (NB_LDPC.c:470); 0 = always
                            run nb_iter_max-1 passes (fixed-iteration throughput mode)               */
     /* syndrome_ems only (NB_LDPC.c:185-201, commented out there; see DESIGN.md "Syndrome path").
@@ -422,9 +439,10 @@ int nbgpu_download_soft_bits(nbgpu_ctx *ctx, float *llr);
  * decoder->M_CtoV_LLR/GF after it. */
 int nbgpu_check_node(nbgpu_ctx *ctx, int node, const float *vllr, const int *vgf,
                      float *cllr, int *cgf, int B);
-/* Steps 2-7 of the sum-product node (ecn_kind = 2) of check node `node` for B input sets: mvc[B][dc][q] -> ctov[B][dc][q],
- * both in symbol order, through the decoder's own device functions.  NBGPU_EINVAL on a context of another ecn_kind;
- * nbgpu_check_node is NBGPU_EINVAL on an ecn_kind = 2 context. */
+/* The dense check node of the context for check node `node` and B input sets: steps 2-7 of the sum-product node
+ * (ecn_kind = 2) or steps 2-5 of the Min-Max node (ecn_kind = 4), mvc[B][dc][q] -> ctov[B][dc][q], both in symbol order,
+ * through the decoder's own device functions.  NBGPU_EINVAL on a context of another ecn_kind; nbgpu_check_node is
+ * NBGPU_EINVAL on an ecn_kind = 2 or 4 context. */
 int nbgpu_check_node_dense(nbgpu_ctx *ctx, int node, const float *mvc, float *ctov, int B);
 /* ElementaryStep (bubble_decoder.h:28) for B independent pairs of n_m-lists (symbols, -1 = absent) */
 int nbgpu_elementary_step(nbgpu_ctx *ctx, const float *in1, const float *in2, const int *idx1,
